@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-seconds/second of the fused MFCC+FFN VAD hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (configs[2]): 1,000 h of synthetic 16 kHz int16 audio PER GPU as 360,000 x 10 s
@@ -16,6 +16,9 @@ metric through the C ABI's host-buffer entry point vadb200_vad_host: pinned host
 kernel -> D2H labels, every step), roofline (algorithmic FP32 flop / kernel time against a live
 FMA microbenchmark; HBM fraction alongside), cpu_baseline (the reference-shaped CPU port on the
 host cores, bounded sample), clocks and launch count.
+
+--dump-outputs DIR saves what the timed launches returned in their last step (a fixed, seeded sample of whole
+utterances' labels) so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import json
@@ -28,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the source tree, which may be read-only
 
 METRIC = "audio_seconds_per_second"
 UNIT = "audio-s/s"
@@ -38,6 +42,7 @@ FP32_NOMINAL_TFLOPS = 74.4     # 148 SM x 128 lanes x 2 x 1.965 GHz (fallback de
 # dram__bytes_read.sum + dram__bytes_write.sum of fused_kernel<2,2> from the committed `ncu --set full`
 # capture (profiles/r3_fused_kernel_2_2_ncu_raw.csv: 5.8241 GB + 0.0227 GB for 17.874 M frames)
 NCU_DRAM_BYTES_PER_FRAME = (5.824133e9 + 22.738688e6) / 17874000.0
+DUMP_LABEL_BYTES = 48 << 20    # --dump-outputs: float32 labels of as many sampled utterances as fit (64 MB cap in all)
 
 
 def parse_args():
@@ -61,7 +66,15 @@ def parse_args():
     ap.add_argument("--streams", type=int, default=4096)
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the cfg2 / cfg4 / cfg5 sub-records")
     ap.add_argument("--parity-utts", type=int, default=4)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, save the last step's labels of a fixed seeded sample of utterances "
+                         "as DIR/labels.npy (float32 [utterances, rows]) and their indices as DIR/utterances.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs saves the GPU path's outputs (--impl ours)")
+    return a
 
 
 # ----------------------------------------------------------------------------------------- clocks
@@ -123,7 +136,8 @@ class ClockSampler(object):
 def run_cpu_port(utts, procs, steps, warmup, utt_seconds, seed):
     cmd = [sys.executable, "-m", "oracle.cpu_bench", "--utts", str(utts), "--procs", str(procs), "--steps", str(steps),
            "--warmup", str(warmup), "--utt-seconds", str(utt_seconds), "--seed", str(seed)]
-    env = dict(os.environ, OMP_NUM_THREADS="1", OPENBLAS_NUM_THREADS="1", MKL_NUM_THREADS="1")
+    env = dict(os.environ, OMP_NUM_THREADS="1", OPENBLAS_NUM_THREADS="1", MKL_NUM_THREADS="1",
+               PYTHONDONTWRITEBYTECODE="1")
     out = subprocess.run(cmd, cwd=ROOT, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=1500)
     if out.returncode != 0:
         raise RuntimeError("cpu_bench failed: " + out.stderr[-400:])
@@ -251,6 +265,21 @@ def parity_sample(h, plan, pcm, labels, n_utt, L, stride, seed, first_utt, k):
             "pcm_bit_identical_to_host_generator": ok_pcm, "labels_equal_oracle_on_decisive_rows": ok_lab,
             "logits_within_1e-3": ok_logit, "max_logit_abs_err": max_err,
             "oracle": "oracle/ref_math.py (float64 restatement pinned to the reference's golden vectors)"}
+
+
+def dump_outputs(out_dir, plan, labels, n_utt, torch):
+    """The labels the timed launches wrote in their last step, for whole utterances drawn with a fixed seed (the
+    same utterances for the same arguments, whatever the build): DIR/labels.npy float32 [k, rows per utterance] and
+    DIR/utterances.npy float64 [k], the utterances' indices in the rank-0 shard."""
+    import numpy as np
+    ro = plan.row_offsets
+    rows = int(ro[1] - ro[0])                                   # uniform layout: every utterance has as many rows
+    k = min(n_utt, DUMP_LABEL_BYTES // (4 * max(rows, 1)))
+    utts = np.sort(np.random.default_rng(0).choice(n_utt, size=k, replace=False))
+    idx = torch.from_numpy(ro[utts][:, None] + np.arange(rows)).to(labels.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "labels.npy"), labels[idx].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "utterances.npy"), utts.astype(np.float64))
 
 
 def stream_record(h, a, torch):
@@ -398,6 +427,9 @@ def main():
     need = n_utt * stride * 2 + n_utt * 1000 + (3 << 30)
     free, _ = torch.cuda.mem_get_info(dev)
     if need > free:  # never drive the box out of memory: shrink and say so
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs: %.0f h per GPU do not fit in free GPU memory; a smaller workload's "
+                             "outputs would not compare with a full run's" % a.hours_per_gpu)
         n_utt = int((free - (4 << 30)) // (stride * 2 + 1000))
         offsets, lengths, stride = batch.uniform_layout(n_utt, L)
         a.hours_per_gpu = n_utt * a.utt_seconds / 3600.0
@@ -454,6 +486,8 @@ def main():
         time.sleep(0.1)
         sampler.stop()
     ms_per_step = ms_total / a.steps
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, plan, labels, n_utt, torch)
     total_audio = sum_over_ranks(audio_s)
     value = total_audio / (ms_per_step * 1e-3)
     speech_frac = float(labels[: min(frames, 50_000_000)].float().mean().item())

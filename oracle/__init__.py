@@ -13,8 +13,7 @@ Pinning status
   (``oracle/reference_shim.py`` imports /root/reference/mfcc.py,
   dataset/file_processing.py and realtime_analysis/sklearn_analyser.py).
   ``oracle/make_golden.py`` froze those outputs into ``tests/golden/*.npz``;
-  ``tests/test_oracle.py`` re-checks the restatement against the fixtures on any
-  box and against the live reference whenever /root/reference is present.
+  ``tests/test_oracle.py`` re-checks the restatement against the fixtures.
 * FFN forward (``ref_math.ffn_forward``): **parity unpinned**.  The reference
   only defines the architecture (learning/ffn_trainer.py:104-116); it never
   runs inference, ships no weights, and its arithmetic lives in Keras 1.x

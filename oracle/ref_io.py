@@ -3,8 +3,8 @@
 Line citations are relative to /root/reference.  ``dataset/sph.py`` and ``dataset/stm_parser.py`` are python-2
 byte-string code (``header[2].split(' ')`` on a file opened 'rb', ``ord(chunk[i])``) and do not run under
 python 3 even through the shim, so these two are restated from the source and are NOT pinned to an execution of
-the reference ("parity unpinned" for SPHERE / STM ingest); ``process_file`` on wav files IS pinned to the live
-reference in tests/test_oracle.py when it is mounted.
+the reference ("parity unpinned" for SPHERE / STM ingest); ``process_file`` on wav files IS pinned to the
+reference's own output (tests/golden/utterances.npz) in tests/test_oracle.py.
 """
 import os
 

@@ -1,10 +1,9 @@
 """Loader that imports the UNMODIFIED reference (python-2 code) under python 3.
 
 TEST INFRASTRUCTURE.  Sources come from /root/reference where it is mounted (the build container)
-or from the byte-identical staged copy oracle/_ref/ (``oracle/make_ref.py``; git-ignored, travels
-to the GPU box).  Used by ``oracle/make_golden.py`` to freeze fixtures, by ``tests/test_oracle.py``
-to re-pin the restatement against the live reference, and by ``oracle/cpu_bench.py`` to time the
-reference's own code.  Recipe: SURVEY.md appendix C.
+or from the byte-identical staged copy oracle/_ref/ (``oracle/make_ref.py``; git-ignored).  Used by
+``oracle/make_golden.py`` to freeze fixtures and by ``oracle/cpu_bench.py`` to time the reference's
+own code.  Recipe: SURVEY.md appendix C.
 """
 import os
 import pickle

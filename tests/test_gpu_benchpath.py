@@ -345,3 +345,37 @@ def test_bit_identical_frames_define_nan_rows(hw):
     sig = np.lib.stride_tricks.sliding_window_view(c, 5, axis=0)[: c.shape[0] - 5].std(axis=2)
     tol = 3e-4 + 2e-4 / np.maximum(np.tile(sig, 3), 1e-12)
     assert np.all(np.abs(fe2 - ref_f)[fin] <= tol[fin])
+
+
+def test_bench_dump_outputs_hold_the_timed_labels(hw, tmp_path):
+    """bench.py --dump-outputs saves the timed step's labels of a seeded sample of utterances: the rows a plan over the
+    same seeded workload gives for those utterances, within the 64 MB cap; --steps sets the number of timed launches."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import torch
+    from vad_b200 import batch, runtime
+    h, w = hw
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    seed, n_utt, L = 77, 14400, 160000                                         # 40 h of 10 s utterances
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                          "--hours-per-gpu", "40", "--seed", str(seed), "--no-e2e", "--no-cpu-baseline",
+                          "--no-extra-configs", "--parity-utts", "0", "--dump-outputs", str(tmp_path / "dump")],
+                         stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-3000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["gpu_launches"] == 2 and line["frames_per_step"] == n_utt * 993
+    got = np.load(str(tmp_path / "dump" / "labels.npy"))
+    utts = np.load(str(tmp_path / "dump" / "utterances.npy"))
+    assert got.dtype == np.float32 and utts.dtype == np.float64 and got.nbytes + utts.nbytes <= 64 << 20
+    ids = utts.astype(np.int64)
+    assert np.array_equal(ids, utts) and np.all(np.diff(ids) > 0) and 0 <= ids[0] and ids[-1] < n_utt
+    assert got.shape == (ids.size, 993) and 10000 < ids.size < n_utt                  # a sample, not the whole output
+    h.set_ffn_impl("tc16")                                                      # bench.py's default FFN
+    off, ln, stride = batch.uniform_layout(n_utt, L)
+    pcm = h.synth_pcm(n_utt, L, seed=seed, first_utt=0, utt_stride=stride)
+    labels = runtime.Plan(h, off, ln, runtime.MODE_VAD).vad(pcm)[0].view(n_utt, 993)
+    assert np.array_equal(got, labels[torch.from_numpy(ids).to(h.device)].float().cpu().numpy())
+    for u in (int(ids[0]), int(ids[-1])):
+        check_vad(got[np.searchsorted(ids, u)].astype(np.uint8), None, synth_utterance(seed, u, L), w)

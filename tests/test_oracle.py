@@ -1,12 +1,11 @@
-"""CPU: pin the oracle restatement (oracle/ref_math.py, oracle/ref_loop.py) against the
-golden vectors frozen from the unmodified reference, and against the live reference when
-/root/reference is mounted (build container only)."""
+"""CPU: pin the oracle restatement (oracle/ref_math.py, oracle/ref_loop.py, oracle/ref_io.py) against
+the golden vectors frozen from the unmodified reference (oracle/make_golden.py)."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle import ref_math as rm, ref_loop, reference_shim
+from oracle import ref_math as rm, ref_loop
 
 
 @pytest.fixture(scope="module")
@@ -134,65 +133,18 @@ def test_ffn_nan_rows_are_nonspeech():
     assert np.all(np.isnan(logits)) and np.array_equal(rm.decide(logits), [0, 0])
 
 
-def test_scale_features_matches_reference_when_mounted():
-    if not reference_shim.available():
-        pytest.skip("reference not mounted")
-    import sys
-    ref = reference_shim.load()
-    sys.path.insert(0, "/root/reference/dataset")
-    import importlib
-    ref_utils = importlib.import_module("utils") if "utils" not in sys.modules else None
-    if ref_utils is None or not hasattr(ref_utils, "scale_features"):
-        spec = importlib.util.spec_from_file_location("ref_dataset_utils", "/root/reference/dataset/utils.py")
-        ref_utils = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref_utils)
-    rng = np.random.default_rng(3)
-    groups = [rng.standard_normal((n, 39)) * 3 + 1 for n in (5, 9)]
-    as_lists = [[(r[:13].copy(), r[13:26].copy(), r[26:].copy()) for r in g] for g in groups]
-    ref_utils.scale_features(as_lists)
-    mine, _ = rm.scale_features(groups)
-    for g, l in zip(mine, as_lists):
-        np.testing.assert_allclose(g, np.array([np.concatenate(r) for r in l]), atol=1e-12)
-
-
-def test_live_reference_when_mounted():
-    if not reference_shim.available():
-        pytest.skip("reference not mounted")
-    ref = reference_shim.load()
-    fb = ref.mfcc.get_mel_filterbanks(300, 8000, ref.FFT_N, 26, 16000)
-    assert np.array_equal(fb, rm.get_mel_filterbanks())
-    rng = np.random.default_rng(11)
-    for amp in (3.0, 300.0, 30000.0):
-        frame = np.clip(rng.standard_normal(400) * amp, -32768, 32767).astype(np.int16)
-        np.testing.assert_allclose(rm.get_mfcc(frame, fb), ref.mfcc.get_mfcc(frame, ref.FFT_N, fb, 13),
-                                   rtol=0, atol=2e-5)
-
-
-def test_ref_io_wav_path_matches_live_process_file_when_mounted(tmp_path):
-    """oracle/ref_io.py's file path (wav read + dataset rows) against the unmodified reference process_file."""
-    if not reference_shim.available():
-        pytest.skip("reference not mounted")
+@pytest.mark.parametrize("name", CASES)
+def test_ref_io_wav_path_matches_reference_process_file(utts, name, tmp_path):
+    """oracle/ref_io.py's file path (wav read + dataset rows) against the rows the unmodified reference's
+    process_file returned for the same PCM written as a 16 kHz wav (tests/golden/utterances.npz)."""
     from scipy.io import wavfile
     from oracle import ref_io
-    from vad_b200.synth import synth_utterance
-    ref = reference_shim.load()
-    pcm = synth_utterance(5, 3, 20000)
+    pcm = utts[name + "/pcm"]
     path = str(tmp_path / "u.wav")
     wavfile.write(path, 16000, pcm)
-
-    class Q(object):
-        v = 0
-
-        def get(self):
-            return self.v
-
-        def put(self, v):
-            self.v = v
-
-    fb = ref.mfcc.get_mel_filterbanks(300, 8000, ref.FFT_N, 26, 16000)
-    feats = ref.file_processing.process_file([path, 400, 160, ref.FFT_N, fb, 13, Q(), None])
-    want = np.array([np.concatenate(f) for f in feats])
     got = rm.dataset_features(rm.mfcc_utterance(ref_io.file_samples(path)))
+    want = utts[name + "/dataset_rows"]
+    assert got.shape == want.shape
     np.testing.assert_allclose(got, want, rtol=0, atol=2e-5)
 
 
