@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define VADB200_VERSION 200
+#define VADB200_VERSION 201
 
 #define VADB200_OK 0
 #define VADB200_E_INVALID (-1)      /* bad argument (null, negative, misaligned) */
@@ -91,6 +91,22 @@ int vadb200_set_ffn_weights(vadb200_handle* h, const float* W1, const float* b1,
  * meet the logit tolerance; applies to vadb200_vad_packed / vadb200_vad_host / vadb200_ffn_predict. */
 int vadb200_set_ffn_impl(vadb200_handle* h, int impl);
 int vadb200_get_ffn_impl(vadb200_handle* h);
+
+/* Opt-in front end and operating point (python_speech_features-style front ends); the defaults reproduce the
+ * reference (no pre-emphasis, rectangular window, argmax == VOICED).  Handle state read at launch, like ffn_impl.
+ * Pre-emphasis y[0] = x[0], y[n] = x[n] - preemph x[n-1] (preemph in [0, 1]) runs over each utterance as a whole
+ * before framing (a bank stream: one signal from its last reset; the per-frame API: each frame on its own); then
+ * the 400 window weights h_window (NULL = rectangular) multiply frame samples 0..399.  Applies to
+ * vadb200_mfcc_packed / _vad_packed / _mfcc_host / _vad_host / _spec_frames / _mfcc_frames / _stream_feed; the
+ * per-frame calls reject a window unless frame_len == 400.  get: h_window (nullable) receives the 400 weights
+ * (ones without a window). */
+int vadb200_set_frontend(vadb200_handle* h, float preemph, const float* h_window /* [400] or NULL */);
+int vadb200_get_frontend(vadb200_handle* h, float* preemph, float* h_window /* nullable */, int* has_window);
+/* speech <=> softmax(logits)[1] >= p_voiced; p_voiced <= 0 restores argmax == VOICED (default), >= 1 or NaN is
+ * rejected.  Logits and features do not depend on it; rows with non-finite features stay label 0.  Applies to
+ * vadb200_vad_packed / _vad_host / _vad_windows / _ffn_predict / _stream_feed.  get: 0 = argmax. */
+int vadb200_set_decision_threshold(vadb200_handle* h, float p_voiced);
+float vadb200_get_decision_threshold(vadb200_handle* h);
 
 /* ---- ragged packed batches (replaces dataset_creator.process_files' Pool.map over files,
  * dataset_creator.py:53-65, and split_into_frames, file_processing.py:80-103) ---------------

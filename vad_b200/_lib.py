@@ -35,6 +35,10 @@ SIGNATURES = {
     "vadb200_set_ffn_weights": (C.c_int, [_P] + [_P] * 8),
     "vadb200_set_ffn_impl": (C.c_int, [_P, C.c_int]),
     "vadb200_get_ffn_impl": (C.c_int, [_P]),
+    "vadb200_set_frontend": (C.c_int, [_P, C.c_float, _P]),
+    "vadb200_get_frontend": (C.c_int, [_P, _P, _P, _P]),
+    "vadb200_set_decision_threshold": (C.c_int, [_P, C.c_float]),
+    "vadb200_get_decision_threshold": (C.c_float, [_P]),
     "vadb200_plan_create": (C.c_int, [_P, _P, _P, _I64, C.c_int, C.POINTER(_P)]),
     "vadb200_plan_destroy": (C.c_int, [_P]),
     "vadb200_plan_total_rows": (_I64, [_P]),

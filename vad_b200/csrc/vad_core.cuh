@@ -90,10 +90,10 @@ struct FfnParams {
   float b3[kH3];
   float W4[kH3 * kNCls];
   float b4[kNCls];
-  float pad_[1];
+  float thresh;                  // decision threshold on p(voiced); <= 0: argmax (vadb200_set_decision_threshold)
 };
 struct alignas(8) FfnBias {      // what the tensor-core FFN needs besides its weight blob
-  float b1[kH1], b2[kH2], b3[kH3], b4[kNCls], pad_[1];
+  float b1[kH1], b2[kH2], b3[kH3], b4[kNCls], thresh;  // thresh: as FfnParams::thresh
   float pre[4];                  // fp16 operand path: power-of-two scale of layer l's input activations (pre[0] == 1)
   float post[4];                 // ... and the exact inverse of (weight scale x activation scale)
   // fp16 path, hidden layers: the next layer's activation scale folded into this layer's epilogue (powers of two,
@@ -255,6 +255,49 @@ VADB_HD void fft_load_f32(const float* fr, int frame_len, int t, float (&xr)[16]
     const int n = 2 * (t + 16 * j);
     xr[j] = (n < frame_len) ? fr[n] : 0.0f;
     xi[j] = (n + 1 < frame_len) ? fr[n + 1] : 0.0f;
+  });
+}
+
+// ---- opt-in front end (vadb200_set_frontend): pre-emphasis y[n] = x[n] - a x[n-1], then window weights ----------
+// w2[m] = (w[2m], w[2m+1]): a 400-point window (ones when none is set; 256 pairs, entries past 400 are 1).
+#if defined(__CUDA_ARCH__)
+VADB_HD cf2 win_pair(const cf2* w2, int m) {  // read-only path: every CTA reads the same 2 KB, it stays in L1
+  const float2 v = __ldg(reinterpret_cast<const float2*>(w2) + m);
+  return cf2{v.x, v.y};
+}
+#else
+VADB_HD cf2 win_pair(const cf2* w2, int m) { return w2[m]; }
+#endif
+// fft_load_pcm2 with the front end.  Word m - 1 carries x[2m - 1] in its high half: for m = 0, w32[-1] must hold the
+// sample before the frame (0 at an utterance start); frame B's word -1 is frame A's data.  The previous word is a
+// second shared-memory load per word (same banks pattern as the first: conflict free).
+VADB_HD void fft_load_pcm2_fe(const uint32_t* w32, int delta, int t, float a, const cf2* w2, f2 (&xr)[16],
+                              f2 (&xi)[16]) {
+  static_for<0, 13>([&](auto J) {
+    constexpr int j = J;
+    const bool on = (j < 12 || t < 8);
+    const int m = t + 16 * j;
+    const uint32_t va = on ? w32[m] : 0u, pa = on ? w32[m - 1] : 0u;
+    const uint32_t vb = on ? w32[delta + m] : 0u, pb = on ? w32[delta + m - 1] : 0u;
+    const cf2 w = on ? win_pair(w2, m) : cf2{0.0f, 0.0f};
+    const f2 lo = mk2(pcm_lo(va), pcm_lo(vb)), hi = mk2(pcm_hi(va), pcm_hi(vb)), prev = mk2(pcm_hi(pa), pcm_hi(pb));
+    xr[j] = vmuls(w.x, vfmas(-a, prev, lo));  // y[2m]     = x[2m]     - a x[2m - 1]
+    xi[j] = vmuls(w.y, vfmas(-a, lo, hi));    // y[2m + 1] = x[2m + 1] - a x[2m]
+  });
+  xr[13] = xi[13] = xr[14] = xi[14] = xr[15] = xi[15] = mk2(0.0f, 0.0f);
+}
+// fft_load_f32 with the front end; each frame is its own signal (y[0] = x[0]).
+VADB_HD void fft_load_f32_fe(const float* fr, int frame_len, int t, float a, const cf2* w2, float (&xr)[16],
+                             float (&xi)[16]) {
+  static_for<0, 16>([&](auto J) {
+    constexpr int j = J;
+    const int m = t + 16 * j, n = 2 * m;
+    const float x0 = (n < frame_len) ? fr[n] : 0.0f;
+    const float x1 = (n + 1 < frame_len) ? fr[n + 1] : 0.0f;
+    const float xp = (n > 0 && n < frame_len) ? fr[n - 1] : 0.0f;
+    const cf2 w = win_pair(w2, m);
+    xr[j] = w.x * fmaf(-a, xp, x0);
+    xi[j] = (n + 1 < frame_len) ? w.y * fmaf(-a, x0, x1) : 0.0f;  // zero padding stays zero
   });
 }
 
@@ -687,6 +730,12 @@ VADB_HD void ffn_forward(const FfnParams& w, const float (&x)[kNFeat], float (&l
 // takes the first maximum, so class 1 must be strictly greater than class 0 and >= class 2.
 VADB_HD uint8_t decide(const float (&logit)[kNCls]) {
   return (logit[1] > logit[0] && logit[1] >= logit[2]) ? 1 : 0;
+}
+// Opt-in operating point: speech <=> softmax(logit)[1] >= th.  th <= 0 keeps the argmax rule.
+VADB_HD uint8_t decide(const float (&logit)[kNCls], float th) {
+  if (!(th > 0.0f)) return decide(logit);
+  const float s = 1.0f + expf(logit[0] - logit[1]) + expf(logit[2] - logit[1]);  // 1 / p(voiced)
+  return (1.0f / s >= th) ? 1 : 0;
 }
 
 }  // namespace vadb

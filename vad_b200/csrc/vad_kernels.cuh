@@ -66,7 +66,14 @@ struct Segment {
   long long pcm_start;  // sample index of the first frame's first sample (multiple of 8)
   long long out_start;  // first output row of the segment
   int n_frames;         // MFCC frames to compute (outputs + 4 in window modes)
-  int pad;
+  int cont;             // 1: the segment continues an utterance (the sample before it is real), 0: utterance start
+};
+
+// Opt-in front end of the fused kernels' fused_fe_kernel variant (vadb200_set_frontend): pre-emphasis coefficient and
+// the handle's window table (vad_core.cuh fft_load_pcm2_fe; all ones when no window is set).
+struct FrontEnd {
+  const cf2* win;
+  float preemph;
 };
 
 // Timing-experiment hooks (phase ablation mask, clock64 stamps) are compiled in only with
@@ -153,17 +160,17 @@ struct ShflXchg {
 };
 
 // Four frames of a warp through the FFT: half-warp h = lanes 16h..16h+15, two frames per thread.
-// w32a: first PCM word of frame A; frame B starts `delta` words later.  ex: this half-warp's
-// transpose scratch (kExchFrame 64-bit slots).
+// ex: this half-warp's transpose scratch (kExchFrame 64-bit slots).
 // store(bin, v): receives |2X|^2 of power bin `bin` for frame A (v.x) and frame B (v.y).
 // before_store() runs after the second DFT16 and before the first power value is stored (the fused kernels put the
 // CTA barrier that protects the previous step's power tile there: by then every warp has long left its mel phase).
-template <int NZ, class PRE, class STORE>
-__device__ __forceinline__ void warp_fft_quad(const uint32_t* w32a, int delta, f2* ex, const cf2* s_tw1,
-                                               const cf2* s_tw2, int lane, PRE&& before_store, STORE&& store) {
+// load(t, xr, xi) fills thread t's inputs (fft_load_pcm2 or, with the front end, fft_load_pcm2_fe).
+template <int NZ, class LOAD, class PRE, class STORE>
+__device__ __forceinline__ void warp_fft_quad(LOAD&& load, f2* ex, const cf2* s_tw1, const cf2* s_tw2, int lane,
+                                               PRE&& before_store, STORE&& store) {
   const int t = lane & 15;
   f2 xr[16], xi[16];
-  fft_load_pcm2(w32a, delta, t, xr, xi);
+  load(t, xr, xi);
   fft_pass1<NZ>(xr, xi, s_tw1, t);
   exch_store_plane(ex, t, xr);
   __syncwarp();
@@ -254,13 +261,14 @@ __device__ __forceinline__ void flush_flat(float* dst, int total, int tid, GEN&&
 }
 
 // One output row per thread: window features -> FFN -> decision (block phase / windows API).
+// th: decision threshold (decide); 0 = argmax.
 __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r)[5][kNCep], int feat_mode,
-                                             uint8_t* labels, float* logits, float* feats, long long row) {
+                                             uint8_t* labels, float* logits, float* feats, long long row, float th) {
   float x[kNFeat];
   const bool ok = window_features(r, feat_mode, x);
   float logit[kNCls];
   ffn_forward(w, x, logit);
-  uint8_t lab = decide(logit);
+  uint8_t lab = decide(logit, th);
   if (!ok) {
     logit[0] = logit[1] = logit[2] = NAN;
     lab = 0;
@@ -287,11 +295,27 @@ template <> struct FfnArgOf<2, 0> { using type = FfnParams; };
 template <> struct FfnArgOf<2, 1> { using type = FfnBias; };
 template <> struct FfnArgOf<2, 2> { using type = FfnBias; };
 
-template <int MODE, int TC>
-__global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constant__ FusedParams p,
-                                                            const __grid_constant__ typename FfnArgOf<MODE, TC>::type ffn) {
+// The decision of the VAD block phase: argmax, or with the front-end variant the handle's threshold.
+template <bool FE, class A>
+__device__ __forceinline__ uint8_t decide_of(const float (&logit)[kNCls], const A& ffn) {
+  if constexpr (FE && !std::is_same<A, FfnNone>::value) return decide(logit, ffn.thresh);
+  else return decide(logit);
+}
+
+// FE: the front-end variant (fused_fe_kernel).  Its PCM stage starts kStageOffFe samples into each buffer and the
+// sample before the step's first frame sits just below it (0 at an utterance start), so fft_load_pcm2_fe finds
+// every frame's previous sample at word -1.  The step's 5360 samples + 8 still fit the 5376-sample buffer.
+constexpr int kStageOffFe = 8;
+static_assert(kStageSamples + kStageOffFe <= kStagePad, "front-end stage offset must fit the PCM buffer");
+
+// tid comes from the kernel: threadIdx.x read inside the kernel carries the launch bound's range (0 .. 255), which the
+// code generation relies on (read here, the default kernels' SASS would change).
+template <int MODE, int TC, bool FE>
+__device__ __forceinline__ void fused_body(const FusedParams& p, const typename FfnArgOf<MODE, TC>::type& ffn,
+                                           const FrontEnd& fe, const int tid) {
   static_assert(TC == 0 || MODE == 2, "tensor-core FFN only exists in VAD mode");
   constexpr int kBlk = TC ? kBlockStepsTc : kBlockSteps;
+  constexpr int kStageOff = FE ? kStageOffFe : 0;
   extern __shared__ __align__(128) unsigned char smem[];
   int16_t* s_pcm = reinterpret_cast<int16_t*>(smem + kOffPcm);
   cf2* s_exch = reinterpret_cast<cf2*>(smem + kOffExch);
@@ -303,7 +327,7 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
   uint64_t* s_bar = reinterpret_cast<uint64_t*>(smem + kOffBar);
   int* s_seg = reinterpret_cast<int*>(smem + kOffSeg);
 
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, h = lane >> 4, t = lane & 15;
+  const int warp = tid >> 5, lane = tid & 31, h = lane >> 4, t = lane & 15;
 
   s_tw1[tid] = p.tw1[tid];
   if (tid < 128) s_tw2[tid] = p.tw2[tid];
@@ -345,13 +369,16 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
     const long long avail = p.pcm_len - start;
     const int nsmp = avail >= kStageSamples ? kStageSamples : (avail > 0 ? static_cast<int>(avail) : 0);
     const int bulk = (nsmp * 2) & ~15;
-    int16_t* dst = s_pcm + buf * kStagePad;
+    int16_t* dst = s_pcm + buf * kStagePad + kStageOff;
     if (tid == 0) {
       mbar_arrive_expect_tx(&s_bar[buf], static_cast<uint32_t>(bulk));
       if (bulk) bulk_g2s(dst, p.pcm + start, static_cast<uint32_t>(bulk), &s_bar[buf]);
     }
     const int tail0 = bulk >> 1;  // < 8 samples past the last whole 16-byte chunk of the buffer
     if (tid < nsmp - tail0) dst[tail0 + tid] = p.pcm[start + tail0 + tid];
+    // the previous sample: part of the utterance unless this is the first step of an utterance's first segment
+    // (published like the tail samples: by warp 0's arrival on "P full" / the barrier after the first load)
+    if (FE && tid == 31) dst[-1] = (step > 0 || seg.cont) ? p.pcm[start - 1] : int16_t(0);
   };
 
   for (;;) {
@@ -402,13 +429,18 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
       };
 
       // ---- FFT phase ---------------------------------------------------------------------
-      const uint32_t* stage32 = reinterpret_cast<const uint32_t*>(s_pcm + buf * kStagePad);
+      const uint32_t* stage32 = reinterpret_cast<const uint32_t*>(s_pcm + buf * kStagePad + kStageOff);
       if (!(VADB_DBG(p) & 1)) {
         // half-warp h: frame slots 4 warp + h and + 2 (PCM 80 words apart per slot -> the two half-warps
         // read different banks), P columns 4 warp + 2 h, + 1
         f2* ex = reinterpret_cast<f2*>(s_exch) + (warp * 2 + h) * kExchFrame;
-        warp_fft_quad<13>(stage32 + (warp * 4 + h) * (kHop / 2), kHop, ex, s_tw1, s_tw2, lane,
-                          [&] { mbar_wait(&s_bar[4], par); }, p2store);
+        const uint32_t* w32a = stage32 + (warp * 4 + h) * (kHop / 2);
+        warp_fft_quad<13>(
+            [&](int tt, f2 (&xr)[16], f2 (&xi)[16]) {
+              if constexpr (FE) fft_load_pcm2_fe(w32a, kHop, tt, fe.preemph, fe.win, xr, xi);
+              else fft_load_pcm2(w32a, kHop, tt, xr, xi);
+            },
+            ex, s_tw1, s_tw2, lane, [&] { mbar_wait(&s_bar[4], par); }, p2store);
       } else {
         mbar_wait(&s_bar[4], par);
       }
@@ -505,7 +537,8 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
               for (int k = 0; k < kNCep; ++k) r[d][k] = s_ring[ring_idx(k, col, kRing)];
             }
             if constexpr (MODE == 2 && TC == 0)
-              classify_row(ffn, r, p.feat_mode, p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2));
+              classify_row(ffn, r, p.feat_mode, p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2),
+                           FE ? ffn.thresh : 0.0f);
           }
           out_done = max(out_done, computed - 2);
         } else {
@@ -559,7 +592,7 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
               ++dbg_n;
               if (valid && hidx == 0) {
                 const bool ok = s_logE[fr] != 0.0f && s_logE[128 + fr] != 0.0f;  // ordered by the tile's bar.syncs
-                uint8_t lab = decide(logit);
+                uint8_t lab = decide_of<FE>(logit, ffn);  // logits are in registers: no TMEM round trip
                 if (!ok) {
                   logit[0] = logit[1] = logit[2] = NAN;
                   lab = 0;
@@ -596,6 +629,20 @@ __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constan
       __threadfence();
     }
   }
+}
+
+template <int MODE, int TC>
+__global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constant__ FusedParams p,
+                                                            const __grid_constant__ typename FfnArgOf<MODE, TC>::type ffn) {
+  fused_body<MODE, TC, false>(p, ffn, FrontEnd{nullptr, 0.0f}, threadIdx.x);
+}
+// The same kernel with the opt-in front end and decision threshold; launched only when the handle sets either, so the
+// default path above keeps its code.
+template <int MODE, int TC>
+__global__ void __launch_bounds__(kThreads, 2) fused_fe_kernel(const __grid_constant__ FusedParams p,
+                                                               const __grid_constant__ typename FfnArgOf<MODE, TC>::type ffn,
+                                                               const __grid_constant__ FrontEnd fe) {
+  fused_body<MODE, TC, true>(p, ffn, fe, threadIdx.x);
 }
 
 // Stand-alone tensor-core FFN over feature rows [n][39] (classifier.predict duck type): one CTA =
@@ -656,7 +703,7 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
   if constexpr (KIND == 2) ffn_tc16_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
   else ffn_tc_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
   if (i < n) {
-    uint8_t lab = decide(logit);
+    uint8_t lab = decide(logit, fb.thresh);
     if (!ok) {
       logit[0] = logit[1] = logit[2] = NAN;
       lab = 0;
@@ -750,8 +797,9 @@ __global__ void __launch_bounds__(kThreads, MINB) exp_fft_kernel(const FusedPara
 // what: 0 -> spectrum [n][256] (get_spec_mag), 1 -> MFCC [n][13] (get_mfcc).
 constexpr int kFramesSmemBytes = kWarps * 2 * kExchFrame * 8 + kBins * kPPitch * 4 + kNMel * 32 * 4 + 384 * 8;
 
+// fe: the handle's front end (fe.win == nullptr: none).
 __global__ void __launch_bounds__(kThreads) frames_kernel(const float* frames, long long n, int frame_len, int what,
-                                                         float* out, const cf2* tw1, const cf2* tw2) {
+                                                         float* out, const cf2* tw1, const cf2* tw2, FrontEnd fe) {
   extern __shared__ __align__(128) unsigned char smem[];
   cf2* s_exch = reinterpret_cast<cf2*>(smem);
   float* s_P = reinterpret_cast<float*>(smem + kWarps * 2 * kExchFrame * 8);
@@ -769,8 +817,12 @@ __global__ void __launch_bounds__(kThreads) frames_kernel(const float* frames, l
     const int fi = warp * 4 + r * 2 + h;
     const long long f = min(f0 + fi, n - 1);  // clamp: surplus slots recompute the last frame
     const float* fr = frames + f * frame_len;
-    warp_fft_pair<16>([&](float (&xr)[16], float (&xi)[16]) { fft_load_f32(fr, frame_len, t, xr, xi); }, ex, s_tw1,
-                      s_tw2, s_P, fi, lane);
+    warp_fft_pair<16>(
+        [&](float (&xr)[16], float (&xi)[16]) {
+          if (fe.win) fft_load_f32_fe(fr, frame_len, t, fe.preemph, fe.win, xr, xi);
+          else fft_load_f32(fr, frame_len, t, xr, xi);
+        },
+        ex, s_tw1, s_tw2, s_P, fi, lane);
   }
   __syncthreads();
   if (what == 0) {
@@ -820,7 +872,7 @@ __global__ void __launch_bounds__(128) windows_kernel(const float* win, long lon
   for (int d = 0; d < 5; ++d)
 #pragma unroll
     for (int k = 0; k < kNCep; ++k) r[d][k] = win[(i * 5 + d) * kNCep + k];
-  classify_row(w, r, feat_mode, labels, logits, feats, i);
+  classify_row(w, r, feat_mode, labels, logits, feats, i, w.thresh);
 }
 
 // classifier.predict duck type (sklearn_analyser.py:71): rows [n][39] -> class {0,1}, logits.
@@ -837,7 +889,7 @@ __global__ void __launch_bounds__(128) ffn_rows_kernel(const float* x, long long
   }
   float logit[kNCls];
   ffn_forward(w, v, logit);
-  uint8_t lab = decide(logit);
+  uint8_t lab = decide(logit, w.thresh);
   if (!ok) {
     logit[0] = logit[1] = logit[2] = NAN;
     lab = 0;
@@ -880,11 +932,14 @@ struct BankParams {
   const cf2* tw1;
   const cf2* tw2;
   int feat_mode;
+  int16_t* prev;          // [n_streams] the raw sample before the 320-sample history (front end only)
+  FrontEnd fe;            // fe.win == nullptr: no front end
 };
 constexpr int kStreamFramePitch = 480;  // samples per staged row: [history 320 | chunk 160] (240 words == 16 mod 32)
 constexpr int kStreamPBytes = kP2Bytes > (kNFeat + kH1 + kH2 + kH3 + kNCep) * 32 * 4
                                   ? kP2Bytes : (kNFeat + kH1 + kH2 + kH3 + kNCep) * 32 * 4;  // P tile, later activations
-constexpr int kStreamSmemBytes = kStepFrames * kStreamFramePitch * 2 + kWarps * 2 * kExchFrame * 8 +
+constexpr int kStreamRowsOff = 16;      // bytes below staged row 0: its word -1 (front end)
+constexpr int kStreamSmemBytes = kStreamRowsOff + kStepFrames * kStreamFramePitch * 2 + kWarps * 2 * kExchFrame * 8 +
                                  kStreamPBytes + kNMel * 32 * 4 + 384 * 8;
 
 // One CTA = 32 streams.  FFT: the fused kernel's packed two-frames-per-thread pass.  The decision
@@ -893,8 +948,8 @@ constexpr int kStreamSmemBytes = kStepFrames * kStreamFramePitch * 2 + kWarps * 
 // handed over through shared memory (the idle P tile); weights are uniform constant-bank operands.
 __global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams p, const __grid_constant__ FfnParams w) {
   extern __shared__ __align__(128) unsigned char smem[];
-  int16_t* s_fr = reinterpret_cast<int16_t*>(smem);
-  cf2* s_exch = reinterpret_cast<cf2*>(smem + kStepFrames * kStreamFramePitch * 2);
+  int16_t* s_fr = reinterpret_cast<int16_t*>(smem + kStreamRowsOff);
+  cf2* s_exch = reinterpret_cast<cf2*>(smem + kStreamRowsOff + kStepFrames * kStreamFramePitch * 2);
   float* s_P = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(s_exch) + kWarps * 2 * kExchFrame * 8);
   float* s_logE = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(s_P) + kStreamPBytes);
   cf2* s_tw1 = reinterpret_cast<cf2*>(s_logE + kNMel * 32);
@@ -927,10 +982,28 @@ __global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams 
       reinterpret_cast<uint32_t*>(p.hist + static_cast<long long>(st) * 320)[wd] =
           reinterpret_cast<const uint32_t*>(s_fr + fi * kStreamFramePitch)[80 + wd];
   }
+  if (p.fe.win) {
+    // Front end: a stream is one signal from its last reset.  The sample before the history goes to the high half of
+    // the row's word -1 (the previous row's last chunk word: the roll above has consumed it), and the stream's new
+    // previous sample is old hist[159], the one before the new history.
+    __syncthreads();
+    if (tid < kStepFrames) {
+      int16_t* row = s_fr + tid * kStreamFramePitch;
+      const int st = min(s0 + tid, p.n_streams - 1);
+      row[-1] = p.prev[st];
+      if (s0 + tid < p.n_streams) p.prev[st] = row[159];
+    }
+    __syncthreads();
+  }
   {
     f2* ex = reinterpret_cast<f2*>(s_exch) + (warp * 2 + h) * kExchFrame;
     const uint32_t* w32 = reinterpret_cast<const uint32_t*>(s_fr + (warp * 4 + h) * kStreamFramePitch);
-    warp_fft_quad<13>(w32, kStreamFramePitch, ex, s_tw1, s_tw2, lane, [] {}, P2Store(s_P, col_of_halfwarp(warp, h), lane & 15));
+    warp_fft_quad<13>(
+        [&](int t, f2 (&xr)[16], f2 (&xi)[16]) {
+          if (p.fe.win) fft_load_pcm2_fe(w32, kStreamFramePitch, t, p.fe.preemph, p.fe.win, xr, xi);
+          else fft_load_pcm2(w32, kStreamFramePitch, t, xr, xi);
+        },
+        ex, s_tw1, s_tw2, lane, [] {}, P2Store(s_P, col_of_halfwarp(warp, h), lane & 15));
   }
   __syncthreads();
   mel2_run_dispatch<kP2Pitch, 32>(warp, s_P + 2 * lane, s_logE + lane);
@@ -1035,7 +1108,7 @@ __global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams 
         bool ok = true;
 #pragma unroll
         for (int k = 0; k < kNCep; ++k) ok = ok && (s_ok[k * 32 + lane] != 0);
-        lab = decide(acc);
+        lab = decide(acc, w.thresh);
         if (ok) {
           lg[0] = acc[0]; lg[1] = acc[1]; lg[2] = acc[2];
         } else {

@@ -49,6 +49,7 @@ long long* g_dbg_ts = nullptr;  // timing experiments only (vadb200_debug_timest
 constexpr int kNumSmFallback = 148;
 constexpr int kPlanCounters = 16;  // launches of one plan that may be in flight at once (any streams)
 constexpr int kHostBufs = 3;
+constexpr int kWinPairs = kFftN / 2;  // window pairs for any frame_len <= 512; entries past 400 stay 1
 
 }  // namespace
 
@@ -80,6 +81,11 @@ struct vadb200_handle {
   unsigned char* d_tc16_blob = nullptr; // canonical fp16 hi/lo weight blob, statically scaled
   bool tc16_ok = false;                 // the fp16 scales are in range for this handle's weights
   int ffn_impl = 2;                     // 0: FP32 CUDA cores, 1: tcgen05 tf32 hi/lo, 2: tcgen05 fp16 hi/lo (default)
+  // opt-in front end (vadb200_set_frontend); the decision threshold lives in par.thresh / bias.thresh
+  float preemph = 0.0f;
+  bool has_window = false;
+  float window[kFrame] = {};
+  cf2* d_win = nullptr;                 // [kWinPairs] window pairs, all ones without a window (per handle: no globals)
 };
 
 struct vadb200_plan {
@@ -111,6 +117,7 @@ struct vadb200_bank {
   int16_t* d_hist = nullptr;
   float* d_ring = nullptr;
   int* d_fed = nullptr;
+  int16_t* d_prev = nullptr;  // the raw sample before each stream's history (front end)
 };
 
 namespace {
@@ -135,6 +142,11 @@ int ensure_attrs(vadb200_handle* h) {
   CU(cudaFuncSetAttribute(fused_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
   CU(cudaFuncSetAttribute(fused_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
   CU(cudaFuncSetAttribute(fused_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
   CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
   CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
   CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
@@ -142,6 +154,9 @@ int ensure_attrs(vadb200_handle* h) {
   h->attr_set = true;
   return 0;
 }
+
+bool frontend_on(const vadb200_handle* h) { return h->preemph != 0.0f || h->has_window; }
+FrontEnd frontend_of(const vadb200_handle* h) { return FrontEnd{h->d_win, h->preemph}; }
 
 int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   vadb200_handle* h = p->h;
@@ -159,6 +174,28 @@ int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   const int per_sm = 2;
 #endif
   const int grid = std::min(n_segs, per_sm * h->num_sms);
+  // the front-end variant runs only when the handle asks for a front end or (VAD) a decision threshold
+  const bool fe = frontend_on(h) || (p->mode == VADB200_MODE_VAD && h->par.thresh > 0.0f);
+  const FrontEnd fea = frontend_of(h);
+  if (fe) {
+    switch (p->mode) {
+      case VADB200_MODE_MFCC: fused_fe_kernel<0, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}, fea); break;
+      case VADB200_MODE_DATASET: fused_fe_kernel<1, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}, fea); break;
+      default:
+        if (h->ffn_impl == 2 && h->tc16_ok) {
+          fp.tc_blob = h->d_tc16_blob;
+          fused_fe_kernel<2, 2><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias, fea);
+        } else if (h->ffn_impl >= 1) {
+          fused_fe_kernel<2, 1><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias, fea);
+        } else {
+          fused_fe_kernel<2, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->par, fea);
+        }
+        break;
+    }
+    g_launches.fetch_add(1);
+    CU(cudaGetLastError());
+    return 0;
+  }
   switch (p->mode) {
     case VADB200_MODE_MFCC: fused_kernel<0, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}); break;
     case VADB200_MODE_DATASET: fused_kernel<1, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}); break;
@@ -249,6 +286,7 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   h->cfg = cfg;
   h->num_sms = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : kNumSmFallback;
   h->fb = mel_filterbank(cfg);
+  std::fill(h->window, h->window + kFrame, 1.0f);  // rectangular
   std::memset(&h->par, 0, sizeof(FfnParams));
   std::memset(&h->bias, 0, sizeof(FfnBias));
   std::memset(&h->tab, 0, sizeof(MelDctTables));
@@ -267,10 +305,17 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   if (e == cudaSuccess) e = cudaMalloc(&h->d_sink, 256);
   if (e == cudaSuccess) e = cudaMalloc(&h->d_tc_blob, kTcBlobBytes);
   if (e == cudaSuccess) e = cudaMalloc(&h->d_tc16_blob, kTc16BlobBytes);
+  if (e == cudaSuccess) e = cudaMalloc(&h->d_win, kWinPairs * sizeof(cf2));
+  if (e == cudaSuccess) {
+    std::vector<cf2> ones(kWinPairs, cf2{1.0f, 1.0f});
+    e = cudaMemcpy(h->d_win, ones.data(), kWinPairs * sizeof(cf2), cudaMemcpyHostToDevice);
+  }
   if (e != cudaSuccess) {
     cudaFree(h->d_tw);
     cudaFree(h->d_sink);
     cudaFree(h->d_tc_blob);
+    cudaFree(h->d_tc16_blob);
+    cudaFree(h->d_win);
     delete h;
     return cuda_fail(e, "vadb200_create");
   }
@@ -304,6 +349,7 @@ int vadb200_destroy(vadb200_handle* h) {
   cudaFree(h->d_sink);
   cudaFree(h->d_tc_blob);
   cudaFree(h->d_tc16_blob);
+  cudaFree(h->d_win);
   delete h;
   return 0;
 }
@@ -344,6 +390,45 @@ int vadb200_set_ffn_impl(vadb200_handle* h, int impl) {
   return 0;
 }
 int vadb200_get_ffn_impl(vadb200_handle* h) { return h ? h->ffn_impl : -1; }
+
+int vadb200_set_frontend(vadb200_handle* h, float preemph, const float* h_window) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (!(preemph >= 0.0f && preemph <= 1.0f)) return fail(VADB200_E_INVALID, "pre-emphasis must be in [0, 1]");
+  if (h_window)
+    for (int i = 0; i < kFrame; ++i)
+      if (!std::isfinite(h_window[i])) return fail(VADB200_E_INVALID, "window weights must be finite");
+  std::vector<cf2> pairs(kWinPairs, cf2{1.0f, 1.0f});
+  if (h_window)
+    for (int m = 0; m < kFrame / 2; ++m) pairs[m] = cf2{h_window[2 * m], h_window[2 * m + 1]};
+  // drained + blocking, like the FFN weights: kernels on any stream see a consistent table
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceSynchronize());
+  CU(cudaMemcpy(h->d_win, pairs.data(), kWinPairs * sizeof(cf2), cudaMemcpyHostToDevice));
+  h->preemph = preemph;
+  h->has_window = h_window != nullptr;
+  if (h_window) std::memcpy(h->window, h_window, sizeof(h->window));
+  else std::fill(h->window, h->window + kFrame, 1.0f);
+  return 0;
+}
+
+int vadb200_get_frontend(vadb200_handle* h, float* preemph, float* h_window, int* has_window) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (preemph) *preemph = h->preemph;
+  if (has_window) *has_window = h->has_window ? 1 : 0;
+  if (h_window) std::memcpy(h_window, h->window, sizeof(h->window));
+  return 0;
+}
+
+int vadb200_set_decision_threshold(vadb200_handle* h, float p_voiced) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (!(p_voiced < 1.0f)) return fail(VADB200_E_INVALID, "threshold must be < 1 (<= 0: argmax)");
+  const float th = p_voiced > 0.0f ? p_voiced : 0.0f;
+  h->par.thresh = th;
+  h->bias.thresh = th;
+  return 0;
+}
+
+float vadb200_get_decision_threshold(vadb200_handle* h) { return h ? h->par.thresh : NAN; }
 
 int vadb200_set_host_chunk_samples(vadb200_handle* h, int64_t samples) {
   if (!h || samples < 4096) return fail(VADB200_E_INVALID, "chunk must be >= 4096 samples");
@@ -396,7 +481,7 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
       s.pcm_start = offs[u] + kHop * o;
       s.out_start = p->row_off[u] + o;
       s.n_frames = static_cast<int>(std::min(seg_rows, r - o) + halo);
-      s.pad = 0;
+      s.cont = o > 0 ? 1 : 0;
       p->segs.push_back(s);
     }
   }
@@ -669,6 +754,7 @@ static int frames_common(vadb200_handle* h, const float* d_frames, int64_t n, in
                          void* stream) {
   if (!h) return fail(VADB200_E_INVALID, "handle is null");
   if (n < 0 || frame_len < 1 || frame_len > kFftN) return fail(VADB200_E_INVALID, "need 1 <= frame_len <= 512, n >= 0");
+  if (h->has_window && frame_len != kFrame) return fail(VADB200_E_INVALID, "a window needs frame_len == 400");
   if (n == 0) return 0;
   if (!d_frames || !d_out) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
@@ -678,7 +764,8 @@ static int frames_common(vadb200_handle* h, const float* d_frames, int64_t n, in
   rc = ensure_tables(h);
   if (rc) return rc;
   const unsigned grid = static_cast<unsigned>((n + kStepFrames - 1) / kStepFrames);
-  frames_kernel<<<grid, kThreads, kFramesSmemBytes, st>>>(d_frames, n, frame_len, what, d_out, h->d_tw, h->d_tw + 256);
+  const FrontEnd fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
+  frames_kernel<<<grid, kThreads, kFramesSmemBytes, st>>>(d_frames, n, frame_len, what, d_out, h->d_tw, h->d_tw + 256, fe);
   g_launches.fetch_add(1);
   CU(cudaGetLastError());
   return 0;
@@ -783,8 +870,9 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
   cudaError_t e = cudaMalloc(&b->d_hist, static_cast<size_t>(n_streams) * 320 * sizeof(int16_t));
   if (e == cudaSuccess) e = cudaMalloc(&b->d_ring, static_cast<size_t>(n_streams) * 5 * kNCep * sizeof(float));
   if (e == cudaSuccess) e = cudaMalloc(&b->d_fed, static_cast<size_t>(n_streams) * sizeof(int));
+  if (e == cudaSuccess) e = cudaMalloc(&b->d_prev, static_cast<size_t>(n_streams) * sizeof(int16_t));
   if (e != cudaSuccess) {
-    cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed);
+    cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev);
     delete b;
     return cuda_fail(e, "vadb200_stream_bank_create");
   }
@@ -798,7 +886,7 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
 int vadb200_stream_bank_destroy(vadb200_bank* b) {
   if (!b) return 0;
   cudaSetDevice(b->h->device);
-  cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed);
+  cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev);
   delete b;
   return 0;
 }
@@ -810,6 +898,7 @@ int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
   CU(cudaMemsetAsync(b->d_hist, 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
   CU(cudaMemsetAsync(b->d_ring, 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
   CU(cudaMemsetAsync(b->d_fed, 0, static_cast<size_t>(b->n) * sizeof(int), st));
+  CU(cudaMemsetAsync(b->d_prev, 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
   return 0;
 }
 
@@ -828,6 +917,8 @@ int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_lab
   bp.n_streams = b->n; bp.hist = b->d_hist; bp.ring = b->d_ring; bp.fed = b->d_fed;
   bp.chunks = d_chunks; bp.labels = d_labels; bp.logits = d_logits;
   bp.tw1 = h->d_tw; bp.tw2 = h->d_tw + 256; bp.feat_mode = VADB200_FEAT_ANALYSER;
+  bp.prev = b->d_prev;
+  bp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
   stream_feed_kernel<<<(b->n + kStepFrames - 1) / kStepFrames, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
   g_launches.fetch_add(1);
   CU(cudaGetLastError());

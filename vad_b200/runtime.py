@@ -116,6 +116,40 @@ class Handle(object):
     def ffn_impl(self):
         return int(self.lib.vadb200_get_ffn_impl(self._h))
 
+    # ---- opt-in front end and operating point ---------------------------------------------------
+    def set_frontend(self, preemph=0.0, window=None):
+        """Pre-emphasis y[n] = x[n] - preemph x[n-1] over each utterance (stream, or frame in the per-frame API), then
+        a 400-point window: an array of 400 weights or "hamming" (np.hamming(400)); None = rectangular.  The defaults
+        are the reference front end."""
+        if isinstance(window, str):
+            if window != "hamming":
+                raise ValueError("window must be an array of 400 weights, 'hamming' or None")
+            window = np.hamming(400)
+        win = None
+        if window is not None:
+            win = np.ascontiguousarray(np.asarray(window, dtype=np.float32))
+            if win.shape != (400,):
+                raise ValueError("window must have 400 weights, got shape %r" % (win.shape,))
+        check(self.lib.vadb200_set_frontend(self._h, float(preemph),
+                                            win.ctypes.data_as(C.c_void_p) if win is not None else C.c_void_p(0)))
+
+    def frontend(self):
+        """(preemph, window as float32[400] or None)."""
+        a = C.c_float()
+        has = C.c_int()
+        win = np.empty(400, dtype=np.float32)
+        check(self.lib.vadb200_get_frontend(self._h, C.byref(a), win.ctypes.data_as(C.c_void_p), C.byref(has)))
+        return float(a.value), (win if has.value else None)
+
+    def set_decision_threshold(self, p=None):
+        """speech <=> softmax(logits)[1] >= p; None (or p <= 0) restores argmax == VOICED."""
+        check(self.lib.vadb200_set_decision_threshold(self._h, 0.0 if p is None else float(p)))
+
+    def decision_threshold(self):
+        """The threshold on p(voiced), or None for the argmax rule."""
+        v = float(self.lib.vadb200_get_decision_threshold(self._h))
+        return v if v > 0.0 else None
+
     # ---- per-frame API --------------------------------------------------------------------
     def _frames_tensor(self, frames):
         t = torch.as_tensor(np.asarray(frames, dtype=np.float32) if not torch.is_tensor(frames) else frames)
