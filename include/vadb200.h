@@ -179,7 +179,10 @@ int vadb200_mfcc_from_spec(vadb200_handle* h, const float* d_spec /* [n][256] */
 int vadb200_vad_windows(vadb200_handle* h, const float* d_windows, int64_t n, int feat_mode,
                         uint8_t* d_labels /* nullable */, float* d_logits /* nullable [n][3] */,
                         float* d_feats /* nullable [n][39] */, void* stream);
-/* classifier.predict duck type (sklearn_analyser.py:71): rows [n][39] -> class in {0,1}. */
+/* classifier.predict duck type (sklearn_analyser.py:71): rows [n][39] -> class in {0,1}.  Caller rows have no
+ * MFCC-derived bound, so under impl 2 (fp16 operands) each 128-row tile is checked against the bounds its fp16 scales
+ * were chosen for (|c or z| <= 1353, |d1| <= 2706, |d2| <= 5416, per feature group); a tile holding any row beyond
+ * them runs on the tf32 operands of impl 1 instead, so any finite row gets finite logits within tolerance. */
 int vadb200_ffn_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t* d_labels,
                         float* d_logits /* nullable [n][3] */, void* stream);
 

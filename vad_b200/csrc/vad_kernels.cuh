@@ -646,13 +646,14 @@ __global__ void __launch_bounds__(kThreads, 2) fused_fe_kernel(const __grid_cons
 }
 
 // Stand-alone tensor-core FFN over feature rows [n][39] (classifier.predict duck type): one CTA =
-// one 128-row tile.  Same tile routine as the fused kernel's block phase.
+// one 128-row tile.  Same tile routines as the fused kernel's block phase.  The fp16 scales hold only for
+// features within the kFeatBound* of their group, which caller rows need not be: with KIND 2 a tile holding
+// any row beyond them runs on the tf32 blob instead (fp16 would overflow to inf and return NaN logits).
 constexpr int kFfnTcSmemBytes = kTcBlobBytes + 64;
-template <int KIND>  // 1: tf32 operands, 2: fp16 operands
-__global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long long n, const unsigned char* blob,
-                                                          uint8_t* labels, float* logits,
+template <int KIND>  // 1: tf32 operands, 2: fp16 operands where the tile's rows allow
+__global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long long n, const unsigned char* blob16,
+                                                          const unsigned char* blob32, uint8_t* labels, float* logits,
                                                           const __grid_constant__ FfnBias fb) {
-  constexpr uint32_t kBlob = KIND == 2 ? kTc16BlobBytes : kTcBlobBytes;
   extern __shared__ __align__(128) unsigned char smem[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kTcBlobBytes);
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + kTcBlobBytes + 32);
@@ -667,18 +668,29 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
   __syncthreads();
   tc_fence_after();
   const uint32_t tm_base = *s_tmem;
-  if (tid == 0) {
-    mbar_arrive_expect_tx(&bars[0], kBlob);
-    bulk_g2s(smem, blob, kBlob, &bars[0]);
+  if (KIND == 1 && tid == 0) {
+    mbar_arrive_expect_tx(&bars[0], kTcBlobBytes);
+    bulk_g2s(smem, blob32, kTcBlobBytes, &bars[0]);
   }
   const long long i = static_cast<long long>(blockIdx.x) * 128 + tid;
   const long long src = i < n ? i : n - 1;
   float v[kNFeat], logit[kNCls];
-  bool ok = true;
+  bool ok = true, wide = false;
 #pragma unroll
   for (int k = 0; k < kNFeat; ++k) {
     v[k] = x[src * kNFeat + k];
     ok = ok && (fabsf(v[k]) <= 3.0e38f);
+    if constexpr (KIND == 2)
+      wide = wide || fabsf(v[k]) > (k < kNCep ? kFeatBoundZ : k < 2 * kNCep ? kFeatBoundD1 : kFeatBoundD2);
+  }
+  bool fp16 = false;
+  if constexpr (KIND == 2) {
+    fp16 = !__syncthreads_or(wide);
+    if (tid == 0) {
+      const uint32_t bytes = fp16 ? kTc16BlobBytes : kTcBlobBytes;
+      mbar_arrive_expect_tx(&bars[0], bytes);
+      bulk_g2s(smem, fp16 ? blob16 : blob32, bytes, &bars[0]);
+    }
   }
   mbar_wait(&bars[0], 0);
   {
@@ -692,7 +704,7 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
       if (col < 24) h0[col] = v[f];
       else h1[col - 24] = v[f];
     }
-    if constexpr (KIND == 2) {
+    if (fp16) {
       tc16_store_a1_half(tl, 0, h0);
       tc16_store_a1_half(tl, 1, h1);
     } else {
@@ -700,7 +712,7 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
       tc_store_a1_half(tl, 1, h1);
     }
   }
-  if constexpr (KIND == 2) ffn_tc16_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
+  if (fp16) ffn_tc16_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
   else ffn_tc_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
   if (i < n) {
     uint8_t lab = decide(logit, fb.thresh);

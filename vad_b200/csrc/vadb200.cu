@@ -824,10 +824,10 @@ int vadb200_ffn_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t*
   if (rc) return rc;
   if (h->ffn_impl >= 2 && h->tc16_ok) {
     ffn_tc_rows_kernel<2><<<static_cast<unsigned>((n + 127) / 128), 128, kFfnTcSmemBytes, st>>>(
-        d_x, n, h->d_tc16_blob, d_labels, d_logits, h->bias);
+        d_x, n, h->d_tc16_blob, h->d_tc_blob, d_labels, d_logits, h->bias);
   } else if (h->ffn_impl >= 1) {
     ffn_tc_rows_kernel<1><<<static_cast<unsigned>((n + 127) / 128), 128, kFfnTcSmemBytes, st>>>(
-        d_x, n, h->d_tc_blob, d_labels, d_logits, h->bias);
+        d_x, n, nullptr, h->d_tc_blob, d_labels, d_logits, h->bias);
   } else {
     ffn_rows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_x, n, d_labels, d_logits, h->par);
   }
