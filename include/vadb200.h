@@ -150,6 +150,38 @@ int vadb200_set_host_chunk_samples(vadb200_handle* h, int64_t samples);
  * (dataset_creator.py:61-65) for a packed batch of decoded files. */
 int vadb200_mfcc_host(vadb200_plan* p, const int16_t* h_pcm, int64_t pcm_len, float* h_out);
 
+/* ---- speech segments (MODE_VAD / MODE_DATASET plans) -------------------------------------------
+ * Frame decisions -> smoothed labels -> speech segments -> speech-only PCM, on the device.  Per utterance, over
+ * its rows (nonzero label = speech), in this order: (1) a non-speech run with speech on both sides and shorter than
+ * min_silence_rows becomes speech; (2) a speech run shorter than min_speech_rows becomes non-speech (a run cut by
+ * the utterance edge counts with the length it has); (3) a row becomes speech when a speech row lies within
+ * pad_rows of it.  0 switches a step off (1 too for steps 1 and 2); each parameter in [0, 1000] rows.  Utterances
+ * never interact.  A segment is a maximal smoothed speech run [r0, r1) and covers the samples
+ * [160 r0 + 440, 160 r1 + 440) of its utterance (row r classifies frame r + 2 and owns its centre hop), so an
+ * utterance has at most ceil(R / 2) segments and 160 samples of speech per smoothed speech row.
+ * Both calls only enqueue work (no synchronisation, no allocation) and can be captured in CUDA graphs; scratch
+ * comes from the caller's workspace, one per stream when a plan runs on several streams at once. */
+int64_t vadb200_plan_max_speech_segments(const vadb200_plan* p);      /* sum over utterances of ceil(R_u / 2) */
+int64_t vadb200_plan_speech_workspace_bytes(const vadb200_plan* p);
+/* d_segments [max][2] int64: start, end samples within the utterance, utterance after utterance;
+ * d_segment_offsets [n_utt + 1]: utterance u owns segments [off[u], off[u + 1]); d_speech_offsets (nullable)
+ * [n_utt + 1]: utterance u's speech samples start at off[u] of the gathered output.  d_smoothed (nullable) [rows]
+ * receives the smoothed 0/1 labels.  Arrays 8-byte aligned, the workspace 16-byte aligned. */
+int vadb200_plan_speech_segments(vadb200_plan* p, const uint8_t* d_labels /* [rows] */,
+                                 int min_speech_rows, int min_silence_rows, int pad_rows,
+                                 uint8_t* d_smoothed /* nullable [rows] */,
+                                 int64_t* d_segments /* [max][2] start, end samples within the utterance */,
+                                 int64_t* d_segment_offsets /* [n_utt + 1] */,
+                                 int64_t* d_speech_offsets /* nullable [n_utt + 1], samples */,
+                                 void* d_workspace, int64_t workspace_bytes, void* stream);
+/* Speech audio: every utterance's segments concatenated in order, utterance after utterance, into d_out
+ * (16-byte aligned, like d_pcm); writes min(d_speech_offsets[n_utt], out_capacity) samples and nothing past
+ * out_capacity.  The three arrays are vadb200_plan_speech_segments' output for this plan. */
+int vadb200_plan_gather_speech(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len,
+                               const int64_t* d_segments, const int64_t* d_segment_offsets,
+                               const int64_t* d_speech_offsets, int16_t* d_out /* 16-byte aligned */,
+                               int64_t out_capacity, void* stream);
+
 /* ---- feature sink and ingest (the steps either side of the path in the offline flow) --------
  * dataset/utils.py:5-32 scale_features on packed dataset rows d_rows [n_rows][39], in place:
  * one scalar mean and one population std per group {mfcc, d1, d2} over all n_rows x 13 values,

@@ -47,6 +47,10 @@ SIGNATURES = {
     "vadb200_plan_segment_count": (_I64, [_P]),
     "vadb200_set_plan_segment_frames": (C.c_int, [_P, C.c_int]),
     "vadb200_mfcc_host": (C.c_int, [_P, _P, _I64, _P]),
+    "vadb200_plan_max_speech_segments": (_I64, [_P]),
+    "vadb200_plan_speech_workspace_bytes": (_I64, [_P]),
+    "vadb200_plan_speech_segments": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _I64, _P]),
+    "vadb200_plan_gather_speech": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _I64, _P]),
     "vadb200_scale_rows": (C.c_int, [_P, _P, _I64, _P, _P]),
     "vadb200_ingest_pcm": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_int, _I64, _P, _P]),
     "vadb200_mfcc_packed": (C.c_int, [_P, _P, _I64, _P, _P]),

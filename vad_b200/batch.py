@@ -71,6 +71,36 @@ def vad_batch(utterances, handle=None, want_logits=False, feat_mode=FEAT_ANALYSE
     return lab
 
 
+def _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode):
+    handle = handle or runtime.default_handle()
+    if not handle.has_ffn:
+        raise RuntimeError("set FFN weights first (Handle.set_ffn_weights)")
+    for v in (min_speech_ms, min_silence_ms, pad_ms):
+        runtime.speech_ms_to_rows(v)               # argument errors before any device work
+    flat, offsets, lengths = pack_utterances(utterances)
+    plan = runtime.Plan(handle, offsets, lengths, MODE_VAD)
+    pcm = flat.to(handle.device)
+    labels, _, _ = plan.vad(pcm, feat_mode=feat_mode)
+    segs, seg_off, sp_off, _ = plan.speech_segments(labels, min_speech_ms, min_silence_ms, pad_ms)
+    return plan, pcm, segs, seg_off, sp_off
+
+
+def speech_segments(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER):
+    """Speech segments of every utterance: a list of int64 [k, 2] arrays of [start, end) samples within the
+    utterance.  One upload, the fused VAD, the segment kernels and one download; the handle's front end and
+    decision threshold apply.  See Plan.speech_segments for the smoothing parameters."""
+    _, _, segs, seg_off, _ = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode)
+    s = segs.cpu().numpy()
+    return [s[seg_off[u]:seg_off[u + 1]] for u in range(len(seg_off) - 1)]
+
+
+def extract_speech(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER):
+    """Speech-only audio of every utterance (its segments concatenated): a list of int16 arrays."""
+    plan, pcm, segs, seg_off, sp_off = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode)
+    out = plan.gather_speech(pcm, segs, seg_off, sp_off).cpu().numpy()
+    return [out[sp_off[u]:sp_off[u + 1]] for u in range(len(sp_off) - 1)]
+
+
 # ---- drop-ins for dataset/file_processing.py ---------------------------------------------------
 def parse_transcription(path, frame_rate):
     """dataset/file_processing.py:106-107 -> dataset/stm_parser.py:5-26."""

@@ -20,6 +20,7 @@
 #include "vad_host_tables.h"
 #include "vad_kernels.cuh"
 #include "ffn_train.cuh"
+#include "vad_segments.cuh"
 
 using namespace vadb;
 
@@ -99,6 +100,14 @@ struct vadb200_plan {
   std::atomic<unsigned> launch_seq{0};
   long long total_rows = 0;
   long long seg_frames = 0;
+  // speech segments (MODE_VAD / MODE_DATASET): tiles of <= kSpeechTile rows of one utterance
+  std::vector<SpeechTile> tiles;
+  std::vector<int> utt_tile;          // n_utt + 1: first tile of each utterance
+  long long max_speech_segs = 0;      // sum over utterances of ceil(R_u / 2)
+  long long* d_row_off = nullptr;     // n_utt + 1 row offsets
+  long long* d_pcm_off = nullptr;     // n_utt sample offsets
+  SpeechTile* d_tiles = nullptr;
+  int* d_utt_tile = nullptr;
 };
 
 struct vadb200_trainer {
@@ -498,8 +507,37 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
     if (e == cudaSuccess)
       e = cudaMemcpy(p->d_segs, p->segs.data(), p->segs.size() * sizeof(Segment), cudaMemcpyHostToDevice);
   }
+  if (mode != VADB200_MODE_MFCC) {
+    p->utt_tile.resize(n_utt + 1);
+    for (long long u = 0; u < n_utt; ++u) {
+      p->utt_tile[u] = static_cast<int>(p->tiles.size());
+      const long long r = p->row_off[u + 1] - p->row_off[u];
+      p->max_speech_segs += (r + 1) / 2;
+      for (long long o = 0; o < r; o += kSpeechTile)
+        p->tiles.push_back(SpeechTile{p->row_off[u] + o, static_cast<int>(std::min<long long>(kSpeechTile, r - o)),
+                                      static_cast<int>(u)});
+    }
+    p->utt_tile[n_utt] = static_cast<int>(p->tiles.size());
+    if (e == cudaSuccess) e = cudaMalloc(&p->d_row_off, (n_utt + 1) * sizeof(long long));
+    if (e == cudaSuccess)
+      e = cudaMemcpy(p->d_row_off, p->row_off.data(), (n_utt + 1) * sizeof(long long), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMalloc(&p->d_utt_tile, (n_utt + 1) * sizeof(int));
+    if (e == cudaSuccess)
+      e = cudaMemcpy(p->d_utt_tile, p->utt_tile.data(), (n_utt + 1) * sizeof(int), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && n_utt > 0) {
+      e = cudaMalloc(&p->d_pcm_off, n_utt * sizeof(long long));
+      if (e == cudaSuccess)
+        e = cudaMemcpy(p->d_pcm_off, p->offsets.data(), n_utt * sizeof(long long), cudaMemcpyHostToDevice);
+    }
+    if (e == cudaSuccess && !p->tiles.empty()) {
+      e = cudaMalloc(&p->d_tiles, p->tiles.size() * sizeof(SpeechTile));
+      if (e == cudaSuccess)
+        e = cudaMemcpy(p->d_tiles, p->tiles.data(), p->tiles.size() * sizeof(SpeechTile), cudaMemcpyHostToDevice);
+    }
+  }
   if (e != cudaSuccess) {
     cudaFree(p->d_counter); cudaFree(p->d_segs);
+    cudaFree(p->d_row_off); cudaFree(p->d_pcm_off); cudaFree(p->d_tiles); cudaFree(p->d_utt_tile);
     delete p;
     return cuda_fail(e, "vadb200_plan_create");
   }
@@ -512,6 +550,10 @@ int vadb200_plan_destroy(vadb200_plan* p) {
   cudaSetDevice(p->h->device);
   cudaFree(p->d_segs);
   cudaFree(p->d_counter);
+  cudaFree(p->d_row_off);
+  cudaFree(p->d_pcm_off);
+  cudaFree(p->d_tiles);
+  cudaFree(p->d_utt_tile);
   delete p;
   return 0;
 }
@@ -1079,6 +1121,103 @@ int vadb200_fp32_peak(vadb200_handle* h, int variant, int iters, double* tflops_
   cudaEventDestroy(e0);
   cudaEventDestroy(e1);
   *tflops_out = best;
+  return 0;
+}
+
+// ---- speech segments (vad_segments.cuh) -----------------------------------------------------------------
+namespace {
+constexpr long long kWsAlign = 256;
+long long ws_round(long long b) { return (b + kWsAlign - 1) / kWsAlign * kWsAlign; }
+// workspace: tile counts int2[n_tiles] | tile prefixes longlong2[n_tiles + 1] | smoothed rows (when not asked)
+struct SpeechWs {
+  long long counts, prefix, smoothed, total;
+};
+SpeechWs speech_ws(const vadb200_plan* p) {
+  SpeechWs w;
+  const long long nt = static_cast<long long>(p->tiles.size());
+  w.counts = 0;
+  w.prefix = ws_round(nt * static_cast<long long>(sizeof(int2)));
+  w.smoothed = w.prefix + ws_round((nt + 1) * static_cast<long long>(sizeof(longlong2)));
+  w.total = w.smoothed + ws_round(p->total_rows);
+  return w;
+}
+bool misaligned(const void* ptr, uintptr_t a) { return (reinterpret_cast<uintptr_t>(ptr) & (a - 1)) != 0; }
+}  // namespace
+
+int64_t vadb200_plan_max_speech_segments(const vadb200_plan* p) {
+  if (!p || p->mode == VADB200_MODE_MFCC) return -1;
+  return p->max_speech_segs;
+}
+
+int64_t vadb200_plan_speech_workspace_bytes(const vadb200_plan* p) {
+  if (!p || p->mode == VADB200_MODE_MFCC) return -1;
+  return speech_ws(p).total;
+}
+
+int vadb200_plan_speech_segments(vadb200_plan* p, const uint8_t* d_labels, int min_speech_rows, int min_silence_rows,
+                                 int pad_rows, uint8_t* d_smoothed, int64_t* d_segments, int64_t* d_segment_offsets,
+                                 int64_t* d_speech_offsets, void* d_workspace, int64_t workspace_bytes, void* stream) {
+  if (!p) return fail(VADB200_E_INVALID, "plan is null");
+  if (p->mode == VADB200_MODE_MFCC) return fail(VADB200_E_INVALID, "speech segments need a MODE_VAD or MODE_DATASET plan");
+  for (int v : {min_speech_rows, min_silence_rows, pad_rows})
+    if (v < 0 || v > kSpeechMaxParam) return fail(VADB200_E_INVALID, "row parameters must lie in [0, 1000]");
+  const SpeechWs ws = speech_ws(p);
+  if (!d_workspace || workspace_bytes < ws.total) return fail(VADB200_E_INVALID, "workspace is null or too small");
+  if (misaligned(d_workspace, 16)) return fail(VADB200_E_INVALID, "workspace must be 16-byte aligned");
+  if (!d_segment_offsets) return fail(VADB200_E_INVALID, "d_segment_offsets is null");
+  if (p->total_rows > 0 && (!d_labels || !d_segments)) return fail(VADB200_E_INVALID, "d_labels / d_segments is null");
+  if (misaligned(d_segments, 8) || misaligned(d_segment_offsets, 8) || misaligned(d_speech_offsets, 8))
+    return fail(VADB200_E_INVALID, "segment and offset arrays must be 8-byte aligned");
+  CU(cudaSetDevice(p->h->device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  unsigned char* wsb = static_cast<unsigned char*>(d_workspace);
+  int2* counts = reinterpret_cast<int2*>(wsb + ws.counts);
+  longlong2* prefix = reinterpret_cast<longlong2*>(wsb + ws.prefix);
+  uint8_t* sm = d_smoothed ? d_smoothed : wsb + ws.smoothed;
+  const int n_tiles = static_cast<int>(p->tiles.size());
+  const SmoothParams sp = smooth_params(min_speech_rows, min_silence_rows, pad_rows);
+  if (n_tiles > 0) {
+    speech_smooth_kernel<<<n_tiles, kSpeechThreads, smooth_smem_bytes(sp.H), st>>>(d_labels, p->d_tiles, p->d_row_off,
+                                                                                 sp, sm, counts);
+    g_launches.fetch_add(1);
+  }
+  speech_scan_kernel<<<1, kSpeechScanThreads, 0, st>>>(counts, n_tiles, prefix);
+  g_launches.fetch_add(1);
+  const long long utt_blocks = (p->n_utt + 1 + kSpeechThreads - 1) / kSpeechThreads;
+  const unsigned grid = static_cast<unsigned>(std::max<long long>(n_tiles, utt_blocks));
+  speech_segments_kernel<<<grid, kSpeechThreads, 0, st>>>(
+      sm, p->d_tiles, p->d_row_off, prefix, n_tiles, p->d_utt_tile, p->n_utt, reinterpret_cast<long long*>(d_segments),
+      reinterpret_cast<long long*>(d_segment_offsets), reinterpret_cast<long long*>(d_speech_offsets));
+  g_launches.fetch_add(1);
+  CU(cudaGetLastError());
+  return 0;
+}
+
+int vadb200_plan_gather_speech(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len, const int64_t* d_segments,
+                               const int64_t* d_segment_offsets, const int64_t* d_speech_offsets, int16_t* d_out,
+                               int64_t out_capacity, void* stream) {
+  if (!p) return fail(VADB200_E_INVALID, "plan is null");
+  if (p->mode == VADB200_MODE_MFCC) return fail(VADB200_E_INVALID, "speech segments need a MODE_VAD or MODE_DATASET plan");
+  int rc = check_pcm(p, d_pcm, pcm_len);
+  if (rc) return rc;
+  if (out_capacity < 0) return fail(VADB200_E_INVALID, "out_capacity < 0");
+  if (!d_segment_offsets || !d_speech_offsets) return fail(VADB200_E_INVALID, "offset arrays are null");
+  if (p->total_rows > 0 && !d_segments) return fail(VADB200_E_INVALID, "d_segments is null");
+  if (out_capacity > 0 && !d_out) return fail(VADB200_E_INVALID, "d_out is null");
+  if (misaligned(d_out, 16)) return fail(VADB200_E_INVALID, "d_out must be 16-byte aligned");
+  if (misaligned(d_segments, 8) || misaligned(d_segment_offsets, 8) || misaligned(d_speech_offsets, 8))
+    return fail(VADB200_E_INVALID, "segment and offset arrays must be 8-byte aligned");
+  if (p->total_rows == 0 || out_capacity == 0) return 0;
+  CU(cudaSetDevice(p->h->device));
+  // output hops are split evenly over a grid sized to keep HBM busy; CTAs past the speech exit at once
+  const long long max_hops = p->total_rows;
+  const unsigned grid = static_cast<unsigned>(std::max<long long>(1, std::min<long long>(8ll * p->h->num_sms, max_hops)));
+  speech_gather_kernel<<<grid, kSpeechThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      d_pcm, p->d_pcm_off, p->n_utt, reinterpret_cast<const long long*>(d_segments),
+      reinterpret_cast<const long long*>(d_segment_offsets), reinterpret_cast<const long long*>(d_speech_offsets), d_out,
+      out_capacity);
+  g_launches.fetch_add(1);
+  CU(cudaGetLastError());
   return 0;
 }
 

@@ -323,6 +323,65 @@ class Plan(object):
         return labels_host, logits_host
 
 
+    # ---- speech segments (vad_segments.cuh) ------------------------------------------------------
+    def speech_segments(self, labels, min_speech_ms=0, min_silence_ms=0, pad_ms=0, want_smoothed=False):
+        """Labels [rows] (uint8 CUDA tensor, nonzero = speech) of a MODE_VAD / MODE_DATASET plan -> smoothed labels and
+        speech segments.  In order, per utterance: silences shorter than ``min_silence_ms`` between speech are
+        filled, speech runs shorter than ``min_speech_ms`` dropped, and the rest padded by ``pad_ms`` on both sides
+        (each ceil(ms / 10) rows, at most 1000; 0 = off).  Returns (segments int64 [k, 2] CUDA tensor of
+        [start, end) samples within each utterance, segment_offsets and speech_offsets as host int64 [n_utt + 1],
+        smoothed uint8 [rows] CUDA tensor or None).  Synchronises once to read the segment count."""
+        if not (torch.is_tensor(labels) and labels.is_cuda and labels.dtype == torch.uint8 and labels.is_contiguous()
+                and labels.dim() == 1 and labels.numel() == self.total_rows):
+            raise TypeError("labels must be a contiguous uint8 CUDA tensor of the plan's %d rows" % self.total_rows)
+        rows = [speech_ms_to_rows(v) for v in (min_speech_ms, min_silence_ms, pad_ms)]
+        dev = labels.device
+        ws_bytes = int(self.lib.vadb200_plan_speech_workspace_bytes(self._p))
+        if ws_bytes < 0:
+            raise ValueError("speech segments need a MODE_VAD or MODE_DATASET plan")
+        ws = getattr(self, "_speech_ws", None)
+        if ws is None or ws.numel() < ws_bytes or ws.device != dev:
+            ws = self._speech_ws = torch.empty((max(ws_bytes, 16),), dtype=torch.uint8, device=dev)
+        max_segs = int(self.lib.vadb200_plan_max_speech_segments(self._p))
+        segs = torch.empty((max(max_segs, 1), 2), dtype=torch.int64, device=dev)
+        offs = torch.empty((2, self.n_utt + 1), dtype=torch.int64, device=dev)
+        smoothed = torch.empty((self.total_rows,), dtype=torch.uint8, device=dev) if want_smoothed else None
+        check(self.lib.vadb200_plan_speech_segments(self._p, _ptr(labels), rows[0], rows[1], rows[2], _ptr(smoothed),
+                                                    _ptr(segs), _ptr(offs[0]), _ptr(offs[1]), _ptr(ws), ws_bytes,
+                                                    self.handle.stream))
+        offs_h = offs.cpu().numpy()
+        return segs[:int(offs_h[0, -1])], offs_h[0].copy(), offs_h[1].copy(), smoothed
+
+    def gather_speech(self, pcm, segments, segment_offsets, speech_offsets, out=None):
+        """Speech audio of every utterance, concatenated in order: an int16 CUDA tensor whose utterance u part is
+        out[speech_offsets[u]:speech_offsets[u + 1]].  The arguments after pcm are speech_segments' output."""
+        self._check_pcm(pcm)
+        dev = pcm.device
+        so = torch.as_tensor(np.asarray(segment_offsets, dtype=np.int64)).to(dev)
+        sp_h = np.asarray(speech_offsets, dtype=np.int64)
+        sp = torch.as_tensor(sp_h).to(dev)
+        if so.numel() != self.n_utt + 1 or sp.numel() != self.n_utt + 1:
+            raise ValueError("offsets must have n_utt + 1 entries")
+        segs = segments if segments.numel() else torch.zeros((1, 2), dtype=torch.int64, device=dev)
+        total = int(sp_h[-1])
+        if out is None:
+            out = torch.empty((total,), dtype=torch.int16, device=dev)
+        check(self.lib.vadb200_plan_gather_speech(self._p, _ptr(pcm), pcm.numel(), _ptr(segs.contiguous()), _ptr(so),
+                                                  _ptr(sp), _ptr(out), out.numel(), self.handle.stream))
+        return out
+
+
+def speech_ms_to_rows(ms):
+    """Duration in ms -> 10 ms rows for the segment parameters: ceil(ms / 10), which must lie in [0, 1000]."""
+    ms = float(ms)
+    if not ms >= 0.0:
+        raise ValueError("durations must be >= 0 ms")
+    rows = int(np.ceil(ms / 10.0))
+    if rows > 1000:
+        raise ValueError("durations must be at most 10000 ms (1000 rows)")
+    return rows
+
+
 class StreamBankHandle(object):
     def __init__(self, handle, n_streams):
         self.handle = handle
