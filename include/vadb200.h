@@ -237,6 +237,37 @@ int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks /* [n][160], de
                         uint8_t* d_labels /* [n], device-visible */, float* d_logits /* nullable */,
                         void* stream);
 
+/* Speech segments for the bank (the offline smoothing of vadb200_plan_speech_segments, online).  Each stream counts
+ * rows from its last reset or end: a feed whose label is not 255 adds row r (chunk r + 7).  With speech on, the feed
+ * of chunk r + 7 + D finalises smoothed row r, D = (G > 1 ? G - 1 : 0) + (S > 1 ? S - 1 : 0) + P rows for
+ * G = min_silence_rows, S = min_speech_rows, P = pad_rows: rows[i] is its label (0 / 1, or 255 when no row is
+ * final this tick) and bounds[i] is 160 r + 440 when row r opens a segment (speech, after non-speech or at r = 0) or
+ * closes one (non-speech after speech), else -1; samples count from the stream's last reset or end.  The rows a
+ * stream finalises, with the tail of its end, are exactly the offline smoothing of its non-255 labels.
+ * All streams share (S, G, P), each in [0, 1000].  set_speech allocates the segment state for these parameters
+ * and resets every stream of the bank; enable = 0 frees it and restores the plain bank (also resetting it).  While
+ * speech is on, vadb200_stream_feed advances the segment state too (its rows are discarded) and
+ * vadb200_stream_bank_reset clears it.  Feeds and ends allocate nothing, never synchronise and can be captured in a
+ * CUDA graph; a graph captured before set_speech holds the previous segment state and must be captured again. */
+int vadb200_stream_bank_set_speech(vadb200_bank* b, int enable, int min_speech_rows, int min_silence_rows,
+                                   int pad_rows, void* stream);
+int vadb200_stream_bank_speech_delay(const vadb200_bank* b);   /* D rows, or -1 when speech is off */
+/* vadb200_stream_feed plus the segment step; VADB200_E_STATE when speech is off */
+int vadb200_stream_feed_speech(vadb200_bank* b, const int16_t* d_chunks /* [n][160], device-visible */,
+                               uint8_t* d_labels /* [n], device-visible */, float* d_logits /* nullable */,
+                               uint8_t* d_rows /* nullable [n] */, int64_t* d_bounds /* nullable [n] */,
+                               void* stream);
+/* Streams with d_end[i] != 0 end and start again; the others are untouched.  With speech on, an ended stream's
+ * pending rows (at most D) are resolved as if its utterance stopped at its last row R - 1 (a trailing silence is
+ * never filled, a trailing speech run counts with the length it has, the pad is clipped): d_tail_rows[i] gets those
+ * rows then 255, d_tail_bounds[i] their bounds, then the close of a segment still open (160 R + 440) or -1, then
+ * -1.  Rows of streams that do not end are not written.  Then the stream's history, MFCC ring, fed count,
+ * front-end previous sample and segment state are zero: its next chunk starts a new signal (255 labels for 7
+ * chunks).  With speech off this is a per-stream reset and the tails are not written. */
+int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end /* [n], device-visible */,
+                                    uint8_t* d_tail_rows /* nullable [n][D] */,
+                                    int64_t* d_tail_bounds /* nullable [n][D + 1] */, void* stream);
+
 /* ---- FFN training (learning/ffn_trainer.py:104-175) ---------------------------------------
  * model.compile(loss='categorical_crossentropy', optimizer='adadelta') + model.train_on_batch for the
  * 39-64-32-16-3 network: forward, backward and the Adadelta update as two hand-written kernels per step,

@@ -139,7 +139,13 @@ class StreamBank(object):
     through pinned host buffers.  A tick is captured once into a CUDA graph and replayed: one graph
     launch per tick.  With ``zero_copy`` (default) the graph is the feed kernel alone: it reads the
     chunks from, and writes the labels to, the pinned host buffers directly over PCIe (each chunk
-    sample is read once), which removes the two copy nodes and their scheduling gaps from the tick."""
+    sample is read once), which removes the two copy nodes and their scheduling gaps from the tick.
+
+    Speech segments (``set_speech``): every stream also runs the offline smoothing of ``Plan.speech_segments``
+    online.  A stream's row r is its label from chunk r + 7 (since its last reset or end); ``feed_speech`` returns
+    for each stream the smoothed row finalised this tick, r - D (255: none), and a segment bound: 160 (r - D) + 440
+    samples when that row opens or closes a segment, else -1.  ``end_streams`` resolves the last D rows of the
+    streams it ends and starts them again, leaving the others untouched."""
 
     NOT_READY = 255
 
@@ -160,37 +166,53 @@ class StreamBank(object):
         self.use_graph = bool(use_graph)
         self.zero_copy = bool(zero_copy)
         self._graphs = {}
+        self.delay = -1          # speech delay D in rows; -1: speech off
+        self.h_rows = self.h_bounds = self.d_rows = self.d_bounds = None
+        self.d_tail_rows = self.d_tail_bounds = None
 
     def reset(self):
         self.bank.reset()
         torch.cuda.synchronize(self.handle.device)
 
-    def _enqueue(self, want_logits):
+    def _enqueue(self, want_logits, speech=False):
         if self.zero_copy:   # pinned host memory is device-visible under UVA: no copy nodes
-            self.bank.feed_ptr(self.h_chunks.data_ptr(), self.h_labels.data_ptr(),
-                               self.h_logits.data_ptr() if want_logits else 0)
+            if speech:
+                self.bank.feed_speech_ptr(self.h_chunks.data_ptr(), self.h_labels.data_ptr(),
+                                          self.h_logits.data_ptr() if want_logits else 0, self.h_rows.data_ptr(),
+                                          self.h_bounds.data_ptr())
+            else:
+                self.bank.feed_ptr(self.h_chunks.data_ptr(), self.h_labels.data_ptr(),
+                                   self.h_logits.data_ptr() if want_logits else 0)
             return
         self.d_chunks.copy_(self.h_chunks, non_blocking=True)
-        self.bank.feed_ptr(self.d_chunks.data_ptr(), self.d_labels.data_ptr(),
-                           self.d_logits.data_ptr() if want_logits else 0)
+        if speech:
+            self.bank.feed_speech_ptr(self.d_chunks.data_ptr(), self.d_labels.data_ptr(),
+                                      self.d_logits.data_ptr() if want_logits else 0, self.d_rows.data_ptr(),
+                                      self.d_bounds.data_ptr())
+            self.h_rows.copy_(self.d_rows, non_blocking=True)
+            self.h_bounds.copy_(self.d_bounds, non_blocking=True)
+        else:
+            self.bank.feed_ptr(self.d_chunks.data_ptr(), self.d_labels.data_ptr(),
+                               self.d_logits.data_ptr() if want_logits else 0)
         self.h_labels.copy_(self.d_labels, non_blocking=True)
         if want_logits:
             self.h_logits.copy_(self.d_logits, non_blocking=True)
 
-    def _tick(self, want_logits):
+    def _tick(self, want_logits, speech=False):
         """One H2D + kernel + D2H; returns after the labels are on the host."""
         if self.use_graph:
-            g = self._graphs.get(want_logits)
+            key = (want_logits, speech)
+            g = self._graphs.get(key)
             if g is None:  # capture once (capturing does not execute: no chunk is consumed)
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g, stream=self.stream):
-                    self._enqueue(want_logits)
-                self._graphs[want_logits] = g
+                    self._enqueue(want_logits, speech)
+                self._graphs[key] = g
             g.replay()                                   # one cudaGraphLaunch on the caller's current stream
             torch.cuda.current_stream(self.handle.device).synchronize()
         else:
             with torch.cuda.stream(self.stream):
-                self._enqueue(want_logits)
+                self._enqueue(want_logits, speech)
             self.stream.synchronize()
 
     def feed(self, chunks, want_logits=False):
@@ -209,3 +231,71 @@ class StreamBank(object):
         launch (H2D + kernel + D2H) is issued and awaited.  Returns a view of ``self.h_labels``."""
         self._tick(False)
         return self.h_labels
+
+    # ---- speech segments ----------------------------------------------------------------------------------------
+    def set_speech(self, min_speech_ms=0, min_silence_ms=0, pad_ms=0):
+        """Turn speech segments on for every stream, with Plan.speech_segments' parameters and ms -> rows rule
+        (each ceil(ms / 10) rows, at most 1000).  Resets the bank; returns the delay D in rows."""
+        rows = [runtime.speech_ms_to_rows(v) for v in (min_speech_ms, min_silence_ms, pad_ms)]
+        dev = self.handle.device
+        self._graphs = {}   # captured ticks hold the previous segment state
+        d = self.bank.set_speech(*rows)
+        if self.h_rows is None:
+            self.h_rows = torch.zeros((self.n,), dtype=torch.uint8).pin_memory()
+            self.h_bounds = torch.zeros((self.n,), dtype=torch.int64).pin_memory()
+            self.d_rows = torch.zeros((self.n,), dtype=torch.uint8, device=dev)
+            self.d_bounds = torch.zeros((self.n,), dtype=torch.int64, device=dev)
+        self.d_tail_rows = torch.empty((self.n, d), dtype=torch.uint8, device=dev)
+        self.d_tail_bounds = torch.empty((self.n, d + 1), dtype=torch.int64, device=dev)
+        torch.cuda.synchronize(dev)
+        self.delay = d
+        return d
+
+    def disable_speech(self):
+        """Back to the plain bank (resets it)."""
+        self._graphs = {}
+        self.bank.disable_speech()
+        torch.cuda.synchronize(self.handle.device)
+        self.delay = -1
+        self.d_tail_rows = self.d_tail_bounds = None
+
+    def feed_speech(self, chunks):
+        """feed() plus the segment step: returns (labels uint8 [n], rows uint8 [n], bounds int64 [n]); see the
+        class notes.  Needs set_speech."""
+        if self.delay < 0:
+            raise RuntimeError("speech is off: call set_speech first")
+        src = torch.as_tensor(np.asarray(chunks, dtype=np.int16) if not torch.is_tensor(chunks) else chunks)
+        if tuple(src.shape) != (self.n, 160):
+            raise ValueError("chunks must have shape (%d, 160)" % self.n)
+        self.h_chunks.copy_(src)
+        self._tick(False, speech=True)
+        return self.h_labels.numpy().copy(), self.h_rows.numpy().copy(), self.h_bounds.numpy().copy()
+
+    def end_streams(self, ids):
+        """End the streams ``ids`` and start them again (their next chunk begins a new signal).  With speech on,
+        returns for each id (tail_rows uint8 [k], tail_bounds int64 [k + 1]): its k <= D pending smoothed rows, their
+        bounds, then the close of a segment still open (160 R + 440 after R rows) or -1.  With speech off the streams
+        are reset and each tail is empty."""
+        ids = [int(i) for i in np.asarray(ids, dtype=np.int64).reshape(-1)]
+        if any(i < 0 or i >= self.n for i in ids):
+            raise ValueError("stream ids must lie in [0, %d)" % self.n)
+        dev = self.handle.device
+        end = np.zeros(self.n, np.uint8)
+        end[ids] = 1
+        speech = self.delay >= 0
+        with torch.cuda.stream(self.stream):
+            d_end = torch.as_tensor(end).to(dev, non_blocking=False)
+            self.bank.end_streams_ptr(d_end.data_ptr(), self.d_tail_rows.data_ptr() if speech else 0,
+                                      self.d_tail_bounds.data_ptr() if speech else 0, stream=self.stream.cuda_stream)
+            if speech:
+                sel = torch.as_tensor(np.asarray(ids, np.int64)).to(dev)
+                rows = self.d_tail_rows.index_select(0, sel).cpu().numpy()
+                bounds = self.d_tail_bounds.index_select(0, sel).cpu().numpy()
+        self.stream.synchronize()
+        if not speech:
+            return [(np.zeros(0, np.uint8), np.zeros(0, np.int64)) for _ in ids]
+        out = []
+        for r, b in zip(rows, bounds):
+            k = int(np.count_nonzero(r != 255))
+            out.append((r[:k].copy(), b[:k + 1].copy()))
+        return out

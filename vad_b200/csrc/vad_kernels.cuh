@@ -958,7 +958,12 @@ constexpr int kStreamSmemBytes = kStreamRowsOff + kStepFrames * kStreamFramePitc
 // tail is spread over all 8 warps with lane = stream: warp w owns cepstral coefficients w, w + 8
 // (DCT, ring push, window features) and then 8 / 4 / 2 neurons of layers 1 / 2 / 3, activations
 // handed over through shared memory (the idle P tile); weights are uniform constant-bank operands.
-__global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams p, const __grid_constant__ FfnParams w) {
+// SEG: the speech variant (stream_feed_speech_kernel) also runs each stream's online smoothing step
+// (vad_segments.cuh seg_step, found when the variant is instantiated with Seg = StreamSeg) on the label warp 0
+// holds, and writes the finalised row and its bound.
+template <bool SEG, class Seg>
+__device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnParams& w, const Seg& sg,
+                                                 const int tid) {
   extern __shared__ __align__(128) unsigned char smem[];
   int16_t* s_fr = reinterpret_cast<int16_t*>(smem + kStreamRowsOff);
   cf2* s_exch = reinterpret_cast<cf2*>(smem + kStreamRowsOff + kStepFrames * kStreamFramePitch * 2);
@@ -972,7 +977,7 @@ __global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams 
   float* s_h2 = s_h1 + kH1 * 32;       // [32][32]
   float* s_h3 = s_h2 + kH2 * 32;       // [16][32]
   int* s_ok = reinterpret_cast<int*>(s_h3 + kH3 * 32);  // [13][32]
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, h = lane >> 4;
+  const int warp = tid >> 5, lane = tid & 31, h = lane >> 4;
   const int s0 = blockIdx.x * kStepFrames;
   s_tw1[tid] = p.tw1[tid];
   if (tid < 128) s_tw2[tid] = p.tw2[tid];
@@ -1134,8 +1139,26 @@ __global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams 
         p.logits[stl * 3 + 1] = lg[1];
         p.logits[stl * 3 + 2] = lg[2];
       }
+      if constexpr (SEG) {  // row fedl - 7 of the stream is this label
+        uint8_t row = 255;
+        long long bound = -1;
+        if (lab != 255) seg_step(sg, stl, fedl - 7, lab != 0, row, bound);
+        if (sg.rows) sg.rows[stl] = row;
+        if (sg.bounds) sg.bounds[stl] = bound;
+      }
     }
   }
+}
+
+__global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams p, const __grid_constant__ FfnParams w) {
+  stream_feed_body<false>(p, w, 0, threadIdx.x);
+}
+// The same tick plus the bank's segment step (vadb200_stream_bank_set_speech); the plain kernel above keeps its code.
+template <class Seg>
+__global__ void __launch_bounds__(kThreads) stream_feed_speech_kernel(const BankParams p,
+                                                                     const __grid_constant__ FfnParams w,
+                                                                     const __grid_constant__ Seg sg) {
+  stream_feed_body<true>(p, w, sg, threadIdx.x);
 }
 
 // ---- feature sink: scale_features (dataset/utils.py:5-32) on packed dataset rows [n][39] ----------------

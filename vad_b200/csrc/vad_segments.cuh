@@ -186,6 +186,203 @@ VADB_SEG_HD bool seg_starts(const uint8_t* s, int o0, int i) { return s[i] && (i
 // Samples of a segment [r0, r1) within its utterance.
 VADB_SEG_HD long long seg_sample(long long r) { return kSpeechHopSamples * r + kSpeechFirstSample; }
 
+// ---- online smoothing for the stream bank -------------------------------------------------------------------
+// The same three steps as a causal cascade, one row in per tick.  Step 1 (gap fill) holds its last d1 = G - 1 rows
+// (G > 1, else it passes rows through) in a bit ring, the length of the trailing non-speech run and whether speech
+// was seen; when speech ends a non-speech run shorter than G that has speech before it, it sets the run's bits.
+// Step 2 (short runs) holds d2 = S - 1 rows and the trailing speech run; when a run shorter than S ends it clears
+// the run's bits.  Step 3 (pad) needs no ring: its row q is speech iff its last speech input lies at or after q - P.
+// Each step emits its oldest row once its ring is full, so after the first H = d1 + d2 + P rows the cascade emits
+// exactly one row per row fed: row r is final when row r + H arrives.  At the end of a stream the steps drain in
+// order with the offline edge rules: a trailing silence is never filled, a trailing speech run is judged with the
+// length it has, and the pad is clipped.
+//
+// State, struct-of-arrays over streams (word k of stream s at [k * n + s]): ring1 [W1][n], ring2 [W2][n] with
+// W = ceil(d / 32), meta [n] and last [n]; all zero is a fresh stream.  A ring slot of input row t is t mod d.
+constexpr uint32_t kSegRunMask = 0x7ffu;  // run lengths are clamped to <= 1000 < 2^11
+constexpr int kSegSeenBit = 11;           // step 1 has seen speech
+constexpr int kSegRun2Shift = 12;         // step 2's trailing speech run
+constexpr int kSegOutBit = 23;            // the last emitted row (a segment is open)
+constexpr int kSegEndThreads = 128;       // streams per CTA of stream_end_kernel
+
+struct StreamSeg {
+  uint32_t* ring1;
+  uint32_t* ring2;
+  uint32_t* meta;  // step 1's trailing non-speech run | seen | step 2's trailing speech run | last emitted row
+  int* last;       // step 3's last speech input + 1 (0: none)
+  long long n;     // streams (the SoA stride)
+  int G, S, P, d1, d2, H;
+  uint8_t* rows;    // [n] finalised row per feed, nullable
+  int64_t* bounds;  // [n] its segment bound, nullable
+};
+
+VADB_SEG_HD int seg_ring_words(int d) { return (d + 31) >> 5; }
+
+VADB_SEG_HD int ring_get(const uint32_t* ring, long long stride, int slot) {
+  return static_cast<int>((ring[(slot >> 5) * stride] >> (slot & 31)) & 1u);
+}
+
+// Set (v = 1) or clear slots [a, b) of a ring, 0 <= a < b <= 32 W.
+VADB_SEG_HD void ring_span(uint32_t* ring, long long stride, int a, int b, int v) {
+  for (int w = a >> 5; w <= (b - 1) >> 5; ++w) {
+    const int lo = (a > 32 * w ? a : 32 * w) - 32 * w, hi = (b < 32 * w + 32 ? b : 32 * w + 32) - 32 * w;
+    const uint32_t m = (hi - lo == 32 ? 0xffffffffu : ((1u << (hi - lo)) - 1u)) << lo;
+    uint32_t& x = ring[w * stride];
+    x = v ? (x | m) : (x & ~m);
+  }
+}
+
+// Set or clear the `len` rows just before the row whose slot is `end` (0 < len <= d): one or two spans.
+VADB_SEG_HD void ring_run(uint32_t* ring, long long stride, int d, int end, int len, int v) {
+  const int a = end >= len ? end - len : end - len + d;
+  if (a + len <= d) {
+    ring_span(ring, stride, a, a + len, v);
+  } else {
+    ring_span(ring, stride, a, d, v);
+    ring_span(ring, stride, 0, a + len - d, v);
+  }
+}
+
+// Push row t (value v) into a ring of d > 0 rows; returns its oldest row t - d, or -1 while t < d.
+VADB_SEG_HD int ring_push(uint32_t* ring, long long stride, int d, int t, int v) {
+  const int slot = t % d;
+  const int out = t >= d ? ring_get(ring, stride, slot) : -1;
+  uint32_t& x = ring[(slot >> 5) * stride];
+  x = (x & ~(1u << (slot & 31))) | (static_cast<uint32_t>(v) << (slot & 31));
+  return out;
+}
+
+// Step 1, input row t of a stream: returns step 1's output row t - d1 (-1: none yet).
+VADB_SEG_HD int seg_fill_push(const StreamSeg& g, uint32_t* ring, long long stride, int t, int v, uint32_t& meta) {
+  if (g.d1 == 0) return v;
+  uint32_t z = meta & kSegRunMask;
+  if (v) {
+    if (z > 0 && ((meta >> kSegSeenBit) & 1u) && z < static_cast<uint32_t>(g.G))
+      ring_run(ring, stride, g.d1, t % g.d1, static_cast<int>(z), 1);
+    z = 0;
+    meta |= 1u << kSegSeenBit;
+  } else if (z < static_cast<uint32_t>(g.G)) {
+    ++z;
+  }
+  meta = (meta & ~kSegRunMask) | z;
+  return ring_push(ring, stride, g.d1, t, v);
+}
+
+// Step 2, input row t: returns its output row t - d2 (-1: none yet).  A short run ends on a non-speech row.
+VADB_SEG_HD int seg_runs_push(const StreamSeg& g, uint32_t* ring, long long stride, int t, int v, uint32_t& meta) {
+  if (g.d2 == 0) return v;
+  uint32_t run = (meta >> kSegRun2Shift) & kSegRunMask;
+  if (v) {
+    if (run < static_cast<uint32_t>(g.S)) ++run;
+  } else {
+    if (run > 0 && run < static_cast<uint32_t>(g.S)) ring_run(ring, stride, g.d2, t % g.d2, static_cast<int>(run), 0);
+    run = 0;
+  }
+  meta = (meta & ~(kSegRunMask << kSegRun2Shift)) | (run << kSegRun2Shift);
+  return ring_push(ring, stride, g.d2, t, v);
+}
+
+// Step 3's row q: speech iff its last speech input (last - 1) lies at or after q - P.
+VADB_SEG_HD int seg_pad_row(int q, int P, int last) { return last > 0 && last - 1 >= q - P ? 1 : 0; }
+
+// Emitted row q with value y: its bound (160 q + 440 when it opens or closes a segment, else -1).
+VADB_SEG_HD long long seg_emit(int q, int y, uint32_t& meta) {
+  const int prev = static_cast<int>((meta >> kSegOutBit) & 1u);
+  meta = (meta & ~(1u << kSegOutBit)) | (static_cast<uint32_t>(y) << kSegOutBit);
+  return y != prev ? seg_sample(q) : -1;
+}
+
+// One row r (value v != 0: speech) of stream s.  Returns the row it finalises, r - H (-1: none), with its value
+// and bound.
+VADB_SEG_HD int seg_step(const StreamSeg& g, long long s, int r, int v, uint8_t& row, long long& bound) {
+  uint32_t meta = g.meta[s];
+  int q = -1;
+  row = 255;
+  bound = -1;
+  int x = seg_fill_push(g, g.ring1 + s, g.n, r, v, meta);
+  if (x >= 0) x = seg_runs_push(g, g.ring2 + s, g.n, r - g.d1, x, meta);
+  if (x >= 0) {
+    const int t3 = r - g.d1 - g.d2;
+    int last = g.last[s];
+    if (x) g.last[s] = last = t3 + 1;
+    if (t3 >= g.P) {
+      q = t3 - g.P;
+      const int y = seg_pad_row(q, g.P, last);
+      row = static_cast<uint8_t>(y);
+      bound = seg_emit(q, y, meta);
+    }
+  }
+  g.meta[s] = meta;
+  return q;
+}
+
+// End of a stream that took R rows: emit(q, value, bound) for its min(R, H) pending rows in order; returns the
+// close of a segment still open (160 R + 440) or -1.  Rings are read and written through (ring1, ring2, stride),
+// which may be a copy of the stream's state; meta and last are the stream's values, updated in place.
+template <class Emit>
+VADB_SEG_HD long long seg_drain(const StreamSeg& g, uint32_t* ring1, uint32_t* ring2, long long stride, int R,
+                                uint32_t& meta, int& last, Emit emit) {
+  int t2 = R - g.d1 > 0 ? R - g.d1 : 0;
+  int t3 = t2 - g.d2 > 0 ? t2 - g.d2 : 0;
+  auto pad_in = [&](int x) {
+    if (x) last = t3 + 1;
+    if (t3 >= g.P) {
+      const int q = t3 - g.P, y = seg_pad_row(q, g.P, last);
+      emit(q, y, seg_emit(q, y, meta));
+    }
+    ++t3;
+  };
+  auto runs_in = [&](int x) {
+    const int y = seg_runs_push(g, ring2, stride, t2++, x, meta);
+    if (y >= 0) pad_in(y);
+  };
+  if (g.d1 > 0)  // step 1: the rows still held, unfilled
+    for (int p = R - g.d1 > 0 ? R - g.d1 : 0; p < R; ++p) runs_in(ring_get(ring1, stride, p % g.d1));
+  if (g.d2 > 0) {  // step 2: the trailing run counts with the length it has
+    const uint32_t run = (meta >> kSegRun2Shift) & kSegRunMask;
+    if (run > 0 && run < static_cast<uint32_t>(g.S)) ring_run(ring2, stride, g.d2, t2 % g.d2, static_cast<int>(run), 0);
+    for (int p = t2 - g.d2 > 0 ? t2 - g.d2 : 0; p < t2; ++p) pad_in(ring_get(ring2, stride, p % g.d2));
+  }
+  for (int q = t3 - g.P > 0 ? t3 - g.P : 0; q < t3; ++q) {  // step 3: the pad clipped at row R
+    const int y = seg_pad_row(q, g.P, last);
+    emit(q, y, seg_emit(q, y, meta));
+  }
+  return (meta >> kSegOutBit) & 1u ? seg_sample(R) : -1;
+}
+
+// End stream s after R rows: its rings move to scratch (word k at scratch[k * sstride]) and the drain runs there;
+// tail_rows [n][H] gets the pending rows then 255, tail_bounds [n][H + 1] their bounds, the close, then -1 (both
+// nullable).  The stream's segment state is zero afterwards.
+VADB_SEG_HD void seg_end(const StreamSeg& g, long long s, int R, uint32_t* scratch, long long sstride,
+                         uint8_t* tail_rows, int64_t* tail_bounds) {
+  const int w1 = g.d1 > 0 ? seg_ring_words(g.d1) : 0, w2 = g.d2 > 0 ? seg_ring_words(g.d2) : 0;
+  for (int k = 0; k < w1; ++k) {
+    scratch[k * sstride] = g.ring1[k * g.n + s];
+    g.ring1[k * g.n + s] = 0;
+  }
+  for (int k = 0; k < w2; ++k) {
+    scratch[(w1 + k) * sstride] = g.ring2[k * g.n + s];
+    g.ring2[k * g.n + s] = 0;
+  }
+  uint32_t meta = g.meta[s];
+  int last = g.last[s];
+  uint8_t* rows = tail_rows ? tail_rows + s * g.H : nullptr;
+  int64_t* bounds = tail_bounds ? tail_bounds + s * (g.H + 1) : nullptr;
+  int j = 0;
+  const long long close = seg_drain(g, scratch, scratch + w1 * sstride, sstride, R, meta, last,
+                                    [&](int, int y, long long b) {
+                                      if (rows) rows[j] = static_cast<uint8_t>(y);
+                                      if (bounds) bounds[j] = b;
+                                      ++j;
+                                    });
+  if (rows)
+    for (int k = j; k < g.H; ++k) rows[k] = 255;
+  if (bounds)
+    for (int k = j; k <= g.H; ++k) bounds[k] = k == j ? close : -1;
+  g.meta[s] = 0;
+  g.last[s] = 0;
+}
+
 #if defined(__CUDACC__)
 
 // Exclusive max of `last` over lower threads (-1 for thread 0) and exclusive min of `first` over higher threads
@@ -449,6 +646,26 @@ __global__ void __launch_bounds__(kSpeechThreads) speech_gather_kernel(
     j += kSpeechThreads;
     __syncthreads();
   }
+}
+
+// Stream bank: end the streams with end[s] != 0.  One thread per stream: with speech on (g.meta != nullptr) it
+// drains the stream's pending rows in shared memory (its rings, lane-strided) and writes the tail; then it zeroes
+// the stream's bank state (history [n][320], MFCC ring [65][n], fed, previous sample) so its next chunk starts a
+// new signal.  Shared memory: (W1 + W2) * kSegEndThreads words.
+__global__ void __launch_bounds__(kSegEndThreads) stream_end_kernel(
+    const StreamSeg g, const uint8_t* __restrict__ end, int n_streams, int16_t* __restrict__ hist,
+    float* __restrict__ mfcc_ring, int* __restrict__ fed, int16_t* __restrict__ prev, uint8_t* __restrict__ tail_rows,
+    int64_t* __restrict__ tail_bounds) {
+  extern __shared__ uint32_t seg_scratch[];
+  const int s = blockIdx.x * kSegEndThreads + threadIdx.x;
+  if (s >= n_streams || !end[s]) return;
+  const int f = fed[s];
+  if (g.meta) seg_end(g, s, f > 7 ? f - 7 : 0, seg_scratch + threadIdx.x, kSegEndThreads, tail_rows, tail_bounds);
+  uint32_t* h32 = reinterpret_cast<uint32_t*>(hist + static_cast<long long>(s) * 320);
+  for (int k = 0; k < 160; ++k) h32[k] = 0;
+  for (int k = 0; k < 65; ++k) mfcc_ring[static_cast<long long>(k) * n_streams + s] = 0.0f;
+  fed[s] = 0;
+  prev[s] = 0;
 }
 
 #endif  // __CUDACC__

@@ -127,6 +127,11 @@ struct vadb200_bank {
   float* d_ring = nullptr;
   int* d_fed = nullptr;
   int16_t* d_prev = nullptr;  // the raw sample before each stream's history (front end)
+  // speech segments (vadb200_stream_bank_set_speech); d_seg == nullptr: off.  One allocation of
+  // [W1 + W2 + 2][n] words: ring1, ring2, meta, last (vad_segments.cuh StreamSeg).
+  SmoothParams sp{};
+  uint32_t* d_seg = nullptr;
+  size_t seg_bytes = 0;
 };
 
 namespace {
@@ -160,6 +165,7 @@ int ensure_attrs(vadb200_handle* h) {
   CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
   CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
   CU(cudaFuncSetAttribute(stream_feed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_feed_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
   h->attr_set = true;
   return 0;
 }
@@ -928,23 +934,33 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
 int vadb200_stream_bank_destroy(vadb200_bank* b) {
   if (!b) return 0;
   cudaSetDevice(b->h->device);
-  cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev);
+  cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev); cudaFree(b->d_seg);
   delete b;
   return 0;
 }
 
-int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
-  if (!b) return fail(VADB200_E_INVALID, "bank is null");
-  CU(cudaSetDevice(b->h->device));
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CU(cudaMemsetAsync(b->d_hist, 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
-  CU(cudaMemsetAsync(b->d_ring, 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
-  CU(cudaMemsetAsync(b->d_fed, 0, static_cast<size_t>(b->n) * sizeof(int), st));
-  CU(cudaMemsetAsync(b->d_prev, 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
-  return 0;
+namespace {
+
+StreamSeg bank_seg(const vadb200_bank* b, uint8_t* d_rows, int64_t* d_bounds) {
+  StreamSeg g{};
+  if (!b->d_seg) return g;
+  const SmoothParams& sp = b->sp;
+  g.n = b->n;
+  g.G = sp.G; g.S = sp.S; g.P = sp.P; g.H = sp.H;
+  g.d1 = sp.G > 1 ? sp.G - 1 : 0;
+  g.d2 = sp.S > 1 ? sp.S - 1 : 0;
+  const long long w1 = g.d1 ? seg_ring_words(g.d1) : 0, w2 = g.d2 ? seg_ring_words(g.d2) : 0;
+  g.ring1 = b->d_seg;
+  g.ring2 = b->d_seg + w1 * b->n;
+  g.meta = b->d_seg + (w1 + w2) * b->n;
+  g.last = reinterpret_cast<int*>(g.meta + b->n);
+  g.rows = d_rows;
+  g.bounds = d_bounds;
+  return g;
 }
 
-int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labels, float* d_logits, void* stream) {
+int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labels, float* d_logits, uint8_t* d_rows,
+                       int64_t* d_bounds, void* stream) {
   if (!b || !d_chunks || !d_labels) return fail(VADB200_E_INVALID, "null argument");
   vadb200_handle* h = b->h;
   if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
@@ -961,7 +977,79 @@ int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_lab
   bp.tw1 = h->d_tw; bp.tw2 = h->d_tw + 256; bp.feat_mode = VADB200_FEAT_ANALYSER;
   bp.prev = b->d_prev;
   bp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
-  stream_feed_kernel<<<(b->n + kStepFrames - 1) / kStepFrames, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
+  const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
+  if (b->d_seg)  // speech on: every feed advances the segment state
+    stream_feed_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par, bank_seg(b, d_rows, d_bounds));
+  else
+    stream_feed_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
+  g_launches.fetch_add(1);
+  CU(cudaGetLastError());
+  return 0;
+}
+
+}  // namespace
+
+int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
+  if (!b) return fail(VADB200_E_INVALID, "bank is null");
+  CU(cudaSetDevice(b->h->device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CU(cudaMemsetAsync(b->d_hist, 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
+  CU(cudaMemsetAsync(b->d_ring, 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
+  CU(cudaMemsetAsync(b->d_fed, 0, static_cast<size_t>(b->n) * sizeof(int), st));
+  CU(cudaMemsetAsync(b->d_prev, 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
+  if (b->d_seg) CU(cudaMemsetAsync(b->d_seg, 0, b->seg_bytes, st));
+  return 0;
+}
+
+int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labels, float* d_logits, void* stream) {
+  return launch_stream_feed(b, d_chunks, d_labels, d_logits, nullptr, nullptr, stream);
+}
+
+int vadb200_stream_bank_set_speech(vadb200_bank* b, int enable, int min_speech_rows, int min_silence_rows,
+                                   int pad_rows, void* stream) {
+  if (!b) return fail(VADB200_E_INVALID, "bank is null");
+  if (enable) {
+    for (int v : {min_speech_rows, min_silence_rows, pad_rows})
+      if (v < 0 || v > kSpeechMaxParam) return fail(VADB200_E_INVALID, "speech parameters must lie in [0, 1000] rows");
+  }
+  CU(cudaSetDevice(b->h->device));
+  CU(cudaFree(b->d_seg));  // waits for work in flight that may still use it
+  b->d_seg = nullptr;
+  b->seg_bytes = 0;
+  if (enable) {
+    const SmoothParams sp = smooth_params(min_speech_rows, min_silence_rows, pad_rows);
+    const int w1 = sp.G > 1 ? seg_ring_words(sp.G - 1) : 0, w2 = sp.S > 1 ? seg_ring_words(sp.S - 1) : 0;
+    const size_t bytes = static_cast<size_t>(w1 + w2 + 2) * b->n * sizeof(uint32_t);
+    cudaError_t e = cudaMalloc(&b->d_seg, bytes);
+    if (e != cudaSuccess) {
+      b->d_seg = nullptr;
+      return cuda_fail(e, "vadb200_stream_bank_set_speech");
+    }
+    b->sp = sp;
+    b->seg_bytes = bytes;
+  }
+  return vadb200_stream_bank_reset(b, stream);
+}
+
+int vadb200_stream_bank_speech_delay(const vadb200_bank* b) { return b && b->d_seg ? b->sp.H : -1; }
+
+int vadb200_stream_feed_speech(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labels, float* d_logits,
+                               uint8_t* d_rows, int64_t* d_bounds, void* stream) {
+  if (!b) return fail(VADB200_E_INVALID, "bank is null");
+  if (!b->d_seg) return fail(VADB200_E_STATE, "speech is off (vadb200_stream_bank_set_speech)");
+  return launch_stream_feed(b, d_chunks, d_labels, d_logits, d_rows, d_bounds, stream);
+}
+
+int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end, uint8_t* d_tail_rows,
+                                    int64_t* d_tail_bounds, void* stream) {
+  if (!b || !d_end) return fail(VADB200_E_INVALID, "null argument");
+  CU(cudaSetDevice(b->h->device));
+  const StreamSeg g = bank_seg(b, nullptr, nullptr);
+  const int words = g.meta ? (g.d1 ? seg_ring_words(g.d1) : 0) + (g.d2 ? seg_ring_words(g.d2) : 0) : 0;
+  stream_end_kernel<<<(b->n + kSegEndThreads - 1) / kSegEndThreads, kSegEndThreads,
+                      static_cast<size_t>(words) * kSegEndThreads * sizeof(uint32_t), static_cast<cudaStream_t>(stream)>>>(
+      g, d_end, b->n, b->d_hist, b->d_ring, b->d_fed, b->d_prev, g.meta ? d_tail_rows : nullptr,
+      g.meta ? d_tail_bounds : nullptr);
   g_launches.fetch_add(1);
   CU(cudaGetLastError());
   return 0;

@@ -408,6 +408,30 @@ class StreamBankHandle(object):
         check(self.lib.vadb200_stream_feed(self._b, C.c_void_p(chunks_ptr), C.c_void_p(labels_ptr),
                                            C.c_void_p(logits_ptr), stream if stream is not None else self.handle.stream))
 
+    # ---- speech segments (vadb200_stream_bank_set_speech) -------------------------------------------
+    def set_speech(self, min_speech_rows, min_silence_rows, pad_rows):
+        """Speech on at (S, G, P) rows, each in [0, 1000]; resets every stream.  Returns the delay D in rows."""
+        check(self.lib.vadb200_stream_bank_set_speech(self._b, 1, int(min_speech_rows), int(min_silence_rows),
+                                                      int(pad_rows), self.handle.stream))
+        return self.speech_delay()
+
+    def disable_speech(self):
+        check(self.lib.vadb200_stream_bank_set_speech(self._b, 0, 0, 0, 0, self.handle.stream))
+
+    def speech_delay(self):
+        """D rows, or -1 when speech is off."""
+        return int(self.lib.vadb200_stream_bank_speech_delay(self._b))
+
+    def feed_speech_ptr(self, chunks_ptr, labels_ptr, logits_ptr=0, rows_ptr=0, bounds_ptr=0, stream=None):
+        check(self.lib.vadb200_stream_feed_speech(self._b, C.c_void_p(chunks_ptr), C.c_void_p(labels_ptr),
+                                                  C.c_void_p(logits_ptr), C.c_void_p(rows_ptr), C.c_void_p(bounds_ptr),
+                                                  stream if stream is not None else self.handle.stream))
+
+    def end_streams_ptr(self, end_ptr, tail_rows_ptr=0, tail_bounds_ptr=0, stream=None):
+        check(self.lib.vadb200_stream_bank_end_streams(self._b, C.c_void_p(end_ptr), C.c_void_p(tail_rows_ptr),
+                                                       C.c_void_p(tail_bounds_ptr),
+                                                       stream if stream is not None else self.handle.stream))
+
 
 _default = {}
 
