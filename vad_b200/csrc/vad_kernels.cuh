@@ -20,9 +20,10 @@
 // The step has no CTA-wide bar.sync: two split-phase mbarriers ("P free", "P full", one arrival per
 // warp) order the power tile; only block steps use CTA barriers.
 // Block phase: MODE 0 / 1 flush MFCC / dataset rows (every 8 steps); MODE 2 builds the 5-frame window
-// features and runs Dense 39-64-32-16-3 -- on FP32 CUDA cores (TC = 0, every 8 steps) or as one
-// tcgen05 tile of 128 frames with TMEM accumulators (TC = 1 tf32, TC = 2 fp16 hi/lo operands; every
-// 4 steps) -- then argmax == VOICED, 1-byte label.
+// features and runs Dense 39-64-32-16-3 -- on FP32 CUDA cores (TC = 0, every 8 steps), as one tcgen05
+// tile of 128 frames with TMEM accumulators (TC = 1, tf32 hi/lo operands, every 4 steps) or as two such
+// tiles of 128 frames side by side in TMEM (TC = 2, fp16 hi/lo operands, every 8 steps) -- then
+// argmax == VOICED, 1-byte label.
 //
 // Reference lines restated: mfcc.py:59-78; dataset/file_processing.py:47-70,99-101;
 // realtime_analysis/sklearn_analyser.py:46-82,103-107; learning/ffn_trainer.py:104-116.
@@ -56,7 +57,9 @@ constexpr int kOffTw2 = kOffTw1 + 256 * 8;
 constexpr int kOffBar = kOffTw2 + 128 * 8;
 constexpr int kOffSeg = kOffBar + 48;                                       // 6 mbarriers: pcm x2, weights, mma, P free, P full
 constexpr int kFusedSmemBytes = kOffSeg + 16;                               // s_seg, s_tmem
-constexpr int kBlockStepsTc = 4;                                            // tensor-core FFN: one M=128 tile
+constexpr int kBlockStepsTc = 4;                                            // tf32 tensor-core FFN: one M=128 tile
+// A block phase reads the window of centres out_done .. computed - 3, i.e. up to kBlockSteps * 32 + 4 ring slots back.
+static_assert(kBlockSteps * kStepFrames + 4 <= kRing, "the MFCC ring must hold a whole block phase's windows");
 static_assert(kTcBlobBytes <= kWarps * 2 * kExchFrame * 8 + kP2Bytes, "weight blob must fit exch + P");
 static_assert(kBlockSteps * kStepFrames * kNFeat * 4 + 16 <= kWarps * 2 * kExchFrame * 8 + kP2Bytes,
               "dataset-row staging tile must fit exch + P");
@@ -100,7 +103,8 @@ struct FusedParams {
   int feat_mode;
   const unsigned char* tc_blob;  // canonical hi/lo tf32 weight blob (ffn_tc.cuh), TC variant only
   long long* dbg_ts;             // timing experiments only: clock64 stamps of CTA 0's block phases [n][16]
-  int debug_skip;                // timing experiments only (env VADB200_DEBUG_SKIP): 1 FFT, 2 mel, 4 DCT, 8 block phase
+  int debug_skip;                // timing experiments only (env VADB200_DEBUG_SKIP): 1 FFT, 2 mel, 4 DCT, 8 block phase,
+                                 // 256 no second fp16 tile (tools/ablate.sh lists the rest)
 };
 
 // ---- PTX wrappers: mbarrier + TMA bulk copy (UBLKCP) --------------------------------------------
@@ -314,7 +318,7 @@ template <int MODE, int TC, bool FE>
 __device__ __forceinline__ void fused_body(const FusedParams& p, const typename FfnArgOf<MODE, TC>::type& ffn,
                                            const FrontEnd& fe, const int tid) {
   static_assert(TC == 0 || MODE == 2, "tensor-core FFN only exists in VAD mode");
-  constexpr int kBlk = TC ? kBlockStepsTc : kBlockSteps;
+  constexpr int kBlk = TC == 1 ? kBlockStepsTc : kBlockSteps;
   constexpr int kStageOff = FE ? kStageOffFe : 0;
   extern __shared__ __align__(128) unsigned char smem[];
   int16_t* s_pcm = reinterpret_cast<int16_t*>(smem + kOffPcm);
@@ -541,8 +545,70 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
                            FE ? ffn.thresh : 0.0f);
           }
           out_done = max(out_done, computed - 2);
+        } else if constexpr (TC == 2) {
+          // ---- fp16 tensor-core FFN: two M = 128 tiles, thread = frame = TMEM lane of tile warp / 4 ---------------
+          const int n_valid = computed - 2 - out_done;  // centres out_done .. computed-3 (<= 256)
+          if (n_valid > 0) {                            // block-uniform (== tc_now)
+            long long* ts = nullptr;
+#if defined(VADB_DEBUG_HOOKS)
+            if (p.dbg_ts && blockIdx.x == 0 && tid == 0 && dbg_n < 64) ts = p.dbg_ts + 16 * dbg_n;
+#endif
+            if (ts) ts[0] = clock64();
+            const bool valid = tid < n_valid;
+            const int c = out_done + (valid ? tid : 0);
+            const long long row = seg.out_start - p.row_base + (c - 2);
+            const uint32_t tl = ffn_tc16_tile2_lane(tm_base, warp);
+            // The frame's 48 layer-1 columns, one 24-column half (coefficient pairs 0-3, then 4-6) at a time.  Validity
+            // stays in a register: ReLU's fmaxf swallows NaNs, so it cannot be read back from the logits.
+            bool ok = true;
+#pragma unroll
+            for (int hidx = 0; hidx < 2; ++hidx) {
+              float xl[24];
+              if (VADB_DBG(p) & 64) {
+#pragma unroll
+                for (int i = 0; i < 24; ++i) xl[i] = 0.5f;
+              } else {
+                ok = (hidx == 0 ? window_features_pairs<0, 4, kRing, 24>(s_ring, c, p.feat_mode, xl)
+                                : window_features_pairs<4, 7, kRing, 24>(s_ring, c, p.feat_mode, xl)) && ok;
+              }
+              tc16_store_a1_half(tl, hidx, xl);
+              if (p.feats && valid) {
+                const int k0 = hidx ? 8 : 0, nk = hidx ? 5 : 8;  // xl[6 (k / 2) + 2 g + k % 2], k relative to k0
+#pragma unroll
+                for (int k = 0; k < 8; ++k)
+#pragma unroll
+                  for (int g = 0; g < 3; ++g)
+                    if (k < nk) p.feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
+              }
+            }
+            if (ts) ts[1] = clock64();
+            if (!(VADB_DBG(p) & 16)) mbar_wait(&s_bar[2], w_par);  // weight blob landed (issued before the DCT phase)
+            if (ts) ts[2] = clock64();
+            float logit[kNCls];
+            // tile 1 only when it holds a valid centre (hook build: mask 256 never issues it, to time one chain)
+            const bool two_tiles = n_valid > 128 && !(VADB_DBG(p) & 256);
+            mma_par = ffn_tc16_tile2(ffn, logit, tm_base, warp, two_tiles, tid == 0, smem_u32(smem + kOffExch), &s_bar[3],
+                                     mma_par, ts);
+            ++dbg_n;
+            if (valid) {
+              uint8_t lab = decide_of<FE>(logit, ffn);  // logits are in registers: no TMEM round trip
+              if (!ok) {
+                logit[0] = logit[1] = logit[2] = NAN;
+                lab = 0;
+              }
+              p.labels[row] = lab;
+              if (p.logits) {
+                p.logits[row * 3 + 0] = logit[0];
+                p.logits[row * 3 + 1] = logit[1];
+                p.logits[row * 3 + 2] = logit[2];
+              }
+            }
+            if (!(VADB_DBG(p) & 16)) w_par ^= 1u;
+            __syncthreads();  // MMAs done reading the blob before the next FFT phase rewrites exch / P
+          }
+          out_done = max(out_done, computed - 2);
         } else {
-          // ---- tensor-core FFN: one M = 128 tile over all 8 warps ------------------------------------
+          // ---- tf32 tensor-core FFN: one M = 128 tile over all 8 warps ------------------------------
           const int n_valid = computed - 2 - out_done;  // centres out_done .. computed-3 (<= 128)
           if (n_valid > 0) {                            // block-uniform (== tc_now)
             unsigned char* wdst = smem + kOffExch;
@@ -571,8 +637,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
               }
               s_logE[tid] = ok_half ? 1.0f : 0.0f;
               if (ts) ts[1] = clock64();
-              if constexpr (TC == 2) tc16_store_a1_half(tl, hidx, xl);
-              else tc_store_a1_half(tl, hidx, xl);
+              tc_store_a1_half(tl, hidx, xl);
               if (p.feats && valid) {
                 const long long row = seg.out_start - p.row_base + (c - 2);
                 const int k0 = hidx ? 8 : 0, nk = hidx ? 5 : 8;  // xl[6 (k / 2) + 2 g + k % 2], k relative to k0
@@ -587,8 +652,6 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
               if constexpr (TC == 1)
                 mma_par = ffn_tc_tile<2>(ffn, logit, tm_base, warp & 3, hidx, tid == 0, smem_u32(wdst), &s_bar[3], mma_par,
                                          ts, VADB_DBG(p));
-              if constexpr (TC == 2)
-                mma_par = ffn_tc16_tile<2>(ffn, logit, tm_base, warp & 3, hidx, tid == 0, smem_u32(wdst), &s_bar[3], mma_par);
               ++dbg_n;
               if (valid && hidx == 0) {
                 const bool ok = s_logE[fr] != 0.0f && s_logE[128 + fr] != 0.0f;  // ordered by the tile's bar.syncs
