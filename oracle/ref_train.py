@@ -4,7 +4,9 @@ learning/ffn_trainer.py:104-120 builds Sequential(Dense64 relu relu Dense32 relu
 compiles it with loss='categorical_crossentropy', optimizer='adadelta'; :148 calls model.train_on_batch.  Keras 1.x
 is neither vendored nor installed, so its arithmetic is restated from its published source (keras/objectives.py,
 keras/optimizers.py of the 1.x line): softmax output clipped to [1e-7, 1 - 1e-7] inside the cross-entropy, mean over
-the batch; Adadelta(lr=1.0, rho=0.95, epsilon=1e-8):
+the batch.  The clip's gradient (Theano T.clip, TF clip_by_value) is zero outside that closed interval, so a row whose
+unclipped true-class probability lies outside it adds its clipped value to the loss and nothing to the gradient.
+Adadelta(lr=1.0, rho=0.95, epsilon=1e-8):
     a <- rho a + (1 - rho) g^2;  u = g sqrt(d + eps) / sqrt(a + eps);  p <- p - lr u;  d <- rho d + (1 - rho) u^2
 All in float64.  ``mixing_order`` restates the class-mixing generator of dataset/__init__.py:38-96.
 """
@@ -32,9 +34,10 @@ def loss_and_grads(p, x, y):
     e = np.exp(z)
     prob = e / e.sum(axis=1, keepdims=True)
     onehot = np.eye(3)[np.asarray(y, dtype=np.int64)]
-    pc = np.clip((prob * onehot).sum(axis=1), 1e-7, 1.0 - 1e-7)
-    loss = float(-np.log(pc).mean())
-    d = (prob - onehot) / b
+    py = (prob * onehot).sum(axis=1)
+    loss = float(-np.log(np.clip(py, 1e-7, 1.0 - 1e-7)).mean())
+    live = (py >= 1e-7) & (py <= 1.0 - 1e-7)        # the clip passes a gradient on the closed interval only
+    d = (prob - onehot) * (live[:, None] / b)
     g = {}
     for i in (4, 3, 2, 1):
         a_prev = acts[i - 1]

@@ -10,23 +10,64 @@ import pytest
 from oracle import ref_math as rm, ref_train as rt
 
 
+def _batch_with_clipped_rows(w, n=23, seed=0):
+    """Rows of N(0, 4) and, among them, rows scaled by 60: two labelled with their least likely class (p_true far
+    below 1e-7: clipped at the low end) and two with their most likely class (p_true far above 1 - 1e-7: clipped at
+    the high end).  Returns x, y and the indices of the clipped rows."""
+    rng = np.random.default_rng(seed)
+    x = rng.standard_normal((n, 39)) * 2
+    y = rng.integers(0, 3, n)
+    low, high = [3, 11], [7, 17]
+    x[low + high] *= 60
+    logits, _ = rm.ffn_forward(x, w)
+    y[low] = logits[low].argmin(axis=1)
+    y[high] = logits[high].argmax(axis=1)
+    prob = np.exp(logits - logits.max(axis=1, keepdims=True))
+    py = (prob / prob.sum(axis=1, keepdims=True))[np.arange(n), y]
+    clipped = np.array(low + high)
+    assert np.all(py[low] < 1e-9) and np.all(1.0 - py[high] < 1e-9)
+    assert np.all((py > 1e-6) & (py < 1.0 - 1e-6) | np.isin(np.arange(n), clipped))   # the rest far from both ends
+    return x, y, clipped
+
+
 def test_oracle_gradients_match_finite_differences():
+    """Every entry of every parameter tensor against central differences of the loss, on a batch whose clipped rows
+    (both ends) sit among ordinary rows: the clip passes no gradient, so those rows contribute nothing."""
     w = rm.glorot_ffn(3)
     st = rt.init_state(w)
-    rng = np.random.default_rng(0)
-    x = rng.standard_normal((23, 39)) * 2
-    y = rng.integers(0, 3, 23)
+    x, y, _ = _batch_with_clipped_rows(w)
     loss, g = rt.loss_and_grads(st["p"], x, y)
-    for k, idx in (("W1", (4, 9)), ("b1", (3,)), ("W2", (5, 7)), ("W3", (1, 2)), ("b3", (0,)), ("W4", (6, 1)), ("b4", (2,))):
-        p2 = {kk: v.copy() for kk, v in st["p"].items()}
-        p2[k][idx] += 1e-6
-        l2, _ = rt.loss_and_grads(p2, x, y)
-        assert abs((l2 - loss) / 1e-6 - g[k][idx]) <= 1e-6 + 1e-4 * abs(g[k][idx])
+    h = 1e-6
+    p2 = {k: v.copy() for k, v in st["p"].items()}
+    for k in rt.KEYS:
+        fd = np.empty_like(g[k])
+        for idx in np.ndindex(*g[k].shape):
+            v = p2[k][idx]
+            p2[k][idx] = v + h
+            lp, _ = rt.loss_and_grads(p2, x, y)
+            p2[k][idx] = v - h
+            lm, _ = rt.loss_and_grads(p2, x, y)
+            p2[k][idx] = v
+            fd[idx] = (lp - lm) / (2 * h)
+        err = np.abs(fd - g[k])
+        assert np.all(err <= 1e-7 + 1e-5 * np.abs(g[k])), (k, np.unravel_index(err.argmax(), err.shape), err.max())
     # Adadelta's first step: a = (1-rho) g^2, u = g sqrt(eps) / sqrt(a + eps)
     before = {k: v.copy() for k, v in st["p"].items()}
     rt.train_on_batch(st, x, y)
     u = g["W4"] * np.sqrt(1e-8) / np.sqrt(0.05 * g["W4"] ** 2 + 1e-8)
     np.testing.assert_allclose(st["p"]["W4"], before["W4"] - u, atol=1e-15)
+
+
+def test_oracle_clipped_rows_only_rescale_the_gradient():
+    """k clipped rows in a batch of n: the gradient is (n - k) / n times the gradient of the batch without them."""
+    w = rm.glorot_ffn(3)
+    p = rt.init_state(w)["p"]
+    x, y, clipped = _batch_with_clipped_rows(w)
+    keep = np.setdiff1d(np.arange(len(y)), clipped)
+    _, g = rt.loss_and_grads(p, x, y)
+    _, g_kept = rt.loss_and_grads(p, x[keep], y[keep])
+    for k in rt.KEYS:
+        np.testing.assert_allclose(g[k], g_kept[k] * (len(keep) / len(y)), rtol=1e-12, atol=1e-15, err_msg=k)
 
 
 def test_mixing_generator_restatements_agree():

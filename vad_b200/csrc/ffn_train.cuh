@@ -4,7 +4,8 @@
 // Dense16 relu Dense3 softmax), loss categorical_crossentropy, optimizer 'adadelta' (Keras-1 defaults lr 1.0,
 // rho 0.95, epsilon 1e-8), model.train_on_batch(batch_x, batch_y).  Restated semantics:
 //   p = softmax(logits);  loss = -mean_i sum_c y_ic log(clip(p_ic, 1e-7, 1 - 1e-7))
-//   g = dloss/dtheta (clip inactive => dlogits = (p - y) / B)
+//   g = dloss/dtheta: dlogits = (p - y) / B, and 0 for a row whose p_true lies outside [1e-7, 1 - 1e-7] (the clip
+//       passes no gradient there, in Theano's T.clip and TF's clip_by_value alike)
 //   a <- rho a + (1 - rho) g^2;  u = g sqrt(d + eps) / sqrt(a + eps);  theta <- theta - lr u;  d <- rho d + (1 - rho) u^2
 //
 // Two kernels per step, both deterministic (no floating-point atomics):
@@ -253,10 +254,14 @@ __global__ void __launch_bounds__(kTr2Threads, 1) ffn_train_grad_kernel(const fl
       const float p[kNCls] = {e0 * inv, e1 * inv, e2 * inv};
       const bool live = r < rows;
       const int cls = live ? y[row0 + r] : 0;
-      const float pc = fminf(fmaxf(cls == 0 ? p[0] : cls == 1 ? p[1] : p[2], 1e-7f), 1.0f - 1e-7f);
-      loss = live ? -logf(pc) : 0.0f;
+      const float py = cls == 0 ? p[0] : cls == 1 ? p[1] : p[2];
+      // the high end as "the other two sum below 1e-7": float32 cannot resolve p_y > 1 - 1e-7 directly
+      const float rest = cls == 0 ? p[1] + p[2] : cls == 1 ? p[0] + p[2] : p[0] + p[1];
+      const bool clipped = py < 1e-7f || rest < 1e-7f;
+      loss = live ? -logf(fminf(fmaxf(py, 1e-7f), 1.0f - 1e-7f)) : 0.0f;
 #pragma unroll
-      for (int o = 0; o < kNCls; ++o) D4[o * kTrainRows + r] = live ? (p[o] - (o == cls ? 1.0f : 0.0f)) * inv_b : 0.0f;
+      for (int o = 0; o < kNCls; ++o)
+        D4[o * kTrainRows + r] = live && !clipped ? (p[o] - (o == cls ? 1.0f : 0.0f)) * inv_b : 0.0f;
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) loss += __shfl_down_sync(0xffffffffu, loss, o);

@@ -91,6 +91,7 @@ struct vadb200_handle {
 
 struct vadb200_plan {
   vadb200_handle* h = nullptr;
+  int device = 0;                     // h->device, kept so destroy never reads a handle destroyed first
   int mode = 0;
   long long n_utt = 0;
   std::vector<long long> offsets, lengths, row_off, utt_seg;  // utt_seg: n_utt + 1
@@ -112,6 +113,7 @@ struct vadb200_plan {
 
 struct vadb200_trainer {
   vadb200_handle* h = nullptr;
+  int device = 0;              // h->device, kept so destroy never reads a handle destroyed first
   long long max_batch = 0;
   float lr = 1.0f, rho = 0.95f, eps = 1e-8f;
   float* d_state = nullptr;    // params | acc_g | acc_u   (3 x kNParams)
@@ -122,6 +124,7 @@ struct vadb200_trainer {
 
 struct vadb200_bank {
   vadb200_handle* h = nullptr;
+  int device = 0;              // h->device, kept so destroy never reads a handle destroyed first
   int n = 0;
   int16_t* d_hist = nullptr;
   float* d_ring = nullptr;
@@ -459,7 +462,7 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
   *out = nullptr;
   vadb200_plan* p = new (std::nothrow) vadb200_plan();
   if (!p) return fail(VADB200_E_NOMEM, "host allocation failed");
-  p->h = h; p->mode = mode; p->n_utt = n_utt;
+  p->h = h; p->device = h->device; p->mode = mode; p->n_utt = n_utt;
   p->offsets.assign(offs, offs + n_utt);
   p->lengths.assign(lens, lens + n_utt);
   p->row_off.resize(n_utt + 1);
@@ -553,7 +556,7 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
 
 int vadb200_plan_destroy(vadb200_plan* p) {
   if (!p) return 0;
-  cudaSetDevice(p->h->device);
+  cudaSetDevice(p->device);
   cudaFree(p->d_segs);
   cudaFree(p->d_counter);
   cudaFree(p->d_row_off);
@@ -914,7 +917,7 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
   CU(cudaSetDevice(h->device));
   vadb200_bank* b = new (std::nothrow) vadb200_bank();
   if (!b) return fail(VADB200_E_NOMEM, "host allocation failed");
-  b->h = h; b->n = n_streams;
+  b->h = h; b->device = h->device; b->n = n_streams;
   cudaError_t e = cudaMalloc(&b->d_hist, static_cast<size_t>(n_streams) * 320 * sizeof(int16_t));
   if (e == cudaSuccess) e = cudaMalloc(&b->d_ring, static_cast<size_t>(n_streams) * 5 * kNCep * sizeof(float));
   if (e == cudaSuccess) e = cudaMalloc(&b->d_fed, static_cast<size_t>(n_streams) * sizeof(int));
@@ -933,7 +936,7 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
 
 int vadb200_stream_bank_destroy(vadb200_bank* b) {
   if (!b) return 0;
-  cudaSetDevice(b->h->device);
+  cudaSetDevice(b->device);
   cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev); cudaFree(b->d_seg);
   delete b;
   return 0;
@@ -1084,7 +1087,7 @@ int vadb200_trainer_create(vadb200_handle* h, int64_t max_batch, float lr, float
   CU(cudaSetDevice(h->device));
   vadb200_trainer* t = new (std::nothrow) vadb200_trainer();
   if (!t) return fail(VADB200_E_NOMEM, "host allocation failed");
-  t->h = h; t->max_batch = max_batch; t->lr = lr; t->rho = rho; t->eps = eps;
+  t->h = h; t->device = h->device; t->max_batch = max_batch; t->lr = lr; t->rho = rho; t->eps = eps;
   const long long n_part = (max_batch + kTrainRows - 1) / kTrainRows;
   cudaError_t e = cudaMalloc(&t->d_state, 3 * kNParams * sizeof(float));
   if (e == cudaSuccess) e = cudaMemset(t->d_state, 0, 3 * kNParams * sizeof(float));
@@ -1107,7 +1110,7 @@ int vadb200_trainer_create(vadb200_handle* h, int64_t max_batch, float lr, float
 
 int vadb200_trainer_destroy(vadb200_trainer* t) {
   if (!t) return 0;
-  cudaSetDevice(t->h->device);
+  cudaSetDevice(t->device);
   cudaFree(t->d_state); cudaFree(t->d_partial); cudaFree(t->d_loss);
   delete t;
   return 0;
@@ -1148,6 +1151,7 @@ int vadb200_train_on_batch(vadb200_trainer* t, const float* d_x, const uint8_t* 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n_tiles = static_cast<int>((n + kTrainRows - 1) / kTrainRows);
   const int n_part = std::min(n_tiles, t->h->num_sms);   // persistent CTAs: one partial gradient each
+  cudaGetLastError();   // the check below is for these launches, not a non-sticky error an earlier call left behind
   ffn_train_grad_kernel<<<n_part, kTr2Threads, kTrain2SmemBytes, st>>>(t->d_state, d_x, d_y, n,
                                                                          1.0f / static_cast<float>(n), t->d_partial);
   ffn_train_update_kernel<<<(kNParams + 1 + 255) / 256, 256, 0, st>>>(t->d_state, t->d_state + kNParams,
