@@ -6,7 +6,8 @@
  * with ctypes and re-exports the reference's function / class names (INTEGRATION.md).
  *
  * Conventions: every function returns 0 on success or a negative VADB200_E_* code and never
- * throws or aborts; vadb200_last_error() gives a thread-local message.  A handle is bound to
+ * throws or aborts; vadb200_last_error() gives a thread-local message.  A *_create function that
+ * fails leaves *out NULL and retains nothing it allocated.  A handle is bound to
  * one CUDA device.  The library keeps NO per-handle state in device globals: FFN weights travel
  * with every launch as kernel parameters, so different handles (= different classifiers, as one
  * SKLearnAnalyzer owns one classifier, sklearn_analyser.py:21-35) may be driven from different

@@ -9,12 +9,15 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "vad_host_tables.h"
@@ -46,15 +49,92 @@ int cuda_fail(cudaError_t e, const char* what) {
     if (e__ != cudaSuccess) return cuda_fail(e__, #expr); \
   } while (0)
 
+// Every kernel launch goes through here: `enqueue` launches n kernels.  The thread's last error is cleared first, so
+// the check reports these launches, not a non-sticky error that an earlier runtime call left behind (a sticky error of
+// a faulted context still surfaces).
+template <class F>
+int launched(int n, F&& enqueue) {
+  cudaGetLastError();
+  enqueue();
+  g_launches.fetch_add(n);
+  CU(cudaGetLastError());
+  return 0;
+}
+
+// Owners of CUDA resources.  Objects free their members on their own device: each destructor body below selects it,
+// and member destructors run after the body.
+struct CudaFree {
+  void operator()(void* p) const { cudaFree(p); }
+};
+struct CudaFreeAsync {  // stream-ordered scratch
+  cudaStream_t st;
+  void operator()(void* p) const { cudaFreeAsync(p, st); }
+};
+struct StreamDestroy {
+  void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+};
+struct EventDestroy {
+  void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+};
+template <class T>
+using DevBuf = std::unique_ptr<T, CudaFree>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+// Frees what b holds, then allocates `bytes` into it; b stays empty on failure.
+template <class T>
+cudaError_t dev_alloc(DevBuf<T>& b, size_t bytes) {
+  b.reset();
+  void* p = nullptr;
+  const cudaError_t e = cudaMalloc(&p, bytes);
+  if (e == cudaSuccess) b.reset(static_cast<T*>(p));
+  return e;
+}
+template <class T>
+cudaError_t dev_upload(DevBuf<T>& b, const T* src, size_t n) {
+  const cudaError_t e = dev_alloc(b, n * sizeof(T));
+  return e == cudaSuccess ? cudaMemcpy(b.get(), src, n * sizeof(T), cudaMemcpyHostToDevice) : e;
+}
+cudaError_t make_stream(Stream& s) {
+  cudaStream_t r = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&r, cudaStreamNonBlocking);
+  s.reset(e == cudaSuccess ? r : nullptr);
+  return e;
+}
+cudaError_t make_event(Event& ev, unsigned flags) {
+  cudaEvent_t r = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&r, flags);
+  ev.reset(e == cudaSuccess ? r : nullptr);
+  return e;
+}
+
 long long* g_dbg_ts = nullptr;  // timing experiments only (vadb200_debug_timestamps)
 constexpr int kNumSmFallback = 148;
 constexpr int kPlanCounters = 16;  // launches of one plan that may be in flight at once (any streams)
 constexpr int kHostBufs = 3;
 constexpr int kWinPairs = kFftN / 2;  // window pairs for any frame_len <= 512; entries past 400 stay 1
 
+// One staging slot of the vad_host pipeline: the chunk's PCM, its results, and the events that order the slot's reuse.
+struct HostBuf {
+  DevBuf<int16_t> stage;
+  DevBuf<uint8_t> labels;
+  DevBuf<float> logits, rows;
+  Event in, done, out;
+};
+// Grows one buffer of every staging slot to `count` elements; contents are not kept.
+template <class T>
+int grow(HostBuf (&slots)[kHostBufs], DevBuf<T> HostBuf::*buf, long long& cap, long long count) {
+  if (count <= cap) return 0;
+  cap = 0;  // a failure part way must not leave a capacity that some slot lacks
+  for (HostBuf& s : slots) CU(dev_alloc(s.*buf, count * sizeof(T)));
+  cap = count;
+  return 0;
+}
+
 }  // namespace
 
 struct vadb200_handle {
+  ~vadb200_handle() { cudaSetDevice(device); }
   int device = 0;
   unsigned long long id = 0;
   unsigned version = 1;
@@ -65,39 +145,36 @@ struct vadb200_handle {
   FfnBias bias;       // the same biases for the tensor-core variant
   int plan_seg_frames = 0;  // 0 = automatic segment length (vadb200_set_plan_segment_frames)
   bool have_ffn = false;
-  cf2* d_tw = nullptr;  // tw1[256] then tw2[128]
+  DevBuf<cf2> d_tw;  // tw1[256] then tw2[128]
   int num_sms = kNumSmFallback;
-  bool attr_set = false;
   long long host_chunk_samples = 32ll << 20;
-  // vad_host pipeline resources (lazy)
-  cudaStream_t s_in = nullptr, s_run = nullptr, s_out = nullptr;
-  cudaEvent_t ev_in[kHostBufs] = {}, ev_done[kHostBufs] = {}, ev_out[kHostBufs] = {};
-  int16_t* d_stage[kHostBufs] = {};
-  uint8_t* d_lab[kHostBufs] = {};
-  float* d_lgt[kHostBufs] = {};
-  float* d_rows[kHostBufs] = {};
-  long long stage_cap = 0, lab_cap = 0, lgt_cap = 0, rows_cap = 0;
-  float* d_sink = nullptr;
-  unsigned char* d_tc_blob = nullptr;   // canonical tf32 hi/lo weight blob (ffn_tc.cuh)
-  unsigned char* d_tc16_blob = nullptr; // canonical fp16 hi/lo weight blob, statically scaled
+  // vad_host pipeline resources (lazy): usable once all streams and events exist
+  bool pipe_ready = false;
+  Stream s_in, s_run, s_out;
+  HostBuf hb[kHostBufs];
+  long long stage_cap = 0, lab_cap = 0, lgt_cap = 0, rows_cap = 0;  // elements in each slot's buffer
+  DevBuf<float> d_sink;
+  DevBuf<unsigned char> d_tc_blob;      // canonical tf32 hi/lo weight blob (ffn_tc.cuh)
+  DevBuf<unsigned char> d_tc16_blob;    // canonical fp16 hi/lo weight blob, statically scaled
   bool tc16_ok = false;                 // the fp16 scales are in range for this handle's weights
   int ffn_impl = 2;                     // 0: FP32 CUDA cores, 1: tcgen05 tf32 hi/lo, 2: tcgen05 fp16 hi/lo (default)
   // opt-in front end (vadb200_set_frontend); the decision threshold lives in par.thresh / bias.thresh
   float preemph = 0.0f;
   bool has_window = false;
   float window[kFrame] = {};
-  cf2* d_win = nullptr;                 // [kWinPairs] window pairs, all ones without a window (per handle: no globals)
+  DevBuf<cf2> d_win;                    // [kWinPairs] window pairs, all ones without a window (per handle: no globals)
 };
 
 struct vadb200_plan {
+  ~vadb200_plan() { cudaSetDevice(device); }
   vadb200_handle* h = nullptr;
   int device = 0;                     // h->device, kept so destroy never reads a handle destroyed first
   int mode = 0;
   long long n_utt = 0;
   std::vector<long long> offsets, lengths, row_off, utt_seg;  // utt_seg: n_utt + 1
   std::vector<Segment> segs;
-  Segment* d_segs = nullptr;
-  int* d_counter = nullptr;   // kPlanCounters self-resetting (next segment, CTAs done) pairs
+  DevBuf<Segment> d_segs;
+  DevBuf<int> d_counter;      // kPlanCounters self-resetting (next segment, CTAs done) pairs
   std::atomic<unsigned> launch_seq{0};
   long long total_rows = 0;
   long long seg_frames = 0;
@@ -105,86 +182,69 @@ struct vadb200_plan {
   std::vector<SpeechTile> tiles;
   std::vector<int> utt_tile;          // n_utt + 1: first tile of each utterance
   long long max_speech_segs = 0;      // sum over utterances of ceil(R_u / 2)
-  long long* d_row_off = nullptr;     // n_utt + 1 row offsets
-  long long* d_pcm_off = nullptr;     // n_utt sample offsets
-  SpeechTile* d_tiles = nullptr;
-  int* d_utt_tile = nullptr;
+  DevBuf<long long> d_row_off;        // n_utt + 1 row offsets
+  DevBuf<long long> d_pcm_off;        // n_utt sample offsets
+  DevBuf<SpeechTile> d_tiles;
+  DevBuf<int> d_utt_tile;
 };
 
 struct vadb200_trainer {
+  ~vadb200_trainer() { cudaSetDevice(device); }
   vadb200_handle* h = nullptr;
   int device = 0;              // h->device, kept so destroy never reads a handle destroyed first
   long long max_batch = 0;
   float lr = 1.0f, rho = 0.95f, eps = 1e-8f;
-  float* d_state = nullptr;    // params | acc_g | acc_u   (3 x kNParams)
-  float* d_partial = nullptr;  // [min(ceil(max_batch / 128), SMs)][kNParams + 1]
-  float* d_loss = nullptr;
+  DevBuf<float> d_state;       // params | acc_g | acc_u   (3 x kNParams)
+  DevBuf<float> d_partial;     // [min(ceil(max_batch / 128), SMs)][kNParams + 1]
+  DevBuf<float> d_loss;
   long long steps = 0;
 };
 
 struct vadb200_bank {
+  ~vadb200_bank() { cudaSetDevice(device); }
   vadb200_handle* h = nullptr;
   int device = 0;              // h->device, kept so destroy never reads a handle destroyed first
   int n = 0;
-  int16_t* d_hist = nullptr;
-  float* d_ring = nullptr;
-  int* d_fed = nullptr;
-  int16_t* d_prev = nullptr;  // the raw sample before each stream's history (front end)
-  // speech segments (vadb200_stream_bank_set_speech); d_seg == nullptr: off.  One allocation of
+  DevBuf<int16_t> d_hist;
+  DevBuf<float> d_ring;
+  DevBuf<int> d_fed;
+  DevBuf<int16_t> d_prev;      // the raw sample before each stream's history (front end)
+  // speech segments (vadb200_stream_bank_set_speech); d_seg empty: off.  One allocation of
   // [W1 + W2 + 2][n] words: ring1, ring2, meta, last (vad_segments.cuh StreamSeg).
   SmoothParams sp{};
-  uint32_t* d_seg = nullptr;
+  DevBuf<uint32_t> d_seg;
   size_t seg_bytes = 0;
 };
 
 namespace {
 
-// Mel weights and the folded DCT matrix are the same for every handle (the kernels are compiled for the
-// reference configuration only), so the __constant__ copy is written once per device and never changes:
-// no handle can observe another handle's state through it.  FFN weights never go through device globals.
-int ensure_tables(vadb200_handle* h) {
-  if (h->device >= 64) return fail(VADB200_E_INVALID, "device index >= 64");
-  std::lock_guard<std::mutex> lk(g_tab_mu);
-  if (g_tab_loaded[h->device]) return 0;
-  CU(cudaMemcpyToSymbol(c_tab, &h->tab, sizeof(MelDctTables), 0, cudaMemcpyHostToDevice));
-  CU(cudaDeviceSynchronize());
-  g_tab_loaded[h->device] = true;
-  return 0;
-}
-
-int ensure_attrs(vadb200_handle* h) {
-  if (h->attr_set) return 0;
-  CU(cudaFuncSetAttribute(fused_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
-  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
-  CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
-  h->attr_set = true;
-  return 0;
-}
-
 bool frontend_on(const vadb200_handle* h) { return h->preemph != 0.0f || h->has_window; }
-FrontEnd frontend_of(const vadb200_handle* h) { return FrontEnd{h->d_win, h->preemph}; }
+FrontEnd frontend_of(const vadb200_handle* h) { return FrontEnd{h->d_win.get(), h->preemph}; }
+
+// The classifier a handle runs: 2 (tcgen05 fp16 hi/lo) when asked for and the weights fit its static scales, else
+// 1 (tcgen05 tf32 hi/lo) when any tensor-core variant is asked for, else 0 (FP32 CUDA cores); and its weight blob.
+struct Classifier {
+  int tc;
+  const unsigned char* blob;
+};
+Classifier classifier_of(const vadb200_handle* h) {
+  if (h->ffn_impl == 2 && h->tc16_ok) return {2, h->d_tc16_blob.get()};
+  if (h->ffn_impl >= 1) return {1, h->d_tc_blob.get()};
+  return {0, nullptr};
+}
+
+template <int MODE, int TC>
+void enqueue_fused(bool fe, int grid, cudaStream_t st, const FusedParams& fp,
+                   const typename FfnArgOf<MODE, TC>::type& ffn, const FrontEnd& fea) {
+  if (fe) fused_fe_kernel<MODE, TC><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn, fea);
+  else fused_kernel<MODE, TC><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn);
+}
 
 int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   vadb200_handle* h = p->h;
   if (n_segs <= 0) return 0;
-  int rc = ensure_attrs(h);
-  if (rc) return rc;
-  rc = ensure_tables(h);
-  if (rc) return rc;
   // each launch takes its own self-resetting counter pair, so one plan can be in flight on several streams
-  fp.counter = p->d_counter + 2 * (p->launch_seq.fetch_add(1) % kPlanCounters);
+  fp.counter = p->d_counter.get() + 2 * (p->launch_seq.fetch_add(1) % kPlanCounters);
 #if defined(VADB_DEBUG_HOOKS)
   const char* gps = std::getenv("VADB200_CTAS_PER_SM");  // occupancy experiments only
   const int per_sm = gps ? std::max(1, std::atoi(gps)) : 2;
@@ -195,52 +255,24 @@ int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   // the front-end variant runs only when the handle asks for a front end or (VAD) a decision threshold
   const bool fe = frontend_on(h) || (p->mode == VADB200_MODE_VAD && h->par.thresh > 0.0f);
   const FrontEnd fea = frontend_of(h);
-  if (fe) {
-    switch (p->mode) {
-      case VADB200_MODE_MFCC: fused_fe_kernel<0, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}, fea); break;
-      case VADB200_MODE_DATASET: fused_fe_kernel<1, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}, fea); break;
-      default:
-        if (h->ffn_impl == 2 && h->tc16_ok) {
-          fp.tc_blob = h->d_tc16_blob;
-          fused_fe_kernel<2, 2><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias, fea);
-        } else if (h->ffn_impl >= 1) {
-          fused_fe_kernel<2, 1><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias, fea);
-        } else {
-          fused_fe_kernel<2, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->par, fea);
-        }
-        break;
-    }
-    g_launches.fetch_add(1);
-    CU(cudaGetLastError());
-    return 0;
-  }
-  switch (p->mode) {
-    case VADB200_MODE_MFCC: fused_kernel<0, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}); break;
-    case VADB200_MODE_DATASET: fused_kernel<1, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, FfnNone{0}); break;
-    default:
-      if (h->ffn_impl == 2 && h->tc16_ok) {
-        fp.tc_blob = h->d_tc16_blob;
-        fused_kernel<2, 2><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias);
-      } else if (h->ffn_impl >= 1) {
-        fused_kernel<2, 1><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->bias);
-      } else {
-        fused_kernel<2, 0><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, h->par);
-      }
-      break;
-  }
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  const Classifier c = classifier_of(h);
+  if (p->mode == VADB200_MODE_VAD) fp.tc_blob = c.blob;
+  return launched(1, [&] {
+    if (p->mode == VADB200_MODE_MFCC) enqueue_fused<0, 0>(fe, grid, st, fp, FfnNone{0}, fea);
+    else if (p->mode == VADB200_MODE_DATASET) enqueue_fused<1, 0>(fe, grid, st, fp, FfnNone{0}, fea);
+    else if (c.tc == 2) enqueue_fused<2, 2>(fe, grid, st, fp, h->bias, fea);
+    else if (c.tc == 1) enqueue_fused<2, 1>(fe, grid, st, fp, h->bias, fea);
+    else enqueue_fused<2, 0>(fe, grid, st, fp, h->par, fea);
+  });
 }
 
 FusedParams base_params(vadb200_plan* p) {
   FusedParams fp;
   std::memset(&fp, 0, sizeof(fp));
-  fp.segs = p->d_segs;
-  fp.counter = p->d_counter;  // launch_fused picks the launch's own pair
-  fp.tw1 = p->h->d_tw;
-  fp.tw2 = p->h->d_tw + 256;
-  fp.tc_blob = p->h->d_tc_blob;
+  fp.segs = p->d_segs.get();
+  fp.counter = p->d_counter.get();  // launch_fused picks the launch's own pair
+  fp.tw1 = p->h->d_tw.get();
+  fp.tw2 = p->h->d_tw.get() + 256;
 #if defined(VADB_DEBUG_HOOKS)
   const char* dbg = std::getenv("VADB200_DEBUG_SKIP");  // timing experiments only; results are garbage
   fp.debug_skip = dbg ? std::atoi(dbg) : 0;
@@ -250,6 +282,17 @@ FusedParams base_params(vadb200_plan* p) {
   fp.dbg_ts = nullptr;
 #endif
   return fp;
+}
+
+// The classifier crosses the C ABI as eight arrays W1, b1, ..., W4, b4; the kNParams parameter vector, which is also
+// how FfnParams begins, holds them back to back from these offsets.
+constexpr int kParamOff[9] = {kOffW1, kOffB1, kOffW2, kOffB2, kOffW3, kOffB3, kOffW4, kOffB4, kNParams};
+static_assert(offsetof(FfnParams, thresh) == kNParams * sizeof(float), "FfnParams starts with the parameter vector");
+void pack_params(const float* const (&src)[8], float* v) {
+  for (int i = 0; i < 8; ++i) std::memcpy(v + kParamOff[i], src[i], (kParamOff[i + 1] - kParamOff[i]) * sizeof(float));
+}
+void unpack_params(const float* v, float* const (&dst)[8]) {
+  for (int i = 0; i < 8; ++i) std::memcpy(dst[i], v + kParamOff[i], (kParamOff[i + 1] - kParamOff[i]) * sizeof(float));
 }
 
 }  // namespace
@@ -292,12 +335,13 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   int ndev = 0;
   CU(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return fail(VADB200_E_INVALID, "no such CUDA device");
+  if (device >= 64) return fail(VADB200_E_INVALID, "device index >= 64");
   CU(cudaSetDevice(device));
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   if (prop.major < 10)
     return fail(VADB200_E_UNSUPPORTED, "kernels are built for sm_100a (B200) only");
-  vadb200_handle* h = new (std::nothrow) vadb200_handle();
+  std::unique_ptr<vadb200_handle> h(new (std::nothrow) vadb200_handle());
   if (!h) return fail(VADB200_E_NOMEM, "host allocation failed");
   h->device = device;
   h->id = g_next_id.fetch_add(1);
@@ -309,65 +353,51 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   std::memset(&h->bias, 0, sizeof(FfnBias));
   std::memset(&h->tab, 0, sizeof(MelDctTables));
   std::string why;
-  if (!pack_mel_weights(h->fb.data(), h->tab.melw, &why)) {
-    delete h;
-    return fail(VADB200_E_UNSUPPORTED, why);
-  }
+  if (!pack_mel_weights(h->fb.data(), h->tab.melw, &why)) return fail(VADB200_E_UNSUPPORTED, why);
   folded_dct(cfg, h->tab.dct);
   pack_mel_pairs(h->fb.data(), h->tab.melw2);
   pack_dct_pairs(h->tab.dct, h->tab.dctp);
   cf2 tw[384];
   fft_twiddles(tw, tw + 256);
-  cudaError_t e = cudaMalloc(&h->d_tw, sizeof(tw));
-  if (e == cudaSuccess) e = cudaMemcpy(h->d_tw, tw, sizeof(tw), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMalloc(&h->d_sink, 256);
-  if (e == cudaSuccess) e = cudaMalloc(&h->d_tc_blob, kTcBlobBytes);
-  if (e == cudaSuccess) e = cudaMalloc(&h->d_tc16_blob, kTc16BlobBytes);
-  if (e == cudaSuccess) e = cudaMalloc(&h->d_win, kWinPairs * sizeof(cf2));
-  if (e == cudaSuccess) {
-    std::vector<cf2> ones(kWinPairs, cf2{1.0f, 1.0f});
-    e = cudaMemcpy(h->d_win, ones.data(), kWinPairs * sizeof(cf2), cudaMemcpyHostToDevice);
-  }
-  if (e != cudaSuccess) {
-    cudaFree(h->d_tw);
-    cudaFree(h->d_sink);
-    cudaFree(h->d_tc_blob);
-    cudaFree(h->d_tc16_blob);
-    cudaFree(h->d_win);
-    delete h;
-    return cuda_fail(e, "vadb200_create");
-  }
+  CU(dev_upload(h->d_tw, tw, 384));
+  CU(dev_alloc(h->d_sink, 256));
+  CU(dev_alloc(h->d_tc_blob, kTcBlobBytes));
+  CU(dev_alloc(h->d_tc16_blob, kTc16BlobBytes));
+  const std::vector<cf2> ones(kWinPairs, cf2{1.0f, 1.0f});
+  CU(dev_upload(h->d_win, ones.data(), kWinPairs));
   // function attributes and the (config-invariant) constant tables now, so that no launch ever
   // synchronises: every device-pointer entry point can be captured into a CUDA graph
-  int rc = ensure_attrs(h);
-  if (!rc) rc = ensure_tables(h);
-  if (rc) {
-    const std::string keep = g_err;
-    vadb200_destroy(h);
-    g_err = keep;
-    return rc;
+  CU(cudaFuncSetAttribute(fused_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
+  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
+  CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
+  CU(cudaFuncSetAttribute(stream_feed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_feed_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
+  // Mel weights and the folded DCT matrix are the same for every handle (the kernels are compiled for the
+  // reference configuration only), so the __constant__ copy is written once per device and never changes:
+  // no handle can observe another handle's state through it.  FFN weights never go through device globals.
+  {
+    std::lock_guard<std::mutex> lk(g_tab_mu);
+    if (!g_tab_loaded[device]) {
+      CU(cudaMemcpyToSymbol(c_tab, &h->tab, sizeof(MelDctTables), 0, cudaMemcpyHostToDevice));
+      CU(cudaDeviceSynchronize());
+      g_tab_loaded[device] = true;
+    }
   }
-  *out = h;
+  *out = h.release();
   return 0;
 }
 
 int vadb200_destroy(vadb200_handle* h) {
-  if (!h) return 0;
-  cudaSetDevice(h->device);
-  for (int i = 0; i < kHostBufs; ++i) {
-    cudaFree(h->d_stage[i]); cudaFree(h->d_lab[i]); cudaFree(h->d_lgt[i]); cudaFree(h->d_rows[i]);
-    if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
-    if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]);
-    if (h->ev_out[i]) cudaEventDestroy(h->ev_out[i]);
-  }
-  if (h->s_in) cudaStreamDestroy(h->s_in);
-  if (h->s_run) cudaStreamDestroy(h->s_run);
-  if (h->s_out) cudaStreamDestroy(h->s_out);
-  cudaFree(h->d_tw);
-  cudaFree(h->d_sink);
-  cudaFree(h->d_tc_blob);
-  cudaFree(h->d_tc16_blob);
-  cudaFree(h->d_win);
   delete h;
   return 0;
 }
@@ -380,11 +410,11 @@ int vadb200_get_filterbank(vadb200_handle* h, double* out) {
 
 int vadb200_set_ffn_weights(vadb200_handle* h, const float* W1, const float* b1, const float* W2, const float* b2,
                             const float* W3, const float* b3, const float* W4, const float* b4) {
-  if (!h || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W4 || !b4) return fail(VADB200_E_INVALID, "null argument");
-  std::memcpy(h->par.W1, W1, sizeof(h->par.W1)); std::memcpy(h->par.b1, b1, sizeof(h->par.b1));
-  std::memcpy(h->par.W2, W2, sizeof(h->par.W2)); std::memcpy(h->par.b2, b2, sizeof(h->par.b2));
-  std::memcpy(h->par.W3, W3, sizeof(h->par.W3)); std::memcpy(h->par.b3, b3, sizeof(h->par.b3));
-  std::memcpy(h->par.W4, W4, sizeof(h->par.W4)); std::memcpy(h->par.b4, b4, sizeof(h->par.b4));
+  const float* src[8] = {W1, b1, W2, b2, W3, b3, W4, b4};
+  if (!h || std::count(src, src + 8, nullptr)) return fail(VADB200_E_INVALID, "null argument");
+  std::vector<float> v(kNParams);
+  pack_params(src, v.data());
+  std::memcpy(&h->par, v.data(), kNParams * sizeof(float));
   std::memcpy(h->bias.b1, b1, sizeof(h->bias.b1)); std::memcpy(h->bias.b2, b2, sizeof(h->bias.b2));
   std::memcpy(h->bias.b3, b3, sizeof(h->bias.b3)); std::memcpy(h->bias.b4, b4, sizeof(h->bias.b4));
   h->have_ffn = true;
@@ -394,10 +424,10 @@ int vadb200_set_ffn_weights(vadb200_handle* h, const float* W1, const float* b1,
   tc_pack_weights(h->par, blob.data());
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(h->d_tc_blob, blob.data(), kTcBlobBytes, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->d_tc_blob.get(), blob.data(), kTcBlobBytes, cudaMemcpyHostToDevice));
   std::vector<unsigned char> blob16(kTc16BlobBytes);
   h->tc16_ok = tc16_pack_weights(h->par, blob16.data(), h->bias);
-  if (h->tc16_ok) CU(cudaMemcpy(h->d_tc16_blob, blob16.data(), kTc16BlobBytes, cudaMemcpyHostToDevice));
+  if (h->tc16_ok) CU(cudaMemcpy(h->d_tc16_blob.get(), blob16.data(), kTc16BlobBytes, cudaMemcpyHostToDevice));
   return 0;
 }
 
@@ -421,7 +451,7 @@ int vadb200_set_frontend(vadb200_handle* h, float preemph, const float* h_window
   // drained + blocking, like the FFN weights: kernels on any stream see a consistent table
   CU(cudaSetDevice(h->device));
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(h->d_win, pairs.data(), kWinPairs * sizeof(cf2), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(h->d_win.get(), pairs.data(), kWinPairs * sizeof(cf2), cudaMemcpyHostToDevice));
   h->preemph = preemph;
   h->has_window = h_window != nullptr;
   if (h_window) std::memcpy(h->window, h_window, sizeof(h->window));
@@ -460,7 +490,7 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
   if (!h || !out || n_utt < 0 || (n_utt > 0 && (!offs || !lens))) return fail(VADB200_E_INVALID, "null / negative argument");
   if (mode < 0 || mode > 2) return fail(VADB200_E_INVALID, "unknown mode");
   *out = nullptr;
-  vadb200_plan* p = new (std::nothrow) vadb200_plan();
+  std::unique_ptr<vadb200_plan> p(new (std::nothrow) vadb200_plan());
   if (!p) return fail(VADB200_E_NOMEM, "host allocation failed");
   p->h = h; p->device = h->device; p->mode = mode; p->n_utt = n_utt;
   p->offsets.assign(offs, offs + n_utt);
@@ -469,10 +499,8 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
   p->utt_seg.resize(n_utt + 1);
   long long rows = 0, prev_end = 0;
   for (long long u = 0; u < n_utt; ++u) {
-    if (offs[u] < 0 || (offs[u] & 7) || lens[u] < 0 || offs[u] < prev_end) {
-      delete p;
+    if (offs[u] < 0 || (offs[u] & 7) || lens[u] < 0 || offs[u] < prev_end)
       return fail(VADB200_E_INVALID, "utterance offsets must be ascending, non-overlapping multiples of 8 samples");
-    }
     prev_end = offs[u] + lens[u];
     p->row_off[u] = rows;
     rows += (mode == VADB200_MODE_MFCC) ? frames_for_length(lens[u]) : outputs_for_length(lens[u]);
@@ -504,18 +532,7 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
     }
   }
   p->utt_seg[n_utt] = static_cast<long long>(p->segs.size());
-  if (p->segs.size() > 0x7fffffffull) {
-    delete p;
-    return fail(VADB200_E_INVALID, "too many segments");
-  }
-  cudaError_t e = cudaSetDevice(h->device);
-  if (e == cudaSuccess) e = cudaMalloc(&p->d_counter, 2 * kPlanCounters * sizeof(int));
-  if (e == cudaSuccess) e = cudaMemset(p->d_counter, 0, 2 * kPlanCounters * sizeof(int));
-  if (e == cudaSuccess && !p->segs.empty()) {
-    e = cudaMalloc(&p->d_segs, p->segs.size() * sizeof(Segment));
-    if (e == cudaSuccess)
-      e = cudaMemcpy(p->d_segs, p->segs.data(), p->segs.size() * sizeof(Segment), cudaMemcpyHostToDevice);
-  }
+  if (p->segs.size() > 0x7fffffffull) return fail(VADB200_E_INVALID, "too many segments");
   if (mode != VADB200_MODE_MFCC) {
     p->utt_tile.resize(n_utt + 1);
     for (long long u = 0; u < n_utt; ++u) {
@@ -527,42 +544,22 @@ int vadb200_plan_create(vadb200_handle* h, const int64_t* offs, const int64_t* l
                                       static_cast<int>(u)});
     }
     p->utt_tile[n_utt] = static_cast<int>(p->tiles.size());
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_row_off, (n_utt + 1) * sizeof(long long));
-    if (e == cudaSuccess)
-      e = cudaMemcpy(p->d_row_off, p->row_off.data(), (n_utt + 1) * sizeof(long long), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_utt_tile, (n_utt + 1) * sizeof(int));
-    if (e == cudaSuccess)
-      e = cudaMemcpy(p->d_utt_tile, p->utt_tile.data(), (n_utt + 1) * sizeof(int), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && n_utt > 0) {
-      e = cudaMalloc(&p->d_pcm_off, n_utt * sizeof(long long));
-      if (e == cudaSuccess)
-        e = cudaMemcpy(p->d_pcm_off, p->offsets.data(), n_utt * sizeof(long long), cudaMemcpyHostToDevice);
-    }
-    if (e == cudaSuccess && !p->tiles.empty()) {
-      e = cudaMalloc(&p->d_tiles, p->tiles.size() * sizeof(SpeechTile));
-      if (e == cudaSuccess)
-        e = cudaMemcpy(p->d_tiles, p->tiles.data(), p->tiles.size() * sizeof(SpeechTile), cudaMemcpyHostToDevice);
-    }
   }
-  if (e != cudaSuccess) {
-    cudaFree(p->d_counter); cudaFree(p->d_segs);
-    cudaFree(p->d_row_off); cudaFree(p->d_pcm_off); cudaFree(p->d_tiles); cudaFree(p->d_utt_tile);
-    delete p;
-    return cuda_fail(e, "vadb200_plan_create");
+  CU(cudaSetDevice(h->device));
+  CU(dev_alloc(p->d_counter, 2 * kPlanCounters * sizeof(int)));
+  CU(cudaMemset(p->d_counter.get(), 0, 2 * kPlanCounters * sizeof(int)));
+  if (!p->segs.empty()) CU(dev_upload(p->d_segs, p->segs.data(), p->segs.size()));
+  if (mode != VADB200_MODE_MFCC) {
+    CU(dev_upload(p->d_row_off, p->row_off.data(), n_utt + 1));
+    CU(dev_upload(p->d_utt_tile, p->utt_tile.data(), n_utt + 1));
+    if (n_utt > 0) CU(dev_upload(p->d_pcm_off, p->offsets.data(), n_utt));
+    if (!p->tiles.empty()) CU(dev_upload(p->d_tiles, p->tiles.data(), p->tiles.size()));
   }
-  *out = p;
+  *out = p.release();
   return 0;
 }
 
 int vadb200_plan_destroy(vadb200_plan* p) {
-  if (!p) return 0;
-  cudaSetDevice(p->device);
-  cudaFree(p->d_segs);
-  cudaFree(p->d_counter);
-  cudaFree(p->d_row_off);
-  cudaFree(p->d_pcm_off);
-  cudaFree(p->d_tiles);
-  cudaFree(p->d_utt_tile);
   delete p;
   return 0;
 }
@@ -624,45 +621,17 @@ int vadb200_vad_packed(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len, u
 // ---- host-buffer pipeline ---------------------------------------------------------------------------------
 static int ensure_host_pipeline(vadb200_handle* h, long long stage_samples, long long rows, bool want_labels,
                                 bool want_logits, long long row_floats) {
-  if (!h->s_in) {
-    CU(cudaStreamCreateWithFlags(&h->s_in, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&h->s_run, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&h->s_out, cudaStreamNonBlocking));
-    for (int i = 0; i < kHostBufs; ++i) {
-      CU(cudaEventCreateWithFlags(&h->ev_in[i], cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&h->ev_done[i], cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&h->ev_out[i], cudaEventDisableTiming));
-    }
+  if (!h->pipe_ready) {
+    for (Stream* s : {&h->s_in, &h->s_run, &h->s_out}) CU(make_stream(*s));
+    for (HostBuf& s : h->hb)
+      for (Event* ev : {&s.in, &s.done, &s.out}) CU(make_event(*ev, cudaEventDisableTiming));
+    h->pipe_ready = true;
   }
-  if (stage_samples > h->stage_cap) {
-    for (int i = 0; i < kHostBufs; ++i) {
-      cudaFree(h->d_stage[i]); h->d_stage[i] = nullptr;
-      CU(cudaMalloc(&h->d_stage[i], stage_samples * sizeof(int16_t)));
-    }
-    h->stage_cap = stage_samples;
-  }
-  if (want_labels && rows > h->lab_cap) {
-    for (int i = 0; i < kHostBufs; ++i) {
-      cudaFree(h->d_lab[i]); h->d_lab[i] = nullptr;
-      CU(cudaMalloc(&h->d_lab[i], rows));
-    }
-    h->lab_cap = rows;
-  }
-  if (want_logits && rows > h->lgt_cap) {
-    for (int i = 0; i < kHostBufs; ++i) {
-      cudaFree(h->d_lgt[i]); h->d_lgt[i] = nullptr;
-      CU(cudaMalloc(&h->d_lgt[i], rows * 3 * sizeof(float)));
-    }
-    h->lgt_cap = rows;
-  }
-  if (row_floats > h->rows_cap) {
-    for (int i = 0; i < kHostBufs; ++i) {
-      cudaFree(h->d_rows[i]); h->d_rows[i] = nullptr;
-      CU(cudaMalloc(&h->d_rows[i], row_floats * sizeof(float)));
-    }
-    h->rows_cap = row_floats;
-  }
-  return 0;
+  int rc = grow(h->hb, &HostBuf::stage, h->stage_cap, stage_samples);
+  if (!rc && want_labels) rc = grow(h->hb, &HostBuf::labels, h->lab_cap, rows);
+  if (!rc && want_logits) rc = grow(h->hb, &HostBuf::logits, h->lgt_cap, rows * 3);
+  if (!rc) rc = grow(h->hb, &HostBuf::rows, h->rows_cap, row_floats);
+  return rc;
 }
 
 // Chunked H2D -> fused kernel -> D2H over three staging buffers and three streams.  VAD plans return
@@ -692,42 +661,44 @@ static int run_host_pipeline(vadb200_plan* p, const int16_t* h_pcm, int64_t pcm_
   int rc = ensure_host_pipeline(h, ((max_span + 7) & ~7ll) + 8, max_rows, h_labels != nullptr, h_logits != nullptr,
                                 width * max_rows);
   if (rc) return rc;
+  cudaStream_t s_in = h->s_in.get(), s_run = h->s_run.get(), s_out = h->s_out.get();
   for (size_t i = 0; i < chunks.size(); ++i) {
     const Chunk& c = chunks[i];
-    const int b = static_cast<int>(i % kHostBufs);
+    const HostBuf& slot = h->hb[i % kHostBufs];
     const long long span = c.s1 - c.s0;
     const long long r0 = p->row_off[c.u0], nrows = p->row_off[c.u1] - r0;
-    if (i >= kHostBufs) CU(cudaStreamWaitEvent(h->s_in, h->ev_done[b], 0));  // stage buffer free again
-    CU(cudaMemcpyAsync(h->d_stage[b], h_pcm + c.s0, span * sizeof(int16_t), cudaMemcpyHostToDevice, h->s_in));
-    CU(cudaEventRecord(h->ev_in[b], h->s_in));
-    CU(cudaStreamWaitEvent(h->s_run, h->ev_in[b], 0));
-    if (i >= kHostBufs) CU(cudaStreamWaitEvent(h->s_run, h->ev_out[b], 0));  // result buffers drained
+    if (i >= kHostBufs) CU(cudaStreamWaitEvent(s_in, slot.done.get(), 0));  // stage buffer free again
+    CU(cudaMemcpyAsync(slot.stage.get(), h_pcm + c.s0, span * sizeof(int16_t), cudaMemcpyHostToDevice, s_in));
+    CU(cudaEventRecord(slot.in.get(), s_in));
+    CU(cudaStreamWaitEvent(s_run, slot.in.get(), 0));
+    if (i >= kHostBufs) CU(cudaStreamWaitEvent(s_run, slot.out.get(), 0));  // result buffers drained
     FusedParams fp = base_params(p);
-    fp.pcm = h->d_stage[b] - c.s0;  // segment sample indices stay absolute
+    fp.pcm = slot.stage.get() - c.s0;  // segment sample indices stay absolute
     fp.pcm_len = c.s1;
-    fp.labels = h_labels ? h->d_lab[b] : nullptr;
-    fp.logits = h_logits ? h->d_lgt[b] : nullptr;
-    fp.rows = width ? h->d_rows[b] : nullptr;
+    fp.labels = h_labels ? slot.labels.get() : nullptr;
+    fp.logits = h_logits ? slot.logits.get() : nullptr;
+    fp.rows = width ? slot.rows.get() : nullptr;
     fp.row_base = r0;
     fp.feat_mode = feat_mode;
     fp.seg_begin = static_cast<int>(p->utt_seg[c.u0]);
     fp.seg_end = static_cast<int>(p->utt_seg[c.u1]);
-    rc = launch_fused(p, fp, fp.seg_end - fp.seg_begin, h->s_run);
+    rc = launch_fused(p, fp, fp.seg_end - fp.seg_begin, s_run);
     if (rc) return rc;
-    CU(cudaEventRecord(h->ev_done[b], h->s_run));
-    CU(cudaStreamWaitEvent(h->s_out, h->ev_done[b], 0));
+    CU(cudaEventRecord(slot.done.get(), s_run));
+    CU(cudaStreamWaitEvent(s_out, slot.done.get(), 0));
     if (nrows > 0) {
-      if (h_labels) CU(cudaMemcpyAsync(h_labels + r0, h->d_lab[b], nrows, cudaMemcpyDeviceToHost, h->s_out));
+      if (h_labels) CU(cudaMemcpyAsync(h_labels + r0, slot.labels.get(), nrows, cudaMemcpyDeviceToHost, s_out));
       if (h_logits)
-        CU(cudaMemcpyAsync(h_logits + r0 * 3, h->d_lgt[b], nrows * 3 * sizeof(float), cudaMemcpyDeviceToHost, h->s_out));
+        CU(cudaMemcpyAsync(h_logits + r0 * 3, slot.logits.get(), nrows * 3 * sizeof(float), cudaMemcpyDeviceToHost,
+                           s_out));
       if (width)
-        CU(cudaMemcpyAsync(h_rows + r0 * width, h->d_rows[b], nrows * width * sizeof(float), cudaMemcpyDeviceToHost,
-                           h->s_out));
+        CU(cudaMemcpyAsync(h_rows + r0 * width, slot.rows.get(), nrows * width * sizeof(float), cudaMemcpyDeviceToHost,
+                           s_out));
     }
-    CU(cudaEventRecord(h->ev_out[b], h->s_out));
+    CU(cudaEventRecord(slot.out.get(), s_out));
   }
-  CU(cudaStreamSynchronize(h->s_out));
-  CU(cudaStreamSynchronize(h->s_run));
+  CU(cudaStreamSynchronize(s_out));
+  CU(cudaStreamSynchronize(s_run));
   return 0;
 }
 
@@ -757,19 +728,19 @@ int vadb200_scale_rows(vadb200_handle* h, float* d_rows, int64_t n_rows, double*
   if (!d_rows) return fail(VADB200_E_INVALID, "d_rows is null");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  double* acc = nullptr;
-  CU(cudaMallocAsync(&acc, 6 * sizeof(double), st));  // stream-ordered scratch: no per-handle state
-  CU(cudaMemsetAsync(acc, 0, 6 * sizeof(double), st));
+  double* scratch = nullptr;
+  CU(cudaMallocAsync(&scratch, 6 * sizeof(double), st));  // stream-ordered scratch: no per-handle state
+  const std::unique_ptr<double, CudaFreeAsync> acc(scratch, CudaFreeAsync{st});
+  CU(cudaMemsetAsync(acc.get(), 0, 6 * sizeof(double), st));
   const long long total = n_rows * kNFeat;
   const int grid = static_cast<int>(std::min<long long>((total + 255) / 256, 8ll * h->num_sms));
-  for (int pass = 0; pass < 3; ++pass) {
-    scale_rows_kernel<<<grid, 256, 0, st>>>(d_rows, n_rows, pass, acc);
-    g_launches.fetch_add(1);
-  }
-  CU(cudaGetLastError());
+  const int rc = launched(3, [&] {
+    for (int pass = 0; pass < 3; ++pass) scale_rows_kernel<<<grid, 256, 0, st>>>(d_rows, n_rows, pass, acc.get());
+  });
+  if (rc) return rc;
   if (h_stats) {
     double raw[6];
-    CU(cudaMemcpyAsync(raw, acc, sizeof(raw), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(raw, acc.get(), sizeof(raw), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     const double cnt = static_cast<double>(n_rows) * kNCep;
     for (int g = 0; g < 3; ++g) {
@@ -777,7 +748,6 @@ int vadb200_scale_rows(vadb200_handle* h, float* d_rows, int64_t n_rows, double*
       h_stats[3 + g] = std::sqrt(raw[3 + g] / cnt);
     }
   }
-  CU(cudaFreeAsync(acc, st));
   return 0;
 }
 
@@ -792,12 +762,11 @@ int vadb200_ingest_pcm(vadb200_handle* h, const void* d_raw, int big_endian, con
   CU(cudaSetDevice(h->device));
   const unsigned gx = static_cast<unsigned>(std::min<long long>((max_len + 255) / 256, 4ll * h->num_sms));
   static_assert(sizeof(long long) == sizeof(int64_t), "int64_t layout");
-  ingest_kernel<<<dim3(gx, static_cast<unsigned>(n_seg)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const uint8_t*>(d_raw), big_endian, reinterpret_cast<const long long*>(d_src_start),
-      reinterpret_cast<const long long*>(d_dst_start), reinterpret_cast<const long long*>(d_len), d_dst);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    ingest_kernel<<<dim3(gx, static_cast<unsigned>(n_seg)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const uint8_t*>(d_raw), big_endian, reinterpret_cast<const long long*>(d_src_start),
+        reinterpret_cast<const long long*>(d_dst_start), reinterpret_cast<const long long*>(d_len), d_dst);
+  });
 }
 
 // ---- per-frame API ---------------------------------------------------------------------------------------
@@ -809,17 +778,13 @@ static int frames_common(vadb200_handle* h, const float* d_frames, int64_t n, in
   if (n == 0) return 0;
   if (!d_frames || !d_out) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
-  int rc = ensure_attrs(h);
-  if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_tables(h);
-  if (rc) return rc;
   const unsigned grid = static_cast<unsigned>((n + kStepFrames - 1) / kStepFrames);
   const FrontEnd fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
-  frames_kernel<<<grid, kThreads, kFramesSmemBytes, st>>>(d_frames, n, frame_len, what, d_out, h->d_tw, h->d_tw + 256, fe);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  const cf2* tw = h->d_tw.get();
+  return launched(1, [&] {
+    frames_kernel<<<grid, kThreads, kFramesSmemBytes, st>>>(d_frames, n, frame_len, what, d_out, tw, tw + 256, fe);
+  });
 }
 
 int vadb200_spec_frames(vadb200_handle* h, const float* d_frames, int64_t n, int frame_len, float* d_spec, void* stream) {
@@ -836,13 +801,8 @@ int vadb200_mfcc_from_spec(vadb200_handle* h, const float* d_spec, int64_t n, fl
   if (!d_spec || !d_mfcc) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int rc = ensure_tables(h);
-  if (rc) return rc;
   const unsigned grid = static_cast<unsigned>((n + kStepFrames - 1) / kStepFrames);
-  spec_to_mfcc_kernel<<<grid, kThreads, 0, st>>>(d_spec, n, d_mfcc);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] { spec_to_mfcc_kernel<<<grid, kThreads, 0, st>>>(d_spec, n, d_mfcc); });
 }
 
 int vadb200_vad_windows(vadb200_handle* h, const float* d_win, int64_t n, int feat_mode, uint8_t* d_labels,
@@ -854,13 +814,10 @@ int vadb200_vad_windows(vadb200_handle* h, const float* d_win, int64_t n, int fe
   if (!d_win) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int rc = ensure_tables(h);
-  if (rc) return rc;
-  windows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels, d_logits, d_feats,
-                                                                       h->par);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    windows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels, d_logits,
+                                                                         d_feats, h->par);
+  });
 }
 
 int vadb200_ffn_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t* d_labels, float* d_logits, void* stream) {
@@ -871,20 +828,18 @@ int vadb200_ffn_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t*
   if (!d_x) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  int rc = ensure_tables(h);
-  if (rc) return rc;
-  if (h->ffn_impl >= 2 && h->tc16_ok) {
-    ffn_tc_rows_kernel<2><<<static_cast<unsigned>((n + 127) / 128), 128, kFfnTcSmemBytes, st>>>(
-        d_x, n, h->d_tc16_blob, h->d_tc_blob, d_labels, d_logits, h->bias);
-  } else if (h->ffn_impl >= 1) {
-    ffn_tc_rows_kernel<1><<<static_cast<unsigned>((n + 127) / 128), 128, kFfnTcSmemBytes, st>>>(
-        d_x, n, nullptr, h->d_tc_blob, d_labels, d_logits, h->bias);
-  } else {
-    ffn_rows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_x, n, d_labels, d_logits, h->par);
-  }
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  const unsigned grid = static_cast<unsigned>((n + 127) / 128);
+  const Classifier c = classifier_of(h);
+  return launched(1, [&] {
+    // a fp16 tile holding a row past the feature bounds runs on the tf32 blob
+    if (c.tc == 2)
+      ffn_tc_rows_kernel<2><<<grid, 128, kFfnTcSmemBytes, st>>>(d_x, n, c.blob, h->d_tc_blob.get(), d_labels, d_logits,
+                                                               h->bias);
+    else if (c.tc == 1)
+      ffn_tc_rows_kernel<1><<<grid, 128, kFfnTcSmemBytes, st>>>(d_x, n, nullptr, c.blob, d_labels, d_logits, h->bias);
+    else
+      ffn_rows_kernel<<<grid, 128, 0, st>>>(d_x, n, d_labels, d_logits, h->par);
+  });
 }
 
 int vadb200_get_deltas(vadb200_handle* h, const float* d_a, const float* d_b, int64_t n, float* d_out, void* stream) {
@@ -892,10 +847,10 @@ int vadb200_get_deltas(vadb200_handle* h, const float* d_a, const float* d_b, in
   if (n == 0) return 0;
   if (!d_a || !d_b || !d_out) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
-  elementwise_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(0, d_a, d_b, n, 1, 0, d_out);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    elementwise_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        0, d_a, d_b, n, 1, 0, d_out);
+  });
 }
 
 int vadb200_lifter(vadb200_handle* h, const float* d_in, int64_t n_rows, int ncoef, int L, float* d_out, void* stream) {
@@ -904,10 +859,10 @@ int vadb200_lifter(vadb200_handle* h, const float* d_in, int64_t n_rows, int nco
   if (!d_in || !d_out) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   const long long n = n_rows * ncoef;
-  elementwise_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(1, d_in, nullptr, n, ncoef, L, d_out);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    elementwise_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        1, d_in, nullptr, n, ncoef, L, d_out);
+  });
 }
 
 // ---- streaming -------------------------------------------------------------------------------------------
@@ -915,29 +870,21 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
   if (!h || !out || n_streams < 1) return fail(VADB200_E_INVALID, "bad argument");
   *out = nullptr;
   CU(cudaSetDevice(h->device));
-  vadb200_bank* b = new (std::nothrow) vadb200_bank();
+  std::unique_ptr<vadb200_bank> b(new (std::nothrow) vadb200_bank());
   if (!b) return fail(VADB200_E_NOMEM, "host allocation failed");
   b->h = h; b->device = h->device; b->n = n_streams;
-  cudaError_t e = cudaMalloc(&b->d_hist, static_cast<size_t>(n_streams) * 320 * sizeof(int16_t));
-  if (e == cudaSuccess) e = cudaMalloc(&b->d_ring, static_cast<size_t>(n_streams) * 5 * kNCep * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(&b->d_fed, static_cast<size_t>(n_streams) * sizeof(int));
-  if (e == cudaSuccess) e = cudaMalloc(&b->d_prev, static_cast<size_t>(n_streams) * sizeof(int16_t));
-  if (e != cudaSuccess) {
-    cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev);
-    delete b;
-    return cuda_fail(e, "vadb200_stream_bank_create");
-  }
-  *out = b;
-  int rc = vadb200_stream_bank_reset(b, nullptr);
+  CU(dev_alloc(b->d_hist, static_cast<size_t>(n_streams) * 320 * sizeof(int16_t)));
+  CU(dev_alloc(b->d_ring, static_cast<size_t>(n_streams) * 5 * kNCep * sizeof(float)));
+  CU(dev_alloc(b->d_fed, static_cast<size_t>(n_streams) * sizeof(int)));
+  CU(dev_alloc(b->d_prev, static_cast<size_t>(n_streams) * sizeof(int16_t)));
+  const int rc = vadb200_stream_bank_reset(b.get(), nullptr);
   if (rc) return rc;
   CU(cudaDeviceSynchronize());  // state is zero before any stream can feed
+  *out = b.release();
   return 0;
 }
 
 int vadb200_stream_bank_destroy(vadb200_bank* b) {
-  if (!b) return 0;
-  cudaSetDevice(b->device);
-  cudaFree(b->d_hist); cudaFree(b->d_ring); cudaFree(b->d_fed); cudaFree(b->d_prev); cudaFree(b->d_seg);
   delete b;
   return 0;
 }
@@ -953,9 +900,9 @@ StreamSeg bank_seg(const vadb200_bank* b, uint8_t* d_rows, int64_t* d_bounds) {
   g.d1 = sp.G > 1 ? sp.G - 1 : 0;
   g.d2 = sp.S > 1 ? sp.S - 1 : 0;
   const long long w1 = g.d1 ? seg_ring_words(g.d1) : 0, w2 = g.d2 ? seg_ring_words(g.d2) : 0;
-  g.ring1 = b->d_seg;
-  g.ring2 = b->d_seg + w1 * b->n;
-  g.meta = b->d_seg + (w1 + w2) * b->n;
+  g.ring1 = b->d_seg.get();
+  g.ring2 = b->d_seg.get() + w1 * b->n;
+  g.meta = b->d_seg.get() + (w1 + w2) * b->n;
   g.last = reinterpret_cast<int*>(g.meta + b->n);
   g.rows = d_rows;
   g.bounds = d_bounds;
@@ -969,25 +916,21 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
   if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
   if (reinterpret_cast<uintptr_t>(d_chunks) & 3) return fail(VADB200_E_INVALID, "chunks must be 4-byte aligned");
   CU(cudaSetDevice(h->device));
-  int rc = ensure_attrs(h);
-  if (rc) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  rc = ensure_tables(h);
-  if (rc) return rc;
   BankParams bp;
-  bp.n_streams = b->n; bp.hist = b->d_hist; bp.ring = b->d_ring; bp.fed = b->d_fed;
+  bp.n_streams = b->n; bp.hist = b->d_hist.get(); bp.ring = b->d_ring.get(); bp.fed = b->d_fed.get();
   bp.chunks = d_chunks; bp.labels = d_labels; bp.logits = d_logits;
-  bp.tw1 = h->d_tw; bp.tw2 = h->d_tw + 256; bp.feat_mode = VADB200_FEAT_ANALYSER;
-  bp.prev = b->d_prev;
+  bp.tw1 = h->d_tw.get(); bp.tw2 = h->d_tw.get() + 256; bp.feat_mode = VADB200_FEAT_ANALYSER;
+  bp.prev = b->d_prev.get();
   bp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
-  if (b->d_seg)  // speech on: every feed advances the segment state
-    stream_feed_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par, bank_seg(b, d_rows, d_bounds));
-  else
-    stream_feed_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    if (b->d_seg)  // speech on: every feed advances the segment state
+      stream_feed_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par,
+                                                                                    bank_seg(b, d_rows, d_bounds));
+    else
+      stream_feed_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
+  });
 }
 
 }  // namespace
@@ -996,11 +939,11 @@ int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
   if (!b) return fail(VADB200_E_INVALID, "bank is null");
   CU(cudaSetDevice(b->h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CU(cudaMemsetAsync(b->d_hist, 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
-  CU(cudaMemsetAsync(b->d_ring, 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
-  CU(cudaMemsetAsync(b->d_fed, 0, static_cast<size_t>(b->n) * sizeof(int), st));
-  CU(cudaMemsetAsync(b->d_prev, 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
-  if (b->d_seg) CU(cudaMemsetAsync(b->d_seg, 0, b->seg_bytes, st));
+  CU(cudaMemsetAsync(b->d_hist.get(), 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
+  CU(cudaMemsetAsync(b->d_ring.get(), 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
+  CU(cudaMemsetAsync(b->d_fed.get(), 0, static_cast<size_t>(b->n) * sizeof(int), st));
+  CU(cudaMemsetAsync(b->d_prev.get(), 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
+  if (b->d_seg) CU(cudaMemsetAsync(b->d_seg.get(), 0, b->seg_bytes, st));
   return 0;
 }
 
@@ -1016,18 +959,13 @@ int vadb200_stream_bank_set_speech(vadb200_bank* b, int enable, int min_speech_r
       if (v < 0 || v > kSpeechMaxParam) return fail(VADB200_E_INVALID, "speech parameters must lie in [0, 1000] rows");
   }
   CU(cudaSetDevice(b->h->device));
-  CU(cudaFree(b->d_seg));  // waits for work in flight that may still use it
-  b->d_seg = nullptr;
+  CU(cudaFree(b->d_seg.release()));  // waits for work in flight that may still use it; reports its failure
   b->seg_bytes = 0;
   if (enable) {
     const SmoothParams sp = smooth_params(min_speech_rows, min_silence_rows, pad_rows);
     const int w1 = sp.G > 1 ? seg_ring_words(sp.G - 1) : 0, w2 = sp.S > 1 ? seg_ring_words(sp.S - 1) : 0;
     const size_t bytes = static_cast<size_t>(w1 + w2 + 2) * b->n * sizeof(uint32_t);
-    cudaError_t e = cudaMalloc(&b->d_seg, bytes);
-    if (e != cudaSuccess) {
-      b->d_seg = nullptr;
-      return cuda_fail(e, "vadb200_stream_bank_set_speech");
-    }
+    CU(dev_alloc(b->d_seg, bytes));
     b->sp = sp;
     b->seg_bytes = bytes;
   }
@@ -1049,13 +987,14 @@ int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end, uint8
   CU(cudaSetDevice(b->h->device));
   const StreamSeg g = bank_seg(b, nullptr, nullptr);
   const int words = g.meta ? (g.d1 ? seg_ring_words(g.d1) : 0) + (g.d2 ? seg_ring_words(g.d2) : 0) : 0;
-  stream_end_kernel<<<(b->n + kSegEndThreads - 1) / kSegEndThreads, kSegEndThreads,
-                      static_cast<size_t>(words) * kSegEndThreads * sizeof(uint32_t), static_cast<cudaStream_t>(stream)>>>(
-      g, d_end, b->n, b->d_hist, b->d_ring, b->d_fed, b->d_prev, g.meta ? d_tail_rows : nullptr,
-      g.meta ? d_tail_bounds : nullptr);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  const size_t smem = static_cast<size_t>(words) * kSegEndThreads * sizeof(uint32_t);
+  return launched(1, [&] {
+    stream_end_kernel<<<(b->n + kSegEndThreads - 1) / kSegEndThreads, kSegEndThreads, smem,
+                        static_cast<cudaStream_t>(stream)>>>(g, d_end, b->n, b->d_hist.get(), b->d_ring.get(),
+                                                             b->d_fed.get(), b->d_prev.get(),
+                                                             g.meta ? d_tail_rows : nullptr,
+                                                             g.meta ? d_tail_bounds : nullptr);
+  });
 }
 
 #if defined(VADB_DEBUG_HOOKS)
@@ -1066,17 +1005,16 @@ int vadb200_exp_fft(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len, int 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   FusedParams fp = base_params(p);
   fp.pcm = d_pcm; fp.pcm_len = pcm_len; fp.seg_begin = 0; fp.seg_end = static_cast<int>(p->segs.size());
-  fp.counter = p->d_counter + 2 * (p->launch_seq.fetch_add(1) % kPlanCounters);
+  fp.counter = p->d_counter.get() + 2 * (p->launch_seq.fetch_add(1) % kPlanCounters);
   const int grid = std::min<int>(fp.seg_end, minb * h->num_sms);
-#define VADB_EXP(M)                                                                                          \
-  {                                                                                                          \
-    CU(cudaFuncSetAttribute(exp_fft_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, kExpSmemBytes)); \
-    exp_fft_kernel<M><<<grid, kThreads, kExpSmemBytes, st>>>(fp, h->d_sink);                                 \
-  }
-  if (minb == 1) VADB_EXP(1) else if (minb == 2) VADB_EXP(2) else if (minb == 3) VADB_EXP(3) else VADB_EXP(4)
-#undef VADB_EXP
-  CU(cudaGetLastError());
-  return 0;
+  const auto run = [&](auto kernel) {
+    CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kExpSmemBytes));
+    return launched(0, [&] { kernel<<<grid, kThreads, kExpSmemBytes, st>>>(fp, h->d_sink.get()); });
+  };
+  if (minb == 1) return run(exp_fft_kernel<1>);
+  if (minb == 2) return run(exp_fft_kernel<2>);
+  if (minb == 3) return run(exp_fft_kernel<3>);
+  return run(exp_fft_kernel<4>);
 }
 #endif
 
@@ -1085,61 +1023,48 @@ int vadb200_trainer_create(vadb200_handle* h, int64_t max_batch, float lr, float
   if (!h || !out || max_batch < 1) return fail(VADB200_E_INVALID, "bad argument");
   *out = nullptr;
   CU(cudaSetDevice(h->device));
-  vadb200_trainer* t = new (std::nothrow) vadb200_trainer();
+  std::unique_ptr<vadb200_trainer> t(new (std::nothrow) vadb200_trainer());
   if (!t) return fail(VADB200_E_NOMEM, "host allocation failed");
   t->h = h; t->device = h->device; t->max_batch = max_batch; t->lr = lr; t->rho = rho; t->eps = eps;
   const long long n_part = (max_batch + kTrainRows - 1) / kTrainRows;
-  cudaError_t e = cudaMalloc(&t->d_state, 3 * kNParams * sizeof(float));
-  if (e == cudaSuccess) e = cudaMemset(t->d_state, 0, 3 * kNParams * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(&t->d_partial, n_part * (kNParams + 1) * sizeof(float));
-  if (e == cudaSuccess) e = cudaMalloc(&t->d_loss, sizeof(float));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(ffn_train_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTrain2SmemBytes);
-  if (e != cudaSuccess) {
-    cudaFree(t->d_state); cudaFree(t->d_partial); cudaFree(t->d_loss);
-    delete t;
-    return cuda_fail(e, "vadb200_trainer_create");
-  }
-  if (h->have_ffn) {  // start from the handle's classifier
-    static_assert(sizeof(FfnParams) >= kNParams * sizeof(float), "FfnParams is the parameter vector");
-    CU(cudaMemcpy(t->d_state, &h->par, kNParams * sizeof(float), cudaMemcpyHostToDevice));
-  }
-  *out = t;
+  CU(dev_alloc(t->d_state, 3 * kNParams * sizeof(float)));
+  CU(cudaMemset(t->d_state.get(), 0, 3 * kNParams * sizeof(float)));
+  CU(dev_alloc(t->d_partial, n_part * (kNParams + 1) * sizeof(float)));
+  CU(dev_alloc(t->d_loss, sizeof(float)));
+  CU(cudaFuncSetAttribute(ffn_train_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTrain2SmemBytes));
+  if (h->have_ffn)  // start from the handle's classifier
+    CU(cudaMemcpy(t->d_state.get(), &h->par, kNParams * sizeof(float), cudaMemcpyHostToDevice));
+  *out = t.release();
   return 0;
 }
 
 int vadb200_trainer_destroy(vadb200_trainer* t) {
-  if (!t) return 0;
-  cudaSetDevice(t->device);
-  cudaFree(t->d_state); cudaFree(t->d_partial); cudaFree(t->d_loss);
   delete t;
   return 0;
 }
 
 int vadb200_trainer_set_weights(vadb200_trainer* t, const float* W1, const float* b1, const float* W2, const float* b2,
                                 const float* W3, const float* b3, const float* W4, const float* b4, int reset_optimizer) {
-  if (!t || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W4 || !b4) return fail(VADB200_E_INVALID, "null argument");
-  std::vector<float> v(kNParams);
   const float* src[8] = {W1, b1, W2, b2, W3, b3, W4, b4};
-  const int off[9] = {kOffW1, kOffB1, kOffW2, kOffB2, kOffW3, kOffB3, kOffW4, kOffB4, kNParams};
-  for (int i = 0; i < 8; ++i) std::memcpy(v.data() + off[i], src[i], (off[i + 1] - off[i]) * sizeof(float));
+  if (!t || std::count(src, src + 8, nullptr)) return fail(VADB200_E_INVALID, "null argument");
+  std::vector<float> v(kNParams);
+  pack_params(src, v.data());
   CU(cudaSetDevice(t->h->device));
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(t->d_state, v.data(), kNParams * sizeof(float), cudaMemcpyHostToDevice));
-  if (reset_optimizer) CU(cudaMemset(t->d_state + kNParams, 0, 2 * kNParams * sizeof(float)));
+  CU(cudaMemcpy(t->d_state.get(), v.data(), kNParams * sizeof(float), cudaMemcpyHostToDevice));
+  if (reset_optimizer) CU(cudaMemset(t->d_state.get() + kNParams, 0, 2 * kNParams * sizeof(float)));
   return 0;
 }
 
 int vadb200_trainer_get_weights(vadb200_trainer* t, float* W1, float* b1, float* W2, float* b2, float* W3, float* b3,
                                 float* W4, float* b4) {
-  if (!t || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W4 || !b4) return fail(VADB200_E_INVALID, "null argument");
+  float* dst[8] = {W1, b1, W2, b2, W3, b3, W4, b4};
+  if (!t || std::count(dst, dst + 8, nullptr)) return fail(VADB200_E_INVALID, "null argument");
   std::vector<float> v(kNParams);
   CU(cudaSetDevice(t->h->device));
   CU(cudaDeviceSynchronize());
-  CU(cudaMemcpy(v.data(), t->d_state, kNParams * sizeof(float), cudaMemcpyDeviceToHost));
-  float* dst[8] = {W1, b1, W2, b2, W3, b3, W4, b4};
-  const int off[9] = {kOffW1, kOffB1, kOffW2, kOffB2, kOffW3, kOffB3, kOffW4, kOffB4, kNParams};
-  for (int i = 0; i < 8; ++i) std::memcpy(dst[i], v.data() + off[i], (off[i + 1] - off[i]) * sizeof(float));
+  CU(cudaMemcpy(v.data(), t->d_state.get(), kNParams * sizeof(float), cudaMemcpyDeviceToHost));
+  unpack_params(v.data(), dst);
   return 0;
 }
 
@@ -1151,17 +1076,18 @@ int vadb200_train_on_batch(vadb200_trainer* t, const float* d_x, const uint8_t* 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n_tiles = static_cast<int>((n + kTrainRows - 1) / kTrainRows);
   const int n_part = std::min(n_tiles, t->h->num_sms);   // persistent CTAs: one partial gradient each
-  cudaGetLastError();   // the check below is for these launches, not a non-sticky error an earlier call left behind
-  ffn_train_grad_kernel<<<n_part, kTr2Threads, kTrain2SmemBytes, st>>>(t->d_state, d_x, d_y, n,
-                                                                         1.0f / static_cast<float>(n), t->d_partial);
-  ffn_train_update_kernel<<<(kNParams + 1 + 255) / 256, 256, 0, st>>>(t->d_state, t->d_state + kNParams,
-                                                                       t->d_state + 2 * kNParams, t->d_partial, n_part,
-                                                                       t->lr, t->rho, t->eps, t->d_loss);
-  g_launches.fetch_add(2);
-  CU(cudaGetLastError());
+  float* state = t->d_state.get();
+  const int rc = launched(2, [&] {
+    ffn_train_grad_kernel<<<n_part, kTr2Threads, kTrain2SmemBytes, st>>>(state, d_x, d_y, n, 1.0f / static_cast<float>(n),
+                                                                           t->d_partial.get());
+    ffn_train_update_kernel<<<(kNParams + 1 + 255) / 256, 256, 0, st>>>(state, state + kNParams, state + 2 * kNParams,
+                                                                         t->d_partial.get(), n_part, t->lr, t->rho,
+                                                                         t->eps, t->d_loss.get());
+  });
+  if (rc) return rc;
   ++t->steps;
   if (h_loss) {
-    CU(cudaMemcpyAsync(h_loss, t->d_loss, sizeof(float), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_loss, t->d_loss.get(), sizeof(float), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
   }
   return 0;
@@ -1175,43 +1101,42 @@ int vadb200_synth_pcm(vadb200_handle* h, int16_t* d_out, int64_t n_utt, int64_t 
   CU(cudaSetDevice(h->device));
   const long long total = n_utt * utt_samples;
   const unsigned grid = static_cast<unsigned>(std::min<long long>((total + 255) / 256, 32ll * h->num_sms));
-  synth_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_out, n_utt, utt_samples, utt_stride, seed, first_utt);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    synth_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_out, n_utt, utt_samples, utt_stride, seed,
+                                                                      first_utt);
+  });
 }
 
 int vadb200_fp32_peak(vadb200_handle* h, int variant, int iters, double* tflops_out) {
   if (!h || !tflops_out || iters < 1 || variant < 0 || variant > 6) return fail(VADB200_E_INVALID, "bad argument");
   CU(cudaSetDevice(h->device));
-  int rc = ensure_tables(h);
-  if (rc) return rc;
-  cudaEvent_t e0, e1;
-  CU(cudaEventCreate(&e0));
-  CU(cudaEventCreate(&e1));
+  Event e0, e1;
+  CU(make_event(e0, cudaEventDefault));
+  CU(make_event(e1, cudaEventDefault));
   const int grid = h->num_sms * 8;
+  float* sink = h->d_sink.get();
   double best = 0.0;
   for (int rep = 0; rep < 5; ++rep) {
-    CU(cudaEventRecord(e0, nullptr));
-    if (variant == 0) fp32_peak_kernel<0><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else if (variant == 1) fp32_peak_kernel<1><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else if (variant == 2) fp32x2_peak_kernel<2><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else if (variant == 3) fp32x2_peak_kernel<3><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else if (variant == 4) fp32mix_peak_kernel<8><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else if (variant == 5) fp32mix_peak_kernel<4><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    else fp32mix_peak_kernel<0><<<grid, 256>>>(h->d_sink, iters, 1.0000001f, 1e-9f);
-    g_launches.fetch_add(1);
-    CU(cudaEventRecord(e1, nullptr));
-    CU(cudaEventSynchronize(e1));
+    CU(cudaEventRecord(e0.get(), nullptr));
+    const int rc = launched(1, [&] {
+      if (variant == 0) fp32_peak_kernel<0><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else if (variant == 1) fp32_peak_kernel<1><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else if (variant == 2) fp32x2_peak_kernel<2><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else if (variant == 3) fp32x2_peak_kernel<3><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else if (variant == 4) fp32mix_peak_kernel<8><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else if (variant == 5) fp32mix_peak_kernel<4><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+      else fp32mix_peak_kernel<0><<<grid, 256>>>(sink, iters, 1.0000001f, 1e-9f);
+    });
+    if (rc) return rc;
+    CU(cudaEventRecord(e1.get(), nullptr));
+    CU(cudaEventSynchronize(e1.get()));
     float ms = 0.f;
-    CU(cudaEventElapsedTime(&ms, e0, e1));
+    CU(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
     const double per_rep = variant <= 1 ? 2.0 * 16 : variant <= 3 ? 4.0 * 16
                          : variant == 4 ? 4.0 * 8 + 2.0 * 8 : variant == 5 ? 4.0 * 8 + 2.0 * 4 : 4.0 * 8;
     const double flops = per_rep * 8 * static_cast<double>(iters) * 256.0 * grid;
     if (rep > 0) best = std::max(best, flops / (ms * 1e-3) / 1e12);
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   *tflops_out = best;
   return 0;
 }
@@ -1268,21 +1193,18 @@ int vadb200_plan_speech_segments(vadb200_plan* p, const uint8_t* d_labels, int m
   uint8_t* sm = d_smoothed ? d_smoothed : wsb + ws.smoothed;
   const int n_tiles = static_cast<int>(p->tiles.size());
   const SmoothParams sp = smooth_params(min_speech_rows, min_silence_rows, pad_rows);
-  if (n_tiles > 0) {
-    speech_smooth_kernel<<<n_tiles, kSpeechThreads, smooth_smem_bytes(sp.H), st>>>(d_labels, p->d_tiles, p->d_row_off,
-                                                                                 sp, sm, counts);
-    g_launches.fetch_add(1);
-  }
-  speech_scan_kernel<<<1, kSpeechScanThreads, 0, st>>>(counts, n_tiles, prefix);
-  g_launches.fetch_add(1);
   const long long utt_blocks = (p->n_utt + 1 + kSpeechThreads - 1) / kSpeechThreads;
   const unsigned grid = static_cast<unsigned>(std::max<long long>(n_tiles, utt_blocks));
-  speech_segments_kernel<<<grid, kSpeechThreads, 0, st>>>(
-      sm, p->d_tiles, p->d_row_off, prefix, n_tiles, p->d_utt_tile, p->n_utt, reinterpret_cast<long long*>(d_segments),
-      reinterpret_cast<long long*>(d_segment_offsets), reinterpret_cast<long long*>(d_speech_offsets));
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(n_tiles > 0 ? 3 : 2, [&] {
+    if (n_tiles > 0)
+      speech_smooth_kernel<<<n_tiles, kSpeechThreads, smooth_smem_bytes(sp.H), st>>>(d_labels, p->d_tiles.get(),
+                                                                                   p->d_row_off.get(), sp, sm, counts);
+    speech_scan_kernel<<<1, kSpeechScanThreads, 0, st>>>(counts, n_tiles, prefix);
+    speech_segments_kernel<<<grid, kSpeechThreads, 0, st>>>(
+        sm, p->d_tiles.get(), p->d_row_off.get(), prefix, n_tiles, p->d_utt_tile.get(), p->n_utt,
+        reinterpret_cast<long long*>(d_segments), reinterpret_cast<long long*>(d_segment_offsets),
+        reinterpret_cast<long long*>(d_speech_offsets));
+  });
 }
 
 int vadb200_plan_gather_speech(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len, const int64_t* d_segments,
@@ -1304,13 +1226,12 @@ int vadb200_plan_gather_speech(vadb200_plan* p, const int16_t* d_pcm, int64_t pc
   // output hops are split evenly over a grid sized to keep HBM busy; CTAs past the speech exit at once
   const long long max_hops = p->total_rows;
   const unsigned grid = static_cast<unsigned>(std::max<long long>(1, std::min<long long>(8ll * p->h->num_sms, max_hops)));
-  speech_gather_kernel<<<grid, kSpeechThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      d_pcm, p->d_pcm_off, p->n_utt, reinterpret_cast<const long long*>(d_segments),
-      reinterpret_cast<const long long*>(d_segment_offsets), reinterpret_cast<const long long*>(d_speech_offsets), d_out,
-      out_capacity);
-  g_launches.fetch_add(1);
-  CU(cudaGetLastError());
-  return 0;
+  return launched(1, [&] {
+    speech_gather_kernel<<<grid, kSpeechThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        d_pcm, p->d_pcm_off.get(), p->n_utt, reinterpret_cast<const long long*>(d_segments),
+        reinterpret_cast<const long long*>(d_segment_offsets), reinterpret_cast<const long long*>(d_speech_offsets),
+        d_out, out_capacity);
+  });
 }
 
 }  // extern "C"
