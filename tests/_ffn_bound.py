@@ -103,7 +103,7 @@ def shim():
     if not os.path.isfile(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
         nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
         inc = os.path.join(os.path.dirname(os.path.dirname(os.path.realpath(nvcc))), "include")
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I", inc, "-o", so, src])
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-I", inc, "-o", so, src])
     lib = C.CDLL(so)
     lib.emul_ffn_blob_bytes.restype = C.c_int
     lib.emul_ffn_pack.restype = C.c_int

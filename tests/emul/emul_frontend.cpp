@@ -157,3 +157,94 @@ int emul_utterance_fe(const int16_t* pcm, long long n_samples, int feat_mode, fl
 }
 
 }  // extern "C"
+
+// ---- float32 power spectra and tables for the spectrum -> MFCC bound (tests/_mfcc_bound.py) ----------------------------
+extern "C" {
+
+// Raw |2X|^2 of every frame of one utterance through the fused kernel's load path: fft_load_pcm2 (use_fe == 0) or
+// fft_load_pcm2_fe (previous sample 0 at the utterance start), pass 1 with NZ = 13, the pair tile and
+// fft_split_store.  out [T][256]: bins kMelFirstBin .. 255 (bin 128 from thread 0's self-paired store); the bins the
+// kernel drops stay NaN, and so does any bin no store reached.
+int emul_power_pcm(const int16_t* pcm, long long n_samples, int use_fe, float preemph, const float* window,
+                   float* out) {
+  if (!g_init) return -1;
+  const FrontEndEmul fe = make_fe(preemph, window);
+  const long long T = frames_for_length(n_samples);
+  const int n = static_cast<int>(T);
+  const int nsteps = (n + kStepFrames - 1) / kStepFrames;
+  std::vector<float> P(kP2RowsAlloc * kP2Pitch);
+  std::vector<int16_t> stage_buf(kStageSamples + 16);
+  for (int s = 0; s < nsteps; ++s) {
+    const long long start = static_cast<long long>(s) * kStepFrames * kHop;
+    const long long avail = std::min<long long>(n_samples - start, kStageSamples);
+    std::memset(stage_buf.data(), 0x55, stage_buf.size() * sizeof(int16_t));
+    int16_t* stage = stage_buf.data() + 8;
+    std::memcpy(stage, pcm + start, static_cast<size_t>(avail) * sizeof(int16_t));
+    stage[-1] = s > 0 ? pcm[start - 1] : int16_t(0);
+    std::fill(P.begin(), P.end(), NAN);
+    for (int w = 0; w < 8; ++w)
+      for (int h = 0; h < 2; ++h) {
+        const uint32_t* w32 = reinterpret_cast<const uint32_t*>(stage) + (4 * w + h) * (kHop / 2);
+        if (use_fe) fft_pair_pcm_fe(w32, kHop, P.data(), col_of_halfwarp(w, h), fe);
+        else fft_pair_pcm(w32, kHop, P.data(), col_of_halfwarp(w, h));
+      }
+    for (int col = 0; col < kStepFrames; ++col) {
+      const long long f = static_cast<long long>(s) * kStepFrames + slot_of_col(col);
+      if (f >= n) continue;
+      for (int k = 0; k < kBins; ++k)
+        out[f * kBins + k] = k >= kMelFirstBin ? P[p2_index(k, col)] : NAN;
+    }
+  }
+  return 0;
+}
+
+// Raw |2X|^2 [n][256] of explicit float frames through frames_kernel's path: fft_load_f32 (use_fe == 0) or
+// fft_load_f32_fe, pass 1 with NZ = 16, one frame per thread.  get_spec_mag is this times 2^-20.
+int emul_power_f32(const float* frames, int n_frames, int frame_len, int use_fe, float preemph, const float* window,
+                   float* out) {
+  if (!g_init) return -1;
+  const FrontEndEmul fe = make_fe(preemph, window);
+  std::vector<float> P(256 * kPPitch);
+  for (int f = 0; f < n_frames; ++f) {
+    const float* fr = frames + static_cast<size_t>(f) * frame_len;
+    std::fill(P.begin(), P.end(), NAN);
+    if (use_fe) fft_frame_f32_fe(fr, frame_len, P.data(), fe);
+    else fft_frame_f32(fr, frame_len, P.data());
+    for (int k = 0; k < 256; ++k) out[static_cast<size_t>(f) * 256 + k] = P[k * kPPitch];
+  }
+  return 0;
+}
+
+// The float32 tables the kernels read, as dense matrices: melw (mel_group: frames_kernel, spec_to_mfcc_kernel) and
+// melw2 (mel2_run: the fused kernels) [26][256], both x 2^-20; dct (dct_coef) and dctp (dct_coef2 / dct_coef4)
+// [13][26].
+int emul_tables(float* melw, float* melw2, float* dct, float* dctp) {
+  if (!g_init) return -1;
+  std::memset(melw, 0, kNMel * kBins * sizeof(float));
+  std::memset(melw2, 0, kNMel * kBins * sizeof(float));
+  for (int m = 0; m < kNMel; ++m) {
+    for (int k = kMelLo[m]; k < kMelHi[m]; ++k) melw[m * kBins + k] = c_tab.melw[kMelOff[m] + k - kMelLo[m]];
+    for (int q = 0; q < mel_nq(m); ++q)
+      for (int e = 0; e < 2; ++e) melw2[m * kBins + 2 * (mel_q0(m) + q) + e] = c_tab.melw2[2 * (mel_qoff(m) + q) + e];
+  }
+  std::memcpy(dct, c_tab.dct, kNCep * kNMel * sizeof(float));
+  for (int k = 0; k < kNCep; ++k)
+    for (int n = 0; n < kNMel; ++n) dctp[k * kNMel + n] = c_tab.dctp[k >> 1][n][k & 1];
+  return 0;
+}
+
+// Read (set == 0) or replace (set != 0) the FFT twiddle tables tw1 [256] and tw2 [128] as (re, im) pairs: the CPU
+// suite's mutants of the replay.  emul_init restores the host's own tables.
+int emul_twiddles(float* tw1, float* tw2, int set) {
+  if (!g_init) return -1;
+  if (set) {
+    std::memcpy(g_tw1, tw1, sizeof(g_tw1));
+    std::memcpy(g_tw2, tw2, sizeof(g_tw2));
+  } else {
+    std::memcpy(tw1, g_tw1, sizeof(g_tw1));
+    std::memcpy(tw2, g_tw2, sizeof(g_tw2));
+  }
+  return 0;
+}
+
+}  // extern "C"

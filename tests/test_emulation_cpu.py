@@ -26,7 +26,7 @@ def emul():
     deps = [SRC] + [os.path.join(ROOT, "vad_b200", "csrc", f) for f in
                     ("vad_core.cuh", "vad_host_tables.h", "vad_tables.h")]
     if not os.path.isfile(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-x", "c++", "-o", SO, SRC])
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-x", "c++", "-o", SO, SRC])
     lib = C.CDLL(SO)
     w = rm.glorot_ffn(0)
     flat = np.concatenate([w[k].ravel() for k in FFN_KEYS]).astype(np.float32)

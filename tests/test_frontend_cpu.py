@@ -24,7 +24,7 @@ def emul():
     deps = [os.path.join(EMUL, f) for f in ("emul_frontend.cpp", "emul.cpp")] + \
         [os.path.join(ROOT, "vad_b200", "csrc", f) for f in ("vad_core.cuh", "vad_host_tables.h", "vad_tables.h")]
     if not os.path.isfile(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", SO,
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-o", SO,
                                os.path.join(EMUL, "emul_frontend.cpp")])
     lib = C.CDLL(SO)
     w = rm.glorot_ffn(0)

@@ -21,7 +21,7 @@ SO = os.path.join(EMUL, "libvademul_seg.so")
 def emul():
     deps = [os.path.join(EMUL, "emul_segments.cpp"), os.path.join(ROOT, "vad_b200", "csrc", "vad_segments.cuh")]
     if not os.path.isfile(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", SO,
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-o", SO,
                                os.path.join(EMUL, "emul_segments.cpp")])
     lib = C.CDLL(SO)
     lib.emul_speech_smooth.restype = C.c_longlong

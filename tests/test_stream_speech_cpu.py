@@ -29,7 +29,7 @@ def delay(S, G, P):
 def emul():
     deps = [os.path.join(EMUL, "emul_stream_speech.cpp"), os.path.join(ROOT, "vad_b200", "csrc", "vad_segments.cuh")]
     if not os.path.isfile(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-o", SO,
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-o", SO,
                                os.path.join(EMUL, "emul_stream_speech.cpp")])
     lib = C.CDLL(SO)
     lib.emul_bank_create.restype = C.c_void_p

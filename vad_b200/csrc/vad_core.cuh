@@ -421,7 +421,9 @@ VADB_HD float log2_energy(float e) {
   // mfcc.py:74: exact zeros -> float64 eps = 2^-52 (exactly representable in fp32)
   e = (e == 0.0f) ? 2.220446049250313e-16f : e;
 #if defined(__CUDA_ARCH__)
-  return __log2f(e);  // MUFU.LG2: <= 2 ulp of the result; parity-tested against the f64 oracle
+  // MUFU.LG2 (CUDA C++ Programming Guide, intrinsic functions): absolute error <= 2^-22 for e in [0.5, 2], else
+  // <= 2 ulp of the result; tests/_mfcc_bound.py holds the MFCC rows to exactly this
+  return __log2f(e);
 #else
   return log2f(e);
 #endif
@@ -589,6 +591,17 @@ VADB_HD void dct_coef4(const float* logE, int p, float& ra, float& rb, float& rc
   ra = r.x; rb = r.y; rc = q.x; rd = q.y;
 }
 
+// A product rounded on its own: nvcc contracts a plain product into the add or subtract that consumes it (FFMA),
+// which the packed path (__fmul2_rn) never does.  The window features' mean and z use it, here and in the stream
+// kernel, so fp32, tc and tc16 classify the same features.
+VADB_HD float mul_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+  return __fmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+
 VADB_HD float vadb_rsqrt(float v) {
 #if defined(__CUDA_ARCH__)
   return rsqrtf(v);  // MUFU.RSQ, <= 2 ulp
@@ -608,12 +621,13 @@ VADB_HD bool window_features(const float (&r)[5][kNCep], int mode, float (&x)[kN
     const float c0 = r[0][k], c1 = r[1][k], c2 = r[2][k], c3 = r[3][k], c4 = r[4][k];
     float z = c2;
     if (mode == 0) {
-      const float mu = ((((c0 + c1) + c2) + c3) + c4) * 0.2f;
+      // mul_rn: rounded like window_features_pairs' FMUL2, so every classifier path sees the same features
+      const float mu = mul_rn((((c0 + c1) + c2) + c3) + c4, 0.2f);
       const float d0 = c0 - mu, d1 = c1 - mu, d2 = c2 - mu, d3 = c3 - mu, d4 = c4 - mu;
       const float var = fmaf(d4, d4, fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)))) * 0.2f;
       // exact-arithmetic semantics of np.std == 0: all five equal -> 0/0 = nan
       const bool alleq = (c0 == c1) && (c1 == c2) && (c2 == c3) && (c3 == c4);
-      z = alleq ? NAN : d2 * vadb_rsqrt(var);
+      z = alleq ? NAN : mul_rn(d2, vadb_rsqrt(var));
       ok = ok && (fabsf(z) <= 3.0e38f);  // false for nan and inf
     }
     x[k] = z;

@@ -1112,11 +1112,11 @@ __device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnP
       float z = r[2];
       bool ok = true;
       if (p.feat_mode == 0) {
-        const float mu = ((((r[0] + r[1]) + r[2]) + r[3]) + r[4]) * 0.2f;
+        const float mu = mul_rn((((r[0] + r[1]) + r[2]) + r[3]) + r[4], 0.2f);   // as window_features
         const float d0 = r[0] - mu, d1 = r[1] - mu, d2 = r[2] - mu, d3 = r[3] - mu, d4 = r[4] - mu;
         const float var = fmaf(d4, d4, fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)))) * 0.2f;
         const bool alleq = (r[0] == r[1]) && (r[1] == r[2]) && (r[2] == r[3]) && (r[3] == r[4]);
-        z = alleq ? NAN : d2 * vadb_rsqrt(var);
+        z = alleq ? NAN : mul_rn(d2, vadb_rsqrt(var));
         ok = fabsf(z) <= 3.0e38f;
       }
       s_x[k * 32 + slot] = z;
