@@ -269,6 +269,36 @@ int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end /* [n]
                                     uint8_t* d_tail_rows /* nullable [n][D] */,
                                     int64_t* d_tail_bounds /* nullable [n][D + 1] */, void* stream);
 
+/* Ragged bank: each stream takes any number of samples per feed, from 0 up to max_feed_samples in [1, 16000]
+ * (1 s), so streams can be fed packets as they arrive (20 ms = 320 samples, 400, 512, ...) and a stream with nothing
+ * new sits a feed out.  A stream that has taken N samples since its last reset or end has completed the frames
+ * f >= 0 with 160 f + 400 <= N; completing frame f >= 5 emits row f - 5, the fixed bank's row (chunk r + 7 emits row
+ * r): it classifies frame f - 3 from the frames f - 5 .. f - 1.  After N samples a stream has emitted the rows of an
+ * offline utterance of N + 1 samples (vadb200_outputs_for_length(N + 1)), bit-identical to the fixed bank's and to
+ * the fused fp32 path's.  K = ceil(max_feed_samples / 160) rows at most per stream and feed
+ * (vadb200_stream_bank_max_rows_per_feed; -1 for NULL or a fixed bank).
+ *
+ * vadb200_stream_feed_ragged: stream i takes d_samples[d_offsets[i] .. d_offsets[i + 1]) (d_samples 2-byte aligned;
+ * both arrays may be pinned host memory: each sample is read once).  d_counts[i] gets the rows it emitted (0 .. K),
+ * d_labels[i][0 .. count) their labels (0 / 1) and 255 in the other slots, d_logits[i][j][3] the logits of rows
+ * j < count (other slots are not written).  A length below 0 or above max_feed_samples gets d_counts[i] = -1 and
+ * all-255 labels and leaves the stream untouched; the offsets live on the device, so this is the kernel's check.
+ * With speech on (vadb200_stream_bank_set_speech) each emitted row runs the segment step in row order: d_rows[i][j]
+ * is the smoothed row that row j finalises (255: none) and d_bounds[i][j] its bound (or -1), 255 / -1 past count;
+ * both may be NULL (the state still advances), and passing either while speech is off is VADB200_E_STATE.  The
+ * front end, threshold and speech settings apply as on the fixed bank; vadb200_stream_bank_reset, _set_speech,
+ * _speech_delay and _end_streams work with their meaning above (an end discards the samples that have not completed
+ * a frame; its tail takes R = the rows the stream has emitted).  vadb200_stream_feed / _feed_speech on a ragged bank,
+ * and vadb200_stream_feed_ragged on a fixed one, are VADB200_E_STATE.  A feed is one kernel launch: it allocates
+ * nothing, never synchronises and can be captured in a CUDA graph; the lengths are read on the device, so one graph
+ * serves any mix of packet sizes. */
+int vadb200_stream_bank_create_ragged(vadb200_handle* h, int n_streams, int max_feed_samples, vadb200_bank** out);
+int vadb200_stream_bank_max_rows_per_feed(const vadb200_bank* b);
+int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const int64_t* d_offsets /* [n + 1] */,
+                               int32_t* d_counts /* [n] */, uint8_t* d_labels /* [n][K] */,
+                               float* d_logits /* nullable [n][K][3] */, uint8_t* d_rows /* nullable [n][K] */,
+                               int64_t* d_bounds /* nullable [n][K] */, void* stream);
+
 /* ---- FFN training (learning/ffn_trainer.py:104-175) ---------------------------------------
  * model.compile(loss='categorical_crossentropy', optimizer='adadelta') + model.train_on_batch for the
  * 39-64-32-16-3 network: forward, backward and the Adadelta update as two hand-written kernels per step,

@@ -145,23 +145,46 @@ class StreamBank(object):
     online.  A stream's row r is its label from chunk r + 7 (since its last reset or end); ``feed_speech`` returns
     for each stream the smoothed row finalised this tick, r - D (255: none), and a segment bound: 160 (r - D) + 440
     samples when that row opens or closes a segment, else -1.  ``end_streams`` resolves the last D rows of the
-    streams it ends and starts them again, leaving the others untouched."""
+    streams it ends and starts them again, leaving the others untouched.
+
+    Ragged bank (``max_feed_samples``, 1 .. 16000): each tick takes any number of samples per stream, up to that cap
+    and including none, through ``feed_samples`` / ``feed_samples_speech`` instead of ``feed`` / ``feed_speech``.  A
+    stream's rows are those of the fixed bank fed the same signal: completing frame f >= 5 (samples
+    [160 f, 160 f + 400)) emits row f - 5, so one tick returns 0 .. K = ceil(max_feed_samples / 160) rows per stream.
+    The packets are packed into one pinned buffer with their offsets, and the captured graph reads the lengths on the
+    device: one graph serves every packet mix.  ``end_streams`` discards a stream's samples that have not completed a
+    frame."""
 
     NOT_READY = 255
+    max_feed = None          # ragged bank: the cap on one stream's samples per tick
 
-    def __init__(self, n_streams, ffn_weights=None, handle=None, use_graph=True, zero_copy=True):
+    def __init__(self, n_streams, ffn_weights=None, handle=None, use_graph=True, zero_copy=True,
+                 max_feed_samples=None):
         self.handle = _handle_for(ffn_weights, handle)
         if not self.handle.has_ffn:
             raise RuntimeError("StreamBank needs FFN weights")
         self.n = int(n_streams)
-        self.bank = runtime.StreamBankHandle(self.handle, self.n)
+        if max_feed_samples is not None:
+            self.max_feed = int(max_feed_samples)
+            if not 1 <= self.max_feed <= 16000:
+                raise ValueError("max_feed_samples must lie in [1, 16000]")
+        self.bank = runtime.StreamBankHandle(self.handle, self.n, self.max_feed)
         dev = self.handle.device
-        self.h_chunks = torch.zeros((self.n, 160), dtype=torch.int16).pin_memory()
-        self.h_labels = torch.zeros((self.n,), dtype=torch.uint8).pin_memory()
-        self.h_logits = torch.zeros((self.n, 3), dtype=torch.float32).pin_memory()
-        self.d_chunks = torch.zeros((self.n, 160), dtype=torch.int16, device=dev)
-        self.d_labels = torch.zeros((self.n,), dtype=torch.uint8, device=dev)
-        self.d_logits = torch.zeros((self.n, 3), dtype=torch.float32, device=dev)
+        if self.max_feed is None:
+            self.h_chunks = torch.zeros((self.n, 160), dtype=torch.int16).pin_memory()
+            self.h_labels = torch.zeros((self.n,), dtype=torch.uint8).pin_memory()
+            self.h_logits = torch.zeros((self.n, 3), dtype=torch.float32).pin_memory()
+            self.d_chunks = torch.zeros((self.n, 160), dtype=torch.int16, device=dev)
+            self.d_labels = torch.zeros((self.n,), dtype=torch.uint8, device=dev)
+            self.d_logits = torch.zeros((self.n, 3), dtype=torch.float32, device=dev)
+        else:
+            self.k = self.bank.max_rows_per_feed()
+            shapes = dict(samples=((self.n * self.max_feed,), torch.int16), offsets=((self.n + 1,), torch.int64),
+                          counts=((self.n,), torch.int32), labels=((self.n, self.k), torch.uint8),
+                          logits=((self.n, self.k, 3), torch.float32))
+            for name, (shape, dtype) in shapes.items():
+                setattr(self, "h_" + name, torch.zeros(shape, dtype=dtype).pin_memory())
+                setattr(self, "d_" + name, None if zero_copy else torch.zeros(shape, dtype=dtype, device=dev))
         self.stream = torch.cuda.Stream(device=dev)
         self.use_graph = bool(use_graph)
         self.zero_copy = bool(zero_copy)
@@ -174,7 +197,24 @@ class StreamBank(object):
         self.bank.reset()
         torch.cuda.synchronize(self.handle.device)
 
+    def _enqueue_ragged(self, want_logits, speech):
+        names = ["samples", "offsets", "counts", "labels"] + (["logits"] if want_logits else []) + \
+            (["rows", "bounds"] if speech else [])
+        side = "h_" if self.zero_copy else "d_"
+        if not self.zero_copy:
+            self.d_samples.copy_(self.h_samples, non_blocking=True)
+            self.d_offsets.copy_(self.h_offsets, non_blocking=True)
+        ptr = {k: getattr(self, side + k).data_ptr() for k in names}
+        self.bank.feed_ragged_ptr(ptr["samples"], ptr["offsets"], ptr["counts"], ptr["labels"], ptr.get("logits", 0),
+                                  ptr.get("rows", 0), ptr.get("bounds", 0))
+        if not self.zero_copy:
+            for k in names[2:]:
+                getattr(self, "h_" + k).copy_(getattr(self, "d_" + k), non_blocking=True)
+
     def _enqueue(self, want_logits, speech=False):
+        if self.max_feed is not None:
+            self._enqueue_ragged(want_logits, speech)
+            return
         if self.zero_copy:   # pinned host memory is device-visible under UVA: no copy nodes
             if speech:
                 self.bank.feed_speech_ptr(self.h_chunks.data_ptr(), self.h_labels.data_ptr(),
@@ -215,8 +255,13 @@ class StreamBank(object):
                 self._enqueue(want_logits, speech)
             self.stream.synchronize()
 
+    def _fixed_only(self, what):
+        if self.max_feed is not None:
+            raise RuntimeError("%s needs a fixed bank: a ragged bank (max_feed_samples) takes feed_samples" % what)
+
     def feed(self, chunks, want_logits=False):
         """chunks: array-like int16 [n, 160] on the host.  Blocks until labels are on the host."""
+        self._fixed_only("feed")
         src = torch.as_tensor(np.asarray(chunks, dtype=np.int16) if not torch.is_tensor(chunks) else chunks)
         if tuple(src.shape) != (self.n, 160):
             raise ValueError("chunks must have shape (%d, 160)" % self.n)
@@ -229,6 +274,7 @@ class StreamBank(object):
     def feed_pinned(self):
         """Low-latency tick: the caller has already written ``self.h_chunks`` (pinned); one graph
         launch (H2D + kernel + D2H) is issued and awaited.  Returns a view of ``self.h_labels``."""
+        self._fixed_only("feed_pinned")
         self._tick(False)
         return self.h_labels
 
@@ -241,10 +287,11 @@ class StreamBank(object):
         self._graphs = {}   # captured ticks hold the previous segment state
         d = self.bank.set_speech(*rows)
         if self.h_rows is None:
-            self.h_rows = torch.zeros((self.n,), dtype=torch.uint8).pin_memory()
-            self.h_bounds = torch.zeros((self.n,), dtype=torch.int64).pin_memory()
-            self.d_rows = torch.zeros((self.n,), dtype=torch.uint8, device=dev)
-            self.d_bounds = torch.zeros((self.n,), dtype=torch.int64, device=dev)
+            shape = (self.n,) if self.max_feed is None else (self.n, self.k)   # ragged: a slot per row
+            self.h_rows = torch.zeros(shape, dtype=torch.uint8).pin_memory()
+            self.h_bounds = torch.zeros(shape, dtype=torch.int64).pin_memory()
+            self.d_rows = torch.zeros(shape, dtype=torch.uint8, device=dev)
+            self.d_bounds = torch.zeros(shape, dtype=torch.int64, device=dev)
         self.d_tail_rows = torch.empty((self.n, d), dtype=torch.uint8, device=dev)
         self.d_tail_bounds = torch.empty((self.n, d + 1), dtype=torch.int64, device=dev)
         torch.cuda.synchronize(dev)
@@ -262,6 +309,7 @@ class StreamBank(object):
     def feed_speech(self, chunks):
         """feed() plus the segment step: returns (labels uint8 [n], rows uint8 [n], bounds int64 [n]); see the
         class notes.  Needs set_speech."""
+        self._fixed_only("feed_speech")
         if self.delay < 0:
             raise RuntimeError("speech is off: call set_speech first")
         src = torch.as_tensor(np.asarray(chunks, dtype=np.int16) if not torch.is_tensor(chunks) else chunks)
@@ -270,6 +318,54 @@ class StreamBank(object):
         self.h_chunks.copy_(src)
         self._tick(False, speech=True)
         return self.h_labels.numpy().copy(), self.h_rows.numpy().copy(), self.h_bounds.numpy().copy()
+
+    # ---- ragged bank ----------------------------------------------------------------------------------------------
+    def _pack(self, chunks):
+        """Check every packet, then pack them into the pinned samples / offsets buffers."""
+        if self.max_feed is None:
+            raise RuntimeError("feed_samples needs a ragged bank: create it with max_feed_samples")
+        if len(chunks) != self.n:
+            raise ValueError("chunks must hold %d arrays, one per stream" % self.n)
+        arrs = [np.asarray(c, dtype=np.int16) for c in chunks]
+        for a in arrs:
+            if a.ndim != 1:
+                raise ValueError("each stream's samples must be a 1-D array")
+            if a.shape[0] > self.max_feed:
+                raise ValueError("a stream took %d samples, more than max_feed_samples = %d"
+                                 % (a.shape[0], self.max_feed))
+        flat, off = self.h_samples.numpy(), self.h_offsets.numpy()
+        pos = 0
+        for i, a in enumerate(arrs):
+            off[i] = pos
+            flat[pos:pos + a.shape[0]] = a
+            pos += a.shape[0]
+        off[self.n] = pos
+
+    def _rows_of(self, buf):
+        counts = self.h_counts.numpy()
+        return [buf[i, :counts[i]].copy() for i in range(self.n)]
+
+    def feed_samples(self, chunks, want_logits=False):
+        """chunks: n 1-D int16 arrays, stream i's new samples (0 .. max_feed_samples of them).  Returns n uint8 arrays
+        of the rows each stream completed this tick (and n float32 [k, 3] logit arrays).  Blocks until they are on the
+        host."""
+        self._pack(chunks)
+        self._tick(want_logits)
+        labels = self._rows_of(self.h_labels.numpy())
+        if want_logits:
+            return labels, self._rows_of(self.h_logits.numpy())
+        return labels
+
+    def feed_samples_speech(self, chunks):
+        """feed_samples plus the segment step: for each stream (labels, rows, bounds), aligned with its labels: rows[j]
+        is the smoothed row that label j finalises (255: none) and bounds[j] its bound (-1: none).  Needs
+        set_speech."""
+        if self.max_feed is not None and self.delay < 0:
+            raise RuntimeError("speech is off: call set_speech first")
+        self._pack(chunks)
+        self._tick(False, speech=True)
+        return list(zip(self._rows_of(self.h_labels.numpy()), self._rows_of(self.h_rows.numpy()),
+                        self._rows_of(self.h_bounds.numpy())))
 
     def end_streams(self, ids):
         """End the streams ``ids`` and start them again (their next chunk begins a new signal).  With speech on,

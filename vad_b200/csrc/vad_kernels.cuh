@@ -33,6 +33,7 @@
 
 #include "vad_core.cuh"
 #include "ffn_tc.cuh"
+#include "vad_ragged.h"
 
 namespace vadb {
 
@@ -1017,6 +1018,161 @@ constexpr int kStreamRowsOff = 16;      // bytes below staged row 0: its word -1
 constexpr int kStreamSmemBytes = kStreamRowsOff + kStepFrames * kStreamFramePitch * 2 + kWarps * 2 * kExchFrame * 8 +
                                  kStreamPBytes + kNMel * 32 * 4 + 384 * 8;
 
+// Shared memory of one bank CTA (32 streams): staged PCM rows, the FFT exchange, the P tile (after the mel phase
+// the activations of the decision tail live there), log-mel energies and twiddles.
+struct StreamSmem {
+  int16_t* fr;
+  cf2* exch;
+  float* P;
+  float* logE;
+  cf2* tw1;
+  cf2* tw2;
+  float* x;   // [39][32]
+  float* h1;  // [64][32]
+  float* h2;  // [32][32]
+  float* h3;  // [16][32]
+  int* ok;    // [13][32]
+  __device__ __forceinline__ explicit StreamSmem(unsigned char* smem) {
+    fr = reinterpret_cast<int16_t*>(smem + kStreamRowsOff);
+    exch = reinterpret_cast<cf2*>(smem + kStreamRowsOff + kStepFrames * kStreamFramePitch * 2);
+    P = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(exch) + kWarps * 2 * kExchFrame * 8);
+    logE = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(P) + kStreamPBytes);
+    tw1 = reinterpret_cast<cf2*>(logE + kNMel * 32);
+    tw2 = tw1 + 256;
+    x = P;
+    h1 = x + kNFeat * 32;
+    h2 = h1 + kH1 * 32;
+    h3 = h2 + kH2 * 32;
+    ok = reinterpret_cast<int*>(h3 + kH3 * 32);
+  }
+};
+
+// The bank's building blocks, shared by the fixed tick (stream_feed_body) and the ragged one (stream_ragged_body).
+// FFT + mel of the 32 staged rows: the fused kernel's packed two-frames-per-thread pass, then log-mel energies.
+__device__ __forceinline__ void stream_fft_mel(const StreamSmem& sm, const FrontEnd& fe, int warp, int lane) {
+  const int h = lane >> 4;
+  {
+    f2* ex = reinterpret_cast<f2*>(sm.exch) + (warp * 2 + h) * kExchFrame;
+    const uint32_t* w32 = reinterpret_cast<const uint32_t*>(sm.fr + (warp * 4 + h) * kStreamFramePitch);
+    warp_fft_quad<13>(
+        [&](int t, f2 (&xr)[16], f2 (&xi)[16]) {
+          if (fe.win) fft_load_pcm2_fe(w32, kStreamFramePitch, t, fe.preemph, fe.win, xr, xi);
+          else fft_load_pcm2(w32, kStreamFramePitch, t, xr, xi);
+        },
+        ex, sm.tw1, sm.tw2, lane, [] {}, P2Store(sm.P, col_of_halfwarp(warp, h), lane & 15));
+  }
+  __syncthreads();
+  mel2_run_dispatch<kP2Pitch, 32>(warp, sm.P + 2 * lane, sm.logE + lane);
+  __syncthreads();
+}
+
+// DCT + MFCC ring + window features: warp = coefficient (w, w + 8), lane = P column, slot = its stream in the CTA.
+// The stream has a new frame when live && frame >= 0: its ring (holding frames -5 .. -1 before it) gives the
+// features and takes the frame.  Otherwise the features are of a zero window and are not used.
+__device__ __forceinline__ void stream_window_features(const StreamSmem& sm, float* ring, long long ns, int st,
+                                                       bool live, int frame, int feat_mode, int warp, int lane,
+                                                       int slot) {
+#pragma unroll
+  for (int rep = 0; rep < 2; ++rep) {
+    const int k = warp + 8 * rep;
+    if (k < kNCep) {                       // warp-uniform
+      const float cnew = dct_coef<32>(sm.logE + lane, k);
+      float r[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+      if (live && frame >= 0) {
+#pragma unroll
+        for (int d = 0; d < 5; ++d) r[d] = ring[(d * kNCep + k) * ns + st];
+#pragma unroll
+        for (int d = 0; d < 4; ++d) ring[(d * kNCep + k) * ns + st] = r[d + 1];
+        ring[(4 * kNCep + k) * ns + st] = cnew;
+      }
+      float z = r[2];
+      bool ok = true;
+      if (feat_mode == 0) {
+        const float mu = mul_rn((((r[0] + r[1]) + r[2]) + r[3]) + r[4], 0.2f);   // as window_features
+        const float d0 = r[0] - mu, d1 = r[1] - mu, d2 = r[2] - mu, d3 = r[3] - mu, d4 = r[4] - mu;
+        const float var = fmaf(d4, d4, fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)))) * 0.2f;
+        const bool alleq = (r[0] == r[1]) && (r[1] == r[2]) && (r[2] == r[3]) && (r[3] == r[4]);
+        z = alleq ? NAN : mul_rn(d2, vadb_rsqrt(var));
+        ok = fabsf(z) <= 3.0e38f;
+      }
+      sm.x[k * 32 + slot] = z;
+      sm.x[(kNCep + k) * 32 + slot] = r[3] - r[1];
+      sm.x[(2 * kNCep + k) * 32 + slot] = (r[4] - z) - (z - r[0]);
+      sm.ok[k * 32 + slot] = ok ? 1 : 0;
+    }
+  }
+}
+
+// FFN layers 1-3, lane = stream (slot order): warp w computes 8 / 4 / 2 neurons; ends with the h3 tile complete.
+__device__ __forceinline__ void stream_ffn_hidden(const StreamSmem& sm, const FfnParams& w, int warp, int lane) {
+  {
+    float acc[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = w.b1[8 * warp + j];
+#pragma unroll 3
+    for (int i = 0; i < kNFeat; ++i) {
+      const float xv = sm.x[i * 32 + lane];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc[j] = fmaf(xv, w.W1[i * kH1 + 8 * warp + j], acc[j]);
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) sm.h1[(8 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
+  }
+  __syncthreads();
+  {
+    float acc[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[j] = w.b2[4 * warp + j];
+#pragma unroll 4
+    for (int i = 0; i < kH1; ++i) {
+      const float a = sm.h1[i * 32 + lane];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) acc[j] = fmaf(a, w.W2[i * kH2 + 4 * warp + j], acc[j]);
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) sm.h2[(4 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
+  }
+  __syncthreads();
+  {
+    float acc[2];
+#pragma unroll
+    for (int j = 0; j < 2; ++j) acc[j] = w.b3[2 * warp + j];
+#pragma unroll 4
+    for (int i = 0; i < kH2; ++i) {
+      const float a = sm.h2[i * 32 + lane];
+#pragma unroll
+      for (int j = 0; j < 2; ++j) acc[j] = fmaf(a, w.W3[i * kH3 + 2 * warp + j], acc[j]);
+    }
+#pragma unroll
+    for (int j = 0; j < 2; ++j) sm.h3[(2 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
+  }
+  __syncthreads();
+}
+
+// Output layer and decision of the stream in this lane; lg gets the logits when every feature is finite (else the
+// label is 0 and lg is left as it is).
+__device__ __forceinline__ uint8_t stream_decide(const StreamSmem& sm, const FfnParams& w, int lane, float (&lg)[3]) {
+  float acc[kNCls];
+#pragma unroll
+  for (int o = 0; o < kNCls; ++o) acc[o] = w.b4[o];
+#pragma unroll
+  for (int i = 0; i < kH3; ++i) {
+    const float a = sm.h3[i * 32 + lane];
+#pragma unroll
+    for (int o = 0; o < kNCls; ++o) acc[o] = fmaf(a, w.W4[i * kNCls + o], acc[o]);
+  }
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < kNCep; ++k) ok = ok && (sm.ok[k * 32 + lane] != 0);
+  uint8_t lab = decide(acc, w.thresh);
+  if (ok) {
+    lg[0] = acc[0]; lg[1] = acc[1]; lg[2] = acc[2];
+  } else {
+    lab = 0;
+  }
+  return lab;
+}
+
 // One CTA = 32 streams.  FFT: the fused kernel's packed two-frames-per-thread pass.  The decision
 // tail is spread over all 8 warps with lane = stream: warp w owns cepstral coefficients w, w + 8
 // (DCT, ring push, window features) and then 8 / 4 / 2 neurons of layers 1 / 2 / 3, activations
@@ -1028,22 +1184,12 @@ template <bool SEG, class Seg>
 __device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnParams& w, const Seg& sg,
                                                  const int tid) {
   extern __shared__ __align__(128) unsigned char smem[];
-  int16_t* s_fr = reinterpret_cast<int16_t*>(smem + kStreamRowsOff);
-  cf2* s_exch = reinterpret_cast<cf2*>(smem + kStreamRowsOff + kStepFrames * kStreamFramePitch * 2);
-  float* s_P = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(s_exch) + kWarps * 2 * kExchFrame * 8);
-  float* s_logE = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(s_P) + kStreamPBytes);
-  cf2* s_tw1 = reinterpret_cast<cf2*>(s_logE + kNMel * 32);
-  cf2* s_tw2 = s_tw1 + 256;
-  // after the mel phase the P tile is dead: activations live there
-  float* s_x = s_P;                    // [39][32]
-  float* s_h1 = s_x + kNFeat * 32;     // [64][32]
-  float* s_h2 = s_h1 + kH1 * 32;       // [32][32]
-  float* s_h3 = s_h2 + kH2 * 32;       // [16][32]
-  int* s_ok = reinterpret_cast<int*>(s_h3 + kH3 * 32);  // [13][32]
-  const int warp = tid >> 5, lane = tid & 31, h = lane >> 4;
+  const StreamSmem sm(smem);
+  int16_t* s_fr = sm.fr;
+  const int warp = tid >> 5, lane = tid & 31;
   const int s0 = blockIdx.x * kStepFrames;
-  s_tw1[tid] = p.tw1[tid];
-  if (tid < 128) s_tw2[tid] = p.tw2[tid];
+  sm.tw1[tid] = p.tw1[tid];
+  if (tid < 128) sm.tw2[tid] = p.tw2[tid];
   // stage [hist 320 | chunk 160] per stream: every chunk sample is read exactly once (the chunks may live in
   // pinned host memory: zero-copy ticks), then roll the history in global memory from the staged copy
   for (int j = tid; j < kStepFrames * 240; j += kThreads) {  // 32-bit words: 160 hist + 80 chunk per stream
@@ -1075,126 +1221,23 @@ __device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnP
     }
     __syncthreads();
   }
-  {
-    f2* ex = reinterpret_cast<f2*>(s_exch) + (warp * 2 + h) * kExchFrame;
-    const uint32_t* w32 = reinterpret_cast<const uint32_t*>(s_fr + (warp * 4 + h) * kStreamFramePitch);
-    warp_fft_quad<13>(
-        [&](int t, f2 (&xr)[16], f2 (&xi)[16]) {
-          if (p.fe.win) fft_load_pcm2_fe(w32, kStreamFramePitch, t, p.fe.preemph, p.fe.win, xr, xi);
-          else fft_load_pcm2(w32, kStreamFramePitch, t, xr, xi);
-        },
-        ex, s_tw1, s_tw2, lane, [] {}, P2Store(s_P, col_of_halfwarp(warp, h), lane & 15));
-  }
-  __syncthreads();
-  mel2_run_dispatch<kP2Pitch, 32>(warp, s_P + 2 * lane, s_logE + lane);
-  __syncthreads();
-  // ---- DCT + ring + window features: warp = coefficient (w, w + 8), lane = P column ----------------
+  stream_fft_mel(sm, p.fe, warp, lane);
   const int slot = slot_of_col(lane);      // stream of this lane inside the CTA
   const int st = s0 + slot;
   const bool live = st < p.n_streams;
-  const long long ns = p.n_streams;
   const int fed = live ? p.fed[st] : 0;    // chunks fed before this one
   const int frame = fed - 2;               // index of the frame completed by this chunk (< 0: none yet)
   // (a row is classified once frame >= 5: the ring then holds frames frame-5 .. frame-1 and frame-3 is the centre)
-#pragma unroll
-  for (int rep = 0; rep < 2; ++rep) {
-    const int k = warp + 8 * rep;
-    if (k < kNCep) {                       // warp-uniform
-      const float cnew = dct_coef<32>(s_logE + lane, k);
-      float r[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
-      if (live && frame >= 0) {
-#pragma unroll
-        for (int d = 0; d < 5; ++d) r[d] = p.ring[(d * kNCep + k) * ns + st];
-#pragma unroll
-        for (int d = 0; d < 4; ++d) p.ring[(d * kNCep + k) * ns + st] = r[d + 1];
-        p.ring[(4 * kNCep + k) * ns + st] = cnew;
-      }
-      float z = r[2];
-      bool ok = true;
-      if (p.feat_mode == 0) {
-        const float mu = mul_rn((((r[0] + r[1]) + r[2]) + r[3]) + r[4], 0.2f);   // as window_features
-        const float d0 = r[0] - mu, d1 = r[1] - mu, d2 = r[2] - mu, d3 = r[3] - mu, d4 = r[4] - mu;
-        const float var = fmaf(d4, d4, fmaf(d3, d3, fmaf(d2, d2, fmaf(d1, d1, d0 * d0)))) * 0.2f;
-        const bool alleq = (r[0] == r[1]) && (r[1] == r[2]) && (r[2] == r[3]) && (r[3] == r[4]);
-        z = alleq ? NAN : mul_rn(d2, vadb_rsqrt(var));
-        ok = fabsf(z) <= 3.0e38f;
-      }
-      s_x[k * 32 + slot] = z;
-      s_x[(kNCep + k) * 32 + slot] = r[3] - r[1];
-      s_x[(2 * kNCep + k) * 32 + slot] = (r[4] - z) - (z - r[0]);
-      s_ok[k * 32 + slot] = ok ? 1 : 0;
-    }
-  }
+  stream_window_features(sm, p.ring, p.n_streams, st, live, frame, p.feat_mode, warp, lane, slot);
   __syncthreads();
-  // ---- FFN, lane = stream (slot order from here on) --------------------------------------------------
-  {
-    float acc[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] = w.b1[8 * warp + j];
-#pragma unroll 3
-    for (int i = 0; i < kNFeat; ++i) {
-      const float xv = s_x[i * 32 + lane];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) acc[j] = fmaf(xv, w.W1[i * kH1 + 8 * warp + j], acc[j]);
-    }
-#pragma unroll
-    for (int j = 0; j < 8; ++j) s_h1[(8 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
-  }
-  __syncthreads();
-  {
-    float acc[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[j] = w.b2[4 * warp + j];
-#pragma unroll 4
-    for (int i = 0; i < kH1; ++i) {
-      const float a = s_h1[i * 32 + lane];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[j] = fmaf(a, w.W2[i * kH2 + 4 * warp + j], acc[j]);
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) s_h2[(4 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
-  }
-  __syncthreads();
-  {
-    float acc[2];
-#pragma unroll
-    for (int j = 0; j < 2; ++j) acc[j] = w.b3[2 * warp + j];
-#pragma unroll 4
-    for (int i = 0; i < kH2; ++i) {
-      const float a = s_h2[i * 32 + lane];
-#pragma unroll
-      for (int j = 0; j < 2; ++j) acc[j] = fmaf(a, w.W3[i * kH3 + 2 * warp + j], acc[j]);
-    }
-#pragma unroll
-    for (int j = 0; j < 2; ++j) s_h3[(2 * warp + j) * 32 + lane] = fmaxf(acc[j], 0.0f);
-  }
-  __syncthreads();
+  stream_ffn_hidden(sm, w, warp, lane);
   if (warp == 0) {
     const int stl = s0 + lane;
     if (stl < p.n_streams) {
       const int fedl = p.fed[stl];
       uint8_t lab = 255;
       float lg[3] = {NAN, NAN, NAN};
-      if (fedl - 2 >= 5) {
-        float acc[kNCls];
-#pragma unroll
-        for (int o = 0; o < kNCls; ++o) acc[o] = w.b4[o];
-#pragma unroll
-        for (int i = 0; i < kH3; ++i) {
-          const float a = s_h3[i * 32 + lane];
-#pragma unroll
-          for (int o = 0; o < kNCls; ++o) acc[o] = fmaf(a, w.W4[i * kNCls + o], acc[o]);
-        }
-        bool ok = true;
-#pragma unroll
-        for (int k = 0; k < kNCep; ++k) ok = ok && (s_ok[k * 32 + lane] != 0);
-        lab = decide(acc, w.thresh);
-        if (ok) {
-          lg[0] = acc[0]; lg[1] = acc[1]; lg[2] = acc[2];
-        } else {
-          lab = 0;
-        }
-      }
+      if (fedl - 2 >= 5) lab = stream_decide(sm, w, lane, lg);
       p.fed[stl] = fedl + 1;
       p.labels[stl] = lab;
       if (p.logits) {
@@ -1222,6 +1265,185 @@ __global__ void __launch_bounds__(kThreads) stream_feed_speech_kernel(const Bank
                                                                      const __grid_constant__ FfnParams w,
                                                                      const __grid_constant__ Seg sg) {
   stream_feed_body<true>(p, w, sg, threadIdx.x);
+}
+
+// ---- ragged bank (vadb200_stream_bank_create_ragged): any number of samples per stream and feed ----------------
+// State per stream: a sample ring int16[R] and the samples taken N (vad_ragged.h), and the MFCC ring [5*13][n] of
+// the fixed bank.  Stream i's packet of this feed is samples[offsets[i] .. offsets[i + 1]).
+struct RaggedParams {
+  int n_streams;
+  int max_feed;               // cap on one packet
+  int ring_len;               // R
+  int max_rows;               // K = ragged_max_rows(max_feed)
+  int16_t* pcm;               // [n_streams][R] sample rings
+  long long* total;           // [n_streams] N
+  float* ring;                // [5*13][n_streams]
+  const int16_t* samples;     // packets, 2-byte aligned
+  const long long* offsets;   // [n_streams + 1]
+  int* counts;                // [n_streams] rows emitted, -1: bad packet length
+  uint8_t* labels;            // [n_streams][K]
+  float* logits;              // nullable [n_streams][K][3]
+  uint8_t* rows;              // nullable [n_streams][K] finalised smoothed rows (speech)
+  int64_t* bounds;            // nullable [n_streams][K] their bounds (speech)
+  const cf2* tw1;
+  const cf2* tw2;
+  int feat_mode;
+  FrontEnd fe;                // fe.win == nullptr: no front end
+};
+constexpr int kRaggedLoads = 8;  // packet samples each thread loads before it stores any (zero-copy reads in flight)
+
+// One CTA = 32 streams, as stream_feed_body.  (1) Read the CTA's 33 offsets once, check each packet length and
+// append the packets to the sample rings: the CTA's packets are one flat run of samples over all 256 threads, each
+// read exactly once (they may live in pinned host memory).  (2) For j below the most frames any of the 32 streams
+// completes, stage frame f0 + j of every stream that has one (its 400 samples and the sample before, from the ring,
+// into the fixed tick's rows), run the fixed tick's FFT, mel, DCT, window features and FFN on it, and emit row
+// f0 + j - 5 of the streams that have it, with the segment step (SEG) in row order.  Staged words, FFT and FFMA
+// order are the fixed tick's, so every row is bit-identical to it.  A CTA with no frame to complete stops after (1).
+template <bool SEG, class Seg>
+__device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const FfnParams& w, const Seg& sg,
+                                                   const int tid) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  const StreamSmem sm(smem);
+  __shared__ long long s_off[kStepFrames + 1];
+  __shared__ long long s_n0[kStepFrames];  // N before this feed
+  __shared__ long long s_f0[kStepFrames];  // first frame this feed completes
+  __shared__ int s_pre[kStepFrames + 1];   // exclusive prefix of the packet lengths (a bad one counts 0)
+  __shared__ int s_base[kStepFrames];      // ring slot of sample N
+  __shared__ int s_w0[kStepFrames];        // ring word of the next frame to stage
+  __shared__ int s_nf[kStepFrames];        // frames this feed completes
+  __shared__ int s_cnt[kStepFrames];       // rows it emits, -1: bad packet length
+  __shared__ int s_jmax;
+  const int warp = tid >> 5, lane = tid & 31;
+  const int s0 = blockIdx.x * kStepFrames;
+  const int nloc = min(kStepFrames, p.n_streams - s0);
+  const int R = p.ring_len, K = p.max_rows;
+  sm.tw1[tid] = p.tw1[tid];
+  if (tid < 128) sm.tw2[tid] = p.tw2[tid];
+  if (tid <= nloc) s_off[tid] = p.offsets[s0 + tid];
+  __syncthreads();
+  if (warp == 0) {
+    int c = 0, nf = 0, cnt = 0;
+    long long n0 = 0, f0 = 0;
+    if (lane < nloc) {
+      const long long c64 = s_off[lane + 1] - s_off[lane];
+      if (c64 < 0 || c64 > p.max_feed) {
+        cnt = -1;                              // not advanced
+      } else {
+        c = static_cast<int>(c64);
+        n0 = p.total[s0 + lane];
+        f0 = ragged_frames(n0);
+        nf = static_cast<int>(ragged_frames(n0 + c) - f0);
+        cnt = static_cast<int>(ragged_rows(n0 + c) - ragged_rows(n0));
+        p.total[s0 + lane] = n0 + c;
+      }
+      p.counts[s0 + lane] = cnt;
+    }
+    int incl = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += v;
+    }
+    s_pre[lane + 1] = incl;
+    if (lane == 0) s_pre[0] = 0;
+    s_n0[lane] = n0;
+    s_f0[lane] = f0;
+    s_nf[lane] = nf;
+    s_cnt[lane] = cnt;
+    s_base[lane] = ragged_slot(n0, R);
+    s_w0[lane] = ragged_frame_word0(f0, R);
+    const int jm = __reduce_max_sync(0xffffffffu, nf);
+    if (lane == 0) s_jmax = jm;
+  }
+  __syncthreads();
+  // (1) append: flat sample q of the CTA belongs to the stream i with s_pre[i] <= q < s_pre[i + 1]
+  const int total = s_pre[kStepFrames];
+  for (int q0 = 0; q0 < total; q0 += kThreads * kRaggedLoads) {
+    int16_t v[kRaggedLoads];
+    int dst[kRaggedLoads];
+#pragma unroll
+    for (int u = 0; u < kRaggedLoads; ++u) {
+      const int q = q0 + u * kThreads + tid;
+      dst[u] = -1;
+      if (q < total) {
+        int i = 0;
+#pragma unroll
+        for (int b = 16; b > 0; b >>= 1)
+          if (s_pre[i + b] <= q) i += b;
+        const int k = q - s_pre[i];
+        v[u] = p.samples[s_off[i] + k];
+        dst[u] = i * R + ragged_wrap(s_base[i] + k, R);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < kRaggedLoads; ++u)
+      if (dst[u] >= 0) p.pcm[static_cast<long long>(s0) * R + dst[u]] = v[u];
+  }
+  // output slots past each stream's count: label 255, row 255, bound -1
+  for (int q = tid; q < nloc * K; q += kThreads) {
+    const int i = q / K, k = q - i * K;
+    if (k >= s_cnt[i]) {
+      const long long o = static_cast<long long>(s0 + i) * K + k;
+      p.labels[o] = 255;
+      if (p.rows) p.rows[o] = 255;
+      if (p.bounds) p.bounds[o] = -1;
+    }
+  }
+  __syncthreads();
+  // (2) frames
+  const int slot = slot_of_col(lane);  // stream of this lane inside the CTA (DCT phase)
+  const int jmax = s_jmax;
+  for (int j = 0; j < jmax; ++j) {
+    for (int q = tid; q < kStepFrames * 200; q += kThreads) {  // 32-bit words: a frame's 400 samples
+      const int i = q / 200, wd = q - i * 200;
+      if (j < s_nf[i])
+        reinterpret_cast<uint32_t*>(sm.fr + i * kStreamFramePitch)[wd] =
+            reinterpret_cast<const uint32_t*>(p.pcm + static_cast<long long>(s0 + i) * R)[ragged_wrap(s_w0[i] + wd, R / 2)];
+    }
+    if (tid < kStepFrames && j < s_nf[tid])  // the sample before the frame: high half of the row's word -1
+      sm.fr[tid * kStreamFramePitch - 1] =
+          s_f0[tid] + j > 0 ? p.pcm[static_cast<long long>(s0 + tid) * R + ragged_pre_slot(s_w0[tid], R)] : 0;
+    __syncthreads();
+    if (tid < kStepFrames) s_w0[tid] = ragged_wrap(s_w0[tid] + 80, R / 2);  // read again after later barriers
+    stream_fft_mel(sm, p.fe, warp, lane);
+    stream_window_features(sm, p.ring, p.n_streams, s0 + slot, j < s_nf[slot], 0, p.feat_mode, warp, lane, slot);
+    __syncthreads();
+    stream_ffn_hidden(sm, w, warp, lane);
+    if (warp == 0 && j < s_nf[lane]) {
+      const long long f = s_f0[lane] + j;
+      if (f >= 5) {                          // row f - 5 of the stream, output slot k
+        const int stl = s0 + lane;
+        float lg[3] = {NAN, NAN, NAN};
+        const uint8_t lab = stream_decide(sm, w, lane, lg);
+        const long long o = static_cast<long long>(stl) * K + (f - max(s_f0[lane], 5ll));
+        p.labels[o] = lab;
+        if (p.logits) {
+          p.logits[o * 3 + 0] = lg[0];
+          p.logits[o * 3 + 1] = lg[1];
+          p.logits[o * 3 + 2] = lg[2];
+        }
+        if constexpr (SEG) {
+          uint8_t row = 255;
+          long long bound = -1;
+          seg_step(sg, stl, static_cast<int>(f - 5), lab != 0, row, bound);
+          if (p.rows) p.rows[o] = row;
+          if (p.bounds) p.bounds[o] = bound;
+        }
+      }
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kThreads) stream_ragged_kernel(const __grid_constant__ RaggedParams p,
+                                                                const __grid_constant__ FfnParams w) {
+  stream_ragged_body<false>(p, w, 0, threadIdx.x);
+}
+// The same feed plus the bank's segment step (Seg = StreamSeg; its rows / bounds pointers are not used).
+template <class Seg>
+__global__ void __launch_bounds__(kThreads) stream_ragged_speech_kernel(const __grid_constant__ RaggedParams p,
+                                                                       const __grid_constant__ FfnParams w,
+                                                                       const __grid_constant__ Seg sg) {
+  stream_ragged_body<true>(p, w, sg, threadIdx.x);
 }
 
 // ---- feature sink: scale_features (dataset/utils.py:5-32) on packed dataset rows [n][39] ----------------

@@ -25,6 +25,8 @@
 
 #include <cstdint>
 
+#include "vad_ragged.h"
+
 #if defined(__CUDACC__)
 #define VADB_SEG_HD __host__ __device__ __forceinline__
 #else
@@ -666,6 +668,22 @@ __global__ void __launch_bounds__(kSegEndThreads) stream_end_kernel(
   for (int k = 0; k < 65; ++k) mfcc_ring[static_cast<long long>(k) * n_streams + s] = 0.0f;
   fed[s] = 0;
   prev[s] = 0;
+}
+
+// Ragged bank: the same for the streams with end[s] != 0, with R the rows the stream has emitted (vad_ragged.h
+// ragged_rows of its sample count N).  Then N and the MFCC ring are zero: samples that have not completed a frame are
+// discarded, and the sample ring needs no clearing (a new signal's frames read only its own samples).
+__global__ void __launch_bounds__(kSegEndThreads) stream_end_ragged_kernel(
+    const StreamSeg g, const uint8_t* __restrict__ end, int n_streams, long long* __restrict__ total,
+    float* __restrict__ mfcc_ring, uint8_t* __restrict__ tail_rows, int64_t* __restrict__ tail_bounds) {
+  extern __shared__ uint32_t seg_scratch[];
+  const int s = blockIdx.x * kSegEndThreads + threadIdx.x;
+  if (s >= n_streams || !end[s]) return;
+  if (g.meta)
+    seg_end(g, s, static_cast<int>(ragged_rows(total[s])), seg_scratch + threadIdx.x, kSegEndThreads, tail_rows,
+            tail_bounds);
+  for (int k = 0; k < 65; ++k) mfcc_ring[static_cast<long long>(k) * n_streams + s] = 0.0f;
+  total[s] = 0;
 }
 
 #endif  // __CUDACC__

@@ -209,6 +209,12 @@ struct vadb200_bank {
   DevBuf<float> d_ring;
   DevBuf<int> d_fed;
   DevBuf<int16_t> d_prev;      // the raw sample before each stream's history (front end)
+  // ragged bank (vadb200_stream_bank_create_ragged; max_feed == 0: the fixed bank, which has d_hist, d_fed, d_prev
+  // instead): per stream a sample ring of ring_len int16 and the samples taken so far (vad_ragged.h)
+  int max_feed = 0;
+  int ring_len = 0;
+  DevBuf<int16_t> d_pcm;
+  DevBuf<long long> d_total;
   // speech segments (vadb200_stream_bank_set_speech); d_seg empty: off.  One allocation of
   // [W1 + W2 + 2][n] words: ring1, ring2, meta, last (vad_segments.cuh StreamSeg).
   SmoothParams sp{};
@@ -382,6 +388,9 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
   CU(cudaFuncSetAttribute(stream_feed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
   CU(cudaFuncSetAttribute(stream_feed_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_ragged_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          kStreamSmemBytes));
   // Mel weights and the folded DCT matrix are the same for every handle (the kernels are compiled for the
   // reference configuration only), so the __constant__ copy is written once per device and never changes:
   // no handle can observe another handle's state through it.  FFN weights never go through device globals.
@@ -884,6 +893,30 @@ int vadb200_stream_bank_create(vadb200_handle* h, int n_streams, vadb200_bank** 
   return 0;
 }
 
+int vadb200_stream_bank_create_ragged(vadb200_handle* h, int n_streams, int max_feed_samples, vadb200_bank** out) {
+  if (out) *out = nullptr;
+  if (!h || !out || n_streams < 1 || max_feed_samples < 1 || max_feed_samples > kRaggedMaxFeed)
+    return fail(VADB200_E_INVALID, "bad argument (max_feed_samples must lie in [1, 16000])");
+  CU(cudaSetDevice(h->device));
+  std::unique_ptr<vadb200_bank> b(new (std::nothrow) vadb200_bank());
+  if (!b) return fail(VADB200_E_NOMEM, "host allocation failed");
+  b->h = h; b->device = h->device; b->n = n_streams;
+  b->max_feed = max_feed_samples;
+  b->ring_len = ragged_ring_samples(max_feed_samples);
+  CU(dev_alloc(b->d_pcm, static_cast<size_t>(n_streams) * b->ring_len * sizeof(int16_t)));
+  CU(dev_alloc(b->d_total, static_cast<size_t>(n_streams) * sizeof(long long)));
+  CU(dev_alloc(b->d_ring, static_cast<size_t>(n_streams) * 5 * kNCep * sizeof(float)));
+  const int rc = vadb200_stream_bank_reset(b.get(), nullptr);
+  if (rc) return rc;
+  CU(cudaDeviceSynchronize());  // state is zero before any stream can feed
+  *out = b.release();
+  return 0;
+}
+
+int vadb200_stream_bank_max_rows_per_feed(const vadb200_bank* b) {
+  return b && b->max_feed ? ragged_max_rows(b->max_feed) : -1;
+}
+
 int vadb200_stream_bank_destroy(vadb200_bank* b) {
   delete b;
   return 0;
@@ -913,6 +946,7 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
                        int64_t* d_bounds, void* stream) {
   if (!b || !d_chunks || !d_labels) return fail(VADB200_E_INVALID, "null argument");
   vadb200_handle* h = b->h;
+  if (b->max_feed) return fail(VADB200_E_STATE, "a ragged bank takes vadb200_stream_feed_ragged");
   if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
   if (reinterpret_cast<uintptr_t>(d_chunks) & 3) return fail(VADB200_E_INVALID, "chunks must be 4-byte aligned");
   CU(cudaSetDevice(h->device));
@@ -939,16 +973,48 @@ int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
   if (!b) return fail(VADB200_E_INVALID, "bank is null");
   CU(cudaSetDevice(b->h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CU(cudaMemsetAsync(b->d_hist.get(), 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
+  if (b->max_feed) {
+    CU(cudaMemsetAsync(b->d_pcm.get(), 0, static_cast<size_t>(b->n) * b->ring_len * sizeof(int16_t), st));
+    CU(cudaMemsetAsync(b->d_total.get(), 0, static_cast<size_t>(b->n) * sizeof(long long), st));
+  } else {
+    CU(cudaMemsetAsync(b->d_hist.get(), 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
+    CU(cudaMemsetAsync(b->d_fed.get(), 0, static_cast<size_t>(b->n) * sizeof(int), st));
+    CU(cudaMemsetAsync(b->d_prev.get(), 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
+  }
   CU(cudaMemsetAsync(b->d_ring.get(), 0, static_cast<size_t>(b->n) * 5 * kNCep * sizeof(float), st));
-  CU(cudaMemsetAsync(b->d_fed.get(), 0, static_cast<size_t>(b->n) * sizeof(int), st));
-  CU(cudaMemsetAsync(b->d_prev.get(), 0, static_cast<size_t>(b->n) * sizeof(int16_t), st));
   if (b->d_seg) CU(cudaMemsetAsync(b->d_seg.get(), 0, b->seg_bytes, st));
   return 0;
 }
 
 int vadb200_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labels, float* d_logits, void* stream) {
   return launch_stream_feed(b, d_chunks, d_labels, d_logits, nullptr, nullptr, stream);
+}
+
+int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const int64_t* d_offsets, int32_t* d_counts,
+                               uint8_t* d_labels, float* d_logits, uint8_t* d_rows, int64_t* d_bounds, void* stream) {
+  if (!b || !d_samples || !d_offsets || !d_counts || !d_labels) return fail(VADB200_E_INVALID, "null argument");
+  if (!b->max_feed) return fail(VADB200_E_STATE, "not a ragged bank (vadb200_stream_bank_create_ragged)");
+  vadb200_handle* h = b->h;
+  if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if ((d_rows || d_bounds) && !b->d_seg) return fail(VADB200_E_STATE, "speech is off (vadb200_stream_bank_set_speech)");
+  if (reinterpret_cast<uintptr_t>(d_samples) & 1) return fail(VADB200_E_INVALID, "samples must be 2-byte aligned");
+  CU(cudaSetDevice(h->device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  RaggedParams rp;
+  rp.n_streams = b->n; rp.max_feed = b->max_feed; rp.ring_len = b->ring_len; rp.max_rows = ragged_max_rows(b->max_feed);
+  rp.pcm = b->d_pcm.get(); rp.total = b->d_total.get(); rp.ring = b->d_ring.get();
+  rp.samples = d_samples; rp.offsets = reinterpret_cast<const long long*>(d_offsets);
+  rp.counts = d_counts; rp.labels = d_labels; rp.logits = d_logits; rp.rows = d_rows; rp.bounds = d_bounds;
+  rp.tw1 = h->d_tw.get(); rp.tw2 = h->d_tw.get() + 256; rp.feat_mode = VADB200_FEAT_ANALYSER;
+  rp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
+  const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
+  return launched(1, [&] {
+    if (b->d_seg)  // speech on: every feed advances the segment state
+      stream_ragged_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par,
+                                                                                      bank_seg(b, nullptr, nullptr));
+    else
+      stream_ragged_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par);
+  });
 }
 
 int vadb200_stream_bank_set_speech(vadb200_bank* b, int enable, int min_speech_rows, int min_silence_rows,
@@ -988,6 +1054,13 @@ int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end, uint8
   const StreamSeg g = bank_seg(b, nullptr, nullptr);
   const int words = g.meta ? (g.d1 ? seg_ring_words(g.d1) : 0) + (g.d2 ? seg_ring_words(g.d2) : 0) : 0;
   const size_t smem = static_cast<size_t>(words) * kSegEndThreads * sizeof(uint32_t);
+  const unsigned grid = (b->n + kSegEndThreads - 1) / kSegEndThreads;
+  if (b->max_feed)
+    return launched(1, [&] {
+      stream_end_ragged_kernel<<<grid, kSegEndThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+          g, d_end, b->n, b->d_total.get(), b->d_ring.get(), g.meta ? d_tail_rows : nullptr,
+          g.meta ? d_tail_bounds : nullptr);
+    });
   return launched(1, [&] {
     stream_end_kernel<<<(b->n + kSegEndThreads - 1) / kSegEndThreads, kSegEndThreads, smem,
                         static_cast<cudaStream_t>(stream)>>>(g, d_end, b->n, b->d_hist.get(), b->d_ring.get(),

@@ -383,12 +383,19 @@ def speech_ms_to_rows(ms):
 
 
 class StreamBankHandle(object):
-    def __init__(self, handle, n_streams):
+    """A stream bank.  With ``max_feed_samples`` (1 .. 16000) it is a ragged bank: each feed takes any number of
+    samples per stream up to that cap (``feed_ragged_ptr``) instead of one 160-sample chunk (``feed_ptr``)."""
+
+    def __init__(self, handle, n_streams, max_feed_samples=None):
         self.handle = handle
         self.lib = handle.lib
         self.n = int(n_streams)
+        self.max_feed = None if max_feed_samples is None else int(max_feed_samples)
         self._b = C.c_void_p()
-        check(self.lib.vadb200_stream_bank_create(handle._h, self.n, C.byref(self._b)))
+        if self.max_feed is None:
+            check(self.lib.vadb200_stream_bank_create(handle._h, self.n, C.byref(self._b)))
+        else:
+            check(self.lib.vadb200_stream_bank_create_ragged(handle._h, self.n, self.max_feed, C.byref(self._b)))
 
     def close(self):
         if getattr(self, "_b", None) is not None and self._b:
@@ -407,6 +414,20 @@ class StreamBankHandle(object):
     def feed_ptr(self, chunks_ptr, labels_ptr, logits_ptr=0, stream=None):
         check(self.lib.vadb200_stream_feed(self._b, C.c_void_p(chunks_ptr), C.c_void_p(labels_ptr),
                                            C.c_void_p(logits_ptr), stream if stream is not None else self.handle.stream))
+
+    def max_rows_per_feed(self):
+        """K: the most rows one ragged feed emits per stream (-1 for a fixed bank)."""
+        return int(self.lib.vadb200_stream_bank_max_rows_per_feed(self._b))
+
+    def feed_ragged_ptr(self, samples_ptr, offsets_ptr, counts_ptr, labels_ptr, logits_ptr=0, rows_ptr=0,
+                        bounds_ptr=0, stream=None):
+        """vadb200_stream_feed_ragged: samples int16, offsets int64 [n + 1], counts int32 [n], labels uint8 [n][K],
+        logits float32 [n][K][3], rows uint8 [n][K], bounds int64 [n][K] (0: NULL)."""
+        check(self.lib.vadb200_stream_feed_ragged(self._b, C.c_void_p(samples_ptr), C.c_void_p(offsets_ptr),
+                                                  C.c_void_p(counts_ptr), C.c_void_p(labels_ptr),
+                                                  C.c_void_p(logits_ptr), C.c_void_p(rows_ptr),
+                                                  C.c_void_p(bounds_ptr),
+                                                  stream if stream is not None else self.handle.stream))
 
     # ---- speech segments (vadb200_stream_bank_set_speech) -------------------------------------------
     def set_speech(self, min_speech_rows, min_silence_rows, pad_rows):
