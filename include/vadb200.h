@@ -87,9 +87,13 @@ int vadb200_set_ffn_weights(vadb200_handle* h, const float* W1, const float* b1,
                             const float* b2, const float* W3, const float* b3, const float* W4,
                             const float* b4);
 
-/* Where the FFN contraction runs: 0 = FP32 CUDA cores (constant-bank FFMA), 1 = tcgen05 tensor cores
- * (kind::tf32, operands split hi/lo into three MMAs, fp32 accumulation in TMEM; the default).  Both
- * meet the logit tolerance; applies to vadb200_vad_packed / vadb200_vad_host / vadb200_ffn_predict. */
+/* Where the FFN contraction runs: 0 = FP32 CUDA cores (constant-bank FFMA); 1 = tcgen05 tensor cores,
+ * kind::tf32 (operands split hi/lo into three products, fp32 accumulation in TMEM); 2 = tcgen05 kind::f16
+ * on statically scaled fp16 hi/lo operands (the default; weights whose scales would be out of range keep
+ * impl 1, and vadb200_ffn_predict runs any 128-row tile holding a row beyond the feature bounds on impl 1).
+ * All three meet the logit tolerance; applies to vadb200_vad_packed / vadb200_vad_host / vadb200_ffn_predict.
+ * For any impl, vadb200_ffn_predict on the feature rows the fused VAD path returns reproduces its labels and
+ * logits bit for bit. */
 int vadb200_set_ffn_impl(vadb200_handle* h, int impl);
 int vadb200_get_ffn_impl(vadb200_handle* h);
 

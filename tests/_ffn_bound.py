@@ -20,8 +20,8 @@ Per implementation (u = 2^-24, the fp32 unit roundoff):
 * ``tc`` (ffn_tc_tile, tf32 hi/lo): x = x_hi + x_lo with x_hi the top 11 significant bits (truncation) and x_lo read
   by the tensor core as tf32, i.e. truncated to 11 bits, which loses the 2 lowest bits of x (< 2^-21 |x|); the
   dropped x_lo w_lo is < 2^-20 |x w|.  Per product: u_prod = 2^-20 + 2 x 2^-21 = 2^-19.
-* ``tc16`` (ffn_tc16_tile: every layer on the 2N scheme) and ``tc16_tile2`` (ffn_tc16_tile2: layer 1 on one
-  accumulator): operands a = h pre[l] and w sw_l, split to nearest in fp16.  Each split half errs by at most 2^-11 of
+* ``tc16`` (ffn_tc16_tile: layer 1 on one accumulator, layers 2-4 on the 2N scheme): operands a = h pre[l] and
+  w sw_l, split to nearest in fp16.  Each split half errs by at most 2^-11 of
   what it rounds, or by half the fp16 subnormal spacing (2^-25) where it is subnormal, so a - a_hi - a_lo is within
   2^-22 |a| + 2^-25, and the dropped a_lo w_lo adds 2^-22 |a w|.  Per product, in unscaled units:
   3 x 2^-22 |h w| + 2^-25 (|w| / pre[l] + |h| / sw_l).  The scales are the ones tc16_pack_weights chooses
@@ -32,7 +32,7 @@ sum has not been measured, so each MMA instruction (8 tf32 or 16 fp16 products p
 truncate its result to fp32 once, toward zero: an error below 2 u |partial sum| <= 2 u |W|^T H.  A layer's output
 sees one such rounding per instruction that accumulates into its column: 2 K/g on the 2N scheme (a_hi B_hi and
 a_lo B_hi share the first N columns; a_hi B_lo goes to the second N, whose sum is below 2^-9 of the first), 3 K/g on
-the single accumulator of tc16_tile2's layer 1.  K is the padded depth (48, 64, 32, 16).  The epilogue adds the two
+the single accumulator of tc16's layer 1.  K is the padded depth (48, 64, 32, 16).  The epilogue adds the two
 halves and the bias (tc) or runs one FFMA with the folded constants (tc16), each rounded to nearest: 2 u (|W|^T H +
 |b|).  Everything above is first order; the constants carry a 2^-9 margin for the second-order terms.
 """
@@ -49,7 +49,7 @@ FFN_KEYS = ("W1", "b1", "W2", "b2", "W3", "b3", "W4", "b4")
 K_PAD = (48, 64, 32, 16)       # kTcK1 .. kTcK4
 N_PAD = (64, 32, 16, 16)       # kTcN1 .. kTcN4
 FEAT_BOUND = np.repeat([1353.0, 2706.0, 5416.0], 13)   # kFeatBoundZ / D1 / D2 (ffn_tc.cuh)
-IMPLS = ("fp32", "tc", "tc16", "tc16_tile2")
+IMPLS = ("fp32", "tc", "tc16")
 U = 2.0 ** -24
 MARGIN = 1.0 + 2.0 ** -9
 
@@ -146,10 +146,10 @@ def relu_keep(z, e):
 
 def ffn_bound(x, w, impl, scales=None):
     """[n, 3] float64 bound on |device logit - float64 logit| of ``impl`` (one of IMPLS) on float32 rows ``x``.
-    ``scales``: tc16_scales(w), computed when None (tc16 impls only)."""
+    ``scales``: tc16_scales(w), computed when None (tc16 only)."""
     if impl not in IMPLS:
         raise ValueError(impl)
-    fp16 = impl.startswith("tc16")
+    fp16 = impl == "tc16"
     if fp16:
         ok, pre, _, sw = scales if scales is not None else tc16_scales(w)
         if not ok:
@@ -168,7 +168,7 @@ def ffn_bound(x, w, impl, scales=None):
             d = K * U / (1 - K * U) * (HW + b)
         else:
             g = 16 if fp16 else 8
-            n_acc = (3 if (impl == "tc16_tile2" and l == 0) else 2) * K_PAD[l] // g
+            n_acc = (3 if (fp16 and l == 0) else 2) * K_PAD[l] // g
             d = 2 * U * n_acc * HW * (1 + 2.0 ** -9)               # truncating accumulation (the a_hi B_lo half below)
             d += 2 * U * (HW + b)                                  # epilogue: two roundings to nearest
             if fp16:

@@ -1,10 +1,10 @@
 """CPU: the per-entry logit bound of tests/_ffn_bound.py against numpy emulations of each device FFN scheme.
 
 The emulations follow the kernels' arithmetic step by step: ffn_forward's FFMA order (fp32), ffn_tc_tile's tf32
-hi/lo split (tc), and the fp16 hi/lo schemes on the very blob tc16_pack_weights packs (read back through
-tests/emul/emul_ffn.cpp and de-swizzled with tc16_pack_layer's index formula): ffn_tc16_tile with every layer on the
-2N scheme, and ffn_tc16_tile2 with layer 1 on one accumulator.  Each tensor-core instruction's sum is truncated to
-fp32, the accumulation the bound assumes.  Every faithful emulation stays within a quarter of the bound; every
+hi/lo split (tc), and ffn_tc16_tile's fp16 hi/lo scheme (tc16: layer 1 on one accumulator, layers 2-4 on the 2N
+scheme) on the very blob tc16_pack_weights packs (read back through tests/emul/emul_ffn.cpp and de-swizzled with
+tc16_pack_layer's index formula).  Each tensor-core instruction's sum is truncated to fp32, the accumulation the
+bound assumes.  Every faithful emulation stays within a quarter of the bound; every
 mutant -- a product dropped in one layer, a subnormal lo flushed, a scale off by two, an unscaled bias, a shifted
 layer-1 column -- exceeds it at least five-fold somewhere."""
 import numpy as np
@@ -123,8 +123,8 @@ def emul_tc(x, w, pk):
         a = np.maximum(z, np.float32(0))
 
 
-def emul_tc16(x, w, pk, tile2, drop=None, flush_lo=False, pre2=None, post2=None, bias_unscaled=False, shift=0):
-    """ffn_tc16_tile (tile2 False) or ffn_tc16_tile2 (True).  Mutations: drop = (layer, "hh" | "hl" | "lh");
+def emul_tc16(x, w, pk, drop=None, flush_lo=False, pre2=None, post2=None, bias_unscaled=False, shift=0):
+    """ffn_tc16_tile.  Mutations: drop = (layer, "hh" | "hl" | "lh");
     flush_lo: subnormal lo halves of the activations become 0; pre2 / post2 = layer whose activation pre-scale /
     weight post-scale is doubled; bias_unscaled: c_l = b_l; shift: layer-1 features one column off."""
     postp = f32(pk["postp"]).copy()
@@ -151,7 +151,7 @@ def emul_tc16(x, w, pk, tile2, drop=None, flush_lo=False, pre2=None, post2=None,
         prods = {"hh": (ah, bh), "hl": (ah, bl), "lh": (al, bh)}
         live = [p for p in ("hh", "hl", "lh") if drop != (l, p)]
         zero = np.zeros((a.shape[0], N), np.float32)
-        if tile2 and l == 0:
+        if l == 0:
             d = mma_chain(zero, [prods[p] for p in live], 16)
         else:
             v = mma_chain(zero, [prods[p] for p in live if p != "hl"], 16)
@@ -167,7 +167,7 @@ def emulate(impl, x, w, pk):
         return emul_fp32(x, w)
     if impl == "tc":
         return emul_tc(x, w, pk)
-    return emul_tc16(x, w, pk, impl == "tc16_tile2")
+    return emul_tc16(x, w, pk)
 
 
 # ---- test rows ------------------------------------------------------------------------------------------------------
@@ -255,20 +255,19 @@ def mutants():
 
 
 @pytest.mark.parametrize("name", MUTANT_SETS)
-@pytest.mark.parametrize("tile2", [True, False])
-def test_mutants_exceed_the_bound_five_fold(name, tile2):
+def test_mutants_exceed_the_bound_five_fold(name):
     """A kernel that loses a product, a lo half, a scale or a column is caught with a margin.  The unscaled-bias
     mutant computes the faithful function where every c_l equals b_l (zero biases, or pre[l+1] == 1 throughout) and
     is only required where it differs."""
     w = SETS[name]
     pk = fb.pack(w)
     ref = fb.forward64(ROWS, w)[0][3]
-    bound = bound_of(name, "tc16_tile2" if tile2 else "tc16")
+    bound = bound_of(name, "tc16")
     weak = {}
     for mname, kw in mutants().items():
         if mname == "bias unscaled" and all(np.array_equal(pk["c"][l], f32(w["b%d" % (l + 1)])) for l in range(3)):
             continue
-        got = emul_tc16(ROWS, w, pk, tile2, **kw)
+        got = emul_tc16(ROWS, w, pk, **kw)
         worst = np.nanmax(np.abs(got - ref) / bound)
         if not worst >= 5.0:
             weak[mname] = worst

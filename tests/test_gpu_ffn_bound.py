@@ -4,7 +4,7 @@ own float32 inputs, and every label against the decision rule applied to the dev
 Inputs are the features the fused kernel writes (want_feats), the windows' features vad_windows writes, and the rows
 given to ffn_predict, so MFCC and feature error play no part and the bound can be tight.  Kernels reached:
 
-* fused_kernel / fused_fe_kernel <2, 2> (ffn_tc16_tile2), <2, 1> (ffn_tc_tile<2>), <2, 0> (classify_row / ffn_forward)
+* fused_kernel / fused_fe_kernel <2, 2> (ffn_tc16_tile<2>), <2, 1> (ffn_tc_tile<2>), <2, 0> (classify_row / ffn_forward)
   under FEAT_ANALYSER and FEAT_DATASET, on utterances whose last block phase holds 1 to 256 centres, catalogue
   signals and digital silence, with segment ends mid-phase;
 * ffn_tc_rows_kernel<2> (ffn_tc16_tile<1>, and its per-tile fall-back to the tf32 blob), ffn_tc_rows_kernel<1>,
@@ -72,11 +72,11 @@ def handles():
             print("  %-34s %-11s %.4f" % (k[0], k[1], WORST[k]))
 
 
-def bound_impl(name, impl, fused):
+def bound_impl(name, impl):
     if impl == "fp32":
         return "fp32"
     if impl == "tc16" and fb.tc16_scales(SETS[name])[0]:
-        return "tc16_tile2" if fused else "tc16"
+        return "tc16"
     return "tc"
 
 
@@ -140,7 +140,7 @@ def test_fused_vad_logits_within_bound(handles, name, fe):
                     torch.cuda.synchronize()
                     labels, logits, feats = labels.cpu().numpy(), logits.cpu().numpy(), feats.cpu().numpy()
                     check("fused%s sf=%d" % ("_fe" if fe else "", sf) if sf in (0, 2048) else
-                          "fused%s mid-phase" % ("_fe" if fe else ""), name, bound_impl(name, impl, True),
+                          "fused%s mid-phase" % ("_fe" if fe else ""), name, bound_impl(name, impl),
                           feats, logits, labels, THETA if fe else None)
                     per_impl[(impl, fm)] = logits
             if name == "beyond_ea61":          # tc16 keeps the tf32 path
@@ -204,7 +204,7 @@ def test_ffn_predict_logits_within_bound(handles, name):
                 tiles[128 * t:128 * (t + 1)] = True
             for impl in IMPLS:
                 labels, logits = got[impl]
-                bi = bound_impl(name, impl, False)
+                bi = bound_impl(name, impl)
                 if bi == "tc16":               # tiles holding a wide row run on the tf32 blob: tc's logits bit for bit
                     assert np.array_equal(logits[tiles].view(np.uint32), got["tc"][1][tiles].view(np.uint32)), n
                     check("ffn_predict", name, "tc", x[tiles], logits[tiles], labels[tiles])

@@ -453,19 +453,6 @@ __host__ __device__ constexpr uint32_t tc16_idesc(int n) {
   return (1u << 4) /* D = f32; A = B = f16 (format 0), both K-major */ | (static_cast<uint32_t>(n >> 3) << 17) |
          (static_cast<uint32_t>(128 >> 4) << 24);
 }
-template <int K, int N>
-__device__ __forceinline__ void tc16_issue_layer(uint32_t tm_base, uint32_t d_col, uint32_t w_smem, uint64_t* done_bar) {
-  constexpr uint32_t lbo = (2 * N / 8) * 128, sbo = 128;   // core matrix = 8 rows x 8 fp16
-  constexpr uint32_t idesc_2n = tc16_idesc(2 * N), idesc_n = tc16_idesc(N);
-  const uint32_t a_hi = tm_base + kTmA, a_lo = tm_base + kTmA + K / 2, d = tm_base + d_col;
-#pragma unroll
-  for (int j = 0; j < K / 16; ++j) {
-    const uint64_t b = tc_smem_desc(w_smem + 2 * j * lbo, lbo, sbo);
-    umma_f16_ts(d, a_hi + 8 * j, b, idesc_2n, j > 0 ? 1u : 0u);
-    umma_f16_ts(d, a_lo + 8 * j, b, idesc_n, 1u);
-  }
-  umma_commit(done_bar);
-}
 // (x0, x1) -> one 32-bit word of hi parts and one of lo parts (element 0 in the low half); the residual is one FADD2
 __device__ __forceinline__ void tc16_split2(f2 x, uint32_t& hi, uint32_t& lo) {
   const __half2 h = __floats2half2_rn(x.x, x.y);
@@ -475,43 +462,30 @@ __device__ __forceinline__ void tc16_split2(f2 x, uint32_t& hi, uint32_t& lo) {
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
-// Epilogue of a hidden layer: D (NOUT fp32 columns at d_col, second half NOUT further) -> x (post-scale x next layer's
-// pre-scale), + scaled bias, ReLU, fp16 hi/lo split -> A operand of the next layer.  Column pairs are processed with
-// packed fp32 arithmetic (tcgen05.ld delivers neighbouring columns in neighbouring registers).
-// cbias: bias x next pre-scale (FfnBias::c1..c3), postp: FfnBias::postp[l].
-template <int NOUT, int HALVES>
-__device__ __forceinline__ void tc16_hidden_epilogue(uint32_t tl, uint32_t d_col, const float* cbias, float postp,
-                                                     int hidx) {
-  constexpr int W = NOUT / HALVES;         // fp32 columns per thread: 64, 32, 16 or 8
-  constexpr int CH = W >= 16 ? 16 : 8;
-  const int base = hidx * W;
+// Epilogue of a hidden layer on the 2N scheme: D (NOUT fp32 columns at d_col, second half NOUT further) -> x (post-scale
+// x next layer's pre-scale), + scaled bias, ReLU, fp16 hi/lo split -> A operand of the next layer.  Column pairs are
+// processed with packed fp32 arithmetic (tcgen05.ld delivers neighbouring columns in neighbouring registers).  One
+// thread per frame.  cbias: bias x next pre-scale (FfnBias::c1..c3), postp: FfnBias::postp[l].
+template <int NOUT>
+__device__ __forceinline__ void tc16_hidden_epilogue(uint32_t tl, uint32_t d_col, const float* cbias, float postp) {
+  static_assert(NOUT % 16 == 0, "16-column chunks");
 #pragma unroll
-  for (int c0 = 0; c0 < W; c0 += CH) {
-    uint32_t v[CH], u[CH], hi[CH / 2], lo[CH / 2];
-    if constexpr (CH == 16) {
-      tmem_ld16(tl + d_col + base + c0, v);
-      tmem_ld16(tl + d_col + NOUT + base + c0, u);
-    } else {
-      tmem_ld8(tl + d_col + base + c0, v);
-      tmem_ld8(tl + d_col + NOUT + base + c0, u);
-    }
+  for (int c0 = 0; c0 < NOUT; c0 += 16) {
+    uint32_t v[16], u[16], hi[8], lo[8];
+    tmem_ld16(tl + d_col + c0, v);
+    tmem_ld16(tl + d_col + NOUT + c0, u);
     tmem_wait_ld();
 #pragma unroll
-    for (int i = 0; i < CH; i += 2) {
+    for (int i = 0; i < 16; i += 2) {
       const f2 d = vadd(mk2(__uint_as_float(v[i]), __uint_as_float(v[i + 1])),
                         mk2(__uint_as_float(u[i]), __uint_as_float(u[i + 1])));
-      f2 a = vfma(d, mk2(postp, postp), mk2(cbias[base + c0 + i], cbias[base + c0 + i + 1]));
+      f2 a = vfma(d, mk2(postp, postp), mk2(cbias[c0 + i], cbias[c0 + i + 1]));
       a.x = fmaxf(a.x, 0.0f);
       a.y = fmaxf(a.y, 0.0f);
       tc16_split2(a, hi[i / 2], lo[i / 2]);
     }
-    if constexpr (CH == 16) {
-      tmem_st8(tl + kTmA + (base + c0) / 2, hi);
-      tmem_st8(tl + kTmA + NOUT / 2 + (base + c0) / 2, lo);
-    } else {
-      tmem_st4(tl + kTmA + (base + c0) / 2, hi);
-      tmem_st4(tl + kTmA + NOUT / 2 + (base + c0) / 2, lo);
-    }
+    tmem_st8(tl + kTmA + c0 / 2, hi);
+    tmem_st8(tl + kTmA + NOUT / 2 + c0 / 2, lo);
   }
   tmem_wait_st();
 }
@@ -529,80 +503,29 @@ __device__ __forceinline__ void tc16_store_a1_half(uint32_t tl, int hidx, const 
   tmem_st8(b + kTcK1 / 2, lo);
   tmem_st4(b + kTcK1 / 2 + 8, lo4);
 }
-// The whole FFN for one 128-frame tile on fp16 operands; same contract as ffn_tc_tile.
-template <int HALVES>
-__device__ __forceinline__ uint32_t ffn_tc16_tile(const FfnBias& fb, float (&logit)[kNCls], uint32_t tm_base, int wq,
-                                                  int hidx, bool is_issuer, uint32_t w_smem, uint64_t* mma_bar,
-                                                  uint32_t par) {
-  const uint32_t tl = tm_base + (static_cast<uint32_t>(32 * wq) << 16);
-  tmem_wait_st();
-  tc_fence_before();
-  tc_bar<HALVES>();
-  if (is_issuer) {
-    tc_fence_after();
-    tc16_issue_layer<kTcK1, kTcN1>(tm_base, kTmD1, w_smem + kTc16Off1, mma_bar);
-  }
-  tc_mbar_wait(mma_bar, par); par ^= 1u;
-  tc_fence_after();
-  tc16_hidden_epilogue<kTcN1, HALVES>(tl, kTmD1, fb.c1, fb.postp[0], hidx);
-  tc_fence_before();
-  tc_bar<HALVES>();
-  if (is_issuer) {
-    tc_fence_after();
-    tc16_issue_layer<kTcK2, kTcN2>(tm_base, kTmD2, w_smem + kTc16Off2, mma_bar);
-  }
-  tc_mbar_wait(mma_bar, par); par ^= 1u;
-  tc_fence_after();
-  tc16_hidden_epilogue<kTcN2, HALVES>(tl, kTmD2, fb.c2, fb.postp[1], hidx);
-  tc_fence_before();
-  tc_bar<HALVES>();
-  if (is_issuer) {
-    tc_fence_after();
-    tc16_issue_layer<kTcK3, kTcN3>(tm_base, kTmD3, w_smem + kTc16Off3, mma_bar);
-  }
-  tc_mbar_wait(mma_bar, par); par ^= 1u;
-  tc_fence_after();
-  tc16_hidden_epilogue<kTcN3, HALVES>(tl, kTmD3, fb.c3, fb.postp[2], hidx);
-  tc_fence_before();
-  tc_bar<HALVES>();
-  if (is_issuer) {
-    tc_fence_after();
-    tc16_issue_layer<kTcK4, kTcN4>(tm_base, kTmD4, w_smem + kTc16Off4, mma_bar);
-  }
-  tc_mbar_wait(mma_bar, par); par ^= 1u;
-  tc_fence_after();
-  if (hidx == 0) {
-    uint32_t v[8], u[8];
-    tmem_ld8(tl + kTmD4, v);
-    tmem_ld8(tl + kTmD4 + kTcN4, u);
-    tmem_wait_ld();
-#pragma unroll
-    for (int o = 0; o < kNCls; ++o) logit[o] = fmaf(__uint_as_float(v[o]) + __uint_as_float(u[o]), fb.post[3], fb.b4[o]);
-  }
-  tc_fence_before();  // the next tile's tcgen05.st must not overtake these loads
-  return par;
-}
 
-// ================================ two fp16 tiles per block phase ======================================
-// The fused kernel's TC = 2 block phase: 256 frames, thread = frame, warp w serves tile w / 4 on TMEM lane quarter
-// w % 4.  Tile t owns columns [128 t, 128 t + 128) of the CTA's 256: the A operand (packed hi | lo, at most 32 + 32
-// columns) in the first 64, the fp32 accumulators in the last 64.  Layer 1's 2N scheme would need 2 x 64 accumulator
-// columns, so layer 1 accumulates all three products into ONE 64-column accumulator, per k-step in the order
-// a_hi.B_hi, a_hi.B_lo, a_lo.B_hi (B_lo is the same descriptor N/8 core matrices further on: the blob is unchanged).
-// Layers 2-4 keep the 2N scheme (2 x 32, 2 x 16 and 2 x 16 columns fit); with one accumulator they ran 0.7 % slower.
-// The block phase's fixed costs (barriers, synchronous DCT, blob copy, four MMA round trips) are paid once per 256
-// frames instead of once per 128.  Each epilogue overwrites A only after that layer's MMAs have completed.
+// ================================ fp16 tiles: one or two per CTA ======================================
+// TILES = 2 is the fused kernel's block phase: 256 frames, thread = frame, warp w serves tile w / 4 on TMEM lane quarter
+// w % 4.  TILES = 1 is ffn_tc_rows_kernel's 128-row tile on warps 0-3.  Tile t owns columns [128 t, 128 t + 128) of the
+// CTA's 256: the A operand (packed hi | lo, at most 32 + 32 columns) in the first 64, the fp32 accumulators in the last
+// 64.  Layer 1's 2N scheme would need 2 x 64 accumulator columns, so layer 1 accumulates all three products into ONE
+// 64-column accumulator, per k-step in the order a_hi.B_hi, a_hi.B_lo, a_lo.B_hi (B_lo is the same descriptor N/8 core
+// matrices further on: the blob is unchanged).  Layers 2-4 keep the 2N scheme (2 x 32, 2 x 16 and 2 x 16 columns fit);
+// with one accumulator they ran 0.7 % slower.  The fused block phase's fixed costs (barriers, synchronous DCT, blob
+// copy, four MMA round trips) are paid once per 256 frames instead of once per 128.  Each epilogue overwrites A only
+// after that layer's MMAs have completed.
 constexpr int kTm2Tile = 128;                                      // TMEM columns per tile
 constexpr int kTm2D1 = 64, kTm2D2 = 64, kTm2D3 = 64, kTm2D4 = 96;  // accumulators, relative to the tile
 static_assert(2 * kTm2Tile == kTmemCols && kTm2D1 + kTcN1 <= kTm2Tile && kTm2D2 + 2 * kTcN2 <= kTm2Tile &&
               kTm2D4 + 2 * kTcN4 <= kTm2Tile && kTcK2 <= kTm2D1, "two tiles share the CTA's TMEM allocation");
 
-// One layer of both tiles (tile 1 only if two_tiles), interleaved MMA by MMA so that the tensor pipe always has an
+// One layer of tile 0 and, if two_tiles, tile 1, interleaved MMA by MMA so that the tensor pipe always has an
 // independent instruction between two that accumulate into the same columns; one commit.  Executed by ONE thread.
-// ONE_ACC: a_hi.B_hi, a_hi.B_lo, a_lo.B_hi into N columns; otherwise the 2N scheme of tc16_issue_layer.
+// ONE_ACC: a_hi.B_hi, a_hi.B_lo, a_lo.B_hi into N columns; otherwise a_hi . [B_hi | B_lo] into 2N columns and
+// a_lo . B_hi into the first N.
 template <int K, int N, bool ONE_ACC>
-__device__ __forceinline__ void tc16_issue_layer2(uint32_t tm_base, uint32_t d_col, uint32_t w_smem, bool two_tiles,
-                                                  uint64_t* done_bar) {
+__device__ __forceinline__ void tc16_issue_layer(uint32_t tm_base, uint32_t d_col, uint32_t w_smem, bool two_tiles,
+                                                 uint64_t* done_bar) {
   constexpr uint32_t lbo = (2 * N / 8) * 128, sbo = 128, lo_off = (N / 8) * 128;
   constexpr int kMmas = ONE_ACC ? 3 : 2;
 #pragma unroll
@@ -643,26 +566,30 @@ __device__ __forceinline__ void tc16_epilogue_1acc(uint32_t tl, uint32_t d_col, 
   }
   tmem_wait_st();
 }
-// The whole FFN for two 128-frame tiles, executed by 256 threads; each thread has stored both halves of its frame's
-// layer-1 A operand (tc16_store_a1_half at tl = ffn_tc16_tile2_lane(...)) and gets its frame's logits.  two_tiles
-// (block-uniform) false: tile 1 holds no valid frame and its MMAs are not issued (the epilogues of warps 4-7 then work
-// on stale columns and their logits are meaningless).  mma_bar / par as in ffn_tc_tile; ts: clock64 stamps 3..15
-// (timing experiments only, same stages as ffn_tc_tile's).
-__device__ __forceinline__ uint32_t ffn_tc16_tile2_lane(uint32_t tm_base, int warp) {
+// The whole FFN for TILES 128-frame tiles, executed by 128 TILES threads; each thread has stored both halves of its
+// frame's layer-1 A operand (tc16_store_a1_half at tl = ffn_tc16_tile_lane(...)) and gets its frame's logits.
+// two_tiles (TILES = 2 only, block-uniform) false: tile 1 holds no valid frame and its MMAs are not issued (the
+// epilogues of warps 4-7 then work on stale columns and their logits are meaningless).  w_smem: shared-memory address
+// of the fp16 weight blob (already landed); mma_bar: mbarrier (count 1) whose current phase parity is `par` (4
+// phases).  ts: clock64 stamps 3..15 (timing experiments only, same stages as ffn_tc_tile's).
+__device__ __forceinline__ uint32_t ffn_tc16_tile_lane(uint32_t tm_base, int warp) {
   return tm_base + kTm2Tile * static_cast<uint32_t>(warp >> 2) + (static_cast<uint32_t>(32 * (warp & 3)) << 16);
 }
-__device__ __forceinline__ uint32_t ffn_tc16_tile2(const FfnBias& fb, float (&logit)[kNCls], uint32_t tm_base, int warp,
-                                                   bool two_tiles, bool is_issuer, uint32_t w_smem, uint64_t* mma_bar,
-                                                   uint32_t par, long long* ts = nullptr) {
-  const uint32_t tl = ffn_tc16_tile2_lane(tm_base, warp);
+template <int TILES>
+__device__ __forceinline__ uint32_t ffn_tc16_tile(const FfnBias& fb, float (&logit)[kNCls], uint32_t tm_base, int warp,
+                                                  bool two_tiles, bool is_issuer, uint32_t w_smem, uint64_t* mma_bar,
+                                                  uint32_t par, long long* ts = nullptr) {
+  static_assert(TILES == 1 || TILES == 2, "one or two tiles");
+  const uint32_t tl = ffn_tc16_tile_lane(tm_base, warp);
+  two_tiles = TILES == 2 && two_tiles;
 #define VADB_TS(i) do { if (ts) ts[i] = clock64(); } while (0)
   tmem_wait_st();
   tc_fence_before();
-  tc_bar<2>();
+  tc_bar<TILES>();
   VADB_TS(3);
   if (is_issuer) {
     tc_fence_after();
-    tc16_issue_layer2<kTcK1, kTcN1, true>(tm_base, kTm2D1, w_smem + kTc16Off1, two_tiles, mma_bar);
+    tc16_issue_layer<kTcK1, kTcN1, true>(tm_base, kTm2D1, w_smem + kTc16Off1, two_tiles, mma_bar);
   }
   VADB_TS(4);
   tc_mbar_wait(mma_bar, par); par ^= 1u;
@@ -671,34 +598,34 @@ __device__ __forceinline__ uint32_t ffn_tc16_tile2(const FfnBias& fb, float (&lo
   tc16_epilogue_1acc<kTcN1>(tl, kTm2D1, fb.c1, fb.postp[0]);
   VADB_TS(6);
   tc_fence_before();
-  tc_bar<2>();
+  tc_bar<TILES>();
   if (is_issuer) {
     tc_fence_after();
-    tc16_issue_layer2<kTcK2, kTcN2, false>(tm_base, kTm2D2, w_smem + kTc16Off2, two_tiles, mma_bar);
+    tc16_issue_layer<kTcK2, kTcN2, false>(tm_base, kTm2D2, w_smem + kTc16Off2, two_tiles, mma_bar);
   }
   VADB_TS(7);
   tc_mbar_wait(mma_bar, par); par ^= 1u;
   tc_fence_after();
   VADB_TS(8);
-  tc16_hidden_epilogue<kTcN2, 1>(tl, kTm2D2, fb.c2, fb.postp[1], 0);
+  tc16_hidden_epilogue<kTcN2>(tl, kTm2D2, fb.c2, fb.postp[1]);
   VADB_TS(9);
   tc_fence_before();
-  tc_bar<2>();
+  tc_bar<TILES>();
   if (is_issuer) {
     tc_fence_after();
-    tc16_issue_layer2<kTcK3, kTcN3, false>(tm_base, kTm2D3, w_smem + kTc16Off3, two_tiles, mma_bar);
+    tc16_issue_layer<kTcK3, kTcN3, false>(tm_base, kTm2D3, w_smem + kTc16Off3, two_tiles, mma_bar);
   }
   VADB_TS(10);
   tc_mbar_wait(mma_bar, par); par ^= 1u;
   tc_fence_after();
   VADB_TS(11);
-  tc16_hidden_epilogue<kTcN3, 1>(tl, kTm2D3, fb.c3, fb.postp[2], 0);
+  tc16_hidden_epilogue<kTcN3>(tl, kTm2D3, fb.c3, fb.postp[2]);
   VADB_TS(12);
   tc_fence_before();
-  tc_bar<2>();
+  tc_bar<TILES>();
   if (is_issuer) {
     tc_fence_after();
-    tc16_issue_layer2<kTcK4, kTcN4, false>(tm_base, kTm2D4, w_smem + kTc16Off4, two_tiles, mma_bar);
+    tc16_issue_layer<kTcK4, kTcN4, false>(tm_base, kTm2D4, w_smem + kTc16Off4, two_tiles, mma_bar);
   }
   VADB_TS(13);
   tc_mbar_wait(mma_bar, par); par ^= 1u;
@@ -712,7 +639,7 @@ __device__ __forceinline__ uint32_t ffn_tc16_tile2(const FfnBias& fb, float (&lo
 #pragma unroll
     for (int o = 0; o < kNCls; ++o) logit[o] = fmaf(__uint_as_float(v[o]) + __uint_as_float(u[o]), fb.post[3], fb.b4[o]);
   }
-  tc_fence_before();  // the next block phase's tcgen05.st must not overtake these loads
+  tc_fence_before();  // the next tile's tcgen05.st must not overtake these loads
   VADB_TS(15);
 #undef VADB_TS
   return par;

@@ -265,6 +265,34 @@ __device__ __forceinline__ void flush_flat(float* dst, int total, int tid, GEN&&
   }
 }
 
+// The rule every classifier path applies to its decision `lab`: a row with a non-finite feature (ok false) gets label
+// 0 and NaN logits.
+__device__ __forceinline__ uint8_t reject_nonfinite(bool ok, uint8_t lab, float (&logit)[kNCls]) {
+  if (!ok) {
+    logit[0] = logit[1] = logit[2] = NAN;
+    lab = 0;
+  }
+  return lab;
+}
+// Stores row `row`'s three logits; logits may be null (not asked for).
+__device__ __forceinline__ void store_logits(float* logits, long long row, const float (&logit)[kNCls]) {
+  if (logits) {
+    logits[row * 3 + 0] = logit[0];
+    logits[row * 3 + 1] = logit[1];
+    logits[row * 3 + 2] = logit[2];
+  }
+}
+// Stores one layer-1 half of a row's features (hidx 0: coefficients 0-7, 1: 8-12), held in the tensor-core column
+// order xl[6 (k / 2) + 2 g + k % 2] (k relative to the half's first coefficient), into the [39] feature row.
+__device__ __forceinline__ void store_feats_half(float* feats, long long row, int hidx, const float (&xl)[24]) {
+  const int k0 = hidx ? 8 : 0, nk = hidx ? 5 : 8;
+#pragma unroll
+  for (int k = 0; k < 8; ++k)
+#pragma unroll
+    for (int g = 0; g < 3; ++g)
+      if (k < nk) feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
+}
+
 // One output row per thread: window features -> FFN -> decision (block phase / windows API).
 // th: decision threshold (decide); 0 = argmax.
 __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r)[5][kNCep], int feat_mode,
@@ -273,17 +301,9 @@ __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r
   const bool ok = window_features(r, feat_mode, x);
   float logit[kNCls];
   ffn_forward(w, x, logit);
-  uint8_t lab = decide(logit, th);
-  if (!ok) {
-    logit[0] = logit[1] = logit[2] = NAN;
-    lab = 0;
-  }
+  const uint8_t lab = reject_nonfinite(ok, decide(logit, th), logit);
   if (labels) labels[row] = lab;
-  if (logits) {
-    logits[row * 3 + 0] = logit[0];
-    logits[row * 3 + 1] = logit[1];
-    logits[row * 3 + 2] = logit[2];
-  }
+  store_logits(logits, row, logit);
   if (feats) {
 #pragma unroll
     for (int i = 0; i < kNFeat; ++i) feats[row * kNFeat + i] = x[i];
@@ -558,7 +578,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
             const bool valid = tid < n_valid;
             const int c = out_done + (valid ? tid : 0);
             const long long row = seg.out_start - p.row_base + (c - 2);
-            const uint32_t tl = ffn_tc16_tile2_lane(tm_base, warp);
+            const uint32_t tl = ffn_tc16_tile_lane(tm_base, warp);
             // The frame's 48 layer-1 columns, one 24-column half (coefficient pairs 0-3, then 4-6) at a time.  Validity
             // stays in a register: ReLU's fmaxf swallows NaNs, so it cannot be read back from the logits.
             bool ok = true;
@@ -573,14 +593,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
                                 : window_features_pairs<4, 7, kRing, 24>(s_ring, c, p.feat_mode, xl)) && ok;
               }
               tc16_store_a1_half(tl, hidx, xl);
-              if (p.feats && valid) {
-                const int k0 = hidx ? 8 : 0, nk = hidx ? 5 : 8;  // xl[6 (k / 2) + 2 g + k % 2], k relative to k0
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-#pragma unroll
-                  for (int g = 0; g < 3; ++g)
-                    if (k < nk) p.feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
-              }
+              if (p.feats && valid) store_feats_half(p.feats, row, hidx, xl);
             }
             if (ts) ts[1] = clock64();
             if (!(VADB_DBG(p) & 16)) mbar_wait(&s_bar[2], w_par);  // weight blob landed (issued before the DCT phase)
@@ -588,21 +601,13 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
             float logit[kNCls];
             // tile 1 only when it holds a valid centre (hook build: mask 256 never issues it, to time one chain)
             const bool two_tiles = n_valid > 128 && !(VADB_DBG(p) & 256);
-            mma_par = ffn_tc16_tile2(ffn, logit, tm_base, warp, two_tiles, tid == 0, smem_u32(smem + kOffExch), &s_bar[3],
-                                     mma_par, ts);
+            mma_par = ffn_tc16_tile<2>(ffn, logit, tm_base, warp, two_tiles, tid == 0, smem_u32(smem + kOffExch),
+                                       &s_bar[3], mma_par, ts);
             ++dbg_n;
             if (valid) {
-              uint8_t lab = decide_of<FE>(logit, ffn);  // logits are in registers: no TMEM round trip
-              if (!ok) {
-                logit[0] = logit[1] = logit[2] = NAN;
-                lab = 0;
-              }
-              p.labels[row] = lab;
-              if (p.logits) {
-                p.logits[row * 3 + 0] = logit[0];
-                p.logits[row * 3 + 1] = logit[1];
-                p.logits[row * 3 + 2] = logit[2];
-              }
+              // logits are in registers: no TMEM round trip
+              p.labels[row] = reject_nonfinite(ok, decide_of<FE>(logit, ffn), logit);
+              store_logits(p.logits, row, logit);
             }
             if (!(VADB_DBG(p) & 16)) w_par ^= 1u;
             __syncthreads();  // MMAs done reading the blob before the next FFT phase rewrites exch / P
@@ -639,15 +644,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
               s_logE[tid] = ok_half ? 1.0f : 0.0f;
               if (ts) ts[1] = clock64();
               tc_store_a1_half(tl, hidx, xl);
-              if (p.feats && valid) {
-                const long long row = seg.out_start - p.row_base + (c - 2);
-                const int k0 = hidx ? 8 : 0, nk = hidx ? 5 : 8;  // xl[6 (k / 2) + 2 g + k % 2], k relative to k0
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-#pragma unroll
-                  for (int g = 0; g < 3; ++g)
-                    if (k < nk) p.feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
-              }
+              if (p.feats && valid) store_feats_half(p.feats, seg.out_start - p.row_base + (c - 2), hidx, xl);
               if (!(VADB_DBG(p) & 16)) mbar_wait(&s_bar[2], w_par);  // weight blob landed (issued before the DCT phase)
               if (ts) ts[2] = clock64();
               if constexpr (TC == 1)
@@ -656,18 +653,11 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
               ++dbg_n;
               if (valid && hidx == 0) {
                 const bool ok = s_logE[fr] != 0.0f && s_logE[128 + fr] != 0.0f;  // ordered by the tile's bar.syncs
-                uint8_t lab = decide_of<FE>(logit, ffn);  // logits are in registers: no TMEM round trip
-                if (!ok) {
-                  logit[0] = logit[1] = logit[2] = NAN;
-                  lab = 0;
-                }
+                // logits are in registers: no TMEM round trip
+                const uint8_t lab = reject_nonfinite(ok, decide_of<FE>(logit, ffn), logit);
                 const long long row = seg.out_start - p.row_base + (c - 2);
                 p.labels[row] = lab;
-                if (p.logits) {
-                  p.logits[row * 3 + 0] = logit[0];
-                  p.logits[row * 3 + 1] = logit[1];
-                  p.logits[row * 3 + 2] = logit[2];
-                }
+                store_logits(p.logits, row, logit);
               }
             }
             if (!(VADB_DBG(p) & 16)) w_par ^= 1u;
@@ -758,7 +748,6 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
   }
   mbar_wait(&bars[0], 0);
   {
-    const uint32_t tl = tm_base + (static_cast<uint32_t>(32 * warp) << 16);
     float h0[24], h1[24];
 #pragma unroll
     for (int i = 0; i < 24; ++i) h0[i] = h1[i] = 0.0f;
@@ -769,27 +758,21 @@ __global__ void __launch_bounds__(128) ffn_tc_rows_kernel(const float* x, long l
       else h1[col - 24] = v[f];
     }
     if (fp16) {
+      const uint32_t tl = ffn_tc16_tile_lane(tm_base, warp);
       tc16_store_a1_half(tl, 0, h0);
       tc16_store_a1_half(tl, 1, h1);
     } else {
+      const uint32_t tl = tm_base + (static_cast<uint32_t>(32 * warp) << 16);
       tc_store_a1_half(tl, 0, h0);
       tc_store_a1_half(tl, 1, h1);
     }
   }
-  if (fp16) ffn_tc16_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
+  if (fp16) ffn_tc16_tile<1>(fb, logit, tm_base, warp, false, tid == 0, smem_u32(smem), &bars[1], 0);
   else ffn_tc_tile<1>(fb, logit, tm_base, warp, 0, tid == 0, smem_u32(smem), &bars[1], 0);
   if (i < n) {
-    uint8_t lab = decide(logit, fb.thresh);
-    if (!ok) {
-      logit[0] = logit[1] = logit[2] = NAN;
-      lab = 0;
-    }
+    const uint8_t lab = reject_nonfinite(ok, decide(logit, fb.thresh), logit);
     if (labels) labels[i] = lab;
-    if (logits) {
-      logits[i * 3 + 0] = logit[0];
-      logits[i * 3 + 1] = logit[1];
-      logits[i * 3 + 2] = logit[2];
-    }
+    store_logits(logits, i, logit);
   }
   tc_fence_before();
   __syncthreads();
@@ -965,17 +948,9 @@ __global__ void __launch_bounds__(128) ffn_rows_kernel(const float* x, long long
   }
   float logit[kNCls];
   ffn_forward(w, v, logit);
-  uint8_t lab = decide(logit, w.thresh);
-  if (!ok) {
-    logit[0] = logit[1] = logit[2] = NAN;
-    lab = 0;
-  }
+  const uint8_t lab = reject_nonfinite(ok, decide(logit, w.thresh), logit);
   if (labels) labels[i] = lab;
-  if (logits) {
-    logits[i * 3 + 0] = logit[0];
-    logits[i * 3 + 1] = logit[1];
-    logits[i * 3 + 2] = logit[2];
-  }
+  store_logits(logits, i, logit);
 }
 
 // mfcc.get_deltas (mfcc.py:81-82: a - b) and mfcc.lifter (mfcc.py:85-93) for standalone callers.
@@ -1417,11 +1392,7 @@ __device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const 
         const uint8_t lab = stream_decide(sm, w, lane, lg);
         const long long o = static_cast<long long>(stl) * K + (f - max(s_f0[lane], 5ll));
         p.labels[o] = lab;
-        if (p.logits) {
-          p.logits[o * 3 + 0] = lg[0];
-          p.logits[o * 3 + 1] = lg[1];
-          p.logits[o * 3 + 2] = lg[2];
-        }
+        store_logits(p.logits, o, lg);
         if constexpr (SEG) {
           uint8_t row = 255;
           long long bound = -1;
