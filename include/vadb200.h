@@ -202,6 +202,53 @@ int vadb200_ingest_pcm(vadb200_handle* h, const void* d_raw, int big_endian, con
                        const int64_t* d_dst_start, const int64_t* d_len, int n_seg, int64_t max_len,
                        int16_t* d_dst, void* stream);
 
+/* ---- audio at other sample rates and formats (DESIGN.md section 5.8) ------------------------------------------
+ * Every other entry point reads 16 kHz mono int16.  These calls turn WAV payloads of any common format, channel
+ * count and sample rate into that: decode to float32 in int16 units, then resample to 16 kHz int16. */
+#define VADB200_PCM_S16 0   /* 16-bit signed: v = s */
+#define VADB200_PCM_U8 1    /* 8-bit unsigned: v = (b - 128) * 256 */
+#define VADB200_PCM_S24 2   /* 24-bit signed, packed 3 bytes: v = s / 256 */
+#define VADB200_PCM_S32 3   /* 32-bit signed: v = s / 65536 */
+#define VADB200_PCM_F32 4   /* IEEE float: v = x * 32768, non-finite samples become 0 */
+#define VADB200_PCM_F64 5   /* IEEE double: v = x * 32768 rounded to float32, non-finite samples become 0 */
+
+typedef struct vadb200_resampler vadb200_resampler;
+
+/* Decode + gather: segment i turns d_len[i] frames, starting at frame d_src_start[i] of the raw stream d_raw
+ * (interleaved frames of `channels` samples in `format`; big_endian != 0 swaps each sample's bytes), into
+ * d_dst[d_dst_start[i] ...] as float32 in int16 units, the mean of the channels (summed in channel order in float32,
+ * then divided by `channels`).  d_raw is aligned to the sample size (1 for u8 / s24, 2, 4, 8), channels in [1, 32],
+ * n_seg <= 65535, max_len = the largest d_len.  Only enqueues work. */
+int vadb200_decode_pcm(vadb200_handle* h, const void* d_raw, int format, int channels, int big_endian,
+                       const int64_t* d_src_start, const int64_t* d_dst_start, const int64_t* d_len, int n_seg,
+                       int64_t max_len, float* d_dst, void* stream);
+
+/* Resampling from src_rate to 16 kHz.  With g = gcd(src_rate, 16000), up = 16000 / g, down = src_rate / g,
+ * half = 10 max(up, down) and h = scipy.signal.firwin(2 half + 1, 1 / max(up, down), window=('kaiser', 5.0)) * up,
+ * an utterance x[0 .. n) becomes y[m] = sum_k x[k] h[m down + half - k up] for m < ceil(n up / down) (zero padding at
+ * both ends: scipy.signal.resample_poly(x, up, down)), computed in float32 from float32 taps, then rounded half to
+ * even and saturated to int16.  Accepted: integer rates in [4000, 384000] with max(up, down) <= 1024; 16000 is the
+ * identity (one tap of 1); any other rate is VADB200_E_UNSUPPORTED.
+ * vadb200_resampled_length: ceil(n up / down), or -1 for an unsupported rate or n < 0.
+ * vadb200_resample_taps: the float64 taps h (h_taps nullable, else 2 half + 1 entries); returns their count or -1. */
+int64_t vadb200_resampled_length(int64_t n, int src_rate);
+int64_t vadb200_resample_taps(int src_rate, double* h_taps);
+/* The resampler owns its float32 polyphase tap table on the handle's device; create allocates and synchronises. */
+int vadb200_resampler_create(vadb200_handle* h, int src_rate, vadb200_resampler** out);
+int vadb200_resampler_destroy(vadb200_resampler* r);
+/* Workspace for a call over n_utt utterances (16-byte aligned device memory; one per stream in flight). */
+int64_t vadb200_resample_workspace_bytes(const vadb200_resampler* r, int64_t n_utt);
+/* A ragged packed batch: utterance u is h_in_lengths[u] samples of d_in from sample h_in_offsets[u] (in_format
+ * VADB200_PCM_S16: int16, 2-byte aligned; VADB200_PCM_F32: float32 in int16 units, 4-byte aligned).  Output
+ * utterance u goes to d_out (16-byte aligned) from h_out_offsets[u] (filled: n_utt + 1 entries, each a multiple of 8
+ * samples, the last the total), whose length is vadb200_resampled_length of the input's; the 8-sample padding
+ * between utterances is not written, nor is anything past h_out_offsets[n_utt], which must be <= out_capacity.
+ * Only enqueues work: it allocates nothing, never synchronises and can be captured in a CUDA graph (the work list
+ * travels in kernel parameters into the workspace). */
+int vadb200_resample_packed(vadb200_resampler* r, int in_format, const void* d_in, const int64_t* h_in_offsets,
+                            const int64_t* h_in_lengths, int64_t n_utt, int16_t* d_out, int64_t out_capacity,
+                            int64_t* h_out_offsets, void* d_workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- per-frame API (mfcc.py:59-78 as the reference calls it: one float frame at a time;
  * batched here over n explicit frames of frame_len <= 512 float32 samples) ------------------ */
 int vadb200_spec_frames(vadb200_handle* h, const float* d_frames, int64_t n, int frame_len,

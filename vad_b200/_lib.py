@@ -53,6 +53,13 @@ SIGNATURES = {
     "vadb200_plan_gather_speech": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _I64, _P]),
     "vadb200_scale_rows": (C.c_int, [_P, _P, _I64, _P, _P]),
     "vadb200_ingest_pcm": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_int, _I64, _P, _P]),
+    "vadb200_decode_pcm": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P, C.c_int, _I64, _P, _P]),
+    "vadb200_resampled_length": (_I64, [_I64, C.c_int]),
+    "vadb200_resample_taps": (_I64, [C.c_int, _P]),
+    "vadb200_resampler_create": (C.c_int, [_P, C.c_int, C.POINTER(_P)]),
+    "vadb200_resampler_destroy": (C.c_int, [_P]),
+    "vadb200_resample_workspace_bytes": (_I64, [_P, _I64]),
+    "vadb200_resample_packed": (C.c_int, [_P, C.c_int, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P]),
     "vadb200_mfcc_packed": (C.c_int, [_P, _P, _I64, _P, _P]),
     "vadb200_vad_packed": (C.c_int, [_P, _P, _I64, _P, _P, _P, C.c_int, _P]),
     "vadb200_vad_host": (C.c_int, [_P, _P, _I64, _P, _P, C.c_int]),

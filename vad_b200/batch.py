@@ -43,60 +43,127 @@ def uniform_layout(n_utt, utt_samples):
     return offsets, lengths, stride
 
 
+def _upload_16k(utterances, handle, sample_rate):
+    """One upload of the batch and, at any rate but 16 kHz, the device resampler -> (int16 CUDA tensor, offsets,
+    lengths) at 16 kHz.  At 16000 Hz this is pack_utterances and one copy, as before."""
+    if int(sample_rate) == config.SAMPLERATE:
+        flat, offsets, lengths = pack_utterances(utterances)
+        return flat.to(handle.device), offsets, lengths
+    return _resample_device(utterances, handle, int(sample_rate))
+
+
+def _resample_device(utterances, handle, sample_rate):
+    r = runtime.Resampler(handle, sample_rate)
+    arrs = [np.asarray(u) for u in utterances]
+    if all(a.dtype == np.int16 for a in arrs):
+        flat, offsets, lengths = pack_utterances(arrs)
+        return r.run(flat.to(handle.device), offsets, lengths)
+    if not all(a.dtype.kind == "f" for a in arrs):
+        raise TypeError("utterances must all be int16 PCM or all floating point in [-1, 1]")
+    wide = any(a.dtype.itemsize > 4 for a in arrs)
+    dt, fmt = (np.float64, runtime.PCM_F64) if wide else (np.float32, runtime.PCM_F32)
+    lengths = np.array([a.size for a in arrs], dtype=np.int64)
+    offsets = np.zeros(len(arrs), dtype=np.int64)
+    if len(arrs) > 1:
+        offsets[1:] = np.cumsum(lengths[:-1])
+    host = np.zeros(max(int(lengths.sum()), 1), dtype=dt)
+    for a, o, n in zip(arrs, offsets, lengths):
+        host[o:o + n] = a.reshape(-1)
+    raw = torch.from_numpy(host.view(np.uint8)).to(handle.device)
+    f32 = torch.empty(host.size, dtype=torch.float32, device=handle.device)
+    keep = lengths > 0                    # decode scales by 32768 on the device, non-finite samples become 0
+    for lo in range(0, int(keep.sum()), 65535):
+        sl = slice(lo, lo + 65535)
+        handle.decode_pcm(raw, fmt, 1, offsets[keep][sl], offsets[keep][sl], lengths[keep][sl], f32)
+    return r.run(f32, offsets, lengths)
+
+
+def resample(utterances, sample_rate, handle=None):
+    """Utterances at ``sample_rate`` -> list of int16 arrays at 16 kHz: scipy.signal.resample_poly's filter on the
+    device, rounded half to even and saturated (include/vadb200.h).  Input is int16 PCM, or floating point in [-1, 1]
+    (the soundfile / torchaudio convention), scaled by 32768 on the device."""
+    handle = handle or runtime.default_handle()
+    pcm, offsets, lengths = _resample_device(utterances, handle, int(sample_rate))
+    host = pcm.cpu().numpy()
+    return [host[o:o + n].copy() for o, n in zip(offsets, lengths)]
+
+
 def _split_rows(t, row_offsets):
     return [t[int(row_offsets[i]):int(row_offsets[i + 1])] for i in range(len(row_offsets) - 1)]
 
 
-def mfcc_batch(utterances, deltas=False, handle=None):
+def mfcc_batch(utterances, deltas=False, handle=None, sample_rate=16000):
     """MFCC of every frame of every utterance.  deltas=False -> list of [T_u, 13] tensors;
-    deltas=True -> list of [T_u - 5, 39] rows [c, d1, d2] (process_file's output)."""
+    deltas=True -> list of [T_u - 5, 39] rows [c, d1, d2] (process_file's output).  At any other ``sample_rate`` the
+    batch is resampled to 16 kHz on the device first (``resample``); rows keep the 16 kHz framing."""
     handle = handle or runtime.default_handle()
-    flat, offsets, lengths = pack_utterances(utterances)
+    pcm, offsets, lengths = _upload_16k(utterances, handle, sample_rate)
     plan = runtime.Plan(handle, offsets, lengths, MODE_DATASET if deltas else MODE_MFCC)
-    out = plan.mfcc(flat.to(handle.device))
+    out = plan.mfcc(pcm)
     return _split_rows(out, plan.row_offsets)
 
 
-def vad_batch(utterances, handle=None, want_logits=False, feat_mode=FEAT_ANALYSER):
-    """Per-frame speech / non-speech labels (uint8) for every utterance; optionally logits."""
+def vad_batch(utterances, handle=None, want_logits=False, feat_mode=FEAT_ANALYSER, sample_rate=16000):
+    """Per-frame speech / non-speech labels (uint8) for every utterance; optionally logits.  At any other
+    ``sample_rate`` the batch is resampled to 16 kHz on the device first; labels keep the 16 kHz framing."""
     handle = handle or runtime.default_handle()
     if not handle.has_ffn:
         raise RuntimeError("set FFN weights first (Handle.set_ffn_weights)")
-    flat, offsets, lengths = pack_utterances(utterances)
+    pcm, offsets, lengths = _upload_16k(utterances, handle, sample_rate)
     plan = runtime.Plan(handle, offsets, lengths, MODE_VAD)
-    labels, logits, _ = plan.vad(flat.to(handle.device), want_logits=want_logits, feat_mode=feat_mode)
+    labels, logits, _ = plan.vad(pcm, want_logits=want_logits, feat_mode=feat_mode)
     lab = _split_rows(labels, plan.row_offsets)
     if want_logits:
         return lab, _split_rows(logits, plan.row_offsets)
     return lab
 
 
-def _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode):
+def _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode, sample_rate):
     handle = handle or runtime.default_handle()
     if not handle.has_ffn:
         raise RuntimeError("set FFN weights first (Handle.set_ffn_weights)")
     for v in (min_speech_ms, min_silence_ms, pad_ms):
         runtime.speech_ms_to_rows(v)               # argument errors before any device work
-    flat, offsets, lengths = pack_utterances(utterances)
+    pcm, offsets, lengths = _upload_16k(utterances, handle, sample_rate)
     plan = runtime.Plan(handle, offsets, lengths, MODE_VAD)
-    pcm = flat.to(handle.device)
     labels, _, _ = plan.vad(pcm, feat_mode=feat_mode)
     segs, seg_off, sp_off, _ = plan.speech_segments(labels, min_speech_ms, min_silence_ms, pad_ms)
     return plan, pcm, segs, seg_off, sp_off
 
 
-def speech_segments(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER):
+def source_bounds(segments, n, sample_rate):
+    """[start, end) bounds at 16 kHz -> the same speech at ``sample_rate`` in an utterance of ``n`` samples there:
+    [floor(a down / up), min(n, ceil(b down / up)))."""
+    s = np.asarray(segments, dtype=np.int64).reshape(-1, 2)
+    g = int(np.gcd(int(sample_rate), config.SAMPLERATE))
+    up, down = config.SAMPLERATE // g, int(sample_rate) // g
+    a = s[:, 0] * down // up
+    b = np.minimum(int(n), -((-s[:, 1] * down) // up))
+    return np.stack([a, b], axis=1)
+
+
+def speech_segments(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER,
+                    sample_rate=16000):
     """Speech segments of every utterance: a list of int64 [k, 2] arrays of [start, end) samples within the
     utterance.  One upload, the fused VAD, the segment kernels and one download; the handle's front end and
-    decision threshold apply.  See Plan.speech_segments for the smoothing parameters."""
-    _, _, segs, seg_off, _ = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode)
+    decision threshold apply.  See Plan.speech_segments for the smoothing parameters.  At any other ``sample_rate``
+    the batch is resampled to 16 kHz on the device first and the bounds come back in the caller's rate
+    (``source_bounds``)."""
+    _, _, segs, seg_off, _ = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode,
+                                         sample_rate)
     s = segs.cpu().numpy()
-    return [s[seg_off[u]:seg_off[u + 1]] for u in range(len(seg_off) - 1)]
+    out = [s[seg_off[u]:seg_off[u + 1]] for u in range(len(seg_off) - 1)]
+    if int(sample_rate) == config.SAMPLERATE:
+        return out
+    return [source_bounds(b, len(u), sample_rate) for b, u in zip(out, utterances)]
 
 
-def extract_speech(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER):
-    """Speech-only audio of every utterance (its segments concatenated): a list of int16 arrays."""
-    plan, pcm, segs, seg_off, sp_off = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode)
+def extract_speech(utterances, handle=None, min_speech_ms=0, min_silence_ms=0, pad_ms=0, feat_mode=FEAT_ANALYSER,
+                   sample_rate=16000):
+    """Speech-only audio of every utterance (its segments concatenated): a list of int16 arrays.  The audio is at
+    16 kHz whatever ``sample_rate`` the input has: it is the resampled signal the decisions were made on."""
+    plan, pcm, segs, seg_off, sp_off = _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode,
+                                                   sample_rate)
     out = plan.gather_speech(pcm, segs, seg_off, sp_off).cpu().numpy()
     return [out[sp_off[u]:sp_off[u + 1]] for u in range(len(sp_off) - 1)]
 
@@ -146,10 +213,11 @@ def _check_frame_args(frame_size, frame_step, fft_n, mel_filterbank, mfcc_num):
     _mfcc._require(fft_n, mel_filterbank, mfcc_num)
 
 
-def _dataset_rows_of_files(jobs, handle):
+def _dataset_rows_of_files(jobs, handle, resample=False):
     """[(fname, transcription_path)] -> (device rows [sum, 39], row_offsets): container parse on the host, then one
-    upload, ``vadb200_ingest_pcm`` (decode + .stm gather) and one MODE_DATASET launch for the whole step."""
-    ing = DeviceIngest(handle)
+    upload, ``vadb200_ingest_pcm`` (decode + .stm gather) and one MODE_DATASET launch for the whole step
+    (``resample``: DeviceIngest's decode and 16 kHz resampling of other formats and rates)."""
+    ing = DeviceIngest(handle, resample=resample)
     for fname, tpath in jobs:
         ing.add(fname, tpath)
     d_pcm, offsets, lengths, _ = ing.run()
@@ -290,7 +358,7 @@ def list_audio_files(files_paths, max_files):
 
 
 def process_files(files_paths, files_type, max_files, csv_writer, transcription_dir=None, handle=None,
-                  files_per_step=None, verbose=True):
+                  files_per_step=None, verbose=True, resample=False):
     """dataset_creator.process_files: list wav / sph files of the given directories (os.listdir order, at most
     max_files), derive each file's .stm path from transcription_dir, and for every step of FILES_PER_STEP files
     (config.py:32) extract the (mfcc, d1, d2) rows, scale them with the step's scalar statistics
@@ -299,7 +367,11 @@ def process_files(files_paths, files_type, max_files, csv_writer, transcription_
     Where the reference maps process_file over a 4-process pool and pickles python lists back, one step here is:
     container headers parsed on the host, one pinned upload of the raw bytes, device decode + .stm gather, one
     MODE_DATASET launch for all files, the two-pass scaling kernels, one download.  The next step's files are read
-    from disk while the GPU works on the current one.  Returns the number of rows written."""
+    from disk while the GPU works on the current one.  Returns the number of rows written.
+
+    ``resample=True`` accepts wav files of any common format, channel count and sample rate and resamples them to
+    16 kHz on the device (``DeviceIngest(resample=True)``); the default reads 16 kHz 16-bit mono as the reference
+    does."""
     handle = handle or runtime.default_handle()
     step = int(files_per_step or config.FILES_PER_STEP)
     if verbose:
@@ -318,7 +390,7 @@ def process_files(files_paths, files_type, max_files, csv_writer, transcription_
     written = 0
     pending = None                                   # (device rows of the previous step), scaled, not yet sunk
     for lo in range(0, len(jobs), step):
-        rows, _ = _dataset_rows_of_files(jobs[lo:lo + step], handle)     # enqueued asynchronously
+        rows, _ = _dataset_rows_of_files(jobs[lo:lo + step], handle, resample)     # enqueued asynchronously
         if rows.shape[0]:
             handle.scale_rows(rows, want_stats=False)
         if pending is not None:                      # sink step k-1 while step k runs on the GPU

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvadb200.so")
-SOURCES = ["vadb200.cu"]
+SOURCES = ["vadb200.cu", "vad_resample.cu"]
 def _deps():
     """Every source the library is compiled from: csrc/*.{cu,cuh,h} and the public header."""
     names = [f for f in sorted(os.listdir(CSRC)) if f.endswith((".cu", ".cuh", ".h"))]

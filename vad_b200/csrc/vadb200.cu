@@ -24,6 +24,7 @@
 #include "vad_kernels.cuh"
 #include "ffn_train.cuh"
 #include "vad_segments.cuh"
+#include "vad_resample.cuh"
 
 using namespace vadb;
 
@@ -220,6 +221,14 @@ struct vadb200_bank {
   SmoothParams sp{};
   DevBuf<uint32_t> d_seg;
   size_t seg_bytes = 0;
+};
+
+struct vadb200_resampler {
+  ~vadb200_resampler() { cudaSetDevice(device); }
+  int device = 0;
+  int num_sms = kNumSmFallback;
+  ResampleDesign d;
+  DevBuf<float> d_taps;        // [up][Ks] float32 polyphase rows (vad_resample.cuh)
 };
 
 namespace {
@@ -1304,6 +1313,124 @@ int vadb200_plan_gather_speech(vadb200_plan* p, const int16_t* d_pcm, int64_t pc
         d_pcm, p->d_pcm_off.get(), p->n_utt, reinterpret_cast<const long long*>(d_segments),
         reinterpret_cast<const long long*>(d_segment_offsets), reinterpret_cast<const long long*>(d_speech_offsets),
         d_out, out_capacity);
+  });
+}
+
+// ---- other sample rates and formats (vad_resample.cuh) ----------------------------------------------------------
+int vadb200_decode_pcm(vadb200_handle* h, const void* d_raw, int format, int channels, int big_endian,
+                       const int64_t* d_src_start, const int64_t* d_dst_start, const int64_t* d_len, int n_seg,
+                       int64_t max_len, float* d_dst, void* stream) {
+  if (format < VADB200_PCM_S16 || format > VADB200_PCM_F64) return fail(VADB200_E_INVALID, "unknown sample format");
+  if (channels < 1 || channels > kMaxChannels) return fail(VADB200_E_INVALID, "channels must be in [1, 32]");
+  if (n_seg < 0 || max_len < 0) return fail(VADB200_E_INVALID, "bad argument");
+  if (n_seg > 65535) return fail(VADB200_E_INVALID, "at most 65535 segments per call");
+  const int align = format == VADB200_PCM_S24 ? 1 : kPcmBytes[format];
+  if (misaligned(d_raw, align)) return fail(VADB200_E_INVALID, "raw stream must be aligned to the sample size");
+  if (misaligned(d_dst, 4)) return fail(VADB200_E_INVALID, "d_dst must be 4-byte aligned");
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (n_seg == 0 || max_len == 0) return 0;
+  if (!d_raw || !d_src_start || !d_dst_start || !d_len || !d_dst) return fail(VADB200_E_INVALID, "null argument");
+  CU(cudaSetDevice(h->device));
+  const unsigned gx = static_cast<unsigned>(std::min<long long>((max_len + 255) / 256, 4ll * h->num_sms));
+  const dim3 grid(gx, static_cast<unsigned>(n_seg));
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const uint8_t* raw = static_cast<const uint8_t*>(d_raw);
+  const long long* src = reinterpret_cast<const long long*>(d_src_start);
+  const long long* dst = reinterpret_cast<const long long*>(d_dst_start);
+  const long long* len = reinterpret_cast<const long long*>(d_len);
+  return launched(1, [&] { enqueue_decode_pcm(format, grid, st, raw, channels, big_endian, src, dst, len, d_dst); });
+}
+
+int64_t vadb200_resampled_length(int64_t n, int src_rate) {
+  int up = 0, down = 0;
+  if (n < 0 || !resample_ratio(src_rate, &up, &down)) return -1;
+  return resampled_length(n, up, down);
+}
+
+int64_t vadb200_resample_taps(int src_rate, double* h_taps) {
+  int up = 0, down = 0;
+  if (!resample_ratio(src_rate, &up, &down)) return -1;
+  const std::vector<double> taps = resample_taps(up, down);
+  if (h_taps) std::memcpy(h_taps, taps.data(), taps.size() * sizeof(double));
+  return static_cast<int64_t>(taps.size());
+}
+
+int vadb200_resampler_create(vadb200_handle* h, int src_rate, vadb200_resampler** out) {
+  if (!out) return fail(VADB200_E_INVALID, "out is null");
+  *out = nullptr;
+  int up = 0, down = 0;
+  if (!resample_ratio(src_rate, &up, &down))
+    return fail(VADB200_E_UNSUPPORTED,
+                "sample rate must be an integer in [4000, 384000] Hz with max(up, down) <= 1024 for 16000 Hz");
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  std::unique_ptr<vadb200_resampler> r(new (std::nothrow) vadb200_resampler());
+  if (!r) return fail(VADB200_E_NOMEM, "host allocation failed");
+  r->device = h->device;
+  r->num_sms = h->num_sms;
+  r->d = resample_design(up, down);
+  CU(cudaSetDevice(h->device));
+  int optin = 0;
+  CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+  if (r->d.smem > static_cast<size_t>(optin)) return fail(VADB200_E_UNSUPPORTED, "resampler tile exceeds shared memory");
+  // the largest opt-in for every resampler: one resampler's attribute never limits another's
+  CU(resample_allow_smem(optin));
+  const std::vector<float> taps = polyphase_taps(r->d, resample_taps(up, down));
+  CU(dev_upload(r->d_taps, taps.data(), taps.size()));
+  *out = r.release();
+  return 0;
+}
+
+int vadb200_resampler_destroy(vadb200_resampler* r) {
+  delete r;
+  return 0;
+}
+
+int64_t vadb200_resample_workspace_bytes(const vadb200_resampler* r, int64_t n_utt) {
+  if (!r || n_utt < 0) return -1;
+  return std::max<int64_t>(n_utt, 1) * static_cast<int64_t>(sizeof(ResampleUtt));
+}
+
+int vadb200_resample_packed(vadb200_resampler* r, int in_format, const void* d_in, const int64_t* h_in_offsets,
+                            const int64_t* h_in_lengths, int64_t n_utt, int16_t* d_out, int64_t out_capacity,
+                            int64_t* h_out_offsets, void* d_workspace, int64_t workspace_bytes, void* stream) {
+  if (!r) return fail(VADB200_E_INVALID, "resampler is null");
+  if (in_format != VADB200_PCM_S16 && in_format != VADB200_PCM_F32)
+    return fail(VADB200_E_INVALID, "in_format must be VADB200_PCM_S16 or VADB200_PCM_F32");
+  if (n_utt < 0 || out_capacity < 0) return fail(VADB200_E_INVALID, "bad argument");
+  if (!h_out_offsets || (n_utt > 0 && (!h_in_offsets || !h_in_lengths)))
+    return fail(VADB200_E_INVALID, "null argument");
+  if (misaligned(d_in, in_format == VADB200_PCM_S16 ? 2 : 4) || misaligned(d_out, 16) || misaligned(d_workspace, 16))
+    return fail(VADB200_E_INVALID, "d_in must be aligned to its sample, d_out and the workspace to 16 bytes");
+  if (n_utt > 0x7fffffffll) return fail(VADB200_E_INVALID, "too many utterances");
+  const ResampleDesign& d = r->d;
+  std::vector<ResampleUtt> utts(static_cast<size_t>(n_utt));
+  long long out_pos = 0, tiles = 0;
+  for (long long u = 0; u < n_utt; ++u) {
+    const long long off = h_in_offsets[u], n = h_in_lengths[u];
+    if (off < 0 || n < 0 || n > (1ll << 40)) return fail(VADB200_E_INVALID, "offsets and lengths must be >= 0");
+    const long long m = resampled_length(n, d.up, d.down);
+    utts[u] = ResampleUtt{off, n, out_pos, tiles};
+    h_out_offsets[u] = out_pos;
+    out_pos += (m + 7) / 8 * 8;
+    tiles += (m + d.T - 1) / d.T;
+  }
+  h_out_offsets[n_utt] = out_pos;
+  if (out_pos > out_capacity) return fail(VADB200_E_INVALID, "out_capacity is smaller than the resampled batch");
+  if (tiles > 0x7fffffffll) return fail(VADB200_E_INVALID, "batch too large for one call");
+  if (tiles == 0) return 0;
+  if (!d_in || !d_out) return fail(VADB200_E_INVALID, "null argument");
+  if (!d_workspace || workspace_bytes < vadb200_resample_workspace_bytes(r, n_utt))
+    return fail(VADB200_E_INVALID, "workspace smaller than vadb200_resample_workspace_bytes");
+  CU(cudaSetDevice(r->device));
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  ResampleUtt* ws = static_cast<ResampleUtt*>(d_workspace);
+  const int n_fill = static_cast<int>((n_utt + kResampleFill - 1) / kResampleFill);
+  ResampleParams a;
+  a.in = d_in; a.out = d_out; a.utts = ws; a.n_utt = static_cast<int>(n_utt); a.taps = r->d_taps.get();
+  a.up = d.up; a.down = d.down; a.half = d.half; a.K = d.K; a.Ks = d.Ks; a.q = d.q; a.H = d.H; a.win = d.win;
+  a.taps_floats = (d.up * d.Ks + 3) / 4 * 4;
+  return launched(n_fill + 1, [&] {
+    enqueue_resample(in_format == VADB200_PCM_S16, a, utts.data(), n_utt, tiles, d.smem, st);
   });
 }
 

@@ -10,6 +10,7 @@ from . import _lib
 from ._lib import check
 
 MODE_MFCC, MODE_DATASET, MODE_VAD = 0, 1, 2
+PCM_S16, PCM_U8, PCM_S24, PCM_S32, PCM_F32, PCM_F64 = 0, 1, 2, 3, 4, 5
 FEAT_ANALYSER, FEAT_DATASET = 0, 1
 FFN_KEYS = ("W1", "b1", "W2", "b2", "W3", "b3", "W4", "b4")
 FFN_SHAPES = {"W1": (39, 64), "b1": (64,), "W2": (64, 32), "b2": (32,), "W3": (32, 16), "b3": (16,),
@@ -31,6 +32,15 @@ def frames_for_length(n_samples):
 
 def outputs_for_length(n_samples):
     return int(_lib.load().vadb200_outputs_for_length(int(n_samples)))
+
+
+def resampled_length(n_samples, src_rate):
+    """Samples at 16 kHz of ``n_samples`` at ``src_rate``: ceil(n up / down), as scipy.signal.resample_poly returns."""
+    n = int(_lib.load().vadb200_resampled_length(int(n_samples), int(src_rate)))
+    if n < 0:
+        raise _lib.VadB200Error(-2 if int(n_samples) >= 0 else -1,
+                                "unsupported sample rate %r or negative length" % (src_rate,))
+    return n
 
 
 def glorot_ffn(seed=0):
@@ -242,6 +252,86 @@ class Handle(object):
         check(self.lib.vadb200_ingest_pcm(self._h, _ptr(raw), 1 if big_endian else 0, _ptr(src), _ptr(dst), _ptr(ln),
                                           int(ln_host.size), int(ln_host.max()), _ptr(out), self.stream))
         return out
+
+
+    def decode_pcm(self, raw, fmt, channels, src_start, dst_start, lengths, out, big_endian=False):
+        """Device decode + gather of any VADB200_PCM_* format: ``raw`` uint8 CUDA tensor of interleaved frames of
+        ``channels`` samples, segment i = ``lengths[i]`` frames from frame ``src_start[i]`` to the float32 tensor
+        ``out[dst_start[i]:]`` in int16 units, the mean of the channels."""
+        ln_host = np.asarray(lengths, dtype=np.int64)
+        if ln_host.size == 0:
+            return out
+        src = torch.as_tensor(np.asarray(src_start, dtype=np.int64)).to(self.device)
+        dst = torch.as_tensor(np.asarray(dst_start, dtype=np.int64)).to(self.device)
+        ln = torch.as_tensor(ln_host).to(self.device)
+        check(self.lib.vadb200_decode_pcm(self._h, _ptr(raw), int(fmt), int(channels), 1 if big_endian else 0,
+                                          _ptr(src), _ptr(dst), _ptr(ln), int(ln_host.size), int(ln_host.max()),
+                                          _ptr(out), self.stream))
+        return out
+
+
+class Resampler(object):
+    """src_rate -> 16 kHz int16 on the device (scipy.signal.resample_poly's filter, rounded half to even and
+    saturated; include/vadb200.h).  Owns the tap table; ``run`` only enqueues work."""
+
+    def __init__(self, handle, src_rate):
+        self.handle = handle
+        self.lib = handle.lib
+        self.src_rate = int(src_rate)
+        self._r = C.c_void_p()
+        check(self.lib.vadb200_resampler_create(handle._h, self.src_rate, C.byref(self._r)))
+        g = int(np.gcd(self.src_rate, 16000))
+        self.up, self.down = 16000 // g, self.src_rate // g
+        self._ws = None
+
+    def close(self):
+        if getattr(self, "_r", None) is not None and self._r:
+            self.lib.vadb200_resampler_destroy(self._r)
+            self._r = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def output_length(self, n):
+        """ceil(n up / down) (vadb200_resampled_length), elementwise for an array."""
+        return (np.asarray(n, dtype=np.int64) * self.up + self.down - 1) // self.down
+
+    def output_offsets(self, lengths):
+        """The packed 8-aligned output offsets ``run`` uses for these input lengths (n_utt + 1 entries)."""
+        m = self.output_length(np.asarray(lengths, dtype=np.int64).reshape(-1))
+        offs = np.zeros(m.size + 1, dtype=np.int64)
+        offs[1:] = np.cumsum((m + 7) // 8 * 8)
+        return offs
+
+    def run(self, d_pcm, offsets, lengths, out=None):
+        """``d_pcm``: 1-D int16 (samples) or float32 (int16 units) CUDA tensor; utterance u = lengths[u] samples from
+        offsets[u].  Returns (int16 CUDA tensor at 16 kHz, offsets16, lengths16); ``out`` (16-byte aligned int16)
+        receives the batch when given."""
+        if not (torch.is_tensor(d_pcm) and d_pcm.is_cuda and d_pcm.dim() == 1 and d_pcm.is_contiguous()
+                and d_pcm.dtype in (torch.int16, torch.float32)):
+            raise TypeError("d_pcm must be a contiguous 1-D int16 or float32 CUDA tensor")
+        fmt = PCM_S16 if d_pcm.dtype == torch.int16 else PCM_F32
+        offs = np.ascontiguousarray(offsets, dtype=np.int64)
+        lens = np.ascontiguousarray(lengths, dtype=np.int64)
+        if offs.shape != lens.shape or offs.ndim != 1:
+            raise ValueError("offsets and lengths must be 1-D arrays of equal length")
+        if lens.size and int((offs + lens).max()) > d_pcm.numel():
+            raise ValueError("an utterance ends past the end of d_pcm")
+        n = int(lens.size)
+        if out is None:
+            out = torch.zeros((int(self.output_offsets(lens)[-1]) + 8,), dtype=torch.int16, device=d_pcm.device)
+        out_offs = np.zeros(n + 1, dtype=np.int64)                   # filled by the library
+        ws_bytes = int(self.lib.vadb200_resample_workspace_bytes(self._r, n))
+        if self._ws is None or self._ws.numel() < ws_bytes or self._ws.device != d_pcm.device:
+            self._ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=d_pcm.device)
+        check(self.lib.vadb200_resample_packed(self._r, fmt, _ptr(d_pcm), offs.ctypes.data_as(C.c_void_p),
+                                               lens.ctypes.data_as(C.c_void_p), n, _ptr(out), out.numel(),
+                                               out_offs.ctypes.data_as(C.c_void_p), _ptr(self._ws), ws_bytes,
+                                               _stream(d_pcm.device)))
+        return out, out_offs[:-1].copy(), self.output_length(lens)
 
 
 class Plan(object):
