@@ -350,6 +350,30 @@ int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const 
                                float* d_logits /* nullable [n][K][3] */, uint8_t* d_rows /* nullable [n][K] */,
                                int64_t* d_bounds /* nullable [n][K] */, void* stream);
 
+/* Ragged bank at another source rate (DESIGN.md section 5.9): each stream takes int16 packets at sample_rate r, a
+ * rate vadb200_resampler_create accepts (else VADB200_E_UNSUPPORTED), of 0 .. max_feed_samples samples, the cap in
+ * [1, r] (else VADB200_E_INVALID; on failure *out is NULL).  With vadb200_resample_packed's up, down, half and
+ * filter, a stream that has taken N source samples since its last reset or end has produced the 16 kHz samples m whose
+ * newest input lies inside them, (m down + half) div up <= N - 1: M(N) = 0 if N up <= half, else
+ * (N up - 1 - half) div down + 1 of them, bit-identical to vadb200_resample_packed's output on the stream's whole
+ * signal (the causal prefix of scipy.signal.resample_poly; latency half / up source samples).  Those samples feed the
+ * 16 kHz ragged bank above unchanged: after N source samples a stream has emitted the rows of an offline 16 kHz
+ * utterance of M(N) + 1 samples.  One feed adds at most cap16 = ceil(max_feed_samples up / down) <= 16000 samples at
+ * 16 kHz, so vadb200_stream_bank_max_rows_per_feed returns ceil(cap16 / 160).
+ *
+ * vadb200_stream_feed_ragged takes source-rate packets (d_samples / d_offsets may be pinned host memory; a packet
+ * sample is read once, apart from the few samples two tiles of one stream share).  A length below 0 or above
+ * max_feed_samples gets count -1 and all-255 labels and leaves the stream's source-rate and 16 kHz state untouched.
+ * Speech bounds are 16 kHz samples, as vadb200_plan_speech_segments gives them.  _end_streams and _reset also zero the
+ * source-rate state: the next packet starts a new signal with zeros before it, and an end discards the source samples
+ * whose 16 kHz samples are not yet ready.  A feed is three kernel launches and an end two; both allocate nothing,
+ * never synchronise and can be captured in a CUDA graph.  sample_rate 16000 creates exactly
+ * vadb200_stream_bank_create_ragged's bank.
+ * vadb200_stream_bank_sample_rate: r, 16000 for every other bank, -1 for NULL. */
+int vadb200_stream_bank_create_ragged_rate(vadb200_handle* h, int n_streams, int max_feed_samples, int sample_rate,
+                                           vadb200_bank** out);
+int vadb200_stream_bank_sample_rate(const vadb200_bank* b);
+
 /* ---- FFN training (learning/ffn_trainer.py:104-175) ---------------------------------------
  * model.compile(loss='categorical_crossentropy', optimizer='adadelta') + model.train_on_batch for the
  * 39-64-32-16-3 network: forward, backward and the Adadelta update as two hand-written kernels per step,

@@ -82,6 +82,8 @@ SIGNATURES = {
     "vadb200_stream_bank_create_ragged": (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(_P)]),
     "vadb200_stream_bank_max_rows_per_feed": (C.c_int, [_P]),
     "vadb200_stream_feed_ragged": (C.c_int, [_P] + [_P] * 7 + [_P]),
+    "vadb200_stream_bank_create_ragged_rate": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.POINTER(_P)]),
+    "vadb200_stream_bank_sample_rate": (C.c_int, [_P]),
     "vadb200_trainer_create": (C.c_int, [_P, _I64, C.c_float, C.c_float, C.c_float, C.POINTER(_P)]),
     "vadb200_trainer_destroy": (C.c_int, [_P]),
     "vadb200_trainer_set_weights": (C.c_int, [_P] + [_P] * 8 + [C.c_int]),

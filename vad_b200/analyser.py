@@ -8,7 +8,7 @@ import pickle
 import numpy as np
 import torch
 
-from . import runtime
+from . import _lib, runtime
 from .runtime import FEAT_ANALYSER
 
 
@@ -153,22 +153,39 @@ class StreamBank(object):
     [160 f, 160 f + 400)) emits row f - 5, so one tick returns 0 .. K = ceil(max_feed_samples / 160) rows per stream.
     The packets are packed into one pinned buffer with their offsets, and the captured graph reads the lengths on the
     device: one graph serves every packet mix.  ``end_streams`` discards a stream's samples that have not completed a
-    frame."""
+    frame.
+
+    A ragged bank at another ``sample_rate`` (a rate ``batch.resample`` accepts) takes int16 packets at that rate, up to
+    ``max_feed_samples`` of them in [1, sample_rate], and resamples each stream to 16 kHz on the device with
+    ``batch.resample``'s filter: after N samples a stream has the rows of ``vad_batch`` on the first M(N) samples of
+    its resampled signal plus one (see include/vadb200.h), which trails the input by half / up source samples (at most
+    1.25 ms).  Rows keep the 16 kHz, 10 ms framing; segment bounds come back in source samples, mapped as
+    ``batch.source_bounds`` maps them."""
 
     NOT_READY = 255
     max_feed = None          # ragged bank: the cap on one stream's samples per tick
+    sample_rate = 16000      # the rate of the samples fed
 
     def __init__(self, n_streams, ffn_weights=None, handle=None, use_graph=True, zero_copy=True,
-                 max_feed_samples=None):
+                 max_feed_samples=None, sample_rate=16000):
+        rate = int(sample_rate)
+        if rate != 16000:    # checked before any device work
+            if max_feed_samples is None:
+                raise ValueError("a fixed bank takes 16 kHz chunks: give max_feed_samples for another sample rate")
+            if int(_lib.load().vadb200_resampled_length(1, rate)) < 0:
+                raise ValueError("unsupported sample rate %r" % (sample_rate,))
+        if max_feed_samples is not None and not 1 <= int(max_feed_samples) <= rate:
+            raise ValueError("max_feed_samples must lie in [1, %d]" % rate)
         self.handle = _handle_for(ffn_weights, handle)
         if not self.handle.has_ffn:
             raise RuntimeError("StreamBank needs FFN weights")
         self.n = int(n_streams)
+        self.sample_rate = rate
         if max_feed_samples is not None:
             self.max_feed = int(max_feed_samples)
-            if not 1 <= self.max_feed <= 16000:
-                raise ValueError("max_feed_samples must lie in [1, 16000]")
-        self.bank = runtime.StreamBankHandle(self.handle, self.n, self.max_feed)
+        g = np.gcd(rate, 16000)
+        self._up, self._down = 16000 // g, rate // g
+        self.bank = runtime.StreamBankHandle(self.handle, self.n, self.max_feed, rate)
         dev = self.handle.device
         if self.max_feed is None:
             self.h_chunks = torch.zeros((self.n, 160), dtype=torch.int16).pin_memory()
@@ -364,8 +381,20 @@ class StreamBank(object):
             raise RuntimeError("speech is off: call set_speech first")
         self._pack(chunks)
         self._tick(False, speech=True)
-        return list(zip(self._rows_of(self.h_labels.numpy()), self._rows_of(self.h_rows.numpy()),
-                        self._rows_of(self.h_bounds.numpy())))
+        rows = self._rows_of(self.h_rows.numpy())
+        return list(zip(self._rows_of(self.h_labels.numpy()), rows,
+                        [self._to_source(b, r == 1) for r, b in zip(rows, self._rows_of(self.h_bounds.numpy()))]))
+
+    def _to_source(self, bounds, opening):
+        """16 kHz segment bounds -> source samples, as batch.source_bounds maps them: an opening bound a (its row is
+        speech) to floor(a down / up), a closing one b to ceil(b down / up); -1 stays -1.  Every bound a stream emits
+        lies before the 16 kHz samples it has produced, and those read only the N source samples it has taken, so
+        ceil(b down / up) <= N: nothing needs clipping."""
+        if self.sample_rate == 16000:
+            return bounds
+        b = np.asarray(bounds, np.int64)
+        up, down = self._up, self._down
+        return np.where(b < 0, b, np.where(opening, b * down // up, -((-b * down) // up)))
 
     def end_streams(self, ids):
         """End the streams ``ids`` and start them again (their next chunk begins a new signal).  With speech on,
@@ -393,5 +422,5 @@ class StreamBank(object):
         out = []
         for r, b in zip(rows, bounds):
             k = int(np.count_nonzero(r != 255))
-            out.append((r[:k].copy(), b[:k + 1].copy()))
+            out.append((r[:k].copy(), self._to_source(b[:k + 1].copy(), np.r_[r[:k] == 1, False])))
         return out

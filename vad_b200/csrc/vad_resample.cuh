@@ -144,6 +144,37 @@ void enqueue_decode_pcm(int fmt, dim3 grid, cudaStream_t st, const uint8_t* raw,
 void enqueue_resample(bool s16, const ResampleParams& a, const ResampleUtt* list, long long n, long long tiles,
                       size_t smem, cudaStream_t st);
 
+// ---- the resampling ragged bank (vad_stream_resample.cu, index math in vad_stream_resample.h) -------------------
+// What the plan step decides for one stream and feed.
+struct SrsFeed {
+  long long n0;    // source samples taken before this feed
+  long long src;   // the packet's first sample in the caller's samples
+  long long out;   // its first new 16 kHz sample in the bank's packed buffer
+  int c;           // packet length (0 for a bad one)
+  int outs;        // 16 kHz samples it adds
+  int rd;          // history buffer holding x[n0 - K + 1 .. n0 - 1]
+  int pad;
+};
+struct StreamResampleParams {
+  int n, cap, cap16;
+  int up, down, half, K, Ks;
+  int hs;                    // history slots per stream: K - 1
+  const float* taps;         // [up][Ks] polyphase rows (polyphase_taps)
+  long long* n_in;           // [n] source samples taken since the last reset or end
+  int* cur;                  // [n] the history buffer the next feed reads
+  int16_t* hist;             // [2][n][hs]
+  SrsFeed* feed;             // [n]
+  int* tile_off;             // [n + 1] first tile of each stream; [n] the feed's tiles
+  long long* off16;          // [n + 1] packed 16 kHz offsets (a bad stream: cap16 + 1 samples, never read)
+  int16_t* pcm16;            // [n (cap16 + 1)] the feed's 16 kHz samples
+  const int16_t* samples;    // the caller's source packets (may be pinned host memory)
+  const long long* offsets;  // [n + 1]
+};
+// Plan (one CTA) then resample (`grid` CTAs looping over the feed's tiles): two launches.
+void enqueue_stream_resample(const StreamResampleParams& p, int grid, cudaStream_t st);
+// Zero n_in and both histories of the streams with end[i] != 0: one launch.
+void enqueue_stream_resample_end(const StreamResampleParams& p, const uint8_t* end, cudaStream_t st);
+
 #if defined(VADB_RESAMPLE_KERNELS)
 __global__ void __launch_bounds__(256) resample_fill_kernel(ResampleUtt* dst, int n, const __grid_constant__ ResampleFill f) {
   for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = f.u[i];

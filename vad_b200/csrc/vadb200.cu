@@ -25,6 +25,7 @@
 #include "ffn_train.cuh"
 #include "vad_segments.cuh"
 #include "vad_resample.cuh"
+#include "vad_stream_resample.h"
 
 using namespace vadb;
 
@@ -216,6 +217,19 @@ struct vadb200_bank {
   int ring_len = 0;
   DevBuf<int16_t> d_pcm;
   DevBuf<long long> d_total;
+  // resampling ragged bank (vadb200_stream_bank_create_ragged_rate at a rate other than 16000): the source-rate side
+  // of vad_stream_resample.cu.  max_feed above is cap16, so the 16 kHz ragged state is sized for one feed's output.
+  int sample_rate = 16000;
+  int src_cap = 0;             // cap on one packet, in source samples; 0: no resampling
+  ResampleDesign rs{};
+  DevBuf<float> d_taps;        // [up][Ks] polyphase rows (polyphase_taps)
+  DevBuf<long long> d_nin;     // [n] source samples taken
+  DevBuf<int> d_cur;           // [n] history buffer the next feed reads
+  DevBuf<int16_t> d_shist;     // [2][n][K - 1] source history
+  DevBuf<SrsFeed> d_feed;      // [n] this feed's plan
+  DevBuf<int> d_tile_off;      // [n + 1]
+  DevBuf<long long> d_off16;   // [n + 1]
+  DevBuf<int16_t> d_pcm16;     // [n (cap16 + 1)]
   // speech segments (vadb200_stream_bank_set_speech); d_seg empty: off.  One allocation of
   // [W1 + W2 + 2][n] words: ring1, ring2, meta, last (vad_segments.cuh StreamSeg).
   SmoothParams sp{};
@@ -922,6 +936,44 @@ int vadb200_stream_bank_create_ragged(vadb200_handle* h, int n_streams, int max_
   return 0;
 }
 
+int vadb200_stream_bank_create_ragged_rate(vadb200_handle* h, int n_streams, int max_feed_samples, int sample_rate,
+                                           vadb200_bank** out) {
+  if (out) *out = nullptr;
+  if (!h || !out) return fail(VADB200_E_INVALID, "null argument");
+  int up = 0, down = 0;
+  if (!resample_ratio(sample_rate, &up, &down))
+    return fail(VADB200_E_UNSUPPORTED,
+                "sample rate must be an integer in [4000, 384000] Hz with max(up, down) <= 1024 for 16000 Hz");
+  if (n_streams < 1 || max_feed_samples < 1 || max_feed_samples > sample_rate)
+    return fail(VADB200_E_INVALID, "bad argument (max_feed_samples must lie in [1, sample_rate])");
+  if (up == 1 && down == 1) return vadb200_stream_bank_create_ragged(h, n_streams, max_feed_samples, out);
+  const int cap16 = srs_cap16(max_feed_samples, up, down);
+  vadb200_bank* raw = nullptr;
+  const int rc = vadb200_stream_bank_create_ragged(h, n_streams, cap16, &raw);
+  if (rc) return rc;
+  std::unique_ptr<vadb200_bank> b(raw);
+  b->sample_rate = sample_rate;
+  b->src_cap = max_feed_samples;
+  b->rs = resample_design(up, down);
+  const size_t n = static_cast<size_t>(n_streams);
+  const std::vector<float> taps = polyphase_taps(b->rs, resample_taps(up, down));
+  CU(dev_upload(b->d_taps, taps.data(), taps.size()));
+  CU(dev_alloc(b->d_nin, n * sizeof(long long)));
+  CU(dev_alloc(b->d_cur, n * sizeof(int)));
+  CU(dev_alloc(b->d_shist, 2 * n * (b->rs.K - 1) * sizeof(int16_t)));
+  CU(dev_alloc(b->d_feed, n * sizeof(SrsFeed)));
+  CU(dev_alloc(b->d_tile_off, (n + 1) * sizeof(int)));
+  CU(dev_alloc(b->d_off16, (n + 1) * sizeof(long long)));
+  CU(dev_alloc(b->d_pcm16, n * (cap16 + 1) * sizeof(int16_t)));
+  const int rc2 = vadb200_stream_bank_reset(b.get(), nullptr);
+  if (rc2) return rc2;
+  CU(cudaDeviceSynchronize());  // state is zero before any stream can feed
+  *out = b.release();
+  return 0;
+}
+
+int vadb200_stream_bank_sample_rate(const vadb200_bank* b) { return b ? b->sample_rate : -1; }
+
 int vadb200_stream_bank_max_rows_per_feed(const vadb200_bank* b) {
   return b && b->max_feed ? ragged_max_rows(b->max_feed) : -1;
 }
@@ -976,6 +1028,24 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
   });
 }
 
+// The source-rate side of a resampling bank for one feed of d_samples / d_offsets (NULL for an end).
+StreamResampleParams srs_params(vadb200_bank* b, const int16_t* d_samples, const int64_t* d_offsets) {
+  StreamResampleParams p;
+  p.n = b->n; p.cap = b->src_cap; p.cap16 = b->max_feed;
+  p.up = b->rs.up; p.down = b->rs.down; p.half = b->rs.half; p.K = b->rs.K; p.Ks = b->rs.Ks; p.hs = b->rs.K - 1;
+  p.taps = b->d_taps.get();
+  p.n_in = b->d_nin.get(); p.cur = b->d_cur.get(); p.hist = b->d_shist.get(); p.feed = b->d_feed.get();
+  p.tile_off = b->d_tile_off.get(); p.off16 = b->d_off16.get(); p.pcm16 = b->d_pcm16.get();
+  p.samples = d_samples; p.offsets = reinterpret_cast<const long long*>(d_offsets);
+  return p;
+}
+
+// CTAs of stream_resample_kernel: enough for every SM to hold eight, never more than a feed can have tiles.
+int srs_grid(const vadb200_bank* b) {
+  const long long most = static_cast<long long>(b->n) * srs_tiles(b->src_cap, b->max_feed);
+  return static_cast<int>(std::min<long long>(most, 8LL * b->h->num_sms));
+}
+
 }  // namespace
 
 int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
@@ -985,6 +1055,11 @@ int vadb200_stream_bank_reset(vadb200_bank* b, void* stream) {
   if (b->max_feed) {
     CU(cudaMemsetAsync(b->d_pcm.get(), 0, static_cast<size_t>(b->n) * b->ring_len * sizeof(int16_t), st));
     CU(cudaMemsetAsync(b->d_total.get(), 0, static_cast<size_t>(b->n) * sizeof(long long), st));
+    if (b->src_cap) {
+      CU(cudaMemsetAsync(b->d_nin.get(), 0, static_cast<size_t>(b->n) * sizeof(long long), st));
+      CU(cudaMemsetAsync(b->d_cur.get(), 0, static_cast<size_t>(b->n) * sizeof(int), st));
+      CU(cudaMemsetAsync(b->d_shist.get(), 0, 2 * static_cast<size_t>(b->n) * (b->rs.K - 1) * sizeof(int16_t), st));
+    }
   } else {
     CU(cudaMemsetAsync(b->d_hist.get(), 0, static_cast<size_t>(b->n) * 320 * sizeof(int16_t), st));
     CU(cudaMemsetAsync(b->d_fed.get(), 0, static_cast<size_t>(b->n) * sizeof(int), st));
@@ -1013,11 +1088,16 @@ int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const 
   rp.n_streams = b->n; rp.max_feed = b->max_feed; rp.ring_len = b->ring_len; rp.max_rows = ragged_max_rows(b->max_feed);
   rp.pcm = b->d_pcm.get(); rp.total = b->d_total.get(); rp.ring = b->d_ring.get();
   rp.samples = d_samples; rp.offsets = reinterpret_cast<const long long*>(d_offsets);
+  if (b->src_cap) {  // resampling bank: the ragged kernel reads the 16 kHz samples the two steps before it leave
+    rp.samples = b->d_pcm16.get();
+    rp.offsets = b->d_off16.get();
+  }
   rp.counts = d_counts; rp.labels = d_labels; rp.logits = d_logits; rp.rows = d_rows; rp.bounds = d_bounds;
   rp.tw1 = h->d_tw.get(); rp.tw2 = h->d_tw.get() + 256; rp.feat_mode = VADB200_FEAT_ANALYSER;
   rp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
-  return launched(1, [&] {
+  return launched(b->src_cap ? 3 : 1, [&] {
+    if (b->src_cap) enqueue_stream_resample(srs_params(b, d_samples, d_offsets), srs_grid(b), st);
     if (b->d_seg)  // speech on: every feed advances the segment state
       stream_ragged_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par,
                                                                                       bank_seg(b, nullptr, nullptr));
@@ -1065,10 +1145,12 @@ int vadb200_stream_bank_end_streams(vadb200_bank* b, const uint8_t* d_end, uint8
   const size_t smem = static_cast<size_t>(words) * kSegEndThreads * sizeof(uint32_t);
   const unsigned grid = (b->n + kSegEndThreads - 1) / kSegEndThreads;
   if (b->max_feed)
-    return launched(1, [&] {
+    return launched(b->src_cap ? 2 : 1, [&] {
       stream_end_ragged_kernel<<<grid, kSegEndThreads, smem, static_cast<cudaStream_t>(stream)>>>(
           g, d_end, b->n, b->d_total.get(), b->d_ring.get(), g.meta ? d_tail_rows : nullptr,
           g.meta ? d_tail_bounds : nullptr);
+      if (b->src_cap)  // and the source-rate state: the next packet starts a new signal
+        enqueue_stream_resample_end(srs_params(b, nullptr, nullptr), d_end, static_cast<cudaStream_t>(stream));
     });
   return launched(1, [&] {
     stream_end_kernel<<<(b->n + kSegEndThreads - 1) / kSegEndThreads, kSegEndThreads, smem,

@@ -474,18 +474,26 @@ def speech_ms_to_rows(ms):
 
 class StreamBankHandle(object):
     """A stream bank.  With ``max_feed_samples`` (1 .. 16000) it is a ragged bank: each feed takes any number of
-    samples per stream up to that cap (``feed_ragged_ptr``) instead of one 160-sample chunk (``feed_ptr``)."""
+    samples per stream up to that cap (``feed_ragged_ptr``) instead of one 160-sample chunk (``feed_ptr``).  A ragged
+    bank at another ``sample_rate`` takes packets at that rate (the cap counted in its samples) and resamples them to
+    16 kHz on the device (vadb200_stream_bank_create_ragged_rate)."""
 
-    def __init__(self, handle, n_streams, max_feed_samples=None):
+    def __init__(self, handle, n_streams, max_feed_samples=None, sample_rate=16000):
         self.handle = handle
         self.lib = handle.lib
         self.n = int(n_streams)
         self.max_feed = None if max_feed_samples is None else int(max_feed_samples)
+        self.sample_rate = int(sample_rate)
         self._b = C.c_void_p()
         if self.max_feed is None:
+            if self.sample_rate != 16000:
+                raise ValueError("a fixed bank takes 16 kHz chunks: give max_feed_samples for another sample rate")
             check(self.lib.vadb200_stream_bank_create(handle._h, self.n, C.byref(self._b)))
-        else:
+        elif self.sample_rate == 16000:
             check(self.lib.vadb200_stream_bank_create_ragged(handle._h, self.n, self.max_feed, C.byref(self._b)))
+        else:
+            check(self.lib.vadb200_stream_bank_create_ragged_rate(handle._h, self.n, self.max_feed, self.sample_rate,
+                                                                   C.byref(self._b)))
 
     def close(self):
         if getattr(self, "_b", None) is not None and self._b:
