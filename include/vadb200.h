@@ -113,6 +113,44 @@ int vadb200_get_frontend(vadb200_handle* h, float* preemph, float* h_window /* n
 int vadb200_set_decision_threshold(vadb200_handle* h, float p_voiced);
 float vadb200_get_decision_threshold(vadb200_handle* h);
 
+/* ---- decision-tree classifier (a fitted sklearn DecisionTreeClassifier, as realtime_analysis/vad.py loads) ------
+ * vadb200_set_tree takes exactly the arrays clf.tree_ and clf.classes_ expose: children_left / children_right (-1 at
+ * a leaf), feature, threshold (float64), value [n_nodes][n_classes] (float64, tree_.value[:, 0, :]) and classes_
+ * (int64 ids, distinct, ascending, each in {0, 1, 2}, config.py:45-47).  Features are the 39 columns of
+ * vadb200_vad_windows' feature rows, in that order.  Malformed input (a child index out of range or not greater than
+ * its parent's, a node with two parents or none, a node with one child, a feature outside [0, 39), a class outside
+ * {0, 1, 2}, a NaN threshold, a negative or non-finite value, more than 2^26 nodes) returns VADB200_E_INVALID and
+ * leaves the handle unchanged.  n_nodes == 0 is vadb200_clear_tree.  Host pointers; drains the device like
+ * vadb200_set_ffn_weights, so it must not race the handle's own launches.
+ * While a tree is set it is the classifier of vadb200_vad_packed / _vad_host / _vad_windows / _stream_feed /
+ * _stream_feed_speech / _stream_feed_ragged (the FFN weights stay set underneath it; vadb200_ffn_predict keeps
+ * running the FFN).  The decision is sklearn's, exactly, on the features the device computed:
+ *   - a node sends x right when x > t32, t32 the largest float32 <= threshold (round toward -inf; >= FLT_MAX: +inf),
+ *     which for float32 x is sklearn's float64 test x <= threshold;
+ *   - argmax (threshold <= 0): speech <=> classes_[argmax(value[leaf])] == 1, ties to the first maximum as
+ *     np.argmax; class 2 (music) is non-speech;
+ *   - threshold p > 0 (vadb200_set_decision_threshold): speech <=> p1 >= (double)p, p1 = value[leaf][class 1] in
+ *     float64 (predict_proba's column; 0 when the tree lacks class 1).
+ * value is taken as predict_proba, as sklearn >= 1.4 stores it (class fractions); a caller holding class counts
+ * divides each row by its sum first.  Where a path returns logits (d_logits / h_logits), a tree writes
+ * float32(value[leaf]) there in the columns of class ids 0, 1, 2 (0 for a class the tree lacks).  A row with a
+ * non-finite feature gets label 0 and NaN in all three columns, as with the FFN. */
+#define VADB200_CLASSIFIER_NONE 0
+#define VADB200_CLASSIFIER_FFN 1
+#define VADB200_CLASSIFIER_TREE 2
+int vadb200_set_tree(vadb200_handle* h, int64_t n_nodes, const int64_t* h_children_left,
+                     const int64_t* h_children_right, const int64_t* h_feature, const double* h_threshold,
+                     const double* h_value, const int64_t* h_classes, int n_classes);
+int vadb200_clear_tree(vadb200_handle* h);
+int vadb200_get_classifier(const vadb200_handle* h);         /* VADB200_CLASSIFIER_*; -1 for NULL */
+int64_t vadb200_tree_node_count(const vadb200_handle* h);    /* 0 without a tree */
+int vadb200_tree_depth(const vadb200_handle* h);             /* internal nodes on the longest path; 0 without */
+/* The tree over feature rows d_x [n][39] (classifier.predict duck type): d_labels [n] (nullable) gets the decision
+ * above, d_proba [n][3] (nullable) the probabilities.  One launch, no allocation, graph-capturable;
+ * VADB200_E_STATE without a tree. */
+int vadb200_tree_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t* d_labels, float* d_proba,
+                         void* stream);
+
 /* ---- ragged packed batches (replaces dataset_creator.process_files' Pool.map over files,
  * dataset_creator.py:53-65, and split_into_frames, file_processing.py:80-103) ---------------
  * Utterance u occupies samples [offsets[u], offsets[u] + lengths[u]) of one int16 buffer;

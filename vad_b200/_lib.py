@@ -39,6 +39,12 @@ SIGNATURES = {
     "vadb200_get_frontend": (C.c_int, [_P, _P, _P, _P]),
     "vadb200_set_decision_threshold": (C.c_int, [_P, C.c_float]),
     "vadb200_get_decision_threshold": (C.c_float, [_P]),
+    "vadb200_set_tree": (C.c_int, [_P, _I64, _P, _P, _P, _P, _P, _P, C.c_int]),
+    "vadb200_clear_tree": (C.c_int, [_P]),
+    "vadb200_get_classifier": (C.c_int, [_P]),
+    "vadb200_tree_node_count": (_I64, [_P]),
+    "vadb200_tree_depth": (C.c_int, [_P]),
+    "vadb200_tree_predict": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
     "vadb200_plan_create": (C.c_int, [_P, _P, _P, _I64, C.c_int, C.POINTER(_P)]),
     "vadb200_plan_destroy": (C.c_int, [_P]),
     "vadb200_plan_total_rows": (_I64, [_P]),

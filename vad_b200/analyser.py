@@ -1,6 +1,6 @@
 """Drop-ins for realtime_analysis/: the ``Analyser`` plugin interface (analyser.py:4-15), a
 fused-GPU ``FusedAnalyser`` with SKLearnAnalyzer's exact feed_frame contract
-(sklearn_analyser.py:15-130), a ``.predict`` duck-typed ``FFNClassifier``
+(sklearn_analyser.py:15-130), ``.predict`` duck-typed ``FFNClassifier`` and ``TreeClassifier``
 (sklearn_analyser.py:71) and a many-stream ``StreamBank`` for 10 ms hop chunks."""
 import abc
 import pickle
@@ -58,14 +58,55 @@ class FFNClassifier(object):
         return self.handle.ffn_predict(np.asarray(x, dtype=np.float32))[1].cpu().numpy()
 
 
+class TreeClassifier(object):
+    """A fitted sklearn DecisionTreeClassifier (or a pickle / .npz path, ``runtime.tree_arrays``) run on the device:
+    ``predict`` / ``predict_proba`` duck types.  ``predict`` returns sklearn's class ids (1 = VOICED; with a handle
+    threshold, 1 where predict_proba[:, 1] >= threshold), ``predict_proba`` float32 columns by class id 0, 1, 2.
+    Without ``handle`` it gets a private one, so it never replaces another object's classifier."""
+
+    def __init__(self, tree, handle=None):
+        self._arrays = runtime.tree_arrays(tree)
+        self.classes_ = self._arrays["classes"]
+        self.handle = handle if handle is not None else runtime.Handle()
+        self.handle.set_tree(self._arrays)
+
+    @staticmethod
+    def classes_of(labels, proba):
+        """Class ids from the device's decision and probabilities: 1 for speech, else 2 where music outweighs
+        silence (the first maximum wins ties, as np.argmax), else 0."""
+        labels = np.asarray(labels)
+        proba = np.asarray(proba)
+        return np.where(labels != 0, 1, np.where(proba[:, 2] > proba[:, 0], 2, 0)).astype(np.int64)
+
+    def predict(self, x):
+        labels, proba = self.handle.tree_predict(np.asarray(x, dtype=np.float32))
+        return self.classes_of(labels.cpu().numpy(), proba.cpu().numpy())
+
+    def predict_proba(self, x):
+        return self.handle.tree_predict(np.asarray(x, dtype=np.float32))[1].cpu().numpy()
+
+
+def _tree_handle(classifier, handle):
+    """The handle a StreamBank runs ``classifier`` (a TreeClassifier, sklearn tree or path) on."""
+    if isinstance(classifier, TreeClassifier):
+        if handle is None or handle is classifier.handle:
+            return classifier.handle
+        classifier = classifier._arrays
+    h = handle if handle is not None else runtime.Handle()
+    h.set_tree(classifier)
+    return h
+
+
 class FusedAnalyser(Analyser):
     """SKLearnAnalyzer (sklearn_analyser.py:15-130) on the GPU.
 
     ``feed_frame(frame)`` takes one whole frame (float / int array of <= 512 samples, vad.py
     feeds 400), returns None for the first five calls, then the raw frame fed three calls
     earlier when it is classified speech, else None.  ``classifier`` may be: None (use the fused
-    FFN with ``ffn_weights``), a path to a pickled object with ``.predict`` (as the reference's
-    ``fname``), or such an object; an external classifier receives the reference's (1, 39)
+    FFN with ``ffn_weights``), a ``TreeClassifier`` (the tree runs on the device next to the
+    features, no per-frame host call; a tree's class 2 still raises AssertionError), a path to a
+    pickled object with ``.predict`` (as the reference's ``fname``), or such an object; an external
+    classifier receives the reference's (1, 39)
     float64 feature row and anything other than class 0 / 1 raises AssertionError
     (sklearn_analyser.py:76-82).  The reference's spectral subtraction is computed and discarded
     there (sklearn_analyser.py:121-123), so it is not reproduced."""
@@ -81,13 +122,17 @@ class FusedAnalyser(Analyser):
             raise NotImplementedError("vad_b200 kernels are compiled for the reference configuration only")
         self.sample_rate, self.fft_n, self.mfcc_num = sample_rate, int(fft_n), mfcc_num
         self.low_hz, self.high_hz, self.fbank_num = low_hz, high_hz, fbank_num
+        self.tree = isinstance(classifier, TreeClassifier)
+        if self.tree:
+            handle = _tree_handle(classifier, handle)
+            classifier = None
         if isinstance(classifier, str):
             with open(classifier, "rb") as f:
                 classifier = pickle.load(f)
         self.classifier = classifier
-        self.handle = _handle_for(ffn_weights if classifier is None else None, handle)
+        self.handle = handle if self.tree else _handle_for(ffn_weights if classifier is None else None, handle)
         self.filterbank = self.handle.filterbank()
-        if classifier is None:
+        if classifier is None and not self.tree:
             if not self.handle.has_ffn:
                 raise RuntimeError("FusedAnalyser needs FFN weights or an external classifier")
         self.frames_buffer = []
@@ -115,7 +160,10 @@ class FusedAnalyser(Analyser):
         processing_frame = self.frames_buffer[self.PROCESSING_FRAME_INDEX]
         window = torch.stack(self.frames_mfcc_buffer)[None]
         labels, logits, feats = self.handle.vad_windows(window, FEAT_ANALYSER, want_feats=self.classifier is not None)
-        if self.classifier is None:
+        if self.tree:
+            self.last_logits = logits[0]
+            cls = int(TreeClassifier.classes_of(labels[:1].cpu().numpy(), logits[:1].cpu().numpy())[0])
+        elif self.classifier is None:
             cls = int(labels[0].item())
             self.last_logits = logits[0]
         else:
@@ -160,14 +208,18 @@ class StreamBank(object):
     ``batch.resample``'s filter: after N samples a stream has the rows of ``vad_batch`` on the first M(N) samples of
     its resampled signal plus one (see include/vadb200.h), which trails the input by half / up source samples (at most
     1.25 ms).  Rows keep the 16 kHz, 10 ms framing; segment bounds come back in source samples, mapped as
-    ``batch.source_bounds`` maps them."""
+    ``batch.source_bounds`` maps them.
+
+    ``classifier`` (a ``TreeClassifier``, fitted sklearn DecisionTreeClassifier, pickle or .npz path) runs every bank
+    on a decision tree instead of the FFN (``Handle.set_tree``).  Captured ticks are recaptured after the handle's
+    classifier or threshold changes."""
 
     NOT_READY = 255
     max_feed = None          # ragged bank: the cap on one stream's samples per tick
     sample_rate = 16000      # the rate of the samples fed
 
     def __init__(self, n_streams, ffn_weights=None, handle=None, use_graph=True, zero_copy=True,
-                 max_feed_samples=None, sample_rate=16000):
+                 max_feed_samples=None, sample_rate=16000, classifier=None):
         rate = int(sample_rate)
         if rate != 16000:    # checked before any device work
             if max_feed_samples is None:
@@ -176,9 +228,12 @@ class StreamBank(object):
                 raise ValueError("unsupported sample rate %r" % (sample_rate,))
         if max_feed_samples is not None and not 1 <= int(max_feed_samples) <= rate:
             raise ValueError("max_feed_samples must lie in [1, %d]" % rate)
-        self.handle = _handle_for(ffn_weights, handle)
-        if not self.handle.has_ffn:
-            raise RuntimeError("StreamBank needs FFN weights")
+        if classifier is not None:   # a decision tree: TreeClassifier, fitted sklearn tree, pickle or .npz path
+            self.handle = _tree_handle(classifier, handle)
+        else:
+            self.handle = _handle_for(ffn_weights, handle)
+        if not self.handle.has_classifier:
+            raise RuntimeError("StreamBank needs FFN weights or a decision tree")
         self.n = int(n_streams)
         self.sample_rate = rate
         if max_feed_samples is not None:
@@ -206,6 +261,7 @@ class StreamBank(object):
         self.use_graph = bool(use_graph)
         self.zero_copy = bool(zero_copy)
         self._graphs = {}
+        self._graph_version = self.handle.classifier_version
         self.delay = -1          # speech delay D in rows; -1: speech off
         self.h_rows = self.h_bounds = self.d_rows = self.d_bounds = None
         self.d_tail_rows = self.d_tail_bounds = None
@@ -258,6 +314,9 @@ class StreamBank(object):
     def _tick(self, want_logits, speech=False):
         """One H2D + kernel + D2H; returns after the labels are on the host."""
         if self.use_graph:
+            if self._graph_version != self.handle.classifier_version:   # captured ticks hold the old classifier
+                self._graphs = {}
+                self._graph_version = self.handle.classifier_version
             key = (want_logits, speech)
             g = self._graphs.get(key)
             if g is None:  # capture once (capturing does not execute: no chunk is consumed)

@@ -107,7 +107,7 @@ def vad_batch(utterances, handle=None, want_logits=False, feat_mode=FEAT_ANALYSE
     """Per-frame speech / non-speech labels (uint8) for every utterance; optionally logits.  At any other
     ``sample_rate`` the batch is resampled to 16 kHz on the device first; labels keep the 16 kHz framing."""
     handle = handle or runtime.default_handle()
-    if not handle.has_ffn:
+    if not handle.has_classifier:
         raise RuntimeError("set FFN weights first (Handle.set_ffn_weights)")
     pcm, offsets, lengths = _upload_16k(utterances, handle, sample_rate)
     plan = runtime.Plan(handle, offsets, lengths, MODE_VAD)
@@ -120,7 +120,7 @@ def vad_batch(utterances, handle=None, want_logits=False, feat_mode=FEAT_ANALYSE
 
 def _speech_run(utterances, handle, min_speech_ms, min_silence_ms, pad_ms, feat_mode, sample_rate):
     handle = handle or runtime.default_handle()
-    if not handle.has_ffn:
+    if not handle.has_classifier:
         raise RuntimeError("set FFN weights first (Handle.set_ffn_weights)")
     for v in (min_speech_ms, min_silence_ms, pad_ms):
         runtime.speech_ms_to_rows(v)               # argument errors before any device work

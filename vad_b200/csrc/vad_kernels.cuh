@@ -23,7 +23,7 @@
 // features and runs Dense 39-64-32-16-3 -- on FP32 CUDA cores (TC = 0, every 8 steps), as one tcgen05
 // tile of 128 frames with TMEM accumulators (TC = 1, tf32 hi/lo operands, every 4 steps) or as two such
 // tiles of 128 frames side by side in TMEM (TC = 2, fp16 hi/lo operands, every 8 steps) -- then
-// argmax == VOICED, 1-byte label.
+// argmax == VOICED, 1-byte label; or walks a decision tree instead (TC = 3, one thread per centre, every 8 steps).
 //
 // Reference lines restated: mfcc.py:59-78; dataset/file_processing.py:47-70,99-101;
 // realtime_analysis/sklearn_analyser.py:46-82,103-107; learning/ffn_trainer.py:104-116.
@@ -34,6 +34,7 @@
 #include "vad_core.cuh"
 #include "ffn_tc.cuh"
 #include "vad_ragged.h"
+#include "vad_tree.cuh"
 
 namespace vadb {
 
@@ -293,6 +294,25 @@ __device__ __forceinline__ void store_feats_half(float* feats, long long row, in
       if (k < nk) feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
 }
 
+// One output row per thread: window features -> tree -> decision (block phase / windows API).  The features pass
+// through this thread's column of a shared-memory tile x[f * stride] (a walk indexes them by node).
+__device__ __forceinline__ void tree_classify_row(const TreeArg& tr, const float (&r)[5][kNCep], int feat_mode,
+                                                  float* xs, int stride, uint8_t* labels, float* logits, float* feats,
+                                                  long long row, float th) {
+  float x[kNFeat];
+  const bool ok = window_features(r, feat_mode, x);
+#pragma unroll
+  for (int i = 0; i < kNFeat; ++i) xs[i * stride] = x[i];
+  float p[kNCls];
+  const uint8_t lab = reject_nonfinite(ok, tree_decide(tree_walk(tr, [&](uint32_t f) { return xs[f * stride]; }), th, p), p);
+  if (labels) labels[row] = lab;
+  store_logits(logits, row, p);
+  if (feats) {
+#pragma unroll
+    for (int i = 0; i < kNFeat; ++i) feats[row * kNFeat + i] = x[i];
+  }
+}
+
 // One output row per thread: window features -> FFN -> decision (block phase / windows API).
 // th: decision threshold (decide); 0 = argmax.
 __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r)[5][kNCep], int feat_mode,
@@ -312,13 +332,15 @@ __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r
 
 // MODE 0: MFCC rows [T][13]; 1: dataset rows [T-5][39]; 2: VAD labels [T-5].
 // TC (MODE 2 only): 0 = FFN on FP32 CUDA cores, 1 = FFN on tcgen05 kind::tf32 (hi/lo split, TMEM accumulators),
-// 2 = tcgen05 kind::f16 on statically scaled fp16 hi/lo operands (half the MMAs, half the weight blob).
+// 2 = tcgen05 kind::f16 on statically scaled fp16 hi/lo operands (half the MMAs, half the weight blob), 3 = decision tree
+// (vad_tree.cuh) on the TC = 0 block phase.
 // FFN argument of the kernel variant: nothing (MFCC / dataset rows), the full FP32 weights, or the biases
 // only (tensor-core FFN: the weights are the per-handle tcgen05 operand blob in global memory).
 template <int MODE, int TC> struct FfnArgOf { using type = FfnNone; };
 template <> struct FfnArgOf<2, 0> { using type = FfnParams; };
 template <> struct FfnArgOf<2, 1> { using type = FfnBias; };
 template <> struct FfnArgOf<2, 2> { using type = FfnBias; };
+template <> struct FfnArgOf<2, 3> { using type = TreeArg; };
 
 // The decision of the VAD block phase: argmax, or with the front-end variant the handle's threshold.
 template <bool FE, class A>
@@ -339,6 +361,7 @@ template <int MODE, int TC, bool FE>
 __device__ __forceinline__ void fused_body(const FusedParams& p, const typename FfnArgOf<MODE, TC>::type& ffn,
                                            const FrontEnd& fe, const int tid) {
   static_assert(TC == 0 || MODE == 2, "tensor-core FFN only exists in VAD mode");
+  constexpr bool kTmem = TC == 1 || TC == 2;  // the tensor-core FFN variants
   constexpr int kBlk = TC == 1 ? kBlockStepsTc : kBlockSteps;
   constexpr int kStageOff = FE ? kStageOffFe : 0;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -368,7 +391,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
   }
   uint32_t tm_base = 0, w_par = 0, mma_par = 0;
   int dbg_n = 0;
-  if (TC) {
+  if (kTmem) {
     if (warp == 0) tmem_alloc(s_tmem, kTmemCols);
     tc_fence_before();
     __syncthreads();
@@ -484,7 +507,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
       warp_arrive(&s_bar[4], lane);
       const int computed = min((s + 1) * kStepFrames, n);
       const bool block_now = (((s + 1) % kBlk) == 0 || s == nsteps - 1) && !(VADB_DBG(p) & 8);
-      const bool tc_now = TC && block_now && (computed - 2 - out_done) > 0;  // block-uniform
+      const bool tc_now = kTmem && block_now && (computed - 2 - out_done) > 0;  // block-uniform
       dct_pending = !block_now;
 
       // A step that is followed by a block phase transforms its own log-mel tile right away, behind a CTA barrier.
@@ -551,7 +574,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
             __syncthreads();  // the next FFT phase rewrites exch / P
           }
           out_done = max(out_done, computed - 2);
-        } else if (!TC) {
+        } else if (TC == 0 || TC == 3) {
           const int c = out_done + tid;
           if (c <= computed - 3) {
             float r[5][kNCep];
@@ -564,7 +587,12 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
             if constexpr (MODE == 2 && TC == 0)
               classify_row(ffn, r, p.feat_mode, p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2),
                            FE ? ffn.thresh : 0.0f);
+            else if constexpr (TC == 3)  // features staged in exch + P, idle until the next FFT phase
+              tree_classify_row(ffn, r, p.feat_mode, reinterpret_cast<float*>(smem + kOffExch) + tid, kThreads,
+                                p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2),
+                                FE ? ffn.thresh : 0.0f);
           }
+          if constexpr (TC == 3) __syncthreads();  // the next FFT phase rewrites the staged features
           out_done = max(out_done, computed - 2);
         } else if constexpr (TC == 2) {
           // ---- fp16 tensor-core FFN: two M = 128 tiles, thread = frame = TMEM lane of tile warp / 4 ---------------
@@ -668,7 +696,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
       }
     }
   }
-  if (TC) {
+  if (kTmem) {
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tm_base, kTmemCols);
@@ -934,6 +962,37 @@ __global__ void __launch_bounds__(128) windows_kernel(const float* win, long lon
   classify_row(w, r, feat_mode, labels, logits, feats, i, w.thresh);
 }
 
+// The same with a decision tree: labels, probabilities (in logits' place) and features.
+static_assert(kNFeat * 128 * 4 <= 48 * 1024, "windows_tree_kernel's feature tile");
+__global__ void __launch_bounds__(128) windows_tree_kernel(const float* win, long long n, int feat_mode, uint8_t* labels,
+                                                           float* proba, float* feats, const __grid_constant__ TreeArg tr) {
+  __shared__ float s_x[kNFeat * 128];
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float r[5][kNCep];
+#pragma unroll
+  for (int d = 0; d < 5; ++d)
+#pragma unroll
+    for (int k = 0; k < kNCep; ++k) r[d][k] = win[(i * 5 + d) * kNCep + k];
+  tree_classify_row(tr, r, feat_mode, s_x + threadIdx.x, 128, labels, proba, feats, i, tr.thresh);
+}
+
+// Decision tree over feature rows [n][39] (vadb200_tree_predict): one thread per row; the walk reads the row from
+// global memory (L1 after the finiteness check).
+__global__ void __launch_bounds__(128) tree_rows_kernel(const float* x, long long n, uint8_t* labels, float* proba,
+                                                        const __grid_constant__ TreeArg tr) {
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float* row = x + i * kNFeat;
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < kNFeat; ++k) ok = ok && (fabsf(row[k]) <= 3.0e38f);
+  float p[kNCls];
+  const uint8_t lab = reject_nonfinite(ok, tree_decide(tree_walk(tr, [&](uint32_t f) { return row[f]; }), tr.thresh, p), p);
+  if (labels) labels[i] = lab;
+  store_logits(proba, i, p);
+}
+
 // classifier.predict duck type (sklearn_analyser.py:71): rows [n][39] -> class {0,1}, logits.
 __global__ void __launch_bounds__(128) ffn_rows_kernel(const float* x, long long n, uint8_t* labels, float* logits,
                                                        const __grid_constant__ FfnParams w) {
@@ -1148,6 +1207,21 @@ __device__ __forceinline__ uint8_t stream_decide(const StreamSmem& sm, const Ffn
   return lab;
 }
 
+// The tree's decision of the stream in this lane (features x[f][lane]); as stream_decide above.
+__device__ __forceinline__ uint8_t stream_decide(const StreamSmem& sm, const TreeArg& tr, int lane, float (&lg)[3]) {
+  float p[kNCls];
+  uint8_t lab = tree_decide(tree_walk(tr, [&](uint32_t f) { return sm.x[f * 32 + lane]; }), tr.thresh, p);
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < kNCep; ++k) ok = ok && (sm.ok[k * 32 + lane] != 0);
+  if (ok) {
+    lg[0] = p[0]; lg[1] = p[1]; lg[2] = p[2];
+  } else {
+    lab = 0;
+  }
+  return lab;
+}
+
 // One CTA = 32 streams.  FFT: the fused kernel's packed two-frames-per-thread pass.  The decision
 // tail is spread over all 8 warps with lane = stream: warp w owns cepstral coefficients w, w + 8
 // (DCT, ring push, window features) and then 8 / 4 / 2 neurons of layers 1 / 2 / 3, activations
@@ -1155,9 +1229,9 @@ __device__ __forceinline__ uint8_t stream_decide(const StreamSmem& sm, const Ffn
 // SEG: the speech variant (stream_feed_speech_kernel) also runs each stream's online smoothing step
 // (vad_segments.cuh seg_step, found when the variant is instantiated with Seg = StreamSeg) on the label warp 0
 // holds, and writes the finalised row and its bound.
-template <bool SEG, class Seg>
-__device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnParams& w, const Seg& sg,
-                                                 const int tid) {
+// W: FfnParams, or TreeArg (stream_feed_tree_kernel: no hidden layers, warp 0 walks the tree).
+template <bool SEG, class Seg, class W>
+__device__ __forceinline__ void stream_feed_body(const BankParams& p, const W& w, const Seg& sg, const int tid) {
   extern __shared__ __align__(128) unsigned char smem[];
   const StreamSmem sm(smem);
   int16_t* s_fr = sm.fr;
@@ -1205,7 +1279,7 @@ __device__ __forceinline__ void stream_feed_body(const BankParams& p, const FfnP
   // (a row is classified once frame >= 5: the ring then holds frames frame-5 .. frame-1 and frame-3 is the centre)
   stream_window_features(sm, p.ring, p.n_streams, st, live, frame, p.feat_mode, warp, lane, slot);
   __syncthreads();
-  stream_ffn_hidden(sm, w, warp, lane);
+  if constexpr (std::is_same<W, FfnParams>::value) stream_ffn_hidden(sm, w, warp, lane);
   if (warp == 0) {
     const int stl = s0 + lane;
     if (stl < p.n_streams) {
@@ -1242,6 +1316,13 @@ __global__ void __launch_bounds__(kThreads) stream_feed_speech_kernel(const Bank
   stream_feed_body<true>(p, w, sg, threadIdx.x);
 }
 
+// The fixed tick with a decision tree (SEG: plus the segment step).
+template <bool SEG, class Seg>
+__global__ void __launch_bounds__(kThreads) stream_feed_tree_kernel(const BankParams p, const __grid_constant__ TreeArg tr,
+                                                                   const __grid_constant__ Seg sg) {
+  stream_feed_body<SEG>(p, tr, sg, threadIdx.x);
+}
+
 // ---- ragged bank (vadb200_stream_bank_create_ragged): any number of samples per stream and feed ----------------
 // State per stream: a sample ring int16[R] and the samples taken N (vad_ragged.h), and the MFCC ring [5*13][n] of
 // the fixed bank.  Stream i's packet of this feed is samples[offsets[i] .. offsets[i + 1]).
@@ -1274,9 +1355,8 @@ constexpr int kRaggedLoads = 8;  // packet samples each thread loads before it s
 // into the fixed tick's rows), run the fixed tick's FFT, mel, DCT, window features and FFN on it, and emit row
 // f0 + j - 5 of the streams that have it, with the segment step (SEG) in row order.  Staged words, FFT and FFMA
 // order are the fixed tick's, so every row is bit-identical to it.  A CTA with no frame to complete stops after (1).
-template <bool SEG, class Seg>
-__device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const FfnParams& w, const Seg& sg,
-                                                   const int tid) {
+template <bool SEG, class Seg, class W>
+__device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const W& w, const Seg& sg, const int tid) {
   extern __shared__ __align__(128) unsigned char smem[];
   const StreamSmem sm(smem);
   __shared__ long long s_off[kStepFrames + 1];
@@ -1383,7 +1463,7 @@ __device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const 
     stream_fft_mel(sm, p.fe, warp, lane);
     stream_window_features(sm, p.ring, p.n_streams, s0 + slot, j < s_nf[slot], 0, p.feat_mode, warp, lane, slot);
     __syncthreads();
-    stream_ffn_hidden(sm, w, warp, lane);
+    if constexpr (std::is_same<W, FfnParams>::value) stream_ffn_hidden(sm, w, warp, lane);
     if (warp == 0 && j < s_nf[lane]) {
       const long long f = s_f0[lane] + j;
       if (f >= 5) {                          // row f - 5 of the stream, output slot k
@@ -1415,6 +1495,14 @@ __global__ void __launch_bounds__(kThreads) stream_ragged_speech_kernel(const __
                                                                        const __grid_constant__ FfnParams w,
                                                                        const __grid_constant__ Seg sg) {
   stream_ragged_body<true>(p, w, sg, threadIdx.x);
+}
+
+// The ragged feed with a decision tree (SEG: plus the segment step).
+template <bool SEG, class Seg>
+__global__ void __launch_bounds__(kThreads) stream_ragged_tree_kernel(const __grid_constant__ RaggedParams p,
+                                                                     const __grid_constant__ TreeArg tr,
+                                                                     const __grid_constant__ Seg sg) {
+  stream_ragged_body<SEG>(p, tr, sg, threadIdx.x);
 }
 
 // ---- feature sink: scale_features (dataset/utils.py:5-32) on packed dataset rows [n][39] ----------------

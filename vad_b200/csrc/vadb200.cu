@@ -165,6 +165,11 @@ struct vadb200_handle {
   bool has_window = false;
   float window[kFrame] = {};
   DevBuf<cf2> d_win;                    // [kWinPairs] window pairs, all ones without a window (per handle: no globals)
+  // decision tree (vadb200_set_tree): nodes [tree_nodes] then leaf entries [tree_nodes] (vad_tree.h); empty: none.
+  // A tree takes precedence over the FFN weights, which stay set underneath it.
+  DevBuf<unsigned char> d_tree;
+  long long tree_nodes = 0;
+  int tree_depth = 0;
 };
 
 struct vadb200_plan {
@@ -247,6 +252,14 @@ struct vadb200_resampler {
 
 namespace {
 
+bool has_tree(const vadb200_handle* h) { return h->tree_nodes > 0; }
+bool has_classifier(const vadb200_handle* h) { return h->have_ffn || has_tree(h); }
+TreeArg tree_arg(const vadb200_handle* h) {
+  const TreeNode* nodes = reinterpret_cast<const TreeNode*>(h->d_tree.get());
+  return TreeArg{nodes, reinterpret_cast<const TreeLeaf*>(nodes + h->tree_nodes), h->tree_depth, h->par.thresh};
+}
+constexpr const char* kNoClassifier = "FFN weights not set (vadb200_set_ffn_weights)";
+
 bool frontend_on(const vadb200_handle* h) { return h->preemph != 0.0f || h->has_window; }
 FrontEnd frontend_of(const vadb200_handle* h) { return FrontEnd{h->d_win.get(), h->preemph}; }
 
@@ -289,6 +302,7 @@ int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   return launched(1, [&] {
     if (p->mode == VADB200_MODE_MFCC) enqueue_fused<0, 0>(fe, grid, st, fp, FfnNone{0}, fea);
     else if (p->mode == VADB200_MODE_DATASET) enqueue_fused<1, 0>(fe, grid, st, fp, FfnNone{0}, fea);
+    else if (has_tree(h)) enqueue_fused<2, 3>(fe, grid, st, fp, tree_arg(h), fea);
     else if (c.tc == 2) enqueue_fused<2, 2>(fe, grid, st, fp, h->bias, fea);
     else if (c.tc == 1) enqueue_fused<2, 1>(fe, grid, st, fp, h->bias, fea);
     else enqueue_fused<2, 0>(fe, grid, st, fp, h->par, fea);
@@ -406,6 +420,16 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   CU(cudaFuncSetAttribute(fused_fe_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
   CU(cudaFuncSetAttribute(fused_fe_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
   CU(cudaFuncSetAttribute(fused_fe_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_kernel<2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
+  CU(cudaFuncSetAttribute(stream_feed_tree_kernel<false, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_feed_tree_kernel<true, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_ragged_tree_kernel<false, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          kStreamSmemBytes));
+  CU(cudaFuncSetAttribute(stream_ragged_tree_kernel<true, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          kStreamSmemBytes));
   CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
   CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
   CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
@@ -470,6 +494,64 @@ int vadb200_set_ffn_impl(vadb200_handle* h, int impl) {
   return 0;
 }
 int vadb200_get_ffn_impl(vadb200_handle* h) { return h ? h->ffn_impl : -1; }
+
+// ---- decision tree (vad_tree.h) ---------------------------------------------------------------------------
+int vadb200_set_tree(vadb200_handle* h, int64_t n_nodes, const int64_t* h_children_left,
+                     const int64_t* h_children_right, const int64_t* h_feature, const double* h_threshold,
+                     const double* h_value, const int64_t* h_classes, int n_classes) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (n_nodes < 0) return fail(VADB200_E_INVALID, "n_nodes < 0");
+  if (n_nodes == 0) return vadb200_clear_tree(h);
+  TreeLayout L;
+  std::string why;
+  if (!tree_convert(n_nodes, h_children_left, h_children_right, h_feature, h_threshold, h_value, h_classes, n_classes,
+                    &L, &why))
+    return fail(VADB200_E_INVALID, "malformed tree: " + why);
+  const size_t nb = L.nodes.size() * sizeof(TreeNode), lb = L.leaves.size() * sizeof(TreeLeaf);
+  CU(cudaSetDevice(h->device));
+  DevBuf<unsigned char> d;
+  CU(dev_alloc(d, nb + lb));
+  // drained + blocking, like the FFN weights: no launch of this handle still reads the tree being replaced
+  CU(cudaDeviceSynchronize());
+  CU(cudaMemcpyAsync(d.get(), L.nodes.data(), nb, cudaMemcpyHostToDevice, nullptr));
+  CU(cudaMemcpyAsync(d.get() + nb, L.leaves.data(), lb, cudaMemcpyHostToDevice, nullptr));
+  CU(cudaStreamSynchronize(nullptr));
+  h->d_tree = std::move(d);
+  h->tree_nodes = n_nodes;
+  h->tree_depth = L.depth;
+  return 0;
+}
+
+int vadb200_clear_tree(vadb200_handle* h) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  CU(cudaSetDevice(h->device));
+  CU(cudaDeviceSynchronize());
+  h->d_tree.reset();
+  h->tree_nodes = 0;
+  h->tree_depth = 0;
+  return 0;
+}
+
+int vadb200_get_classifier(const vadb200_handle* h) {
+  if (!h) return -1;
+  return has_tree(h) ? VADB200_CLASSIFIER_TREE : h->have_ffn ? VADB200_CLASSIFIER_FFN : VADB200_CLASSIFIER_NONE;
+}
+int64_t vadb200_tree_node_count(const vadb200_handle* h) { return h ? h->tree_nodes : -1; }
+int vadb200_tree_depth(const vadb200_handle* h) { return h ? h->tree_depth : -1; }
+
+int vadb200_tree_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t* d_labels, float* d_proba,
+                         void* stream) {
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (!has_tree(h)) return fail(VADB200_E_STATE, "no decision tree set (vadb200_set_tree)");
+  if (n < 0) return fail(VADB200_E_INVALID, "n < 0");
+  if (n == 0) return 0;
+  if (!d_x) return fail(VADB200_E_INVALID, "null argument");
+  CU(cudaSetDevice(h->device));
+  return launched(1, [&] {
+    tree_rows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+        d_x, n, d_labels, d_proba, tree_arg(h));
+  });
+}
 
 int vadb200_set_frontend(vadb200_handle* h, float preemph, const float* h_window) {
   if (!h) return fail(VADB200_E_INVALID, "handle is null");
@@ -639,7 +721,7 @@ int vadb200_vad_packed(vadb200_plan* p, const int16_t* d_pcm, int64_t pcm_len, u
   int rc = check_pcm(p, d_pcm, pcm_len);
   if (rc) return rc;
   if (p->mode != VADB200_MODE_VAD) return fail(VADB200_E_INVALID, "plan was not created for MODE_VAD");
-  if (!p->h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!has_classifier(p->h)) return fail(VADB200_E_STATE, kNoClassifier);
   if (p->total_rows > 0 && !d_labels) return fail(VADB200_E_INVALID, "d_labels is null");
   if (feat_mode != VADB200_FEAT_ANALYSER && feat_mode != VADB200_FEAT_DATASET) return fail(VADB200_E_INVALID, "unknown feat_mode");
   CU(cudaSetDevice(p->h->device));
@@ -738,7 +820,7 @@ int vadb200_vad_host(vadb200_plan* p, const int16_t* h_pcm, int64_t pcm_len, uin
                      int feat_mode) {
   if (!p) return fail(VADB200_E_INVALID, "plan is null");
   if (p->mode != VADB200_MODE_VAD) return fail(VADB200_E_INVALID, "plan was not created for MODE_VAD");
-  if (!p->h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!has_classifier(p->h)) return fail(VADB200_E_STATE, kNoClassifier);
   if (feat_mode != VADB200_FEAT_ANALYSER && feat_mode != VADB200_FEAT_DATASET) return fail(VADB200_E_INVALID, "unknown feat_mode");
   if (p->total_rows == 0) return 0;
   if (!h_pcm || !h_labels) return fail(VADB200_E_INVALID, "null argument");
@@ -840,12 +922,17 @@ int vadb200_mfcc_from_spec(vadb200_handle* h, const float* d_spec, int64_t n, fl
 int vadb200_vad_windows(vadb200_handle* h, const float* d_win, int64_t n, int feat_mode, uint8_t* d_labels,
                         float* d_logits, float* d_feats, void* stream) {
   if (!h) return fail(VADB200_E_INVALID, "handle is null");
-  if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!has_classifier(h)) return fail(VADB200_E_STATE, kNoClassifier);
   if (n < 0) return fail(VADB200_E_INVALID, "n < 0");
   if (n == 0) return 0;
   if (!d_win) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (has_tree(h))
+    return launched(1, [&] {
+      windows_tree_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels,
+                                                                                d_logits, d_feats, tree_arg(h));
+    });
   return launched(1, [&] {
     windows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels, d_logits,
                                                                          d_feats, h->par);
@@ -1008,7 +1095,7 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
   if (!b || !d_chunks || !d_labels) return fail(VADB200_E_INVALID, "null argument");
   vadb200_handle* h = b->h;
   if (b->max_feed) return fail(VADB200_E_STATE, "a ragged bank takes vadb200_stream_feed_ragged");
-  if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!has_classifier(h)) return fail(VADB200_E_STATE, kNoClassifier);
   if (reinterpret_cast<uintptr_t>(d_chunks) & 3) return fail(VADB200_E_INVALID, "chunks must be 4-byte aligned");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1019,6 +1106,13 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
   bp.prev = b->d_prev.get();
   bp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
+  if (has_tree(h))
+    return launched(1, [&] {
+      if (b->d_seg)
+        stream_feed_tree_kernel<true><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, tree_arg(h), bank_seg(b, d_rows, d_bounds));
+      else
+        stream_feed_tree_kernel<false><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, tree_arg(h), StreamSeg{});
+    });
   return launched(1, [&] {
     if (b->d_seg)  // speech on: every feed advances the segment state
       stream_feed_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par,
@@ -1079,7 +1173,7 @@ int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const 
   if (!b || !d_samples || !d_offsets || !d_counts || !d_labels) return fail(VADB200_E_INVALID, "null argument");
   if (!b->max_feed) return fail(VADB200_E_STATE, "not a ragged bank (vadb200_stream_bank_create_ragged)");
   vadb200_handle* h = b->h;
-  if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!has_classifier(h)) return fail(VADB200_E_STATE, kNoClassifier);
   if ((d_rows || d_bounds) && !b->d_seg) return fail(VADB200_E_STATE, "speech is off (vadb200_stream_bank_set_speech)");
   if (reinterpret_cast<uintptr_t>(d_samples) & 1) return fail(VADB200_E_INVALID, "samples must be 2-byte aligned");
   CU(cudaSetDevice(h->device));
@@ -1098,7 +1192,13 @@ int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const 
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
   return launched(b->src_cap ? 3 : 1, [&] {
     if (b->src_cap) enqueue_stream_resample(srs_params(b, d_samples, d_offsets), srs_grid(b), st);
-    if (b->d_seg)  // speech on: every feed advances the segment state
+    if (has_tree(h)) {
+      if (b->d_seg)
+        stream_ragged_tree_kernel<true><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, tree_arg(h),
+                                                                                  bank_seg(b, nullptr, nullptr));
+      else
+        stream_ragged_tree_kernel<false><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, tree_arg(h), StreamSeg{});
+    } else if (b->d_seg)  // speech on: every feed advances the segment state
       stream_ragged_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par,
                                                                                       bank_seg(b, nullptr, nullptr));
     else

@@ -2,6 +2,8 @@
 batch -> segment table), StreamBankHandle.  PyTorch is used only to own device / pinned memory
 and to name the CUDA stream; every numeric result comes from libvadb200.so kernels."""
 import ctypes as C
+import os
+import pickle
 
 import numpy as np
 import torch
@@ -65,6 +67,59 @@ def load_ffn_npz(path):
     return {k: np.asarray(z[k], dtype=np.float32) for k in FFN_KEYS}
 
 
+TREE_KEYS = ("children_left", "children_right", "feature", "threshold", "value", "classes")
+
+
+def tree_arrays(tree):
+    """The arrays vadb200_set_tree takes, as a dict of TREE_KEYS, from a fitted sklearn DecisionTreeClassifier (found
+    by its ``tree_`` / ``classes_``, so sklearn is only needed by a caller that already has one), a path to a pickle of
+    one (the reference's ``fname``) or to an ``.npz`` written by ``save_tree_npz``, or such a dict.  ``value`` is
+    [n_nodes, n_classes] predict_proba rows: class counts (a tree from sklearn < 1.4) are divided by their row sum, as
+    that sklearn's predict_proba did."""
+    if isinstance(tree, (str, os.PathLike)):
+        if str(tree).endswith(".npz"):
+            return load_tree_npz(tree)
+        with open(tree, "rb") as f:
+            tree = pickle.load(f)
+    if hasattr(tree, "tree_") and hasattr(tree, "classes_"):
+        if getattr(tree, "n_outputs_", 1) != 1:
+            raise ValueError("only single-output trees are supported")
+        if getattr(tree, "n_features_in_", 39) != 39:
+            raise ValueError("the tree must take the 39 window features")
+        t = tree.tree_
+        d = dict(children_left=t.children_left, children_right=t.children_right, feature=t.feature,
+                 threshold=t.threshold, value=np.asarray(t.value)[:, 0, :], classes=tree.classes_)
+    elif all(k in tree for k in TREE_KEYS):
+        d = {k: tree[k] for k in TREE_KEYS}
+    else:
+        raise TypeError("expected a fitted DecisionTreeClassifier, a pickle or .npz path, or a dict of %r" % (TREE_KEYS,))
+    classes = np.asarray(d["classes"])
+    try:
+        cls = classes.astype(np.int64)
+    except (TypeError, ValueError):
+        raise ValueError("class labels must be the ids 0, 1, 2, got %r" % (classes,))
+    if not np.array_equal(cls, classes):
+        raise ValueError("class labels must be the ids 0, 1, 2, got %r" % (classes,))
+    value = np.array(d["value"], dtype=np.float64).reshape(len(np.asarray(d["children_left"])), cls.size)
+    s = value.sum(axis=1)
+    counts = (s > 0) & (np.abs(s - 1.0) > 1e-9)
+    value[counts] /= s[counts, None]
+    out = {k: np.ascontiguousarray(d[k], dtype=np.int64) for k in ("children_left", "children_right", "feature")}
+    out.update(threshold=np.ascontiguousarray(d["threshold"], dtype=np.float64), value=np.ascontiguousarray(value),
+               classes=np.ascontiguousarray(cls))
+    return out
+
+
+def save_tree_npz(path, tree):
+    """Write a tree's arrays (``tree_arrays``) to ``path``: a deployment then runs it without sklearn installed."""
+    np.savez(path, **tree_arrays(tree))
+
+
+def load_tree_npz(path):
+    z = np.load(path)
+    return {k: z[k] for k in TREE_KEYS}
+
+
 class Handle(object):
     """One per (process, device): owns the mel / DCT / twiddle tables and the FFN weights."""
 
@@ -82,6 +137,8 @@ class Handle(object):
         self.lib.vadb200_default_config(C.byref(cfg))
         check(self.lib.vadb200_create(C.byref(cfg), self.device.index, C.byref(self._h)))
         self.has_ffn = False
+        self.has_tree = False
+        self.classifier_version = 0   # changes with the classifier a launch captures (weights, tree, threshold)
         if ffn_weights is not None:
             self.set_ffn_weights(ffn_weights)
 
@@ -114,6 +171,51 @@ class Handle(object):
             arrs.append(a)
         check(self.lib.vadb200_set_ffn_weights(self._h, *[a.ctypes.data_as(C.c_void_p) for a in arrs]))
         self.has_ffn = True
+        self.classifier_version += 1
+
+    # ---- decision tree ------------------------------------------------------------------------------
+    def set_tree(self, tree):
+        """Classify with a decision tree on every VAD path of this handle: a fitted sklearn DecisionTreeClassifier, a
+        path to a pickle of one or to an .npz of its arrays (``tree_arrays``).  The decision matches sklearn's
+        predict (argmax) or predict_proba[:, 1] >= threshold exactly on the features the device computes; logits
+        outputs receive float32 predict_proba by class id.  FFN weights stay set underneath (``clear_tree``)."""
+        a = tree_arrays(tree)
+        n = int(a["children_left"].shape[0])
+        for k in ("children_right", "feature", "threshold"):
+            if a[k].shape != (n,):
+                raise ValueError("%s must have %d entries" % (k, n))
+        p = {k: v.ctypes.data_as(C.c_void_p) for k, v in a.items()}
+        check(self.lib.vadb200_set_tree(self._h, n, p["children_left"], p["children_right"], p["feature"],
+                                        p["threshold"], p["value"], p["classes"], int(a["classes"].size)))
+        self.has_tree = n > 0
+        self.classifier_version += 1
+
+    def clear_tree(self):
+        """Back to the FFN (if its weights are set)."""
+        check(self.lib.vadb200_clear_tree(self._h))
+        self.has_tree = False
+        self.classifier_version += 1
+
+    @property
+    def has_classifier(self):
+        return self.has_ffn or self.has_tree
+
+    @property
+    def tree_node_count(self):
+        return int(self.lib.vadb200_tree_node_count(self._h))
+
+    @property
+    def tree_depth(self):
+        return int(self.lib.vadb200_tree_depth(self._h))
+
+    def tree_predict(self, x):
+        """Feature rows [n, 39] -> (labels uint8 [n], probabilities float32 [n, 3] by class id), CUDA tensors."""
+        t = torch.as_tensor(x).to(device=self.device, dtype=torch.float32).contiguous().reshape(-1, 39)
+        n = t.shape[0]
+        labels = torch.empty((n,), dtype=torch.uint8, device=self.device)
+        proba = torch.empty((n, 3), dtype=torch.float32, device=self.device)
+        check(self.lib.vadb200_tree_predict(self._h, _ptr(t), n, _ptr(labels), _ptr(proba), self.stream))
+        return labels, proba
 
     def set_ffn_impl(self, impl):
         """0 / "fp32": CUDA-core FFMA; 1 / "tc": tcgen05 kind::tf32 on hi/lo operands; 2 / "tc16" (default):
@@ -154,6 +256,7 @@ class Handle(object):
     def set_decision_threshold(self, p=None):
         """speech <=> softmax(logits)[1] >= p; None (or p <= 0) restores argmax == VOICED."""
         check(self.lib.vadb200_set_decision_threshold(self._h, 0.0 if p is None else float(p)))
+        self.classifier_version += 1
 
     def decision_threshold(self):
         """The threshold on p(voiced), or None for the argmax rule."""
