@@ -8,8 +8,8 @@ given to ffn_predict, so MFCC and feature error play no part and the bound can b
   under FEAT_ANALYSER and FEAT_DATASET, on utterances whose last block phase holds 1 to 256 centres, catalogue
   signals and digital silence, with segment ends mid-phase;
 * ffn_tc_rows_kernel<2> (ffn_tc16_tile<1>, and its per-tile fall-back to the tf32 blob), ffn_tc_rows_kernel<1>,
-  ffn_rows_kernel;
-* windows_kernel (classify_row);
+  rows_kernel<FfnParams>;
+* windows_kernel<FfnParams> (classify_row);
 * stream_feed_kernel's classifier, through its logits equalling the fused fp32 path's bit for bit.
 
 Rows whose features are not finite must come out NaN with label 0."""

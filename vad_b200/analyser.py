@@ -12,18 +12,27 @@ from . import _lib, runtime
 from .runtime import FEAT_ANALYSER
 
 
-def _handle_for(weights, handle):
-    """One analyser == one classifier (sklearn_analyser.py:21-35): weights given without an explicit
-    handle get a PRIVATE handle, so constructing a second object can never replace the classifier of
-    an earlier one.  The process-wide default handle serves only the weight-free mfcc.* functions and
-    objects that ask for it explicitly."""
-    if weights is None:
+def _handle_for(tree, ffn_weights, handle):
+    """The handle an object runs on.  One analyser == one classifier (sklearn_analyser.py:21-35): a decision tree
+    (a TreeClassifier, fitted sklearn tree, pickle or .npz path) or FFN weights given without an explicit handle get a
+    PRIVATE handle, so constructing a second object can never replace the classifier of an earlier one; an explicit
+    handle receives them (the caller owns it and asked for this).  A TreeClassifier runs on its own handle unless
+    another one is given.  With neither, the process-wide default handle, which serves only the weight-free mfcc.*
+    functions and objects that ask for it explicitly."""
+    if isinstance(tree, TreeClassifier):
+        if handle is None or handle is tree.handle:
+            return tree.handle
+        tree = tree._arrays
+    if tree is None and ffn_weights is None:
         return handle or runtime.default_handle()
-    w = runtime.load_ffn_npz(weights) if isinstance(weights, str) else weights
-    if handle is None:
-        return runtime.Handle(ffn_weights=w)
-    handle.set_ffn_weights(w)      # explicit handle: the caller owns it and asked for this
-    return handle
+    if tree is None and isinstance(ffn_weights, str):
+        ffn_weights = runtime.load_ffn_npz(ffn_weights)
+    h = handle if handle is not None else runtime.Handle()
+    if tree is not None:
+        h.set_tree(tree)
+    else:
+        h.set_ffn_weights(ffn_weights)
+    return h
 
 
 class Analyser:
@@ -46,7 +55,7 @@ class FFNClassifier(object):
     (1 = VOICED, config.py:46; the FFN's music class 2 maps to 0), evaluated on the GPU."""
 
     def __init__(self, weights=None, handle=None):
-        self.handle = _handle_for(weights, handle)
+        self.handle = _handle_for(None, weights, handle)
         if not self.handle.has_ffn:
             raise RuntimeError("FFNClassifier needs FFN weights")
 
@@ -86,17 +95,6 @@ class TreeClassifier(object):
         return self.handle.tree_predict(np.asarray(x, dtype=np.float32))[1].cpu().numpy()
 
 
-def _tree_handle(classifier, handle):
-    """The handle a StreamBank runs ``classifier`` (a TreeClassifier, sklearn tree or path) on."""
-    if isinstance(classifier, TreeClassifier):
-        if handle is None or handle is classifier.handle:
-            return classifier.handle
-        classifier = classifier._arrays
-    h = handle if handle is not None else runtime.Handle()
-    h.set_tree(classifier)
-    return h
-
-
 class FusedAnalyser(Analyser):
     """SKLearnAnalyzer (sklearn_analyser.py:15-130) on the GPU.
 
@@ -123,16 +121,13 @@ class FusedAnalyser(Analyser):
         self.sample_rate, self.fft_n, self.mfcc_num = sample_rate, int(fft_n), mfcc_num
         self.low_hz, self.high_hz, self.fbank_num = low_hz, high_hz, fbank_num
         self.tree = isinstance(classifier, TreeClassifier)
-        if self.tree:
-            handle = _tree_handle(classifier, handle)
-            classifier = None
         if isinstance(classifier, str):
             with open(classifier, "rb") as f:
                 classifier = pickle.load(f)
-        self.classifier = classifier
-        self.handle = handle if self.tree else _handle_for(ffn_weights if classifier is None else None, handle)
+        self.handle = _handle_for(classifier if self.tree else None, ffn_weights if classifier is None else None, handle)
+        self.classifier = None if self.tree else classifier
         self.filterbank = self.handle.filterbank()
-        if classifier is None and not self.tree:
+        if self.classifier is None and not self.tree:
             if not self.handle.has_ffn:
                 raise RuntimeError("FusedAnalyser needs FFN weights or an external classifier")
         self.frames_buffer = []
@@ -228,10 +223,8 @@ class StreamBank(object):
                 raise ValueError("unsupported sample rate %r" % (sample_rate,))
         if max_feed_samples is not None and not 1 <= int(max_feed_samples) <= rate:
             raise ValueError("max_feed_samples must lie in [1, %d]" % rate)
-        if classifier is not None:   # a decision tree: TreeClassifier, fitted sklearn tree, pickle or .npz path
-            self.handle = _tree_handle(classifier, handle)
-        else:
-            self.handle = _handle_for(ffn_weights, handle)
+        # classifier: a decision tree (TreeClassifier, fitted sklearn tree, pickle or .npz path), else the FFN
+        self.handle = _handle_for(classifier, ffn_weights if classifier is None else None, handle)
         if not self.handle.has_classifier:
             raise RuntimeError("StreamBank needs FFN weights or a decision tree")
         self.n = int(n_streams)

@@ -1,6 +1,6 @@
 // vad_kernels.cuh -- sm_100a kernels of the fused MFCC + FFN VAD path.
 //
-// fused_kernel<MODE, TC>: persistent CTAs (2 per SM, 256 threads) pull *segments* (runs of
+// fused_kernel<MODE, CLS>: persistent CTAs (2 per SM, 256 threads) pull *segments* (runs of
 // consecutive frames of one utterance) from an atomic work counter.  Per 32-frame step:
 //   1. PCM for the step (5360 int16 = 31 hops + one frame) arrives in shared memory by one
 //      TMA bulk copy (cp.async.bulk + mbarrier), double-buffered one step ahead; overlapping
@@ -20,10 +20,10 @@
 // The step has no CTA-wide bar.sync: two split-phase mbarriers ("P free", "P full", one arrival per
 // warp) order the power tile; only block steps use CTA barriers.
 // Block phase: MODE 0 / 1 flush MFCC / dataset rows (every 8 steps); MODE 2 builds the 5-frame window
-// features and runs Dense 39-64-32-16-3 -- on FP32 CUDA cores (TC = 0, every 8 steps), as one tcgen05
-// tile of 128 frames with TMEM accumulators (TC = 1, tf32 hi/lo operands, every 4 steps) or as two such
-// tiles of 128 frames side by side in TMEM (TC = 2, fp16 hi/lo operands, every 8 steps) -- then
-// argmax == VOICED, 1-byte label; or walks a decision tree instead (TC = 3, one thread per centre, every 8 steps).
+// features and runs Dense 39-64-32-16-3 -- on FP32 CUDA cores (CLS = kClsFp32, every 8 steps), as one tcgen05
+// tile of 128 frames with TMEM accumulators (kClsTf32, tf32 hi/lo operands, every 4 steps) or as two such
+// tiles of 128 frames side by side in TMEM (kClsFp16, fp16 hi/lo operands, every 8 steps) -- then
+// argmax == VOICED, 1-byte label; or walks a decision tree instead (kClsTree, one thread per centre, every 8 steps).
 //
 // Reference lines restated: mfcc.py:59-78; dataset/file_processing.py:47-70,99-101;
 // realtime_analysis/sklearn_analyser.py:46-82,103-107; learning/ffn_trainer.py:104-116.
@@ -103,7 +103,7 @@ struct FusedParams {
   float* rows;
   long long row_base;     // subtracted from Segment::out_start (chunked host runs)
   int feat_mode;
-  const unsigned char* tc_blob;  // canonical hi/lo tf32 weight blob (ffn_tc.cuh), TC variant only
+  const unsigned char* tc_blob;  // canonical hi/lo tf32 weight blob (ffn_tc.cuh), tensor-core variants only
   long long* dbg_ts;             // timing experiments only: clock64 stamps of CTA 0's block phases [n][16]
   int debug_skip;                // timing experiments only (env VADB200_DEBUG_SKIP): 1 FFT, 2 mel, 4 DCT, 8 block phase,
                                  // 256 no second fp16 tile (tools/ablate.sh lists the rest)
@@ -294,36 +294,39 @@ __device__ __forceinline__ void store_feats_half(float* feats, long long row, in
       if (k < nk) feats[row * kNFeat + g * kNCep + k0 + k] = xl[6 * (k >> 1) + 2 * g + (k & 1)];
 }
 
-// One output row per thread: window features -> tree -> decision (block phase / windows API).  The features pass
-// through this thread's column of a shared-memory tile x[f * stride] (a walk indexes them by node).
-__device__ __forceinline__ void tree_classify_row(const TreeArg& tr, const float (&r)[5][kNCep], int feat_mode,
-                                                  float* xs, int stride, uint8_t* labels, float* logits, float* feats,
-                                                  long long row, float th) {
-  float x[kNFeat];
-  const bool ok = window_features(r, feat_mode, x);
+// The classifier kinds a kernel can run (its CLS template parameter): the FFN on FP32 CUDA cores, on tcgen05
+// kind::tf32 (hi/lo split, TMEM accumulators), on tcgen05 kind::f16 with statically scaled fp16 hi/lo operands (half
+// the MMAs, half the weight blob), or a decision tree (vad_tree.cuh).  The values are part of kernel names
+// (fused_kernel<2, 2> is VAD mode on the fp16 FFN).
+constexpr int kClsFp32 = 0, kClsTf32 = 1, kClsFp16 = 2, kClsTree = 3;
+
+// The decision step of classify_row for the features x of one row: logits or leaf probabilities in out.  The tree
+// walks them from this thread's column of a shared-memory tile xs[f * stride] (a walk indexes them by node); the FFN
+// needs no tile.  th: decision threshold (decide); 0 = argmax.
+__device__ __forceinline__ uint8_t decide_row(const FfnParams& w, const float (&x)[kNFeat], float*, int, float th,
+                                              float (&out)[kNCls]) {
+  ffn_forward(w, x, out);
+  return decide(out, th);
+}
+__device__ __forceinline__ uint8_t decide_row(const TreeArg& tr, const float (&x)[kNFeat], float* xs, int stride,
+                                              float th, float (&out)[kNCls]) {
 #pragma unroll
   for (int i = 0; i < kNFeat; ++i) xs[i * stride] = x[i];
-  float p[kNCls];
-  const uint8_t lab = reject_nonfinite(ok, tree_decide(tree_walk(tr, [&](uint32_t f) { return xs[f * stride]; }), th, p), p);
-  if (labels) labels[row] = lab;
-  store_logits(logits, row, p);
-  if (feats) {
-#pragma unroll
-    for (int i = 0; i < kNFeat; ++i) feats[row * kNFeat + i] = x[i];
-  }
+  return tree_decide(tree_walk(tr, [&](uint32_t f) { return xs[f * stride]; }), th, out);
 }
 
-// One output row per thread: window features -> FFN -> decision (block phase / windows API).
-// th: decision threshold (decide); 0 = argmax.
-__device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r)[5][kNCep], int feat_mode,
-                                             uint8_t* labels, float* logits, float* feats, long long row, float th) {
+// One output row per thread: window features -> classifier W (FfnParams or TreeArg) -> decision (block phase /
+// windows API).  xs, stride: the tree's feature column (decide_row).
+template <class W>
+__device__ __forceinline__ void classify_row(const W& w, const float (&r)[5][kNCep], int feat_mode, float* xs,
+                                             int stride, uint8_t* labels, float* logits, float* feats, long long row,
+                                             float th) {
   float x[kNFeat];
   const bool ok = window_features(r, feat_mode, x);
-  float logit[kNCls];
-  ffn_forward(w, x, logit);
-  const uint8_t lab = reject_nonfinite(ok, decide(logit, th), logit);
+  float out[kNCls];
+  const uint8_t lab = reject_nonfinite(ok, decide_row(w, x, xs, stride, th, out), out);
   if (labels) labels[row] = lab;
-  store_logits(logits, row, logit);
+  store_logits(logits, row, out);
   if (feats) {
 #pragma unroll
     for (int i = 0; i < kNFeat; ++i) feats[row * kNFeat + i] = x[i];
@@ -331,16 +334,14 @@ __device__ __forceinline__ void classify_row(const FfnParams& w, const float (&r
 }
 
 // MODE 0: MFCC rows [T][13]; 1: dataset rows [T-5][39]; 2: VAD labels [T-5].
-// TC (MODE 2 only): 0 = FFN on FP32 CUDA cores, 1 = FFN on tcgen05 kind::tf32 (hi/lo split, TMEM accumulators),
-// 2 = tcgen05 kind::f16 on statically scaled fp16 hi/lo operands (half the MMAs, half the weight blob), 3 = decision tree
-// (vad_tree.cuh) on the TC = 0 block phase.
-// FFN argument of the kernel variant: nothing (MFCC / dataset rows), the full FP32 weights, or the biases
-// only (tensor-core FFN: the weights are the per-handle tcgen05 operand blob in global memory).
-template <int MODE, int TC> struct FfnArgOf { using type = FfnNone; };
-template <> struct FfnArgOf<2, 0> { using type = FfnParams; };
-template <> struct FfnArgOf<2, 1> { using type = FfnBias; };
-template <> struct FfnArgOf<2, 2> { using type = FfnBias; };
-template <> struct FfnArgOf<2, 3> { using type = TreeArg; };
+// CLS (MODE 2 only): the classifier kind; the tree runs on the kClsFp32 block phase.
+// Classifier argument of the kernel variant: nothing (MFCC / dataset rows), the full FP32 weights, the biases only
+// (tensor-core FFN: the weights are the per-handle tcgen05 operand blob in global memory), or the tree.
+template <int MODE, int CLS> struct ClsArgOf { using type = FfnNone; };
+template <> struct ClsArgOf<2, kClsFp32> { using type = FfnParams; };
+template <> struct ClsArgOf<2, kClsTf32> { using type = FfnBias; };
+template <> struct ClsArgOf<2, kClsFp16> { using type = FfnBias; };
+template <> struct ClsArgOf<2, kClsTree> { using type = TreeArg; };
 
 // The decision of the VAD block phase: argmax, or with the front-end variant the handle's threshold.
 template <bool FE, class A>
@@ -357,12 +358,12 @@ static_assert(kStageSamples + kStageOffFe <= kStagePad, "front-end stage offset 
 
 // tid comes from the kernel: threadIdx.x read inside the kernel carries the launch bound's range (0 .. 255), which the
 // code generation relies on (read here, the default kernels' SASS would change).
-template <int MODE, int TC, bool FE>
-__device__ __forceinline__ void fused_body(const FusedParams& p, const typename FfnArgOf<MODE, TC>::type& ffn,
+template <int MODE, int CLS, bool FE>
+__device__ __forceinline__ void fused_body(const FusedParams& p, const typename ClsArgOf<MODE, CLS>::type& ffn,
                                            const FrontEnd& fe, const int tid) {
-  static_assert(TC == 0 || MODE == 2, "tensor-core FFN only exists in VAD mode");
-  constexpr bool kTmem = TC == 1 || TC == 2;  // the tensor-core FFN variants
-  constexpr int kBlk = TC == 1 ? kBlockStepsTc : kBlockSteps;
+  static_assert(CLS == kClsFp32 || MODE == 2, "a classifier only exists in VAD mode");
+  constexpr bool kTmem = CLS == kClsTf32 || CLS == kClsFp16;  // the tensor-core FFN variants
+  constexpr int kBlk = CLS == kClsTf32 ? kBlockStepsTc : kBlockSteps;
   constexpr int kStageOff = FE ? kStageOffFe : 0;
   extern __shared__ __align__(128) unsigned char smem[];
   int16_t* s_pcm = reinterpret_cast<int16_t*>(smem + kOffPcm);
@@ -515,7 +516,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
         if (tc_now) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // exch/P generic accesses before the TMA overwrite
         __syncthreads();
         if (tc_now && tid == 0 && !(VADB_DBG(p) & 16)) {  // exch + P are idle until the next FFT phase: land the weight blob during the DCT
-          constexpr uint32_t blob_bytes = TC == 2 ? kTc16BlobBytes : kTcBlobBytes;
+          constexpr uint32_t blob_bytes = CLS == kClsFp16 ? kTc16BlobBytes : kTcBlobBytes;
           mbar_arrive_expect_tx(&s_bar[2], blob_bytes);
           bulk_g2s(smem + kOffExch, p.tc_blob, blob_bytes, &s_bar[2]);
         }
@@ -574,7 +575,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
             __syncthreads();  // the next FFT phase rewrites exch / P
           }
           out_done = max(out_done, computed - 2);
-        } else if (TC == 0 || TC == 3) {
+        } else if constexpr (CLS == kClsFp32 || CLS == kClsTree) {
           const int c = out_done + tid;
           if (c <= computed - 3) {
             float r[5][kNCep];
@@ -584,17 +585,13 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
 #pragma unroll
               for (int k = 0; k < kNCep; ++k) r[d][k] = s_ring[ring_idx(k, col, kRing)];
             }
-            if constexpr (MODE == 2 && TC == 0)
-              classify_row(ffn, r, p.feat_mode, p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2),
-                           FE ? ffn.thresh : 0.0f);
-            else if constexpr (TC == 3)  // features staged in exch + P, idle until the next FFT phase
-              tree_classify_row(ffn, r, p.feat_mode, reinterpret_cast<float*>(smem + kOffExch) + tid, kThreads,
-                                p.labels, p.logits, p.feats, seg.out_start - p.row_base + (c - 2),
-                                FE ? ffn.thresh : 0.0f);
+            if constexpr (MODE == 2)  // a tree stages the features in exch + P, idle until the next FFT phase
+              classify_row(ffn, r, p.feat_mode, reinterpret_cast<float*>(smem + kOffExch) + tid, kThreads, p.labels,
+                           p.logits, p.feats, seg.out_start - p.row_base + (c - 2), FE ? ffn.thresh : 0.0f);
           }
-          if constexpr (TC == 3) __syncthreads();  // the next FFT phase rewrites the staged features
+          if constexpr (CLS == kClsTree) __syncthreads();  // the next FFT phase rewrites the staged features
           out_done = max(out_done, computed - 2);
-        } else if constexpr (TC == 2) {
+        } else if constexpr (CLS == kClsFp16) {
           // ---- fp16 tensor-core FFN: two M = 128 tiles, thread = frame = TMEM lane of tile warp / 4 ---------------
           const int n_valid = computed - 2 - out_done;  // centres out_done .. computed-3 (<= 256)
           if (n_valid > 0) {                            // block-uniform (== tc_now)
@@ -675,7 +672,7 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
               if (p.feats && valid) store_feats_half(p.feats, seg.out_start - p.row_base + (c - 2), hidx, xl);
               if (!(VADB_DBG(p) & 16)) mbar_wait(&s_bar[2], w_par);  // weight blob landed (issued before the DCT phase)
               if (ts) ts[2] = clock64();
-              if constexpr (TC == 1)
+              if constexpr (CLS == kClsTf32)
                 mma_par = ffn_tc_tile<2>(ffn, logit, tm_base, warp & 3, hidx, tid == 0, smem_u32(wdst), &s_bar[3], mma_par,
                                          ts, VADB_DBG(p));
               ++dbg_n;
@@ -713,18 +710,18 @@ __device__ __forceinline__ void fused_body(const FusedParams& p, const typename 
   }
 }
 
-template <int MODE, int TC>
+template <int MODE, int CLS>
 __global__ void __launch_bounds__(kThreads, 2) fused_kernel(const __grid_constant__ FusedParams p,
-                                                            const __grid_constant__ typename FfnArgOf<MODE, TC>::type ffn) {
-  fused_body<MODE, TC, false>(p, ffn, FrontEnd{nullptr, 0.0f}, threadIdx.x);
+                                                            const __grid_constant__ typename ClsArgOf<MODE, CLS>::type ffn) {
+  fused_body<MODE, CLS, false>(p, ffn, FrontEnd{nullptr, 0.0f}, threadIdx.x);
 }
 // The same kernel with the opt-in front end and decision threshold; launched only when the handle sets either, so the
 // default path above keeps its code.
-template <int MODE, int TC>
+template <int MODE, int CLS>
 __global__ void __launch_bounds__(kThreads, 2) fused_fe_kernel(const __grid_constant__ FusedParams p,
-                                                               const __grid_constant__ typename FfnArgOf<MODE, TC>::type ffn,
+                                                               const __grid_constant__ typename ClsArgOf<MODE, CLS>::type ffn,
                                                                const __grid_constant__ FrontEnd fe) {
-  fused_body<MODE, TC, true>(p, ffn, fe, threadIdx.x);
+  fused_body<MODE, CLS, true>(p, ffn, fe, threadIdx.x);
 }
 
 // Stand-alone tensor-core FFN over feature rows [n][39] (classifier.predict duck type): one CTA =
@@ -949,9 +946,17 @@ __global__ void __launch_bounds__(kThreads) spec_to_mfcc_kernel(const float* spe
   }
 }
 
-// 5-frame MFCC windows [n][5][13] -> features / logits / labels (one thread per window).
+// 5-frame MFCC windows [n][5][13] -> features / logits (a tree: probabilities) / labels (one thread per window).
+// W: FfnParams, or TreeArg with a [39][128] shared feature tile.
+static_assert(kNFeat * 128 * 4 <= 48 * 1024, "windows_kernel's tree feature tile");
+template <class W>
 __global__ void __launch_bounds__(128) windows_kernel(const float* win, long long n, int feat_mode, uint8_t* labels,
-                                                      float* logits, float* feats, const __grid_constant__ FfnParams w) {
+                                                      float* logits, float* feats, const __grid_constant__ W w) {
+  float* xs = nullptr;
+  if constexpr (std::is_same<W, TreeArg>::value) {
+    __shared__ float s_x[kNFeat * 128];
+    xs = s_x + threadIdx.x;
+  }
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float r[5][kNCep];
@@ -959,57 +964,40 @@ __global__ void __launch_bounds__(128) windows_kernel(const float* win, long lon
   for (int d = 0; d < 5; ++d)
 #pragma unroll
     for (int k = 0; k < kNCep; ++k) r[d][k] = win[(i * 5 + d) * kNCep + k];
-  classify_row(w, r, feat_mode, labels, logits, feats, i, w.thresh);
+  classify_row(w, r, feat_mode, xs, 128, labels, logits, feats, i, w.thresh);
 }
 
-// The same with a decision tree: labels, probabilities (in logits' place) and features.
-static_assert(kNFeat * 128 * 4 <= 48 * 1024, "windows_tree_kernel's feature tile");
-__global__ void __launch_bounds__(128) windows_tree_kernel(const float* win, long long n, int feat_mode, uint8_t* labels,
-                                                           float* proba, float* feats, const __grid_constant__ TreeArg tr) {
-  __shared__ float s_x[kNFeat * 128];
-  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  float r[5][kNCep];
-#pragma unroll
-  for (int d = 0; d < 5; ++d)
-#pragma unroll
-    for (int k = 0; k < kNCep; ++k) r[d][k] = win[(i * 5 + d) * kNCep + k];
-  tree_classify_row(tr, r, feat_mode, s_x + threadIdx.x, 128, labels, proba, feats, i, tr.thresh);
-}
-
-// Decision tree over feature rows [n][39] (vadb200_tree_predict): one thread per row; the walk reads the row from
-// global memory (L1 after the finiteness check).
-__global__ void __launch_bounds__(128) tree_rows_kernel(const float* x, long long n, uint8_t* labels, float* proba,
-                                                        const __grid_constant__ TreeArg tr) {
-  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const float* row = x + i * kNFeat;
-  bool ok = true;
-#pragma unroll
-  for (int k = 0; k < kNFeat; ++k) ok = ok && (fabsf(row[k]) <= 3.0e38f);
-  float p[kNCls];
-  const uint8_t lab = reject_nonfinite(ok, tree_decide(tree_walk(tr, [&](uint32_t f) { return row[f]; }), tr.thresh, p), p);
-  if (labels) labels[i] = lab;
-  store_logits(proba, i, p);
-}
-
-// classifier.predict duck type (sklearn_analyser.py:71): rows [n][39] -> class {0,1}, logits.
-__global__ void __launch_bounds__(128) ffn_rows_kernel(const float* x, long long n, uint8_t* labels, float* logits,
-                                                       const __grid_constant__ FfnParams w) {
-  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+// The decision step of rows_kernel for a row in global memory; ok: whether every feature is finite.  The FFN reads the
+// row into registers as it checks it, the tree checks it and walks it where it is (L1 after the check).
+__device__ __forceinline__ uint8_t decide_row(const FfnParams& w, const float* row, bool& ok, float (&out)[kNCls]) {
   float v[kNFeat];
-  bool ok = true;
 #pragma unroll
   for (int k = 0; k < kNFeat; ++k) {
-    v[k] = x[i * kNFeat + k];
+    v[k] = row[k];
     ok = ok && (fabsf(v[k]) <= 3.0e38f);
   }
-  float logit[kNCls];
-  ffn_forward(w, v, logit);
-  const uint8_t lab = reject_nonfinite(ok, decide(logit, w.thresh), logit);
+  ffn_forward(w, v, out);
+  return decide(out, w.thresh);
+}
+__device__ __forceinline__ uint8_t decide_row(const TreeArg& tr, const float* row, bool& ok, float (&out)[kNCls]) {
+#pragma unroll
+  for (int k = 0; k < kNFeat; ++k) ok = ok && (fabsf(row[k]) <= 3.0e38f);
+  return tree_decide(tree_walk(tr, [&](uint32_t f) { return row[f]; }), tr.thresh, out);
+}
+
+// classifier.predict duck type (sklearn_analyser.py:71) and vadb200_tree_predict: rows [n][39] -> class, logits (a
+// tree: probabilities); one thread per row.
+template <class W>
+__global__ void __launch_bounds__(128) rows_kernel(const float* x, long long n, uint8_t* labels, float* logits,
+                                                   const __grid_constant__ W w) {
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  bool ok = true;
+  float out[kNCls];
+  const uint8_t d = decide_row(w, x + i * kNFeat, ok, out);
+  const uint8_t lab = reject_nonfinite(ok, d, out);
   if (labels) labels[i] = lab;
-  store_logits(logits, i, logit);
+  store_logits(logits, i, out);
 }
 
 // mfcc.get_deltas (mfcc.py:81-82: a - b) and mfcc.lifter (mfcc.py:85-93) for standalone callers.
@@ -1222,14 +1210,18 @@ __device__ __forceinline__ uint8_t stream_decide(const StreamSmem& sm, const Tre
   return lab;
 }
 
+// The segment state a bank kernel hands its body: its StreamSeg, or 0 when it takes none (the plain FFN kernels).
+__device__ __forceinline__ int seg_arg() { return 0; }
+template <class Seg>
+__device__ __forceinline__ const Seg& seg_arg(const Seg& sg) { return sg; }
+
 // One CTA = 32 streams.  FFT: the fused kernel's packed two-frames-per-thread pass.  The decision
 // tail is spread over all 8 warps with lane = stream: warp w owns cepstral coefficients w, w + 8
 // (DCT, ring push, window features) and then 8 / 4 / 2 neurons of layers 1 / 2 / 3, activations
 // handed over through shared memory (the idle P tile); weights are uniform constant-bank operands.
-// SEG: the speech variant (stream_feed_speech_kernel) also runs each stream's online smoothing step
-// (vad_segments.cuh seg_step, found when the variant is instantiated with Seg = StreamSeg) on the label warp 0
-// holds, and writes the finalised row and its bound.
-// W: FfnParams, or TreeArg (stream_feed_tree_kernel: no hidden layers, warp 0 walks the tree).
+// SEG: the speech variant also runs each stream's online smoothing step (vad_segments.cuh seg_step, found when the
+// variant is instantiated with Seg = StreamSeg) on the label warp 0 holds, and writes the finalised row and its bound.
+// W: FfnParams, or TreeArg (no hidden layers, warp 0 walks the tree).
 template <bool SEG, class Seg, class W>
 __device__ __forceinline__ void stream_feed_body(const BankParams& p, const W& w, const Seg& sg, const int tid) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -1305,22 +1297,12 @@ __device__ __forceinline__ void stream_feed_body(const BankParams& p, const W& w
   }
 }
 
-__global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams p, const __grid_constant__ FfnParams w) {
-  stream_feed_body<false>(p, w, 0, threadIdx.x);
-}
-// The same tick plus the bank's segment step (vadb200_stream_bank_set_speech); the plain kernel above keeps its code.
-template <class Seg>
-__global__ void __launch_bounds__(kThreads) stream_feed_speech_kernel(const BankParams p,
-                                                                     const __grid_constant__ FfnParams w,
-                                                                     const __grid_constant__ Seg sg) {
-  stream_feed_body<true>(p, w, sg, threadIdx.x);
-}
-
-// The fixed tick with a decision tree (SEG: plus the segment step).
-template <bool SEG, class Seg>
-__global__ void __launch_bounds__(kThreads) stream_feed_tree_kernel(const BankParams p, const __grid_constant__ TreeArg tr,
-                                                                   const __grid_constant__ Seg sg) {
-  stream_feed_body<SEG>(p, tr, sg, threadIdx.x);
+// The fixed tick of classifier W, with the bank's segment step (vadb200_stream_bank_set_speech) when SEG; sg: the
+// segment state (StreamSeg), or nothing (the plain FFN tick) or an unused StreamSeg (the plain tree tick) without it.
+template <bool SEG, class W, class... Seg>
+__global__ void __launch_bounds__(kThreads) stream_feed_kernel(const BankParams p, const __grid_constant__ W w,
+                                                              const __grid_constant__ Seg... sg) {
+  stream_feed_body<SEG>(p, w, seg_arg(sg...), threadIdx.x);
 }
 
 // ---- ragged bank (vadb200_stream_bank_create_ragged): any number of samples per stream and feed ----------------
@@ -1485,24 +1467,13 @@ __device__ __forceinline__ void stream_ragged_body(const RaggedParams& p, const 
   }
 }
 
+// The ragged feed of classifier W, with the segment step when SEG (sg as stream_feed_kernel; the rows / bounds
+// pointers of a StreamSeg are not used).
+template <bool SEG, class W, class... Seg>
 __global__ void __launch_bounds__(kThreads) stream_ragged_kernel(const __grid_constant__ RaggedParams p,
-                                                                const __grid_constant__ FfnParams w) {
-  stream_ragged_body<false>(p, w, 0, threadIdx.x);
-}
-// The same feed plus the bank's segment step (Seg = StreamSeg; its rows / bounds pointers are not used).
-template <class Seg>
-__global__ void __launch_bounds__(kThreads) stream_ragged_speech_kernel(const __grid_constant__ RaggedParams p,
-                                                                       const __grid_constant__ FfnParams w,
-                                                                       const __grid_constant__ Seg sg) {
-  stream_ragged_body<true>(p, w, sg, threadIdx.x);
-}
-
-// The ragged feed with a decision tree (SEG: plus the segment step).
-template <bool SEG, class Seg>
-__global__ void __launch_bounds__(kThreads) stream_ragged_tree_kernel(const __grid_constant__ RaggedParams p,
-                                                                     const __grid_constant__ TreeArg tr,
-                                                                     const __grid_constant__ Seg sg) {
-  stream_ragged_body<SEG>(p, tr, sg, threadIdx.x);
+                                                                const __grid_constant__ W w,
+                                                                const __grid_constant__ Seg... sg) {
+  stream_ragged_body<SEG>(p, w, seg_arg(sg...), threadIdx.x);
 }
 
 // ---- feature sink: scale_features (dataset/utils.py:5-32) on packed dataset rows [n][39] ----------------

@@ -253,33 +253,98 @@ struct vadb200_resampler {
 namespace {
 
 bool has_tree(const vadb200_handle* h) { return h->tree_nodes > 0; }
-bool has_classifier(const vadb200_handle* h) { return h->have_ffn || has_tree(h); }
-TreeArg tree_arg(const vadb200_handle* h) {
-  const TreeNode* nodes = reinterpret_cast<const TreeNode*>(h->d_tree.get());
-  return TreeArg{nodes, reinterpret_cast<const TreeLeaf*>(nodes + h->tree_nodes), h->tree_depth, h->par.thresh};
-}
+bool has_classifier(const vadb200_handle* h) { return vadb200_get_classifier(h) != VADB200_CLASSIFIER_NONE; }
 constexpr const char* kNoClassifier = "FFN weights not set (vadb200_set_ffn_weights)";
 
 bool frontend_on(const vadb200_handle* h) { return h->preemph != 0.0f || h->has_window; }
 FrontEnd frontend_of(const vadb200_handle* h) { return FrontEnd{h->d_win.get(), h->preemph}; }
 
-// The classifier a handle runs: 2 (tcgen05 fp16 hi/lo) when asked for and the weights fit its static scales, else
-// 1 (tcgen05 tf32 hi/lo) when any tensor-core variant is asked for, else 0 (FP32 CUDA cores); and its weight blob.
-struct Classifier {
-  int tc;
-  const unsigned char* blob;
+// Sets of classifier kinds (vad_kernels.cuh kCls*): bit k stands for kind k.
+constexpr unsigned cls_bit(int kind) { return 1u << kind; }
+constexpr unsigned kKindsAll = cls_bit(kClsFp32) | cls_bit(kClsTf32) | cls_bit(kClsFp16) | cls_bit(kClsTree);
+constexpr unsigned kKindsFfn = cls_bit(kClsFp32) | cls_bit(kClsTf32) | cls_bit(kClsFp16);
+constexpr unsigned kKindsTreeFp32 = cls_bit(kClsTree) | cls_bit(kClsFp32);
+
+// The tensor-core FFN's operands: the fp16 blob (kClsFp16 only), the tf32 blob (kClsTf32's weights, and ffn_predict's
+// fallback for a kClsFp16 tile with a row past the fp16 scales) and the biases.
+struct TcFfn {
+  const unsigned char* blob16;
+  const unsigned char* blob32;
+  FfnBias bias;
 };
-Classifier classifier_of(const vadb200_handle* h) {
-  if (h->ffn_impl == 2 && h->tc16_ok) return {2, h->d_tc16_blob.get()};
-  if (h->ffn_impl >= 1) return {1, h->d_tc_blob.get()};
-  return {0, nullptr};
+// A classifier as kernels take it: its kind and the argument of that kind.
+struct Classifier {
+  int kind;
+  const FfnParams* ffn;  // kClsFp32: the handle's weights (launches copy them into the kernel parameters)
+  TcFfn tc;              // kClsTf32, kClsFp16
+  TreeArg tree;          // kClsTree
+};
+
+// The classifier a launch runs, given the kinds its entry point can run:
+//   entry point                                 kinds           runs
+//   vad_packed, vad_host (launch_fused)         kKindsAll       the tree, else the fp16 tcgen05 FFN (ffn_impl 2 and
+//                                                               the weights fit its static scales), else the tf32
+//                                                               tcgen05 FFN (ffn_impl >= 1), else the FP32 FFN
+//   ffn_predict                                 kKindsFfn       the same without the tree (a tree is ignored)
+//   tree_predict                                kClsTree        the tree
+//   vad_windows, fixed and ragged banks         kKindsTreeFp32  the tree, else the FP32 FFN (ffn_impl ignored)
+// The entry point has checked that the handle holds a classifier it can run.
+Classifier classifier_of(const vadb200_handle* h, unsigned kinds) {
+  Classifier c{};
+  if ((kinds & cls_bit(kClsTree)) && has_tree(h)) {
+    const TreeNode* nodes = reinterpret_cast<const TreeNode*>(h->d_tree.get());
+    c.kind = kClsTree;
+    c.tree = TreeArg{nodes, reinterpret_cast<const TreeLeaf*>(nodes + h->tree_nodes), h->tree_depth, h->par.thresh};
+  } else if ((kinds & cls_bit(kClsFp16)) && h->ffn_impl == 2 && h->tc16_ok) {
+    c.kind = kClsFp16;
+    c.tc = TcFfn{h->d_tc16_blob.get(), h->d_tc_blob.get(), h->bias};
+  } else if ((kinds & cls_bit(kClsTf32)) && h->ffn_impl >= 1) {
+    c.kind = kClsTf32;
+    c.tc = TcFfn{nullptr, h->d_tc_blob.get(), h->bias};
+  } else {
+    c.kind = kClsFp32;
+    c.ffn = &h->par;
+  }
+  return c;
 }
 
-template <int MODE, int TC>
+// Calls f(kind, argument) for classifier c, with the kind as a std::integral_constant; f is instantiated for the kinds
+// in KINDS only, so each entry point's kernel families have exactly the variants it can launch.
+template <unsigned KINDS, class F>
+void with_classifier(const Classifier& c, F&& f) {
+  switch (c.kind) {
+    case kClsFp32: if constexpr ((KINDS & cls_bit(kClsFp32)) != 0) f(std::integral_constant<int, kClsFp32>{}, *c.ffn); break;
+    case kClsTf32: if constexpr ((KINDS & cls_bit(kClsTf32)) != 0) f(std::integral_constant<int, kClsTf32>{}, c.tc); break;
+    case kClsFp16: if constexpr ((KINDS & cls_bit(kClsFp16)) != 0) f(std::integral_constant<int, kClsFp16>{}, c.tc); break;
+    case kClsTree: if constexpr ((KINDS & cls_bit(kClsTree)) != 0) f(std::integral_constant<int, kClsTree>{}, c.tree); break;
+  }
+}
+
+// Calls f(SEG, sg...) with the segment arguments of a bank tick of kind K: with speech on the bank's StreamSeg;
+// without it none for the FFN and an unused StreamSeg for the tree (the kernels' parameter lists).
+template <int K, class F>
+void with_bank_seg(bool speech, const StreamSeg& sg, F&& f) {
+  if (speech) f(std::true_type{}, sg);
+  else if constexpr (K == kClsTree) f(std::false_type{}, StreamSeg{});
+  else f(std::false_type{});
+}
+
+// Lets the fixed and ragged bank kernels of one variant take kStreamSmemBytes of dynamic shared memory.  The casts
+// name the variants: the host compiler resolves a kernel with a parameter pack to no other pointer type.
+template <bool SEG, class W, class... Seg>
+cudaError_t bank_smem(const Seg&...) {
+  const cudaError_t e = cudaFuncSetAttribute((void (*)(const BankParams, const W, const Seg...))stream_feed_kernel<SEG, W, Seg...>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes);
+  if (e != cudaSuccess) return e;
+  return cudaFuncSetAttribute((void (*)(const RaggedParams, const W, const Seg...))stream_ragged_kernel<SEG, W, Seg...>,
+                              cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes);
+}
+
+template <int MODE, int CLS>
 void enqueue_fused(bool fe, int grid, cudaStream_t st, const FusedParams& fp,
-                   const typename FfnArgOf<MODE, TC>::type& ffn, const FrontEnd& fea) {
-  if (fe) fused_fe_kernel<MODE, TC><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn, fea);
-  else fused_kernel<MODE, TC><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn);
+                   const typename ClsArgOf<MODE, CLS>::type& ffn, const FrontEnd& fea) {
+  if (fe) fused_fe_kernel<MODE, CLS><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn, fea);
+  else fused_kernel<MODE, CLS><<<grid, kThreads, kFusedSmemBytes, st>>>(fp, ffn);
 }
 
 int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
@@ -297,15 +362,18 @@ int launch_fused(vadb200_plan* p, FusedParams fp, int n_segs, cudaStream_t st) {
   // the front-end variant runs only when the handle asks for a front end or (VAD) a decision threshold
   const bool fe = frontend_on(h) || (p->mode == VADB200_MODE_VAD && h->par.thresh > 0.0f);
   const FrontEnd fea = frontend_of(h);
-  const Classifier c = classifier_of(h);
-  if (p->mode == VADB200_MODE_VAD) fp.tc_blob = c.blob;
   return launched(1, [&] {
-    if (p->mode == VADB200_MODE_MFCC) enqueue_fused<0, 0>(fe, grid, st, fp, FfnNone{0}, fea);
-    else if (p->mode == VADB200_MODE_DATASET) enqueue_fused<1, 0>(fe, grid, st, fp, FfnNone{0}, fea);
-    else if (has_tree(h)) enqueue_fused<2, 3>(fe, grid, st, fp, tree_arg(h), fea);
-    else if (c.tc == 2) enqueue_fused<2, 2>(fe, grid, st, fp, h->bias, fea);
-    else if (c.tc == 1) enqueue_fused<2, 1>(fe, grid, st, fp, h->bias, fea);
-    else enqueue_fused<2, 0>(fe, grid, st, fp, h->par, fea);
+    if (p->mode == VADB200_MODE_MFCC) enqueue_fused<0, kClsFp32>(fe, grid, st, fp, FfnNone{0}, fea);
+    else if (p->mode == VADB200_MODE_DATASET) enqueue_fused<1, kClsFp32>(fe, grid, st, fp, FfnNone{0}, fea);
+    else with_classifier<kKindsAll>(classifier_of(h, kKindsAll), [&](auto kind, const auto& w) {
+      constexpr int K = decltype(kind)::value;
+      if constexpr (K == kClsTf32 || K == kClsFp16) {
+        fp.tc_blob = K == kClsFp16 ? w.blob16 : w.blob32;
+        enqueue_fused<2, K>(fe, grid, st, fp, w.bias, fea);
+      } else {
+        enqueue_fused<2, K>(fe, grid, st, fp, w, fea);
+      }
+    });
   });
 }
 
@@ -409,35 +477,36 @@ int vadb200_create(const vadb200_config* c, int device, vadb200_handle** out) {
   const std::vector<cf2> ones(kWinPairs, cf2{1.0f, 1.0f});
   CU(dev_upload(h->d_win, ones.data(), kWinPairs));
   // function attributes and the (config-invariant) constant tables now, so that no launch ever
-  // synchronises: every device-pointer entry point can be captured into a CUDA graph
-  CU(cudaFuncSetAttribute(fused_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_kernel<2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(fused_fe_kernel<2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFusedSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_tree_kernel<false, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_tree_kernel<true, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_ragged_tree_kernel<false, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_ragged_tree_kernel<true, StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
-  CU(cudaFuncSetAttribute(ffn_tc_rows_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFfnTcSmemBytes));
-  CU(cudaFuncSetAttribute(frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFramesSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_feed_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_ragged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kStreamSmemBytes));
-  CU(cudaFuncSetAttribute(stream_ragged_speech_kernel<StreamSeg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          kStreamSmemBytes));
+  // synchronises: every device-pointer entry point can be captured into a CUDA graph.  Every variant over 48 KB of
+  // dynamic shared memory: each classifying family's, for every kind the family's entry points can launch.
+  cudaError_t attr = cudaSuccess;
+  auto smem = [&](auto kernel, int bytes) {
+    if (attr == cudaSuccess) attr = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  };
+  smem(fused_kernel<0, kClsFp32>, kFusedSmemBytes);
+  smem(fused_fe_kernel<0, kClsFp32>, kFusedSmemBytes);
+  smem(fused_kernel<1, kClsFp32>, kFusedSmemBytes);
+  smem(fused_fe_kernel<1, kClsFp32>, kFusedSmemBytes);
+  smem(frames_kernel, kFramesSmemBytes);
+  for (const int kind : {kClsFp32, kClsTf32, kClsFp16, kClsTree}) {
+    Classifier c{};
+    c.kind = kind;
+    c.ffn = &h->par;
+    with_classifier<kKindsAll>(c, [&](auto k, const auto& w) {
+      constexpr int K = decltype(k)::value;
+      smem(fused_kernel<2, K>, kFusedSmemBytes);
+      smem(fused_fe_kernel<2, K>, kFusedSmemBytes);
+      if constexpr (K == kClsTf32 || K == kClsFp16) smem(ffn_tc_rows_kernel<K>, kFfnTcSmemBytes);
+      if constexpr ((kKindsTreeFp32 & cls_bit(K)) != 0) {
+        using W = std::decay_t<decltype(w)>;
+        for (const bool speech : {false, true})
+          with_bank_seg<K>(speech, StreamSeg{}, [&](auto seg, const auto&... sg) {
+            if (attr == cudaSuccess) attr = bank_smem<decltype(seg)::value, W>(sg...);
+          });
+      }
+    });
+  }
+  if (attr != cudaSuccess) return cuda_fail(attr, "cudaFuncSetAttribute");
   // Mel weights and the folded DCT matrix are the same for every handle (the kernels are compiled for the
   // reference configuration only), so the __constant__ copy is written once per device and never changes:
   // no handle can observe another handle's state through it.  FFN weights never go through device globals.
@@ -548,8 +617,8 @@ int vadb200_tree_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t
   if (!d_x) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   return launched(1, [&] {
-    tree_rows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-        d_x, n, d_labels, d_proba, tree_arg(h));
+    rows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+        d_x, n, d_labels, d_proba, classifier_of(h, cls_bit(kClsTree)).tree);
   });
 }
 
@@ -928,36 +997,32 @@ int vadb200_vad_windows(vadb200_handle* h, const float* d_win, int64_t n, int fe
   if (!d_win) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (has_tree(h))
-    return launched(1, [&] {
-      windows_tree_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels,
-                                                                                d_logits, d_feats, tree_arg(h));
-    });
   return launched(1, [&] {
-    windows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels, d_logits,
-                                                                         d_feats, h->par);
+    with_classifier<kKindsTreeFp32>(classifier_of(h, kKindsTreeFp32), [&](auto, const auto& w) {
+      windows_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(d_win, n, feat_mode, d_labels, d_logits,
+                                                                           d_feats, w);
+    });
   });
 }
 
 int vadb200_ffn_predict(vadb200_handle* h, const float* d_x, int64_t n, uint8_t* d_labels, float* d_logits, void* stream) {
   if (!h) return fail(VADB200_E_INVALID, "handle is null");
-  if (!h->have_ffn) return fail(VADB200_E_STATE, "FFN weights not set (vadb200_set_ffn_weights)");
+  if (!h->have_ffn) return fail(VADB200_E_STATE, kNoClassifier);
   if (n < 0) return fail(VADB200_E_INVALID, "n < 0");
   if (n == 0) return 0;
   if (!d_x) return fail(VADB200_E_INVALID, "null argument");
   CU(cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const unsigned grid = static_cast<unsigned>((n + 127) / 128);
-  const Classifier c = classifier_of(h);
   return launched(1, [&] {
-    // a fp16 tile holding a row past the feature bounds runs on the tf32 blob
-    if (c.tc == 2)
-      ffn_tc_rows_kernel<2><<<grid, 128, kFfnTcSmemBytes, st>>>(d_x, n, c.blob, h->d_tc_blob.get(), d_labels, d_logits,
-                                                               h->bias);
-    else if (c.tc == 1)
-      ffn_tc_rows_kernel<1><<<grid, 128, kFfnTcSmemBytes, st>>>(d_x, n, nullptr, c.blob, d_labels, d_logits, h->bias);
-    else
-      ffn_rows_kernel<<<grid, 128, 0, st>>>(d_x, n, d_labels, d_logits, h->par);
+    with_classifier<kKindsFfn>(classifier_of(h, kKindsFfn), [&](auto kind, const auto& w) {
+      constexpr int K = decltype(kind)::value;
+      if constexpr (K == kClsFp32)
+        rows_kernel<<<grid, 128, 0, st>>>(d_x, n, d_labels, d_logits, w);
+      else  // a fp16 tile holding a row past the feature bounds runs on the tf32 blob
+        ffn_tc_rows_kernel<K><<<grid, 128, kFfnTcSmemBytes, st>>>(d_x, n, w.blob16, w.blob32, d_labels, d_logits,
+                                                                 w.bias);
+    });
   });
 }
 
@@ -1106,19 +1171,13 @@ int launch_stream_feed(vadb200_bank* b, const int16_t* d_chunks, uint8_t* d_labe
   bp.prev = b->d_prev.get();
   bp.fe = frontend_on(h) ? frontend_of(h) : FrontEnd{nullptr, 0.0f};
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
-  if (has_tree(h))
-    return launched(1, [&] {
-      if (b->d_seg)
-        stream_feed_tree_kernel<true><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, tree_arg(h), bank_seg(b, d_rows, d_bounds));
-      else
-        stream_feed_tree_kernel<false><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, tree_arg(h), StreamSeg{});
-    });
   return launched(1, [&] {
-    if (b->d_seg)  // speech on: every feed advances the segment state
-      stream_feed_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par,
-                                                                                    bank_seg(b, d_rows, d_bounds));
-    else
-      stream_feed_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(bp, h->par);
+    with_classifier<kKindsTreeFp32>(classifier_of(h, kKindsTreeFp32), [&](auto kind, const auto& w) {
+      // speech on: every feed advances the segment state
+      with_bank_seg<decltype(kind)::value>(b->d_seg != nullptr, bank_seg(b, d_rows, d_bounds), [&](auto seg, const auto&... sg) {
+        stream_feed_kernel<decltype(seg)::value><<<grid, kThreads, kStreamSmemBytes, st>>>(bp, w, sg...);
+      });
+    });
   });
 }
 
@@ -1192,17 +1251,12 @@ int vadb200_stream_feed_ragged(vadb200_bank* b, const int16_t* d_samples, const 
   const unsigned grid = (b->n + kStepFrames - 1) / kStepFrames;
   return launched(b->src_cap ? 3 : 1, [&] {
     if (b->src_cap) enqueue_stream_resample(srs_params(b, d_samples, d_offsets), srs_grid(b), st);
-    if (has_tree(h)) {
-      if (b->d_seg)
-        stream_ragged_tree_kernel<true><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, tree_arg(h),
-                                                                                  bank_seg(b, nullptr, nullptr));
-      else
-        stream_ragged_tree_kernel<false><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, tree_arg(h), StreamSeg{});
-    } else if (b->d_seg)  // speech on: every feed advances the segment state
-      stream_ragged_speech_kernel<StreamSeg><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par,
-                                                                                      bank_seg(b, nullptr, nullptr));
-    else
-      stream_ragged_kernel<<<grid, kThreads, kStreamSmemBytes, st>>>(rp, h->par);
+    with_classifier<kKindsTreeFp32>(classifier_of(h, kKindsTreeFp32), [&](auto kind, const auto& w) {
+      // speech on: every feed advances the segment state
+      with_bank_seg<decltype(kind)::value>(b->d_seg != nullptr, bank_seg(b, nullptr, nullptr), [&](auto seg, const auto&... sg) {
+        stream_ragged_kernel<decltype(seg)::value><<<grid, kThreads, kStreamSmemBytes, st>>>(rp, w, sg...);
+      });
+    });
   });
 }
 
