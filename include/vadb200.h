@@ -48,6 +48,7 @@ typedef struct vadb200_handle vadb200_handle;
 typedef struct vadb200_plan vadb200_plan;
 typedef struct vadb200_bank vadb200_bank;
 typedef struct vadb200_trainer vadb200_trainer;
+typedef struct vadb200_tree_fitter vadb200_tree_fitter;
 
 /* config.py:20-27.  Only the reference values are accepted by the fused kernels. */
 typedef struct vadb200_config {
@@ -430,6 +431,49 @@ int vadb200_trainer_get_weights(vadb200_trainer* t, float* W1, float* b1, float*
                                 float* b3, float* W4, float* b4);
 int vadb200_train_on_batch(vadb200_trainer* t, const float* d_x, const uint8_t* d_y, int64_t n,
                            float* h_loss, void* stream);
+
+/* ---- decision-tree fit (learning/decision_classifier_trainer.py: DecisionTreeClassifier(...).fit(X, y)) -----------
+ * The tree sklearn 1.9's DecisionTreeClassifier(criterion="gini", splitter="best", max_features=None, max_depth,
+ * min_samples_split, min_samples_leaf, min_impurity_decrease) builds on d_x [n][39] float32 and class ids d_y [n] in
+ * {0, 1, 2}, array for array and bit for bit, at every node where sklearn's choice does not depend on its random
+ * feature order:
+ *   - classes = the ids present, ascending; min_samples_split is raised to 2 min_samples_leaf; max_depth <= 0 is
+ *     unbounded.  A node is a leaf when depth >= max_depth, n < min_samples_split, n < 2 min_samples_leaf,
+ *     impurity <= DBL_EPSILON, it has no candidate, or improvement + DBL_EPSILON < min_impurity_decrease.
+ *   - Within a node sorted by feature f, position p is a candidate iff x[p] > x[p-1] + 1e-7f in float32 and both sides
+ *     keep min_samples_leaf rows.  Its proxy is -(n_r g_r) - (n_l g_l), g = 1.0 - sum(count^2) / (n n), in float64
+ *     without fused multiply-adds; the threshold is double(x[p-1]) / 2.0 + double(x[p]) / 2.0.
+ *   - The maximum proxy wins; within a feature the earliest position, across features THE LOWEST FEATURE INDEX.
+ *     sklearn takes the first maximum in an order drawn from random_state, which no level-wise builder can reproduce,
+ *     so every fit reports tied_nodes, the nodes where a second feature reached the same float64 maximum:
+ *     tied_nodes == 0 => sklearn builds this same tree for every random_state.
+ *   - Output in sklearn's numbering (depth-first preorder, left child first): children -1, feature -2 and threshold
+ *     -2.0 at leaves; value [nodes][n_classes] = count / n_node_samples (tree_.value[:, 0, :] of sklearn >= 1.4), so
+ *     the arrays go to vadb200_set_tree as they are.  The tree depends on neither the row order nor the stream.
+ * A fitter owns about 1.05 KB of device memory per max_rows row (max_rows <= 2^30 - 8), allocated at create.  A fit
+ * reads one small count per tree level, so it synchronises `stream` and cannot be captured in a CUDA graph (like
+ * vadb200_train_on_batch with h_loss).  Bad input (a non-finite feature, a class id > 2, n <= 0 or > max_rows, bad
+ * params, a NULL pointer) returns VADB200_E_INVALID; a tree of more than 2^26 nodes is VADB200_E_UNSUPPORTED; either
+ * leaves the previous result readable.  The fitter is independent of the handle's classifier (fitting installs no
+ * tree) and may be destroyed after its handle. */
+typedef struct vadb200_tree_fit_params {
+  int32_t max_depth;             /* <= 0: unbounded */
+  int32_t min_samples_split;     /* >= 2 */
+  int32_t min_samples_leaf;      /* >= 1 */
+  int32_t reserved;
+  double min_impurity_decrease;  /* >= 0, finite */
+} vadb200_tree_fit_params;
+void vadb200_default_tree_fit_params(vadb200_tree_fit_params* p);       /* sklearn's defaults */
+int vadb200_tree_fitter_create(vadb200_handle* h, int64_t max_rows, vadb200_tree_fitter** out);
+int vadb200_tree_fitter_destroy(vadb200_tree_fitter* f);
+int vadb200_tree_fit(vadb200_tree_fitter* f, const float* d_x /* [n][39] */, const uint8_t* d_y, int64_t n,
+                     const vadb200_tree_fit_params* p, void* stream);    /* synchronises stream */
+int64_t vadb200_tree_fit_node_count(const vadb200_tree_fitter* f);       /* 0 before the first fit */
+/* The last successful fit; every pointer nullable; VADB200_E_STATE before the first fit. */
+int vadb200_tree_fit_result(const vadb200_tree_fitter* f, int64_t* h_children_left, int64_t* h_children_right,
+                            int64_t* h_feature, double* h_threshold, double* h_value /* [nodes][n_classes] */,
+                            double* h_impurity, int64_t* h_n_node_samples, int64_t* h_classes /* [3] */,
+                            int* n_classes, int64_t* tied_nodes);
 
 /* ---- bench support -------------------------------------------------------------------------
  * Counter-based integer synthetic PCM, bit-identical to vad_b200/synth.py. */

@@ -13,6 +13,11 @@ class VadB200Error(RuntimeError):
         self.code = code
 
 
+class TreeFitParams(C.Structure):
+    _fields_ = [("max_depth", C.c_int32), ("min_samples_split", C.c_int32), ("min_samples_leaf", C.c_int32),
+                ("reserved", C.c_int32), ("min_impurity_decrease", C.c_double)]
+
+
 class Config(C.Structure):
     _fields_ = [("sample_rate", C.c_int32), ("frame_size", C.c_int32), ("frame_step", C.c_int32),
                 ("fft_n", C.c_int32), ("n_filters", C.c_int32), ("n_mfcc", C.c_int32),
@@ -95,6 +100,12 @@ SIGNATURES = {
     "vadb200_trainer_set_weights": (C.c_int, [_P] + [_P] * 8 + [C.c_int]),
     "vadb200_trainer_get_weights": (C.c_int, [_P] + [_P] * 8),
     "vadb200_train_on_batch": (C.c_int, [_P, _P, _P, _I64, _P, _P]),
+    "vadb200_default_tree_fit_params": (None, [_P]),
+    "vadb200_tree_fitter_create": (C.c_int, [_P, _I64, C.POINTER(_P)]),
+    "vadb200_tree_fitter_destroy": (C.c_int, [_P]),
+    "vadb200_tree_fit": (C.c_int, [_P, _P, _P, _I64, _P, _P]),
+    "vadb200_tree_fit_node_count": (_I64, [_P]),
+    "vadb200_tree_fit_result": (C.c_int, [_P] * 11),
     "vadb200_synth_pcm": (C.c_int, [_P, _P, _I64, _I64, _I64, C.c_uint32, _I64, _P]),
     "vadb200_fp32_peak": (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(C.c_double)]),
     "vadb200_launch_count": (_I64, []),

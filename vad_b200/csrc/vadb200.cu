@@ -8,6 +8,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cfloat>
 #include <cmath>
 #include <cstddef>
 #include <cstdio>
@@ -26,6 +27,7 @@
 #include "vad_segments.cuh"
 #include "vad_resample.cuh"
 #include "vad_stream_resample.h"
+#include "vad_tree_fit.cuh"
 
 using namespace vadb;
 
@@ -205,6 +207,35 @@ struct vadb200_trainer {
   DevBuf<float> d_partial;     // [min(ceil(max_batch / 128), SMs)][kNParams + 1]
   DevBuf<float> d_loss;
   long long steps = 0;
+};
+
+// Decision-tree fitter (vad_tree_fit.cuh): every buffer is sized for max_rows at create.
+struct vadb200_tree_fitter {
+  ~vadb200_tree_fitter() { cudaSetDevice(device); }
+  int device = 0;              // the handle's device; the fitter keeps no pointer to the handle
+  long long max_rows = 0;
+  int stride = 0;              // column stride: max_rows rounded up to 8
+  int max_open = 0;            // open nodes a level can hold: each has >= 2 rows
+  int node_cap = 0;            // min(2 max_rows - 1, 2^26)
+  DevBuf<float> d_val[2];      // [39][stride] sorted values, double-buffered
+  DevBuf<uint32_t> d_rl[2];    // [39][stride] row << 2 | label
+  DevBuf<uint8_t> d_side;      // [max_rows]
+  DevBuf<int> d_pos_node;      // [max_rows]
+  DevBuf<unsigned long long> d_chunk_cnt;  // [39][chunks]
+  DevBuf<int4> d_chunk_pre;    // [39][chunks + 1]
+  DevBuf<TfOpen> d_open[2];    // [max_open] this level, next level
+  DevBuf<unsigned long long> d_best_key;   // [max_open][39]
+  DevBuf<int> d_best_pos;      // [max_open][39]
+  DevBuf<TfDec> d_dec;         // [max_open]
+  DevBuf<int> d_scan;          // [max_open][kTfScanItems]
+  DevBuf<TfRec> d_rec;         // [node_cap] breadth-first records
+  DevBuf<int> d_stats;         // [kTfStats]
+  // the last successful fit, in sklearn's preorder numbering
+  std::vector<int64_t> left, right, feature, n_samples;
+  std::vector<double> threshold, value, impurity;
+  int64_t classes[3] = {0, 0, 0};
+  int n_classes = 0;
+  int64_t tied = 0;
 };
 
 struct vadb200_bank {
@@ -1408,6 +1439,241 @@ int vadb200_train_on_batch(vadb200_trainer* t, const float* d_x, const uint8_t* 
     CU(cudaMemcpyAsync(h_loss, t->d_loss.get(), sizeof(float), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
   }
+  return 0;
+}
+
+// ---- decision-tree fit (learning/decision_classifier_trainer.py: DecisionTreeClassifier.fit) -------------------
+void vadb200_default_tree_fit_params(vadb200_tree_fit_params* p) {
+  if (!p) return;
+  p->max_depth = 0;
+  p->min_samples_split = 2;
+  p->min_samples_leaf = 1;
+  p->reserved = 0;
+  p->min_impurity_decrease = 0.0;
+}
+
+int vadb200_tree_fitter_create(vadb200_handle* h, int64_t max_rows, vadb200_tree_fitter** out) {
+  if (!out) return fail(VADB200_E_INVALID, "out is null");
+  *out = nullptr;
+  if (!h) return fail(VADB200_E_INVALID, "handle is null");
+  if (max_rows < 1 || max_rows > kTfMaxRows - 8) return fail(VADB200_E_INVALID, "max_rows must be in [1, 2^30 - 8]");
+  CU(cudaSetDevice(h->device));
+  std::unique_ptr<vadb200_tree_fitter> f(new (std::nothrow) vadb200_tree_fitter());
+  if (!f) return fail(VADB200_E_NOMEM, "host allocation failed");
+  f->device = h->device;
+  f->max_rows = max_rows;
+  f->stride = static_cast<int>((max_rows + 7) / 8 * 8);
+  f->max_open = static_cast<int>(max_rows / 2 + 1);
+  f->node_cap = static_cast<int>(std::min<long long>(2 * max_rows - 1, kTfMaxNodes));
+  const size_t cols = static_cast<size_t>(kTfFeat) * f->stride;
+  const size_t chunks = (max_rows + kTfChunk - 1) / kTfChunk;
+  for (int b = 0; b < 2; ++b) {
+    CU(dev_alloc(f->d_val[b], cols * sizeof(float)));
+    CU(dev_alloc(f->d_rl[b], cols * sizeof(uint32_t)));
+    CU(dev_alloc(f->d_open[b], f->max_open * sizeof(TfOpen)));
+  }
+  CU(dev_alloc(f->d_side, max_rows));
+  CU(dev_alloc(f->d_pos_node, max_rows * sizeof(int)));
+  CU(dev_alloc(f->d_chunk_cnt, kTfFeat * chunks * sizeof(unsigned long long)));
+  CU(dev_alloc(f->d_chunk_pre, kTfFeat * (chunks + 1) * sizeof(int4)));
+  CU(dev_alloc(f->d_best_key, static_cast<size_t>(f->max_open) * kTfFeat * sizeof(unsigned long long)));
+  CU(dev_alloc(f->d_best_pos, static_cast<size_t>(f->max_open) * kTfFeat * sizeof(int)));
+  CU(dev_alloc(f->d_dec, f->max_open * sizeof(TfDec)));
+  CU(dev_alloc(f->d_scan, static_cast<size_t>(f->max_open) * kTfScanItems * sizeof(int)));
+  CU(dev_alloc(f->d_rec, static_cast<size_t>(f->node_cap) * sizeof(TfRec)));
+  CU(dev_alloc(f->d_stats, kTfStats * sizeof(int)));
+  *out = f.release();
+  return 0;
+}
+
+int vadb200_tree_fitter_destroy(vadb200_tree_fitter* f) {
+  delete f;
+  return 0;
+}
+
+int64_t vadb200_tree_fit_node_count(const vadb200_tree_fitter* f) {
+  return f ? static_cast<int64_t>(f->left.size()) : 0;
+}
+
+// sklearn Gini::node_impurity on the host: 1.0 - sq_count / (w * w) (x86-64 host code is never contracted to FMA).
+static double gini_host(const int* c, int n) {
+  double sq = 0.0;
+  for (int j = 0; j < 3; ++j) sq += static_cast<double>(c[j]) * static_cast<double>(c[j]);
+  const double w = n;
+  return 1.0 - sq / (w * w);
+}
+
+int vadb200_tree_fit(vadb200_tree_fitter* f, const float* d_x, const uint8_t* d_y, int64_t n,
+                     const vadb200_tree_fit_params* p, void* stream) {
+  if (!f || !d_x || !d_y || !p) return fail(VADB200_E_INVALID, "null argument");
+  if (n < 1 || n > f->max_rows) return fail(VADB200_E_INVALID, "n must be in [1, max_rows]");
+  if (p->min_samples_split < 2 || p->min_samples_leaf < 1 || !(p->min_impurity_decrease >= 0.0) ||
+      !std::isfinite(p->min_impurity_decrease))
+    return fail(VADB200_E_INVALID, "need min_samples_split >= 2, min_samples_leaf >= 1, finite min_impurity_decrease >= 0");
+  CU(cudaSetDevice(f->device));
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int rows = static_cast<int>(n), stride = f->stride;
+  int* stats = f->d_stats.get();
+  int h_stats[kTfStats];
+  int cur = 0;
+  CU(cudaMemsetAsync(stats, 0, kTfStats * sizeof(int), st));
+  int rc = launched(1, [&] { tf_validate(d_x, d_y, n, stride, f->d_val[0].get(), f->d_rl[0].get(), stats, st); });
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(h_stats, stats, sizeof(h_stats), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (h_stats[0]) return fail(VADB200_E_INVALID, "non-finite feature value");
+  if (h_stats[1]) return fail(VADB200_E_INVALID, "class id > 2");
+
+  // Presort: 16 stable 2-bit LSD passes over the order-preserving image of every column's float32 values.
+  const auto chunks_of = [](int m) { return (m + kTfChunk - 1) / kTfChunk; };
+  for (int shift = 0; shift < 32; shift += 2) {
+    const int nc = chunks_of(rows);
+    rc = launched(3, [&] {
+      tf_count(kTfByDigit, shift, f->d_val[cur].get(), f->d_rl[cur].get(), nullptr, rows, stride, nc,
+               f->d_chunk_cnt.get(), st);
+      tf_chunk_scan(f->d_chunk_cnt.get(), nc, f->d_chunk_pre.get(), st);
+      tf_radix_scatter(shift, f->d_val[cur].get(), f->d_rl[cur].get(), rows, stride, nc, f->d_chunk_pre.get(),
+                       f->d_val[cur ^ 1].get(), f->d_rl[cur ^ 1].get(), st);
+    });
+    if (rc) return rc;
+    cur ^= 1;
+  }
+
+  TfParams prm;
+  prm.max_depth = p->max_depth > 0 ? p->max_depth : 0;
+  prm.min_leaf = p->min_samples_leaf;
+  prm.min_split = static_cast<int>(std::max<long long>(p->min_samples_split, 2ll * p->min_samples_leaf));
+  prm.min_decrease = p->min_impurity_decrease;
+  prm.n_total = static_cast<double>(n);
+  TfOpen root;
+  root.s = 0;
+  root.e = rows;
+  root.depth = 0;
+  root.id = 0;
+  for (int j = 0; j < 3; ++j) {
+    root.c[j] = h_stats[2 + j];
+    root.base[j] = 0;
+  }
+  root.imp = gini_host(root.c, rows);
+  TfRec rrec;
+  rrec.left = rrec.right = -1;
+  rrec.feature = -2;
+  rrec.n = rows;
+  for (int j = 0; j < 3; ++j) rrec.c[j] = root.c[j];
+  rrec.pad = 0;
+  rrec.thr = -2.0;
+  rrec.imp = root.imp;
+  CU(cudaMemcpyAsync(f->d_rec.get(), &rrec, sizeof(rrec), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(f->d_open[0].get(), &root, sizeof(root), cudaMemcpyHostToDevice, st));
+  const bool root_leaf = rows < prm.min_split || rows < 2 * prm.min_leaf || root.imp <= DBL_EPSILON;
+  int n_open = root_leaf ? 0 : 1, n_act = rows, next_id = 1, oc = 0;
+  while (n_open > 0) {
+    const int nc = chunks_of(n_act);
+    const float* val = f->d_val[cur].get();
+    const uint32_t* rl = f->d_rl[cur].get();
+    const TfOpen* open = f->d_open[oc].get();
+    int4* pre = f->d_chunk_pre.get();
+    CU(cudaMemsetAsync(f->d_best_key.get(), 0, static_cast<size_t>(n_open) * kTfFeat * sizeof(unsigned long long), st));
+    CU(cudaMemsetAsync(f->d_best_pos.get(), 0x7f, static_cast<size_t>(n_open) * kTfFeat * sizeof(int), st));
+    rc = launched(12, [&] {
+      tf_node_map(open, n_open, n_act, f->d_pos_node.get(), st);
+      tf_count(kTfByLabel, 0, val, rl, nullptr, n_act, stride, nc, f->d_chunk_cnt.get(), st);
+      tf_chunk_scan(f->d_chunk_cnt.get(), nc, pre, st);
+      for (int phase = 0; phase < 2; ++phase)
+        tf_search(phase, val, rl, n_act, stride, nc, pre, f->d_pos_node.get(), open, prm.min_leaf,
+                  f->d_best_key.get(), f->d_best_pos.get(), st);
+      tf_decide(rl, stride, pre, nc, open, n_open, f->d_best_key.get(), f->d_best_pos.get(), prm, f->d_dec.get(),
+                f->d_scan.get(), st);
+      tf_level_scan(f->d_scan.get(), n_open, stats + 6, st);
+      tf_emit(val, stride, open, n_open, f->d_dec.get(), f->d_scan.get(), next_id, f->node_cap, f->d_rec.get(),
+              f->d_open[oc ^ 1].get(), stats, st);
+      tf_flag(rl, n_act, stride, f->d_pos_node.get(), f->d_dec.get(), f->d_side.get(), st);
+      tf_count(kTfBySide, 0, val, rl, f->d_side.get(), n_act, stride, nc, f->d_chunk_cnt.get(), st);
+      tf_chunk_scan(f->d_chunk_cnt.get(), nc, pre, st);
+      tf_partition(val, rl, n_act, stride, nc, pre, f->d_pos_node.get(), f->d_dec.get(), f->d_side.get(),
+                   f->d_val[cur ^ 1].get(), f->d_rl[cur ^ 1].get(), st);
+    });
+    if (rc) return rc;
+    int tot[kTfScanItems];
+    CU(cudaMemcpyAsync(tot, stats + 6, sizeof(tot), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (static_cast<long long>(next_id) + 2ll * tot[0] > f->node_cap)
+      return fail(VADB200_E_UNSUPPORTED, "the tree would exceed 2^26 nodes (vadb200_set_tree's limit)");
+    next_id += 2 * tot[0];
+    n_open = tot[1];
+    n_act = tot[2] + tot[3];
+    oc ^= 1;
+    cur ^= 1;
+  }
+
+  std::vector<TfRec> rec(next_id);
+  CU(cudaMemcpyAsync(rec.data(), f->d_rec.get(), next_id * sizeof(TfRec), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(h_stats, stats, sizeof(h_stats), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+
+  // Renumber breadth-first records to sklearn's depth-first preorder, left child first.
+  std::vector<int> pre_id(next_id), order;
+  order.reserve(next_id);
+  std::vector<int> stack(1, 0);
+  while (!stack.empty()) {
+    const int k = stack.back();
+    stack.pop_back();
+    pre_id[k] = static_cast<int>(order.size());
+    order.push_back(k);
+    if (rec[k].left >= 0) {
+      stack.push_back(rec[k].right);
+      stack.push_back(rec[k].left);
+    }
+  }
+  int64_t classes[3];
+  int nk = 0;
+  for (int j = 0; j < 3; ++j)
+    if (h_stats[2 + j] > 0) classes[nk++] = j;
+  const size_t m = order.size();
+  std::vector<int64_t> left(m), right(m), feature(m), n_samples(m);
+  std::vector<double> threshold(m), value(m * nk), impurity(m);
+  for (size_t i = 0; i < m; ++i) {
+    const TfRec& r = rec[order[i]];
+    left[i] = r.left >= 0 ? pre_id[r.left] : -1;
+    right[i] = r.right >= 0 ? pre_id[r.right] : -1;
+    feature[i] = r.feature;
+    threshold[i] = r.thr;
+    impurity[i] = r.imp;
+    n_samples[i] = r.n;
+    for (int j = 0; j < nk; ++j)  // sklearn >= 1.4's tree_.value: count / weighted_n_node_samples
+      value[i * nk + j] = static_cast<double>(r.c[classes[j]]) / static_cast<double>(r.n);
+  }
+  f->left.swap(left);
+  f->right.swap(right);
+  f->feature.swap(feature);
+  f->n_samples.swap(n_samples);
+  f->threshold.swap(threshold);
+  f->value.swap(value);
+  f->impurity.swap(impurity);
+  for (int j = 0; j < 3; ++j) f->classes[j] = j < nk ? classes[j] : 0;
+  f->n_classes = nk;
+  f->tied = h_stats[5];
+  return 0;
+}
+
+int vadb200_tree_fit_result(const vadb200_tree_fitter* f, int64_t* h_children_left, int64_t* h_children_right,
+                            int64_t* h_feature, double* h_threshold, double* h_value, double* h_impurity,
+                            int64_t* h_n_node_samples, int64_t* h_classes, int* n_classes, int64_t* tied_nodes) {
+  if (!f) return fail(VADB200_E_INVALID, "fitter is null");
+  if (f->left.empty()) return fail(VADB200_E_STATE, "no fit yet");
+  const auto put = [](auto* dst, const auto& src) {
+    if (dst) std::copy(src.begin(), src.end(), dst);
+  };
+  put(h_children_left, f->left);
+  put(h_children_right, f->right);
+  put(h_feature, f->feature);
+  put(h_threshold, f->threshold);
+  put(h_value, f->value);
+  put(h_impurity, f->impurity);
+  put(h_n_node_samples, f->n_samples);
+  if (h_classes) std::copy(f->classes, f->classes + f->n_classes, h_classes);
+  if (n_classes) *n_classes = f->n_classes;
+  if (tied_nodes) *tied_nodes = f->tied;
   return 0;
 }
 

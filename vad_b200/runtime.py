@@ -373,6 +373,72 @@ class Handle(object):
         return out
 
 
+class TreeFitter(object):
+    """Fits sklearn 1.9's DecisionTreeClassifier(criterion="gini") on the device (vadb200_tree_fit): the tree is
+    sklearn's, bit for bit, at every node where sklearn's choice does not depend on its random feature order; where
+    features tie on the best proxy the lowest index wins and the node counts in ``tied_nodes``, so tied_nodes == 0
+    means sklearn builds this same tree for every random_state.  Reserves its device memory for ``max_rows`` rows
+    (about 1.05 KB each).  Fitting installs no tree: pass the result to ``Handle.set_tree``."""
+
+    def __init__(self, handle, max_rows):
+        self.handle = handle
+        self.lib = handle.lib
+        self.max_rows = int(max_rows)
+        self._f = C.c_void_p()
+        check(self.lib.vadb200_tree_fitter_create(handle._h, self.max_rows, C.byref(self._f)))
+
+    def close(self):
+        if getattr(self, "_f", None) is not None and self._f:
+            self.lib.vadb200_tree_fitter_destroy(self._f)
+            self._f = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def node_count(self):
+        return int(self.lib.vadb200_tree_fit_node_count(self._f))
+
+    def fit(self, x, y, max_depth=None, min_samples_split=2, min_samples_leaf=1, min_impurity_decrease=0.0,
+            stream=None):
+        """x: [n, 39] float32 CUDA tensor, y: [n] uint8 CUDA tensor of class ids 0 / 1 / 2 (rows with a non-finite
+        feature are rejected).  Runs on ``stream`` (a torch.cuda.Stream; the handle's by default) and synchronises it.  Returns the dict of
+        ``tree_arrays``' keys plus impurity, n_node_samples and tied_nodes."""
+        if not (torch.is_tensor(x) and x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 2
+                and x.shape[1] == 39):
+            raise TypeError("x must be a contiguous [n, 39] float32 CUDA tensor")
+        if not (torch.is_tensor(y) and y.is_cuda and y.dtype == torch.uint8 and y.is_contiguous()
+                and y.shape == (x.shape[0],)):
+            raise TypeError("y must be a contiguous [n] uint8 CUDA tensor")
+        p = _lib.TreeFitParams()
+        self.lib.vadb200_default_tree_fit_params(C.byref(p))
+        p.max_depth = 0 if max_depth is None else int(max_depth)
+        p.min_samples_split = int(min_samples_split)
+        p.min_samples_leaf = int(min_samples_leaf)
+        p.min_impurity_decrease = float(min_impurity_decrease)
+        check(self.lib.vadb200_tree_fit(self._f, _ptr(x), _ptr(y), x.shape[0], C.byref(p),
+                                        self.handle.stream if stream is None else C.c_void_p(stream.cuda_stream)))
+        return self.result()
+
+    def result(self):
+        """The last successful fit (see ``fit``)."""
+        m = self.node_count
+        out = {k: np.empty(m, np.int64) for k in ("children_left", "children_right", "feature", "n_node_samples")}
+        out.update(threshold=np.empty(m), impurity=np.empty(m), value=np.empty((m, 3)), classes=np.empty(3, np.int64))
+        nk, tied = C.c_int(), C.c_int64()
+        a = lambda k: out[k].ctypes.data_as(C.c_void_p)  # noqa: E731
+        check(self.lib.vadb200_tree_fit_result(self._f, a("children_left"), a("children_right"), a("feature"),
+                                               a("threshold"), a("value"), a("impurity"), a("n_node_samples"),
+                                               a("classes"), C.byref(nk), C.byref(tied)))
+        out["value"] = np.ascontiguousarray(out["value"].reshape(-1)[:m * nk.value].reshape(m, nk.value))
+        out["classes"] = out["classes"][:nk.value].copy()
+        out["tied_nodes"] = int(tied.value)
+        return out
+
+
 class Resampler(object):
     """src_rate -> 16 kHz int16 on the device (scipy.signal.resample_poly's filter, rounded half to even and
     saturated; include/vadb200.h).  Owns the tap table; ``run`` only enqueues work."""

@@ -1,4 +1,5 @@
-"""FFN training on the device: drop-in for the training loop of learning/ffn_trainer.py:104-175.
+"""Classifier training on the device: drop-ins for learning/ffn_trainer.py:104-175 (``FFNTrainer``, ``train``) and
+learning/decision_classifier_trainer.py (``fit_tree``).
 
 ``FFNTrainer.train_on_batch(x, y)`` is Keras-1 ``model.train_on_batch`` for the reference's network and compile
 settings (categorical cross-entropy, Adadelta lr 1.0 / rho 0.95 / eps 1e-8) as two CUDA kernels per step
@@ -154,3 +155,56 @@ def train(trainer, sources, epochs=EPOCHS_NUM, batch_size=4096, val_fraction=0.2
     if save_prefix:
         trainer.save(save_prefix + "_full_training.npz")
     return history
+
+
+# learning/decision_classifier_trainer.py's grid-search best (cross_validation.res)
+TREE_MAX_DEPTH = 25
+TREE_MIN_SAMPLES_LEAF = 20
+TREE_MIN_SAMPLES_SPLIT = 22
+
+
+def fit_tree(sources, val_fraction=0.25, max_depth=TREE_MAX_DEPTH, min_samples_leaf=TREE_MIN_SAMPLES_LEAF,
+             min_samples_split=TREE_MIN_SAMPLES_SPLIT, seed=0, save_path=None, handle=None, log=print):
+    """The flow of learning/decision_classifier_trainer.py on the device.  ``sources``: list of (rows [n_c, 39] float32
+    CUDA tensor, class id).  Rows with a non-finite feature are dropped (and counted in the log); a random
+    ``val_fraction`` of each source is held out; the tree is fitted on the rest (``runtime.TreeFitter``) and scored on
+    the held-out rows with ``Handle.tree_predict`` (clf.score: the class of the largest probability equals the label).
+    ``save_path``: the tree's arrays go to an .npz (``runtime.save_tree_npz``; replaces cPickle.dump).
+    Returns (tree dict, held-out accuracy; NaN without held-out rows)."""
+    handle = handle or runtime.Handle()
+    g = torch.Generator(device="cpu").manual_seed(int(seed))
+    fit_x, fit_y, val_x, val_y = [], [], [], []
+    for rows, cls in sources:
+        ok = torch.isfinite(rows).all(dim=1)
+        dropped = int((~ok).sum())
+        if dropped and log:
+            log("class %d: dropped %d rows with a non-finite feature" % (cls, dropped))
+        rows = rows[ok]
+        perm = torch.randperm(rows.shape[0], generator=g).to(rows.device)
+        n_val = int(rows.shape[0] * val_fraction)
+        for xs, ys, part in ((val_x, val_y, perm[:n_val]), (fit_x, fit_y, perm[n_val:])):
+            xs.append(rows[part])
+            ys.append(torch.full((part.shape[0],), cls, dtype=torch.uint8, device=rows.device))
+    x, y = torch.cat(fit_x).contiguous(), torch.cat(fit_y).contiguous()
+    fitter = runtime.TreeFitter(handle, x.shape[0])
+    try:
+        tree = fitter.fit(x, y, max_depth=max_depth, min_samples_split=min_samples_split,
+                          min_samples_leaf=min_samples_leaf)
+    finally:
+        fitter.close()
+    vx, vy = torch.cat(val_x).contiguous(), torch.cat(val_y)
+    accuracy = float("nan")
+    if vx.shape[0]:
+        scorer = runtime.Handle(handle.device)
+        try:
+            scorer.set_tree(tree)
+            _, proba = scorer.tree_predict(vx)
+            accuracy = float((proba.argmax(dim=1) == vy.long()).double().mean())
+        finally:
+            scorer.close()
+    if log:
+        log("tree: %d nodes, %d tied, fitted on %d rows, held-out accuracy %.4f"
+            % (tree["feature"].shape[0], tree["tied_nodes"], x.shape[0], accuracy))
+    if save_path:
+        runtime.save_tree_npz(save_path, tree)
+    return tree, accuracy
